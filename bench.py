@@ -1,8 +1,11 @@
 #!/usr/bin/env python
 """Benchmark of the CarMPC batch-evaluation hot path on B200 (contract: see the task brief / DESIGN.md).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+``--dump-outputs DIR`` writes what the last timed step computed as ``DIR/*.npy`` (see ``dump_outputs``): the inputs are
+fixed, so two builds run with the same arguments can be compared output for output.
 
 Headline line (one JSON object on stdout, rank 0): terminal-set samples/s on BASELINE config 2
 (RoadMultipleCarsEnv H-rep, 100^4 = 10^8-point float64 SoA grid, resident in HBM).  One "step" = one
@@ -212,6 +215,29 @@ def _pinned_copy_gbs(torch, dev, nbytes=1 << 30):
     return 3 * nbytes / (e0.elapsed_time(e1) * 1e-3) / 1e9
 
 
+DUMP_SAMPLES = 1 << 22             # grid points drawn for flags_sample.npy (about 16 MB of float32)
+
+
+def dump_outputs(out_dir: str, bits, members: int, n: int) -> None:
+    """Writes what one membership step hands its caller (the bitset of the n grid points and the member count) as
+    float arrays that two builds can be compared by with any tolerance:
+
+    * ``members.npy``: the member count (float64, shape (1,));
+    * ``group_members.npy``: members of every 1024-point group of the grid, in grid order (float64); a flag that
+      differs changes one entry;
+    * ``flags_sample.npy``: the 0 / 1 flags (float32) of the grid points
+      ``np.unique(np.random.default_rng(0).integers(0, n, DUMP_SAMPLES))``, in that order."""
+    import torch
+    shifts = torch.arange(32, dtype=torch.int32, device=bits.device)
+    flags = ((bits[:(n + 31) // 32, None] >> shifts) & 1).reshape(-1)[:n]
+    groups = torch.nn.functional.pad(flags, (0, -n % 1024)).reshape(-1, 1024).sum(1)
+    idx = torch.from_numpy(np.unique(np.random.default_rng(0).integers(0, n, DUMP_SAMPLES))).to(bits.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "members.npy"), np.array([members], dtype=np.float64))
+    np.save(os.path.join(out_dir, "group_members.npy"), groups.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "flags_sample.npy"), flags[idx].cpu().numpy().astype(np.float32))
+
+
 def run_ours(args, rank: int, world: int, local_rank: int):
     import torch
     import torch.distributed as dist
@@ -350,6 +376,12 @@ def run_ours(args, rank: int, world: int, local_rank: int):
     members = int(total.item())
     if window is not None:
         window.check()
+    if args.dump_outputs and rank == 0:
+        if not distributed:
+            last_bits = bits[(args.steps - 1) & 1]
+        else:
+            last_bits = window.result_bits() if window is not None else full_bits
+        dump_outputs(args.dump_outputs, last_bits, members, n)
 
     # ---- outside the timed steps: the gathered result of the last step against an independent evaluation -----------
     verify = None
@@ -627,11 +659,14 @@ def run_ours(args, rank: int, world: int, local_rank: int):
 
 
 def main():
+    sys.dont_write_bytecode = True     # the tree bench.py runs from may be read-only; it gets no bytecode caches either
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=200)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the member count and flags of the last timed step to DIR/*.npy (GPU arm, rank 0)")
     ap.add_argument("--mode", type=int, default=1, help="membership kernel: 0 = float64, 1 = float32 screen + float64 re-check")
     ap.add_argument("--layout", default="cyclic", choices=["cyclic", "contiguous"],
                     help="how the one sample set is sharded over the ranks (N > 1)")
@@ -653,6 +688,10 @@ def main():
     ap.add_argument("--cl-runs", type=int, default=100_000)
     ap.add_argument("--cl-steps", type=int, default=200)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

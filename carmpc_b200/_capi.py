@@ -24,6 +24,12 @@ class QPOpts(ctypes.Structure):
                 ("scaling_iters", ctypes.c_int32), ("polish", ctypes.c_int32)]
 
 
+class DisturbanceModel(ctypes.Structure):
+    """``carmpc_disturbance_model`` (include/carmpc.h)."""
+    _fields_ = [("Bd", ctypes.c_double * 4), ("Cd", ctypes.c_double * 3), ("L1", ctypes.c_double * 12),
+                ("L2", ctypes.c_double * 3), ("Bd_plant", ctypes.c_double * 4), ("Cd_plant", ctypes.c_double * 3)]
+
+
 _vp, _dp, _i64, _i32 = ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int
 
 #: name -> (restype, argtypes); every function include/carmpc.h declares
@@ -65,6 +71,9 @@ SIGNATURES = {
     "carmpc_qp_tensor_mode": (_i32, [_vp, _i32, ctypes.POINTER(_i64)]),
     "carmpc_closed_loop": (_i32, [_vp, _i32, _dp, _dp, _dp, _dp, _dp, ctypes.c_double, ctypes.c_double, _i32,
                                   _i32, _dp, _dp, _i64, _dp, _vp, _dp, _dp, ctypes.POINTER(_i64), _vp]),
+    "carmpc_closed_loop_disturbance": (_i32, [_vp, _dp, _dp, _dp, ctypes.POINTER(DisturbanceModel), _dp, ctypes.c_double,
+                                              ctypes.c_double, _i32, _i32, _dp, _dp, _dp, _dp, _i64, _dp, _dp, _vp, _dp,
+                                              _dp, _dp, ctypes.POINTER(_i64), _vp]),
     "carmpc_measure_peak": (_i32, [_i32, ctypes.POINTER(ctypes.c_double)]),
 }
 

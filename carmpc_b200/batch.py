@@ -489,3 +489,66 @@ class BatchQP(_Handle):
             out["inputs"].data_ptr() if want_inputs else None, ctypes.byref(total), _stream_ptr(stream)))
         out["total_iters"] = int(total.value)
         return out
+
+    def closed_loop_disturbance(self, x_init, steps: int, A, B, C, Bd, Cd, L1, L2, x_ref=None, Bd_plant=None,
+                                Cd_plant=None, d_plant=None, xhat_init=None, dhat_init=None, dt: float = 0.2,
+                                l1: float = 3.5, warm_start=True, want_traj: bool = False, want_inputs: bool = False,
+                                want_dhat: bool = False, stream=None) -> dict:
+        """Closed loops of the disturbance-estimating output-feedback controller (``MPCOutputFBWithDisturbance``,
+        ``carmpc_closed_loop_disturbance``): the loop of ``closed_loop`` with a scalar disturbance estimate ``d^`` kept
+        beside ``x^`` by the augmented observer (``Bd`` (4,), ``Cd`` (3,), gains ``L1`` (4, 3), ``L2`` (3,); no defaults,
+        see ``carmpc_b200.observer``), and the QP of each run taking ``d^`` as its disturbance.  This handle's ``Gc`` must
+        come from a controller with the same ``Bd`` (or be zero).  The plant gets a constant disturbance ``d_plant`` per
+        run ((R,) float64 CUDA tensor, None: 0) through ``Bd_plant`` (4,) after its Euler step and ``Cd_plant`` (3,) in its
+        output (None: zeros).  ``dhat_init``: (R,) CUDA tensor (None: 0).  ``warm_start``: 0 / 1 (True) / 2 as in
+        ``closed_loop``.  Returns ``final`` (4, R), ``dhat`` (R,), ``fail_step`` (R,) int32, ``total_iters`` and
+        optionally ``traj`` (steps, 4, R), ``inputs`` (steps, 2, R), ``dhat_traj`` (steps, R)."""
+        torch = _torch()
+        if not (x_init.is_cuda and x_init.dtype == torch.float64 and x_init.dim() == 2 and x_init.shape[0] == 4
+                and x_init.is_contiguous()):
+            raise ValueError("x_init must be a contiguous (4, R) float64 CUDA tensor")
+        R = x_init.shape[1]
+        dev = x_init.device
+        for name, t in (("d_plant", d_plant), ("dhat_init", dhat_init)):
+            if t is not None and not (t.is_cuda and t.dtype == torch.float64 and t.numel() == R and t.is_contiguous()):
+                raise ValueError(f"{name} must be a contiguous float64 CUDA tensor of R elements")
+        if xhat_init is not None and not (xhat_init.is_cuda and xhat_init.dtype == torch.float64
+                                          and tuple(xhat_init.shape) == (4, R) and xhat_init.is_contiguous()):
+            raise ValueError("xhat_init must be a contiguous (4, R) float64 CUDA tensor")
+
+        def vec(a, n, name):
+            v = _f64(a).ravel()
+            if v.size != n:
+                raise ValueError(f"{name} must have {n} entries")
+            return v
+
+        dm = _capi.DisturbanceModel()
+        dm.Bd[:] = vec(Bd, 4, "Bd").tolist()
+        dm.Cd[:] = vec(Cd, 3, "Cd").tolist()
+        dm.L1[:] = vec(L1, 12, "L1 (4 x 3)").tolist()
+        dm.L2[:] = vec(L2, 3, "L2").tolist()
+        dm.Bd_plant[:] = vec(np.zeros(4) if Bd_plant is None else Bd_plant, 4, "Bd_plant").tolist()
+        dm.Cd_plant[:] = vec(np.zeros(3) if Cd_plant is None else Cd_plant, 3, "Cd_plant").tolist()
+        xref = _f64(self.pq.goal if x_ref is None else x_ref)
+        A_, B_, C_ = _f64(A), _f64(B), _f64(C)
+        out = {"final": torch.empty((4, R), dtype=torch.float64, device=dev),
+               "dhat": torch.empty(R, dtype=torch.float64, device=dev),
+               "fail_step": torch.empty(R, dtype=torch.int32, device=dev)}
+        if want_traj:
+            out["traj"] = torch.empty((steps, 4, R), dtype=torch.float64, device=dev)
+        if want_inputs:
+            out["inputs"] = torch.empty((steps, 2, R), dtype=torch.float64, device=dev)
+        if want_dhat:
+            out["dhat_traj"] = torch.empty((steps, R), dtype=torch.float64, device=dev)
+        total = ctypes.c_int64(0)
+        check(self._lib.carmpc_closed_loop_disturbance(
+            self._h, _capi.ptr(A_), _capi.ptr(B_), _capi.ptr(C_), ctypes.byref(dm), _capi.ptr(xref), float(dt),
+            float(l1), int(steps), int(warm_start), x_init.data_ptr(),
+            xhat_init.data_ptr() if xhat_init is not None else None,
+            dhat_init.data_ptr() if dhat_init is not None else None,
+            d_plant.data_ptr() if d_plant is not None else None, R, out["final"].data_ptr(), out["dhat"].data_ptr(),
+            out["fail_step"].data_ptr(), out["traj"].data_ptr() if want_traj else None,
+            out["inputs"].data_ptr() if want_inputs else None, out["dhat_traj"].data_ptr() if want_dhat else None,
+            ctypes.byref(total), _stream_ptr(stream)))
+        out["total_iters"] = int(total.value)
+        return out

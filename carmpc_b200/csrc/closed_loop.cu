@@ -6,6 +6,13 @@
 // the state itself for state feedback, then one condensed QP per run (lib/mpc.py:461-478 / :318-335).  A run whose QP is
 // infeasible stops there, as the reference raises OutsideTheRegionOfAttractionError.
 //
+// The disturbance mode (carmpc_closed_loop_disturbance) is the controller for constant disturbances
+// (MPCOutputFBWithDisturbance): the plant gets a constant per-run disturbance d_r after its Euler step (Bd_p d_r) and in
+// its output (Cd_p d_r); the augmented observer keeps a scalar estimate d^ beside x^,
+//     i = y - C x^ - Cd d^ ,   x^' = A x^ + Bd d^ + B u_prev + L1 i ,   d^' = d^ + L2 . i ,
+// and the QP of the run takes d^' as its disturbance c (bounds shifted by Gc c).  The d^ buffer itself is the c array
+// the QP stages read, so its address is fixed across steps and the captured step graph stays valid.
+//
 // One thread per run for plant + observer (4 state and 2 input registers); the QPs of all live runs go through the
 // batched solver with the previous step's ADMM state as warm start.
 #include <math.h>
@@ -21,8 +28,9 @@ namespace {
 
 struct LoopConst {
     double A[16], B[8], C[12], L[12];
+    double Bd[4], Cd[3], L2[3], Bdp[4], Cdp[3];     // mode 2: disturbance model, its observer gain, how d_r enters the plant
     double dt, l1;
-    int mode;            // 0 state feedback, 1 output feedback
+    int mode;            // 0 state feedback, 1 output feedback, 2 output feedback with a disturbance estimate
 };
 
 // plant step with the previous input, observer update, estimate -> QP input; builds the list of live runs
@@ -30,7 +38,8 @@ __global__ void __launch_bounds__(256)
 loop_advance_kernel(const LoopConst K, int64_t runs, double* __restrict__ x, double* __restrict__ xhat,
                     const double* __restrict__ u_prev, const int32_t* __restrict__ fail_step,
                     double* __restrict__ est, int* __restrict__ live_list, int* __restrict__ live_count,
-                    double* __restrict__ traj_step, const int* __restrict__ step_dev) {
+                    double* __restrict__ traj_step, const int* __restrict__ step_dev,
+                    double* __restrict__ dhat, const double* __restrict__ d_plant) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= runs) return;
     // replayed steps (CUDA graph) read the step number on the device: traj_step is then the base of the trajectory
@@ -49,10 +58,46 @@ loop_advance_kernel(const LoopConst K, int64_t runs, double* __restrict__ x, dou
         s[1] = r1 * K.dt + s[1];
         s[2] = r2 * K.dt + s[2];
         s[3] = r3 * K.dt + s[3];
+        double dr = 0.0;
+        if (K.mode == 2) {
+            // the run's true constant disturbance, added after the Euler step (component-wise)
+            if (d_plant != nullptr) dr = d_plant[i];
+#pragma unroll
+            for (int c = 0; c < 4; ++c) s[c] = s[c] + K.Bdp[c] * dr;
+        }
 #pragma unroll
         for (int c = 0; c < 4; ++c) x[c * runs + i] = s[c];
         double e[4];
-        if (K.mode == 1) {
+        if (K.mode == 2) {
+            // augmented observer: y = C s + Cd_p d_r measured, innovation against C x^ + Cd d^
+            double xh[4], innov[3];
+            const double dh = dhat[i];
+#pragma unroll
+            for (int c = 0; c < 4; ++c) xh[c] = xhat[c * runs + i];
+#pragma unroll
+            for (int r = 0; r < 3; ++r) {
+                double y = K.Cdp[r] * dr, yh = K.Cd[r] * dh;
+#pragma unroll
+                for (int c = 0; c < 4; ++c) { y += K.C[r * 4 + c] * s[c]; yh += K.C[r * 4 + c] * xh[c]; }
+                innov[r] = y - yh;
+            }
+            double dn = dh;
+#pragma unroll
+            for (int r = 0; r < 4; ++r) {
+                double t = K.Bd[r] * dh;
+#pragma unroll
+                for (int c = 0; c < 4; ++c) t += K.A[r * 4 + c] * xh[c];
+                t += K.B[r * 2 + 0] * u[0] + K.B[r * 2 + 1] * u[1];
+#pragma unroll
+                for (int c = 0; c < 3; ++c) t += K.L[r * 3 + c] * innov[c];
+                e[r] = t;
+            }
+#pragma unroll
+            for (int c = 0; c < 3; ++c) dn += K.L2[c] * innov[c];
+#pragma unroll
+            for (int c = 0; c < 4; ++c) xhat[c * runs + i] = e[c];
+            dhat[i] = dn;                  // = the QP's disturbance c of this run
+        } else if (K.mode == 1) {
             double xh[4], innov[3];
 #pragma unroll
             for (int c = 0; c < 4; ++c) xh[c] = xhat[c * runs + i];
@@ -107,12 +152,15 @@ loop_apply_kernel(int64_t runs, int step, const int* __restrict__ live_list, int
     }
 }
 
-// replayed steps: the input log of this step, then the step number moves on (one thread, after everything that read it)
+// replayed steps: the input (and disturbance-estimate) logs of this step, then the step number moves on (one thread, after
+// everything that read it)
 __global__ void __launch_bounds__(256)
-loop_log_kernel(int64_t runs, const double* __restrict__ u_prev, double* __restrict__ u_log, const int* __restrict__ step_dev) {
+loop_log_kernel(int64_t runs, const double* __restrict__ u_prev, double* __restrict__ u_log, const double* __restrict__ dhat,
+                double* __restrict__ dhat_log, const int* __restrict__ step_dev) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= 2 * runs) return;
-    u_log[(size_t)*step_dev * 2 * runs + i] = u_prev[i];
+    if (u_log != nullptr) u_log[(size_t)*step_dev * 2 * runs + i] = u_prev[i];
+    if (dhat_log != nullptr && i < runs) dhat_log[(size_t)*step_dev * runs + i] = dhat[i];
 }
 __global__ void loop_next_kernel(int* step_dev) { *step_dev += 1; }
 __global__ void loop_set_kernel(int* step_dev, int v) { *step_dev = v; }
@@ -120,6 +168,164 @@ __global__ void loop_set_kernel(int* step_dev, int v) { *step_dev = v; }
 __global__ void fill_i32(int32_t* p, int64_t n, int32_t v) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) p[i] = v;
+}
+
+// Mode-2 state and logs of a run set (all nullable: d^ starts at 0, d_r is 0, d^ is kept in a buffer of the driver).
+struct LoopDisturbance {
+    const double* dhat_init;
+    const double* d_plant;
+    double* dhat_final;
+    double* dhat_log;
+};
+
+// The loop shared by every mode: host-driven first steps, then one captured CUDA graph with the step number on the device.
+int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int steps, int warm_start, const double* d_x_init,
+                    const double* d_xhat_init, int64_t runs, double* d_final, int32_t* d_fail_step, double* d_traj,
+                    double* d_u_log, const LoopDisturbance& D, int64_t* h_total_iters, void* stream) {
+    if (q->host_only) { set_error("carmpc_closed_loop: this QP handle was created without a CUDA device"); return CARMPC_ERR_CUDA; }
+    QPBusyGuard guard(q->busy);
+    CARMPC_REQUIRE(guard.acquired, "this QP handle is in use by another call (one call per handle at a time)");
+    const bool dist = K.mode == 2;
+    // The loop runs on its own (capturable) stream, ordered after the caller's stream by an event and joined at the end by
+    // the final synchronisation: the legacy default stream cannot be captured into a graph.
+    cudaStream_t user_st = (cudaStream_t)stream, st = nullptr;
+    cudaEvent_t ev = nullptr;
+    bool graph_ok = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking) == cudaSuccess &&
+                    cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) == cudaSuccess;
+    if (graph_ok) graph_ok = cudaEventRecord(ev, user_st) == cudaSuccess && cudaStreamWaitEvent(st, ev, 0) == cudaSuccess;
+    if (!graph_ok) { cudaGetLastError(); if (st) cudaStreamDestroy(st); st = user_st; }
+
+    const int mt = q->admm.mt;
+    double *x = d_final, *xhat = nullptr, *est = nullptr, *u_prev = nullptr, *u0 = nullptr, *dhat_own = nullptr;
+    int32_t* status = nullptr;
+    int *live_list = nullptr, *live_count = nullptr;
+    float* warm = nullptr;
+    int rc = CARMPC_OK;
+    auto cleanup = [&]() { if (st != user_st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); } if (ev) cudaEventDestroy(ev);
+                           q->defer_total = 0; q->certify_with_c = 0;
+                           cudaFree(xhat); cudaFree(est); cudaFree(u_prev); cudaFree(u0); cudaFree(status); cudaFree(live_list);
+                           cudaFree(live_count); cudaFree(warm); cudaFree(dhat_own); };
+#define TRY(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) { set_error("%s: %s", #call, cudaGetErrorString(e__)); cleanup(); return CARMPC_ERR_CUDA; } } while (0)
+    TRY(cudaMalloc(&xhat, sizeof(double) * 4 * runs));
+    TRY(cudaMalloc(&est, sizeof(double) * 4 * runs));
+    TRY(cudaMalloc(&u_prev, sizeof(double) * 2 * runs));
+    TRY(cudaMalloc(&u0, sizeof(double) * 2 * runs));
+    TRY(cudaMalloc(&status, sizeof(int32_t) * runs));
+    TRY(cudaMalloc(&live_list, sizeof(int) * runs));
+    TRY(cudaMalloc(&live_count, sizeof(int) * 2));      // [0] live runs of the step, [1] step number of replayed steps
+    if (warm_start) TRY(cudaMalloc(&warm, sizeof(float) * (size_t)mt * runs));
+    // mode 2: the disturbance estimate of every run, which is also the QP's per-run c (fixed address: graph-safe)
+    double* dhat = nullptr;
+    if (dist) {
+        dhat = D.dhat_final;
+        if (dhat == nullptr) { TRY(cudaMalloc(&dhat_own, sizeof(double) * runs)); dhat = dhat_own; }
+        if (D.dhat_init != nullptr) {
+            if (D.dhat_init != dhat) TRY(cudaMemcpyAsync(dhat, D.dhat_init, sizeof(double) * runs, cudaMemcpyDeviceToDevice, st));
+        } else {
+            TRY(cudaMemsetAsync(dhat, 0, sizeof(double) * runs, st));
+        }
+    }
+    const double* c_qp = dhat;
+    if (x != d_x_init) TRY(cudaMemcpyAsync(x, d_x_init, sizeof(double) * 4 * runs, cudaMemcpyDeviceToDevice, st));
+    TRY(cudaMemcpyAsync(xhat, d_xhat_init ? d_xhat_init : d_x_init, sizeof(double) * 4 * runs, cudaMemcpyDeviceToDevice, st));
+    TRY(cudaMemsetAsync(u_prev, 0, sizeof(double) * 2 * runs, st));
+    const int blocks = (int)((runs + 255) / 256);
+    fill_i32<<<blocks, 256, 0, st>>>(d_fail_step, runs, -1);
+    int64_t total_iters = 0;
+    bool warm_valid = false;
+    // the iteration total accumulates on the device over the steps (one read at the end instead of one per step)
+    rc = q->ensure_workspace(runs);
+    if (rc != CARMPC_OK) { cleanup(); return rc; }
+    TRY(cudaMemsetAsync(q->ws_total_iters, 0, sizeof(unsigned long long), st));
+    q->defer_total = 1;
+    // host-driven steps run the filter / decide certificates on the disturbance-shifted bounds too
+    q->certify_with_c = dist ? 1 : 0;
+    // One enqueue-only step (every count stays on the device).  step_dev == nullptr: the step number k comes from the host.
+    auto enqueue_step = [&](int k, const int* step_dev) -> int {
+        cudaError_t e = cudaMemsetAsync(live_count, 0, sizeof(int), st);
+        if (e != cudaSuccess) { set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return CARMPC_ERR_CUDA; }
+        loop_advance_kernel<<<blocks, 256, 0, st>>>(K, runs, x, xhat, u_prev, d_fail_step, est, live_list, live_count,
+                                                    d_traj ? (step_dev ? d_traj : d_traj + (size_t)k * 4 * runs) : nullptr, step_dev,
+                                                    dhat, D.d_plant);
+        const int rc2 = q->solve_enqueue(est, runs, h_xref, c_qp, live_list, live_count, runs, u0, status, warm, st);
+        if (rc2 != CARMPC_OK) return rc2;
+        loop_apply_kernel<<<blocks, 256, 0, st>>>(runs, k, live_list, (int)runs, live_count, u0, status, u_prev, d_fail_step, step_dev);
+        if (step_dev) {
+            if (d_u_log || D.dhat_log)
+                loop_log_kernel<<<(int)((2 * runs + 255) / 256), 256, 0, st>>>(runs, u_prev, d_u_log, dhat, D.dhat_log, step_dev);
+        } else {
+            if (d_u_log) e = cudaMemcpyAsync(d_u_log + (size_t)k * 2 * runs, u_prev, sizeof(double) * 2 * runs, cudaMemcpyDeviceToDevice, st);
+            if (e == cudaSuccess && D.dhat_log)
+                e = cudaMemcpyAsync(D.dhat_log + (size_t)k * runs, dhat, sizeof(double) * runs, cudaMemcpyDeviceToDevice, st);
+            if (e != cudaSuccess) { set_error("cudaMemcpyAsync: %s", cudaGetErrorString(e)); return CARMPC_ERR_CUDA; }
+        }
+        if (step_dev) loop_next_kernel<<<1, 1, 0, st>>>(live_count + 1);
+        return CARMPC_OK;
+    };
+    for (int k = 0; k < steps; ++k) {
+        if (warm_valid && warm_start != 2) {
+            // Every later step only enqueues: the number of live runs, of runs whose active set changed, of second-pass and
+            // fallback samples all stay on the device (kernels sized for the upper bound read them there), so the steps
+            // run back to back on the GPU without a host round trip.  The first such step is launched kernel by kernel
+            // (it also fills the kernel-attribute caches); the remaining ones are ONE captured CUDA graph replayed with
+            // the step number on the device, so that a slow host (thousands of small launches otherwise) cannot stretch
+            // the loop.
+            if (!graph_ok || k + 2 >= steps || k < 2) {
+                rc = enqueue_step(k, nullptr);
+                if (rc != CARMPC_OK) { cleanup(); return rc; }
+                continue;
+            }
+            cudaGraph_t graph = nullptr;
+            cudaGraphExec_t exec = nullptr;
+            loop_set_kernel<<<1, 1, 0, st>>>(live_count + 1, k);
+            if (cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
+                // no capture possible here (e.g. the caller is capturing itself): launch the steps one by one
+                cudaGetLastError();
+                graph_ok = false;
+                rc = enqueue_step(k, nullptr);
+                if (rc != CARMPC_OK) { cleanup(); return rc; }
+                continue;
+            }
+            rc = enqueue_step(k, live_count + 1);
+            cudaError_t ce = cudaStreamEndCapture(st, &graph);
+            if (rc == CARMPC_OK && ce != cudaSuccess) { set_error("cudaStreamEndCapture: %s", cudaGetErrorString(ce)); rc = CARMPC_ERR_CUDA; }
+            if (rc == CARMPC_OK && cudaGraphInstantiate(&exec, graph, 0) != cudaSuccess) { set_error("cudaGraphInstantiate failed"); rc = CARMPC_ERR_CUDA; }
+            for (; rc == CARMPC_OK && k < steps; ++k)
+                if (cudaGraphLaunch(exec, st) != cudaSuccess) { set_error("cudaGraphLaunch failed"); rc = CARMPC_ERR_CUDA; }
+            if (exec) cudaGraphExecDestroy(exec);
+            if (graph) cudaGraphDestroy(graph);
+            if (rc != CARMPC_OK) { cudaGetLastError(); cleanup(); return rc; }
+            break;
+        }
+        TRY(cudaMemsetAsync(live_count, 0, sizeof(int), st));
+        loop_advance_kernel<<<blocks, 256, 0, st>>>(K, runs, x, xhat, u_prev, d_fail_step, est, live_list, live_count,
+                                                    d_traj ? d_traj + (size_t)k * 4 * runs : nullptr, nullptr, dhat, D.d_plant);
+        int live = 0;
+        TRY(cudaMemcpyAsync(&live, live_count, sizeof(int), cudaMemcpyDeviceToHost, st));
+        TRY(cudaStreamSynchronize(st));
+        if (live > 0) {
+            // from the second step on, the active set certified at the previous step is tried first
+            rc = q->solve(est, runs, h_xref, c_qp, live_list, live, u0, nullptr, status, nullptr, nullptr, warm,
+                          warm_valid ? 1 : 0, warm ? 1 : 0, st, warm_valid ? 1 : 0);
+            if (rc != CARMPC_OK) { cleanup(); return rc; }
+            warm_valid = warm != nullptr;
+            loop_apply_kernel<<<(live + 255) / 256, 256, 0, st>>>(runs, k, live_list, live, nullptr, u0, status, u_prev, d_fail_step, nullptr);
+        }
+        if (d_u_log)      // the input each run will apply at the next plant step (unchanged for stopped runs)
+            TRY(cudaMemcpyAsync(d_u_log + (size_t)k * 2 * runs, u_prev, sizeof(double) * 2 * runs, cudaMemcpyDeviceToDevice, st));
+        if (D.dhat_log)   // the estimate the QP of this step used (unchanged for stopped runs)
+            TRY(cudaMemcpyAsync(D.dhat_log + (size_t)k * runs, dhat, sizeof(double) * runs, cudaMemcpyDeviceToDevice, st));
+    }
+    q->defer_total = 0;
+    unsigned long long total_dev = 0;
+    TRY(cudaMemcpyAsync(&total_dev, q->ws_total_iters, sizeof(total_dev), cudaMemcpyDeviceToHost, st));
+    TRY(cudaStreamSynchronize(st));
+    total_iters = (int64_t)total_dev;
+    TRY(cudaGetLastError());
+#undef TRY
+    cleanup();
+    if (h_total_iters) *h_total_iters = total_iters;
+    return CARMPC_OK;
 }
 
 }  // namespace
@@ -143,16 +349,6 @@ extern "C" int carmpc_closed_loop(void* qp, int mode, const double* h_A, const d
     if (h_total_iters) *h_total_iters = 0;
     if (runs == 0) return CARMPC_OK;
     CARMPC_REQUIRE(d_x_init && d_final && d_fail_step, "null device pointer");
-    QPBusyGuard guard(q->busy);
-    CARMPC_REQUIRE(guard.acquired, "this QP handle is in use by another call (one call per handle at a time)");
-    // The loop runs on its own (capturable) stream, ordered after the caller's stream by an event and joined at the end by
-    // the final synchronisation: the legacy default stream cannot be captured into a graph.
-    cudaStream_t user_st = (cudaStream_t)stream, st = nullptr;
-    cudaEvent_t ev = nullptr;
-    bool graph_ok = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking) == cudaSuccess &&
-                    cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) == cudaSuccess;
-    if (graph_ok) graph_ok = cudaEventRecord(ev, user_st) == cudaSuccess && cudaStreamWaitEvent(st, ev, 0) == cudaSuccess;
-    if (!graph_ok) { cudaGetLastError(); if (st) cudaStreamDestroy(st); st = user_st; }
     LoopConst K;
     memset(&K, 0, sizeof(K));
     memcpy(K.A, h_A, sizeof(K.A));
@@ -160,116 +356,46 @@ extern "C" int carmpc_closed_loop(void* qp, int mode, const double* h_A, const d
     if (h_C) memcpy(K.C, h_C, sizeof(K.C));
     if (h_L) memcpy(K.L, h_L, sizeof(K.L));
     K.dt = dt; K.l1 = l1; K.mode = mode;
+    const LoopDisturbance none = {nullptr, nullptr, nullptr, nullptr};
+    return closed_loop_run(q, K, h_xref, steps, warm_start, d_x_init, d_xhat_init, runs, d_final, d_fail_step, d_traj, d_u_log,
+                           none, h_total_iters, stream);
+}
 
-    const int mt = q->admm.mt;
-    double *x = d_final, *xhat = nullptr, *est = nullptr, *u_prev = nullptr, *u0 = nullptr;
-    int32_t* status = nullptr;
-    int *live_list = nullptr, *live_count = nullptr;
-    float* warm = nullptr;
-    int rc = CARMPC_OK;
-    auto cleanup = [&]() { if (st != user_st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); } if (ev) cudaEventDestroy(ev);
-                           q->defer_total = 0; cudaFree(xhat); cudaFree(est); cudaFree(u_prev); cudaFree(u0); cudaFree(status); cudaFree(live_list); cudaFree(live_count); cudaFree(warm); };
-#define TRY(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) { set_error("%s: %s", #call, cudaGetErrorString(e__)); cleanup(); return CARMPC_ERR_CUDA; } } while (0)
-    TRY(cudaMalloc(&xhat, sizeof(double) * 4 * runs));
-    TRY(cudaMalloc(&est, sizeof(double) * 4 * runs));
-    TRY(cudaMalloc(&u_prev, sizeof(double) * 2 * runs));
-    TRY(cudaMalloc(&u0, sizeof(double) * 2 * runs));
-    TRY(cudaMalloc(&status, sizeof(int32_t) * runs));
-    TRY(cudaMalloc(&live_list, sizeof(int) * runs));
-    TRY(cudaMalloc(&live_count, sizeof(int) * 2));      // [0] live runs of the step, [1] step number of replayed steps
-    if (warm_start) TRY(cudaMalloc(&warm, sizeof(float) * (size_t)mt * runs));
-    if (x != d_x_init) TRY(cudaMemcpyAsync(x, d_x_init, sizeof(double) * 4 * runs, cudaMemcpyDeviceToDevice, st));
-    TRY(cudaMemcpyAsync(xhat, d_xhat_init ? d_xhat_init : d_x_init, sizeof(double) * 4 * runs, cudaMemcpyDeviceToDevice, st));
-    TRY(cudaMemsetAsync(u_prev, 0, sizeof(double) * 2 * runs, st));
-    const int blocks = (int)((runs + 255) / 256);
-    fill_i32<<<blocks, 256, 0, st>>>(d_fail_step, runs, -1);
-    int64_t total_iters = 0;
-    bool warm_valid = false;
-    // the iteration total accumulates on the device over the steps (one read at the end instead of one per step)
-    rc = q->ensure_workspace(runs);
-    if (rc != CARMPC_OK) { cleanup(); return rc; }
-    TRY(cudaMemsetAsync(q->ws_total_iters, 0, sizeof(unsigned long long), st));
-    q->defer_total = 1;
-    // One enqueue-only step (every count stays on the device).  step_dev == nullptr: the step number k comes from the host.
-    auto enqueue_step = [&](int k, const int* step_dev) -> int {
-        cudaError_t e = cudaMemsetAsync(live_count, 0, sizeof(int), st);
-        if (e != cudaSuccess) { set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return CARMPC_ERR_CUDA; }
-        loop_advance_kernel<<<blocks, 256, 0, st>>>(K, runs, x, xhat, u_prev, d_fail_step, est, live_list, live_count,
-                                                    d_traj ? (step_dev ? d_traj : d_traj + (size_t)k * 4 * runs) : nullptr, step_dev);
-        const int rc2 = q->solve_enqueue(est, runs, h_xref, live_list, live_count, runs, u0, status, warm, st);
-        if (rc2 != CARMPC_OK) return rc2;
-        loop_apply_kernel<<<blocks, 256, 0, st>>>(runs, k, live_list, (int)runs, live_count, u0, status, u_prev, d_fail_step, step_dev);
-        if (d_u_log) {
-            if (step_dev) {
-                loop_log_kernel<<<(int)((2 * runs + 255) / 256), 256, 0, st>>>(runs, u_prev, d_u_log, step_dev);
-            } else {
-                e = cudaMemcpyAsync(d_u_log + (size_t)k * 2 * runs, u_prev, sizeof(double) * 2 * runs, cudaMemcpyDeviceToDevice, st);
-                if (e != cudaSuccess) { set_error("cudaMemcpyAsync: %s", cudaGetErrorString(e)); return CARMPC_ERR_CUDA; }
-            }
-        }
-        if (step_dev) loop_next_kernel<<<1, 1, 0, st>>>(live_count + 1);
-        return CARMPC_OK;
-    };
-    for (int k = 0; k < steps; ++k) {
-        if (warm_valid && warm_start != 2) {
-            // Every later step only enqueues: the number of live runs, of runs whose active set changed, of second-pass and
-            // fallback samples all stay on the device (kernels sized for the upper bound read them there), so the steps
-            // run back to back on the GPU without a host round trip.  The first such step is launched kernel by kernel
-            // (it also fills the kernel-attribute caches); the remaining ones are ONE captured CUDA graph replayed with
-            // the step number on the device, so that a slow host (thousands of small launches otherwise) cannot stretch
-            // the loop.
-            if (!graph_ok || k + 2 >= steps || k < 2) {
-                rc = enqueue_step(k, nullptr);
-                if (rc != CARMPC_OK) { q->defer_total = 0; cleanup(); return rc; }
-                continue;
-            }
-            cudaGraph_t graph = nullptr;
-            cudaGraphExec_t exec = nullptr;
-            loop_set_kernel<<<1, 1, 0, st>>>(live_count + 1, k);
-            if (cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
-                // no capture possible here (e.g. the caller is capturing itself): launch the steps one by one
-                cudaGetLastError();
-                graph_ok = false;
-                rc = enqueue_step(k, nullptr);
-                if (rc != CARMPC_OK) { q->defer_total = 0; cleanup(); return rc; }
-                continue;
-            }
-            rc = enqueue_step(k, live_count + 1);
-            cudaError_t ce = cudaStreamEndCapture(st, &graph);
-            if (rc == CARMPC_OK && ce != cudaSuccess) { set_error("cudaStreamEndCapture: %s", cudaGetErrorString(ce)); rc = CARMPC_ERR_CUDA; }
-            if (rc == CARMPC_OK && cudaGraphInstantiate(&exec, graph, 0) != cudaSuccess) { set_error("cudaGraphInstantiate failed"); rc = CARMPC_ERR_CUDA; }
-            for (; rc == CARMPC_OK && k < steps; ++k)
-                if (cudaGraphLaunch(exec, st) != cudaSuccess) { set_error("cudaGraphLaunch failed"); rc = CARMPC_ERR_CUDA; }
-            if (exec) cudaGraphExecDestroy(exec);
-            if (graph) cudaGraphDestroy(graph);
-            if (rc != CARMPC_OK) { cudaGetLastError(); q->defer_total = 0; cleanup(); return rc; }
-            break;
-        }
-        TRY(cudaMemsetAsync(live_count, 0, sizeof(int), st));
-        loop_advance_kernel<<<blocks, 256, 0, st>>>(K, runs, x, xhat, u_prev, d_fail_step, est, live_list, live_count,
-                                                    d_traj ? d_traj + (size_t)k * 4 * runs : nullptr, nullptr);
-        int live = 0;
-        TRY(cudaMemcpyAsync(&live, live_count, sizeof(int), cudaMemcpyDeviceToHost, st));
-        TRY(cudaStreamSynchronize(st));
-        if (live > 0) {
-            // from the second step on, the active set certified at the previous step is tried first
-            rc = q->solve(est, runs, h_xref, nullptr, live_list, live, u0, nullptr, status, nullptr, nullptr, warm,
-                          warm_valid ? 1 : 0, warm ? 1 : 0, st, warm_valid ? 1 : 0);
-            if (rc != CARMPC_OK) { q->defer_total = 0; cleanup(); return rc; }
-            warm_valid = warm != nullptr;
-            loop_apply_kernel<<<(live + 255) / 256, 256, 0, st>>>(runs, k, live_list, live, nullptr, u0, status, u_prev, d_fail_step, nullptr);
-        }
-        if (d_u_log)      // the input each run will apply at the next plant step (unchanged for stopped runs)
-            TRY(cudaMemcpyAsync(d_u_log + (size_t)k * 2 * runs, u_prev, sizeof(double) * 2 * runs, cudaMemcpyDeviceToDevice, st));
-    }
-    q->defer_total = 0;
-    unsigned long long total_dev = 0;
-    TRY(cudaMemcpyAsync(&total_dev, q->ws_total_iters, sizeof(total_dev), cudaMemcpyDeviceToHost, st));
-    TRY(cudaStreamSynchronize(st));
-    total_iters = (int64_t)total_dev;
-    TRY(cudaGetLastError());
-#undef TRY
-    cleanup();
-    if (h_total_iters) *h_total_iters = total_iters;
-    return CARMPC_OK;
+extern "C" int carmpc_closed_loop_disturbance(void* qp, const double* h_A, const double* h_B, const double* h_C,
+                                              const carmpc_disturbance_model* dm, const double* h_xref, double dt, double l1,
+                                              int steps, int warm_start, const double* d_x_init, const double* d_xhat_init,
+                                              const double* d_dhat_init, const double* d_d_plant, int64_t runs,
+                                              double* d_final, double* d_dhat_final, int32_t* d_fail_step, double* d_traj,
+                                              double* d_u_log, double* d_dhat_log, int64_t* h_total_iters, void* stream) {
+    QPHandle* q = check_handle<QPHandle>(qp, kQP);
+    CARMPC_REQUIRE(q != nullptr, "not a QP handle");
+    CARMPC_REQUIRE(h_A && h_B && h_C && h_xref, "null model pointer");
+    CARMPC_REQUIRE(dm != nullptr, "null disturbance model");
+    CARMPC_REQUIRE(steps >= 0 && runs >= 0 && runs < (int64_t)1 << 31, "steps / runs");
+    CARMPC_REQUIRE(warm_start >= 0 && warm_start <= 2, "warm_start must be 0, 1 or 2");
+    CARMPC_REQUIRE(dt > 0 && l1 > 0, "dt, l1");
+    bool finite = true;
+    const double* gains[] = {dm->Bd, dm->Cd, dm->L1, dm->L2, dm->Bd_plant, dm->Cd_plant};
+    const int counts[] = {4, 3, 12, 3, 4, 3};
+    for (int g = 0; g < 6; ++g)
+        for (int j = 0; j < counts[g]; ++j) finite = finite && isfinite(gains[g][j]);
+    CARMPC_REQUIRE(finite, "disturbance model and observer gains must be finite");
+    if (h_total_iters) *h_total_iters = 0;
+    if (runs == 0) return CARMPC_OK;
+    CARMPC_REQUIRE(d_x_init && d_final && d_fail_step, "null device pointer");
+    LoopConst K;
+    memset(&K, 0, sizeof(K));
+    memcpy(K.A, h_A, sizeof(K.A));
+    memcpy(K.B, h_B, sizeof(K.B));
+    memcpy(K.C, h_C, sizeof(K.C));
+    memcpy(K.L, dm->L1, sizeof(K.L));
+    memcpy(K.Bd, dm->Bd, sizeof(K.Bd));
+    memcpy(K.Cd, dm->Cd, sizeof(K.Cd));
+    memcpy(K.L2, dm->L2, sizeof(K.L2));
+    memcpy(K.Bdp, dm->Bd_plant, sizeof(K.Bdp));
+    memcpy(K.Cdp, dm->Cd_plant, sizeof(K.Cdp));
+    K.dt = dt; K.l1 = l1; K.mode = 2;
+    const LoopDisturbance D = {d_dhat_init, d_d_plant, d_dhat_final, d_dhat_log};
+    return closed_loop_run(q, K, h_xref, steps, warm_start, d_x_init, d_xhat_init, runs, d_final, d_fail_step, d_traj, d_u_log,
+                           D, h_total_iters, stream);
 }

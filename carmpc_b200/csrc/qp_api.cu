@@ -273,11 +273,14 @@ int QPHandle::solve(const double* d_x0, int64_t stride, const double* xref, cons
         CARMPC_CUDA(cudaStreamSynchronize(st));
     }
     const int* second_list = ws_failed;
-    if (n_failed > 0 && d_c == nullptr) {
+    // The certificate kernels take the disturbance shift as well; the public entry points keep their results with a
+    // disturbance (max_iter instead of a certified "infeasible"), only the closed loop turns them on (certify_with_c).
+    const bool certify = d_c == nullptr || certify_with_c;
+    if (n_failed > 0 && certify) {
         // most of what the first pass could not settle is barely infeasible: the exact certificate test on the first-pass
         // state removes those before the (long) tighter pass
         CARMPC_CUDA(cudaMemsetAsync(ws_counters + 7, 0, sizeof(int), st));
-        rc = farkas_filter_launch(this, ws_failed, n_failed, status, ab.warm, d_x0, stride, d_u0, d_objective, d_u_full,
+        rc = farkas_filter_launch(this, ws_failed, n_failed, status, ab.warm, d_x0, stride, d_c, d_u0, d_objective, d_u_full,
                                   ws_polished, ws_overflow, ws_counters + 7, st);
         if (rc != CARMPC_OK) return rc;
         ++last_launches;
@@ -298,10 +301,10 @@ int QPHandle::solve(const double* d_x0, int64_t stride, const double* xref, cons
         rc = polish_launch(this, pb, st);
         if (rc != CARMPC_OK) return rc;
         // whoever is still at "max_iter" is almost always barely infeasible: the dual iterate of its final ADMM state,
-        // evaluated exactly, settles it (the disturbance-shifted form has no certificate kernel: those keep max_iter)
-        if (d_c == nullptr) {
-            rc = farkas_decide_launch(this, second_list, n_failed, status, ab.warm, d_x0, stride, d_u0, d_objective, d_u_full,
-                                      ws_polished, st);
+        // evaluated exactly, settles it
+        if (certify) {
+            rc = farkas_decide_launch(this, second_list, n_failed, status, ab.warm, d_x0, stride, d_c, d_u0, d_objective,
+                                      d_u_full, ws_polished, st);
             if (rc != CARMPC_OK) return rc;
             ++last_launches;
         }
@@ -327,8 +330,9 @@ int QPHandle::solve(const double* d_x0, int64_t stride, const double* xref, cons
     return CARMPC_OK;
 }
 
-int QPHandle::solve_enqueue(const double* d_x0, int64_t stride, const double* xref, const int* d_idx, const int* d_count,
-                            int64_t max_count, double* d_u0, int32_t* d_status, float* d_warm, cudaStream_t st) {
+int QPHandle::solve_enqueue(const double* d_x0, int64_t stride, const double* xref, const double* d_c, const int* d_idx,
+                            const int* d_count, int64_t max_count, double* d_u0, int32_t* d_status, float* d_warm,
+                            cudaStream_t st) {
     if (host_only) { set_error("carmpc_qp: this handle was created without a CUDA device; there is no CPU solver"); return CARMPC_ERR_CUDA; }
     if (!host.opts.polish) { set_error("solve_enqueue needs the float64 polish (opts.polish = 1)"); return CARMPC_ERR_INVALID; }
     int rc = ensure_workspace(stride);
@@ -337,9 +341,10 @@ int QPHandle::solve_enqueue(const double* d_x0, int64_t stride, const double* xr
     const int cap = (int)max_count;
     int* status = d_status;
 
+    // every stage below (pu, p0, the polish passes, ab, the certificates, the fallback) sees the same disturbance d_c
     PolishBatch pb;
     memset(&pb, 0, sizeof(pb));
-    pb.x0 = d_x0; pb.stride = stride;
+    pb.x0 = d_x0; pb.stride = stride; pb.cdist = d_c;
     for (int c = 0; c < 4; ++c) pb.xref[c] = xref[c];
     pb.sign = ws_sign; pb.u_admm = ws_u; pb.status = status; pb.u0 = d_u0; pb.polished = ws_polished;
     pb.rounds = -1; pb.stats = ws_polish_stats; pb.sign_out = ws_sign;
@@ -361,7 +366,7 @@ int QPHandle::solve_enqueue(const double* d_x0, int64_t stride, const double* xr
     // 2. ADMM (warm-started from the previous step's state) for the runs whose set changed, then the polish
     AdmmBatch ab;
     memset(&ab, 0, sizeof(ab));
-    ab.x0 = d_x0; ab.stride = stride;
+    ab.x0 = d_x0; ab.stride = stride; ab.cdist = d_c;
     for (int c = 0; c < 4; ++c) ab.xref[c] = xref[c];
     ab.idx_list = ws_failed0; ab.count = cap; ab.count_dev = ws_counters + 5; ab.narrow = 1; ab.next = ws_counters + 0;
     ab.sign = ws_sign; ab.u_admm = ws_u; ab.status = status; ab.iters = ws_iters;
@@ -373,7 +378,7 @@ int QPHandle::solve_enqueue(const double* d_x0, int64_t stride, const double* xr
     pb.n_failed = ws_counters + 1; pb.failed_list = ws_failed; pb.final_pass = 0;
     rc = polish_launch(this, pb, st);
     if (rc != CARMPC_OK) return rc;
-    rc = farkas_verify_launch(this, ws_failed0, cap, status, d_warm, d_x0, stride, nullptr, xref, ws_failed, ws_counters + 1, st,
+    rc = farkas_verify_launch(this, ws_failed0, cap, status, d_warm, d_x0, stride, d_c, xref, ws_failed, ws_counters + 1, st,
                               ws_counters + 5);
     if (rc != CARMPC_OK) return rc;
 
@@ -385,10 +390,10 @@ int QPHandle::solve_enqueue(const double* d_x0, int64_t stride, const double* xr
     pb.idx_list = ws_failed; pb.count_dev = ws_counters + 1; pb.n_failed = ws_counters + 3; pb.final_pass = 1;
     rc = polish_launch(this, pb, st);
     if (rc != CARMPC_OK) return rc;
-    rc = farkas_decide_launch(this, ws_failed, cap, status, d_warm, d_x0, stride, d_u0, nullptr, nullptr, ws_polished, st,
+    rc = farkas_decide_launch(this, ws_failed, cap, status, d_warm, d_x0, stride, d_c, d_u0, nullptr, nullptr, ws_polished, st,
                               ws_counters + 1);
     if (rc != CARMPC_OK) return rc;
-    rc = farkas_verify_launch(this, ws_failed, cap, status, d_warm, d_x0, stride, nullptr, xref, ws_overflow, ws_counters + 13, st,
+    rc = farkas_verify_launch(this, ws_failed, cap, status, d_warm, d_x0, stride, d_c, xref, ws_overflow, ws_counters + 13, st,
                               ws_counters + 1);
     if (rc != CARMPC_OK) return rc;
     int handled = 0;

@@ -280,12 +280,12 @@ int farkas_export_launch(QPHandle* q, const int* d_anchors, int count, const int
                          const double* d_x0, int64_t stride, cudaStream_t st);
 // before the second pass: samples the certificate of their first-pass state proves infeasible are done, the rest is listed
 int farkas_filter_launch(QPHandle* q, const int* d_list, int count, int* d_status, const float* d_warm, const double* d_x0,
-                         int64_t stride, double* d_u0, double* d_objective, double* d_u_full, int8_t* d_polished,
-                         int* d_survivors, int* d_n_survivors, cudaStream_t st);
+                         int64_t stride, const double* d_c, double* d_u0, double* d_objective, double* d_u_full,
+                         int8_t* d_polished, int* d_survivors, int* d_n_survivors, cudaStream_t st);
 // samples that ran out of ADMM iterations: a valid certificate from their final ADMM state makes them proven infeasible
 int farkas_decide_launch(QPHandle* q, const int* d_list, int count, int* d_status, const float* d_warm, const double* d_x0,
-                         int64_t stride, double* d_u0, double* d_objective, double* d_u_full, int8_t* d_polished,
-                         cudaStream_t st, const int* d_count = nullptr);
+                         int64_t stride, const double* d_c, double* d_u0, double* d_objective, double* d_u_full,
+                         int8_t* d_polished, cudaStream_t st, const int* d_count = nullptr);
 // ADMM verdicts "infeasible" are only accepted with a float64 certificate: the others re-enter the second pass
 int farkas_verify_launch(QPHandle* q, const int* d_list, int count, int* d_status, const float* d_warm, const double* d_x0,
                          int64_t stride, const double* d_c, const double* xref, int* d_failed, int* d_n_failed, cudaStream_t st,
@@ -325,6 +325,9 @@ struct QPHandle : HandleBase {
     unsigned long long* ws_polish_stats = nullptr;   // [kPolishStats] histogram of the polish launches of the last solve
     int stats_hold = 0;
     int defer_total = 0;                         // closed loop: ws_total_iters accumulates over the steps, read once at the end
+    int certify_with_c = 0;                      // closed loop with a disturbance estimate: solve() also runs the filter /
+                                                 // decide certificates on the disturbance-shifted bounds (the public
+                                                 // entry points keep max_iter there)
     int* ws_overflow = nullptr;
     int* ws_unproven = nullptr;                  // samples the second pass left without a proof (float64 fallback)
     int* ws_counters = nullptr;                  // [0] work counter, [1] n_failed
@@ -354,8 +357,9 @@ struct QPHandle : HandleBase {
     // The same pipeline for a warm-started sequence (closed loop), with every sample count left on the device: the list
     // d_idx holds *d_count <= max_count entries, the previous step's certified active sets are tried first, and nothing
     // is read back - the call only enqueues (no host synchronisation), so consecutive steps run back to back on the GPU.
-    int solve_enqueue(const double* d_x0, int64_t stride, const double* xref, const int* d_idx, const int* d_count,
-                      int64_t max_count, double* d_u0, int32_t* d_status, float* d_warm, cudaStream_t st);
+    // d_c (nullable): per-sample disturbance estimate, indexed like d_x0; every stage shifts its bounds by Gc c.
+    int solve_enqueue(const double* d_x0, int64_t stride, const double* xref, const double* d_c, const int* d_idx,
+                      const int* d_count, int64_t max_count, double* d_u0, int32_t* d_status, float* d_warm, cudaStream_t st);
     // anchors (seed[i] == i or out of range) cold, then every other sample from its anchor's certified active set
     int solve_seeded(const double* d_x0, int64_t batch, const double* xref, const double* d_c, const int* d_seed,
                      double* d_u0, double* d_objective, int32_t* d_status, int32_t* d_iters, double* d_u_full,

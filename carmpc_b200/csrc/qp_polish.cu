@@ -629,19 +629,21 @@ int farkas_export_launch(QPHandle* qh, const int* d_anchors, int count, const in
 }
 
 int farkas_decide_launch(QPHandle* qh, const int* d_list, int count, int* d_status, const float* d_warm, const double* d_x0,
-                         int64_t stride, double* d_u0, double* d_objective, double* d_u_full, int8_t* d_polished,
-                         cudaStream_t st, const int* d_count) {
+                         int64_t stride, const double* d_c, double* d_u0, double* d_objective, double* d_u_full,
+                         int8_t* d_polished, cudaStream_t st, const int* d_count) {
     FarkasArgs f = {};
     f.list = d_list; f.count = count; f.count_dev = d_count; f.mode = 1; f.status = d_status; f.warm = d_warm; f.x0 = d_x0; f.stride = stride;
+    f.cdist = d_c;
     f.u0 = d_u0; f.objective = d_objective; f.u_full = d_u_full; f.polished = d_polished; f.stats = qh->ws_polish_stats;
     return farkas_launch(qh, f, st);
 }
 
 int farkas_filter_launch(QPHandle* qh, const int* d_list, int count, int* d_status, const float* d_warm, const double* d_x0,
-                         int64_t stride, double* d_u0, double* d_objective, double* d_u_full, int8_t* d_polished,
-                         int* d_survivors, int* d_n_survivors, cudaStream_t st) {
+                         int64_t stride, const double* d_c, double* d_u0, double* d_objective, double* d_u_full,
+                         int8_t* d_polished, int* d_survivors, int* d_n_survivors, cudaStream_t st) {
     FarkasArgs f = {};
     f.list = d_list; f.count = count; f.mode = 2; f.status = d_status; f.warm = d_warm; f.x0 = d_x0; f.stride = stride;
+    f.cdist = d_c;
     f.u0 = d_u0; f.objective = d_objective; f.u_full = d_u_full; f.polished = d_polished; f.stats = qh->ws_polish_stats;
     f.survivors = d_survivors; f.n_survivors = d_n_survivors;
     return farkas_launch(qh, f, st);

@@ -311,6 +311,32 @@ int carmpc_closed_loop(void* qp, int mode, const double* h_A, const double* h_B,
                        int32_t* d_fail_step, double* d_traj, double* d_u_log, int64_t* h_total_iters,
                        void* stream);
 
+/* Closed loops of the disturbance-estimating output-feedback controller (MPCOutputFBWithDisturbance, lib/mpc.py:329-396):
+ * the same loop, with a constant scalar disturbance per run and an augmented observer.  Step k of a run:
+ *   s  = s + dt * f(s, u_prev);   s = s + Bd_plant * d_r          (plant: Euler step, then the true disturbance)
+ *   y  = C s + Cd_plant * d_r
+ *   i  = y - C x^ - Cd d^;   x^' = A x^ + Bd d^ + B u_prev + L1 i;   d^' = d^ + L2 . i
+ *   QP at x0 = x^', c = d^' (bounds shifted by Gc c), x_ref = h_xref
+ * The QP handle's Gc must describe the same Bd (BatchQP.from_controller of a controller with that Bd); a handle whose Gc
+ * is zero is allowed (c then has no effect).  Infeasible or undecided QPs stop the run (d_fail_step), as in
+ * carmpc_closed_loop; "infeasible" verdicts carry a float64 certificate of the disturbance-shifted problem.
+ * Non-finite gains are rejected; a non-finite d^ or state of one run makes that run's QP infeasible.
+ *   dm: model and gains (L1 4x3 row-major).  d_x_init, d_xhat_init (nullable: x_init): SoA 4 x runs.
+ *   d_dhat_init (nullable: 0), d_d_plant (nullable: 0, the per-run d_r), d_dhat_final (nullable): runs float64.
+ *   d_traj, d_u_log as in carmpc_closed_loop; d_dhat_log (nullable): steps x runs, d^ the QP of each step used.
+ * warm_start 0 / 1 / 2 as in carmpc_closed_loop. */
+typedef struct carmpc_disturbance_model {
+    double Bd[4], Cd[3], L1[12], L2[3];   /* controller: disturbance model and observer gains (L1 4x3 row-major) */
+    double Bd_plant[4], Cd_plant[3];      /* how the true per-run disturbance enters the plant state / output    */
+} carmpc_disturbance_model;
+
+int carmpc_closed_loop_disturbance(void* qp, const double* h_A, const double* h_B, const double* h_C,
+                                   const carmpc_disturbance_model* dm, const double* h_xref, double dt, double l1,
+                                   int steps, int warm_start, const double* d_x_init, const double* d_xhat_init,
+                                   const double* d_dhat_init, const double* d_d_plant, int64_t runs, double* d_final,
+                                   double* d_dhat_final, int32_t* d_fail_step, double* d_traj, double* d_u_log,
+                                   double* d_dhat_log, int64_t* h_total_iters, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Device micro-benchmarks used as roofline denominators that MEASURED_PEAKS.json does not carry.
  * which: 0 = FP32 FFMA TFLOP/s (uniform multiplier), 1 = FP64 DFMA TFLOP/s, 2 = HBM copy GB/s (read+write),

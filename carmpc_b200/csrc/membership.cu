@@ -155,6 +155,12 @@ struct ScreenConst {         // float32 error-bound constants of the polytope
 constexpr int kExit64 = 4;       // rows between "whole warp already outside" votes, float64 path
 constexpr int kRowBlock = 8;     // ... float32 screen (the float32 row image is padded to a multiple of it)
 
+// Largest bound beta(p) = beta0 + beta1 |p|_1 for which the screen may decide.  Every intermediate of a row's float32 chain
+// is at most (|b_r| + sum |a_rk| |p_k|) (1 + 2^-21) <= (bmax + l1max |p|_1) (1 + 2^-21), and the constants are built with
+// beta0 >= 8 u bmax, beta1 >= 8 u l1max (8 u = 2^-21), so that sum is at most beta(p) 2^21.  At beta(p) <= 1e31 it is below
+// 2.2e37 < FLT_MAX / 15: no product or partial sum can overflow to +-inf, which the rounding bound does not cover.
+constexpr float kScreenMaxBound = 1e31f;
+
 // float64 decision of the NS samples of this thread: the contract chain, every row, rows in host-sorted order
 __device__ __forceinline__ void decide64(const double* __restrict__ s_rows, int rows, const double (&x)[kNS],
                                          const double (&y)[kNS], const double (&p)[kNS], const double (&v)[kNS],
@@ -241,12 +247,11 @@ __device__ __forceinline__ void screen32(const RowF32* __restrict__ s_rows32, in
     float nbeta[kNS], ibeta[kNS], mmin[kNS];
 #pragma unroll
     for (int k = 0; k < kNS; ++k) {
-        // |x| + |y| + |psi| + |v| >= max |coordinate|, and (unlike fmaxf) it propagates NaN / inf into the bound,
-        // which then fails both "surely in" and "surely out": such samples are decided by the float64 chain
+        // |x| + |y| + |psi| + |v| >= max |coordinate|, and (unlike fmaxf) it propagates NaN / inf into the bound
         const float psum = (fabsf(xf[k]) + fabsf(yf[k])) + (fabsf(pf[k]) + fabsf(vf[k]));
         nbeta[k] = -fmaf(sc.beta1, psum, sc.beta0);
         ibeta[k] = fmaf(sc.in1, psum, sc.in0);
-        mmin[k] = in[k] ? INFINITY : -INFINITY;              // padding lanes count as "already outside"
+        mmin[k] = in[k] ? kScreenMaxBound : -INFINITY;       // padding lanes count as "already outside"; for the cap see below
     }
     // samples in pairs: the four fmas of a row run as FFMA2 (same IEEE result per sample as fmaf, half the issue slots)
     f32x2 x2[kNS / 2], y2[kNS / 2], p2[kNS / 2], v2[kNS / 2];
@@ -277,7 +282,12 @@ __device__ __forceinline__ void screen32(const RowF32* __restrict__ s_rows32, in
     }
 #pragma unroll
     for (int k = 0; k < kNS; ++k) {
-        const bool sure_in = mmin[k] > ibeta[k], sure_out = mmin[k] < nbeta[k];
+        // No decision where the bound exceeds kScreenMaxBound or is NaN: the float32 chain may have overflowed (its margin
+        // can be a wrong +-inf; the early exit above may act on it, which only skips rows), the coordinates are not finite,
+        // or the beta pair is infinite because the rows have no faithful float32 image.  The float64 chain decides those.
+        // "Surely inside" needs mmin > ibeta >= bound, and mmin never exceeds its start value kScreenMaxBound, so only
+        // "surely outside" needs the explicit test (one compare per sample instead of two).
+        const bool sure_in = mmin[k] > ibeta[k], sure_out = mmin[k] < nbeta[k] && nbeta[k] >= -kScreenMaxBound;
         amb[k] = in[k] && !sure_in && !sure_out;
         in[k] = in[k] && sure_in;
     }
@@ -617,7 +627,7 @@ struct GridDesc {
 };
 
 // implicit tensor grid: coordinates come from four short axes staged in shared memory, no HBM reads at all
-__global__ void __launch_bounds__(kThreads)
+__global__ void __launch_bounds__(kThreads, 4)        // 4 CTAs per SM: the launch below sizes the grid for that
 membership_grid_kernel(const double* __restrict__ g_rows, const RowF32* __restrict__ g_rows32, int rows, int rows_padded,
                        const ScreenConst sc, const double* __restrict__ g_axes, GridDesc gd, int64_t n,
                        uint32_t* __restrict__ bits, unsigned long long* __restrict__ count) {
@@ -1160,6 +1170,7 @@ int carmpc_polytope_create(const double* h_Ab, int rows, void** handle) {
     std::vector<RowF32> r32(pad_rows(rows) > 0 ? pad_rows(rows) : 8);
     for (RowF32& q : r32) { q.na0 = q.na1 = q.na2 = q.na3 = 0.f; q.b = INFINITY; q.pad0 = q.pad1 = q.pad2 = 0.f; }
     double l1max = 0.0, bmax = 0.0;
+    bool faithful = true;            // every coefficient and every finite b has a finite float32 image
     for (int i = 0; i < rows; ++i) {
         const double* a = h_Ab + 5 * order[i];
         for (int k = 0; k < 5; ++k) sorted[5 * i + k] = a[k];
@@ -1168,17 +1179,34 @@ int carmpc_polytope_create(const double* h_Ab, int rows, void** handle) {
         q.b = (float)a[4];
         q.pad0 = q.pad1 = q.pad2 = 0.f;
         r32[i] = q;
+        faithful = faithful && std::isfinite(q.na0) && std::isfinite(q.na1) && std::isfinite(q.na2) && std::isfinite(q.na3) &&
+                   (isinf(a[4]) || std::isfinite(q.b));
         l1max = std::max(l1max, fabs(a[0]) + fabs(a[1]) + fabs(a[2]) + fabs(a[3]));
         if (!isinf(a[4])) bmax = std::max(bmax, fabs(a[4]));
     }
-    // Rounding-error bound of the float32 margin  fma(-a3, v, fma(-a2, psi, fma(-a1, y, fma(-a0, x, b))))  against the
-    // exact  b - a . p :  each input is rounded once (relative 2^-24), each of the <= 4 fmas rounds once, so
-    // |error| <= (4 + 2 + 1) 2^-24 (|b| + sum |a_k| |p_k|) (1 + O(2^-24)); the float64 chain's own error (2^-51 of the
-    // same magnitude) and overflow to inf (coordinates above 1e30 give an inf bound) are covered by using 8 and
-    // rounding the two constants up.
-    const double u8 = 8.0 * 5.9604644775390625e-08;
-    P->beta0 = nextafterf((float)(u8 * bmax * 1.000001 + 1e-37), INFINITY);
-    P->beta1 = nextafterf((float)(u8 * l1max * 1.000001 + 1e-37), INFINITY);
+    // Rounding-error bound of the float32 margin  m = fma(-a3, v, fma(-a2, psi, fma(-a1, y, fma(-a0, x, b))))  against the
+    // exact  b - a . p , as long as no float32 value in it overflows:
+    //   - b, the coefficients and the coordinates are rounded once to float32 (relative 2^-24), and each of the <= 4 fmas
+    //     rounds once (relative 2^-24 of an intermediate, which is at most |b| + sum |a_k| |p_k| up to O(2^-24)), so
+    //     |error| <= (4 + 2 + 1) 2^-24 (|b| + sum |a_k| |p_k|) (1 + O(2^-24));
+    //   - below the normal range a rounding is off by up to 2^-150 in absolute terms instead: for b, a coefficient or an fma
+    //     result that costs at most 2^-150 (4 + |p|_1), inside the 1e-37 floors; for a coordinate (subnormal or zero in
+    //     float32) it costs |a_k| 2^-150 each, at most l1max 2^-150 in all: the l1max 2^-149 term of beta0;
+    //   - the float64 chain's own error (2^-51 of the same magnitude) is covered by using 8 instead of 7 and by rounding the
+    //     two constants up.
+    // The no-overflow condition is enforced, not assumed.  A polytope whose coefficients or finite bounds have no finite
+    // float32 image, or whose constants reach 1e30, gets an infinite beta pair: no sample is decided in float32 and mode 1
+    // returns what the float64 chain returns for every sample.  Otherwise screen32 leaves every sample whose bound exceeds
+    // kScreenMaxBound (non-finite and huge coordinates among them) to the float64 chain.  Rows with b = +inf stay on the
+    // screen: their float32 margin is exactly +inf, which is right.
+    const double u8 = 8.0 * 5.9604644775390625e-08, tiny = 1.401298464324817e-45;      // 2^-149
+    const double b0 = u8 * bmax * 1.000001 + l1max * tiny + 1e-37, b1 = u8 * l1max * 1.000001 + 1e-37;
+    if (faithful && b0 < 1e30 && b1 < 1e30) {
+        P->beta0 = nextafterf((float)b0, INFINITY);
+        P->beta1 = nextafterf((float)b1, INFINITY);
+    } else {
+        P->beta0 = P->beta1 = INFINITY;
+    }
     P->h_rows = sorted;
     h_Ab = sorted.data();
     auto fail = [&](int code) { delete P; return code; };
@@ -1343,9 +1371,12 @@ int carmpc_rollout_create(const double* h_Ak, const double* h_Acon, const double
     // built here in long double, stored as float32 and evaluated like the H-rep screen; a sample is decided by the
     // screen only when its smallest margin clears the bound
     //     8 u32 (|b'| + sum |g_k| |p_k|)   float32 evaluation (as for the H-rep rows)
+    //   + l1max 2^-149                     coordinates below float32's normal range (as for the H-rep rows)
     //   + c64 G (sum |p_k| + |goal|_1)     float64 step-by-step rollout vs the exact linear functional, with
     //                                      G = max entry of |a_r| |A_k|^t and c64 = 16 (k + 3) 2^-53,
-    // everything else is re-evaluated by the float64 contract chain (rollout64).
+    // everything else is re-evaluated by the float64 contract chain (rollout64).  As for the H-rep rows the bound needs the
+    // float32 chain not to overflow: the screen is built only when every expanded row has a finite float32 image and both
+    // constants stay below 1e30, and screen32 decides no sample whose bound exceeds kScreenMaxBound.
     const long total_rows = (long)s * (k_steps + 1) + (long)rin * (input_check_mode == 1 ? k_steps + 1 : 1);
     if (total_rows > 0 && total_rows <= kMaxRows) {
         std::vector<RowF32> r32(pad_rows((int)total_rows));
@@ -1371,7 +1402,8 @@ int carmpc_rollout_create(const double* h_Ak, const double* h_Acon, const double
             q.pad0 = q.pad1 = q.pad2 = 0.f;
             for (int j = 0; j < 4; ++j) R->h_rows64.push_back((double)g[j]);
             R->h_rows64.push_back(b == INFINITY ? INFINITY : (double)bp);
-            finite = finite && std::isfinite(q.na0) && std::isfinite(q.na1) && std::isfinite(q.na2) && std::isfinite(q.na3) && !std::isnan(q.b);
+            finite = finite && std::isfinite(q.na0) && std::isfinite(q.na1) && std::isfinite(q.na2) && std::isfinite(q.na3) &&
+                     (std::isinf(b) || std::isfinite(q.b));
             if (b == INFINITY) q.b = INFINITY;
             r32[w++] = q;
             l1max = std::max(l1max, l1);
@@ -1393,7 +1425,9 @@ int carmpc_rollout_create(const double* h_Ak, const double* h_Acon, const double
             for (int i = 0; i < 16; ++i) { M[i] = N[i]; Mabs[i] = Na[i]; }
         }
         const long double u8 = 8.0L * 5.9604644775390625e-08L, c64 = 16.0L * (k_steps + 3) * 1.1102230246251565e-16L;
-        const long double b0 = u8 * bmax * 1.000001L + c64 * gabs_max * goal1 + 1e-37L, b1 = u8 * l1max * 1.000001L + c64 * gabs_max + 1e-37L;
+        const long double tiny = 1.401298464324817e-45L;                                   // 2^-149: coordinates below float32's normal range
+        const long double b0 = u8 * bmax * 1.000001L + l1max * tiny + c64 * gabs_max * goal1 + 1e-37L,
+                          b1 = u8 * l1max * 1.000001L + c64 * gabs_max + 1e-37L;
         if (finite && std::isfinite((double)b0) && std::isfinite((double)b1) && (double)b0 < 1e30 && (double)b1 < 1e30) {
             R->beta0 = nextafterf((float)b0, INFINITY);
             R->beta1 = nextafterf((float)b1, INFINITY);

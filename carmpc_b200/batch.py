@@ -354,13 +354,17 @@ class BatchQP(_Handle):
 
     # ---- device tensors ---------------------------------------------------------------------------
     def solve(self, x0, x_ref=None, c=None, want_u_full: bool = False, warm=None, warm_in: bool = False,
-              warm_out: bool = False, stream=None, seed=None) -> dict:
+              warm_out: bool = False, stream=None, seed=None, want_certificate: bool = False) -> dict:
         """``x0``: (4, B) float64 CUDA tensor (SoA).  Returns a dict of CUDA tensors: ``u0`` (2, B), ``objective``
         (B,), ``status`` (B,) int32, ``iters`` (B,) int32 and optionally ``u_full`` (B, 2N).
 
         ``seed`` (int32 CUDA tensor of B entries, e.g. ``grids.lattice_seeds``): sample ``i`` first tries the certified
         active set of sample ``seed[i]`` (an anchor: ``seed[a] == a``) and runs ADMM only if that does not certify;
-        ``out["seeded"]`` counts the samples that needed no ADMM iteration.  Same results as the cold solve."""
+        ``out["seeded"]`` counts the samples that needed no ADMM iteration.  Same results as the cold solve.
+
+        ``want_certificate``: also ``out["certificate"]``, a (B, m + n + k) float64 CUDA tensor in the row space of the
+        handle (``carmpc_qp_solve_certified``): the KKT multipliers of solved samples, the Farkas ray of infeasible ones,
+        zeros for undecided ones.  The other outputs are bit-identical to a solve without it (not with ``warm``)."""
         torch = _torch()
         if not (x0.is_cuda and x0.dtype == torch.float64 and x0.dim() == 2 and x0.shape[0] == 4 and x0.is_contiguous()):
             raise ValueError("x0 must be a contiguous (4, B) float64 CUDA tensor")
@@ -380,6 +384,20 @@ class BatchQP(_Handle):
                 raise ValueError("seed and warm are alternative starting points")
             if not (seed.is_cuda and seed.dtype == torch.int32 and seed.numel() == B and seed.is_contiguous()):
                 raise ValueError("seed must be a contiguous int32 CUDA tensor of B entries")
+        if want_certificate:
+            if warm is not None:
+                raise ValueError("certificates are exported by cold and seeded solves, not warm-started ones")
+            out["certificate"] = torch.empty((B, self.m + self.n + len(self.pq.pre_hi)), dtype=torch.float64, device=dev)
+            seeded = ctypes.c_int64(0)
+            check(self._lib.carmpc_qp_solve_certified(
+                self._h, x0.data_ptr(), _capi.ptr(xref), c.data_ptr() if c is not None else None,
+                seed.data_ptr() if seed is not None else None, B, out["u0"].data_ptr(), out["objective"].data_ptr(),
+                out["status"].data_ptr(), out["iters"].data_ptr(), out["u_full"].data_ptr() if want_u_full else None,
+                out["certificate"].data_ptr(), ctypes.byref(seeded), _stream_ptr(stream)))
+            if seed is not None:
+                out["seeded"] = int(seeded.value)
+            return out
+        if seed is not None:
             seeded = ctypes.c_int64(0)
             check(self._lib.carmpc_qp_solve_seeded(
                 self._h, x0.data_ptr(), _capi.ptr(xref), c.data_ptr() if c is not None else None, seed.data_ptr(), B,

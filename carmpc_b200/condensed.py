@@ -23,7 +23,7 @@ Two exact reductions are applied, neither changes the feasible set or the minimi
 """
 from __future__ import annotations
 
-from dataclasses import dataclass
+from dataclasses import dataclass, field
 
 import numpy as np
 
@@ -52,6 +52,9 @@ class ParametricQP:
     # provenance of each general row: index into the one-sided stack (hi side, lo side or -1)
     src_hi: np.ndarray
     src_lo: np.ndarray
+    # the same for the u-independent rows (certificate.to_one_sided); empty: none recorded
+    pre_src_hi: np.ndarray = field(default_factory=lambda: np.zeros(0, dtype=np.int64))
+    pre_src_lo: np.ndarray = field(default_factory=lambda: np.zeros(0, dtype=np.int64))
 
     @property
     def n(self) -> int:
@@ -139,4 +142,4 @@ def build_parametric_qp(controller, merge_rows: bool = True) -> ParametricQP:
         Gc=np.ascontiguousarray(Gc[keep]), lb=lb, ub=ub, Px=np.ascontiguousarray(Gx[param_only]),
         Pc=np.ascontiguousarray(Gc[param_only]), pre_lo=lo[param_only], pre_hi=hi[param_only],
         goal=np.array(controller.goal, dtype=float), T=T, S=S, rows_x=rows_x, rows_b=rows_b,
-        src_hi=src_hi[keep], src_lo=src_lo[keep])
+        src_hi=src_hi[keep], src_lo=src_lo[keep], pre_src_hi=src_hi[param_only], pre_src_lo=src_lo[param_only])

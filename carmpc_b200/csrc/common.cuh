@@ -13,7 +13,8 @@ namespace carmpc {
 constexpr int kNumSMsFallback = 148;     // B200: 2 dies x 74 SMs
 constexpr int kWarp = 32;
 
-enum HandleKind : uint32_t { kPolytope = 0x504f4c59u, kRollout = 0x524f4c4cu, kQP = 0x51504144u, kShard = 0x53485244u };
+enum HandleKind : uint32_t { kPolytope = 0x504f4c59u, kRollout = 0x524f4c4cu, kQP = 0x51504144u, kShard = 0x53485244u,
+                         kQPCheck = 0x51434b52u };
 
 struct HandleBase {
     uint32_t kind;

@@ -189,6 +189,7 @@ int QPHandle::solve(const double* d_x0, int64_t stride, const double* xref, cons
     pb.rounds = host.opts.polish ? -1 : 0;
     pb.final_pass = host.opts.polish ? 0 : 1;
     pb.stats = ws_polish_stats;
+    pb.cert = cert;
     if (!stats_hold) CARMPC_CUDA(cudaMemsetAsync(ws_polish_stats, 0, sizeof(unsigned long long) * kPolishStats, st));
     // warm-started sequences and seeded maps keep the certified (repaired) active set
     if ((d_warm && warm_out) || keep_sign) pb.sign_out = ws_sign;
@@ -538,10 +539,10 @@ int carmpc_qp_create(int n, int m, int k, const double* h_H, const double* h_F, 
         q->tc = q->tc_parts[0];
     }
     PolishTables& p = q->polish;
-    p.n = n; p.m = m; p.mt = m + n;
+    p.n = n; p.m = m; p.mt = m + n; p.kpre = k;
 #define UP(vec, field) do { rc = upload(q, h.vec, &p.field); if (rc != CARMPC_OK) { delete q; return rc; } } while (0)
     UP(H, H); UP(Hinv, Hinv); UP(F, F); UP(Uu, Uu); UP(AUu, AUu); UP(AH, AH); UP(AHA, AHA); UP(Gx, Gx); UP(Gc, Gc); UP(hi, hi); UP(lo, lo);
-    UP(G, G); UP(Eg, Eg);
+    UP(G, G); UP(Eg, Eg); UP(rsign, rsign);
 #undef UP
     {
         ExactTables& e = q->exact;
@@ -675,6 +676,36 @@ int carmpc_qp_solve_seeded(void* qp, const double* d_x0, const double* h_xref, c
     const int rc = q->solve_seeded(d_x0, batch, h_xref, d_c, d_seed, d_u0, d_objective, d_status, d_iters, d_u_full,
                                    (cudaStream_t)stream);
     if (rc == CARMPC_OK && h_seeded) *h_seeded = q->last_reused;
+    return rc;
+}
+
+int carmpc_qp_solve_certified(void* qp, const double* d_x0, const double* h_xref, const double* d_c, const int32_t* d_seed,
+                              int64_t batch, double* d_u0, double* d_objective, int32_t* d_status, int32_t* d_iters,
+                              double* d_u_full, double* d_cert, int64_t* h_seeded, void* stream) {
+    QPHandle* q = check_handle<QPHandle>(qp, kQP);
+    CARMPC_REQUIRE(q != nullptr, "not a QP handle");
+    CARMPC_REQUIRE(batch >= 0 && batch < (int64_t)1 << 31, "batch");
+    CARMPC_REQUIRE(h_xref != nullptr, "h_xref");
+    CARMPC_REQUIRE(q->host.opts.polish != 0, "certificates come from the float64 polish (opts.polish = 1)");
+    if (h_seeded) *h_seeded = 0;
+    if (batch == 0) { q->last_total_iters = 0; q->last_launches = 0; return CARMPC_OK; }
+    CARMPC_REQUIRE(d_x0 && d_status && d_cert, "d_x0, d_status and d_cert are required");
+    QPBusyGuard guard(q->busy);
+    CARMPC_REQUIRE(guard.acquired, "this QP handle is in use by another call (one call per handle at a time)");
+    if (q->host_only) { set_error("carmpc_qp: this handle was created without a CUDA device; there is no CPU solver"); return CARMPC_ERR_CUDA; }
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t width = (size_t)q->host.m + q->host.n + q->host.kpre;
+    CARMPC_CUDA(cudaMemsetAsync(d_cert, 0, sizeof(double) * width * batch, st));
+    struct ResetOnExit { double*& p; ~ResetOnExit() { p = nullptr; } } reset_cert{q->cert};     // also on error returns
+    q->cert = d_cert;
+    int rc;
+    if (d_seed != nullptr) {
+        rc = q->solve_seeded(d_x0, batch, h_xref, d_c, d_seed, d_u0, d_objective, d_status, d_iters, d_u_full, st);
+        if (rc == CARMPC_OK && h_seeded) *h_seeded = q->last_reused;
+    } else {
+        q->use_records = 0;
+        rc = q->solve(d_x0, batch, h_xref, d_c, nullptr, batch, d_u0, d_objective, d_status, d_iters, d_u_full, nullptr, 0, 0, st);
+    }
     return rc;
 }
 

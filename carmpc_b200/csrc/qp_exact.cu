@@ -163,6 +163,15 @@ __device__ __forceinline__ bool exact_farkas(const PolishTables& T, const ExactW
     return isfinite(c0) && isfinite(a0) && a0 > 0.0 && c0 < -1e-9 * a0;
 }
 
+// Certificate row of a ray exact_farkas accepted (y in S.v): the general part in the caller's orientation, the box part by
+// the same expression the test used, zeros on the u-independent rows.
+__device__ __forceinline__ void store_ray(const PolishTables& T, const ExactWs& S, double* row, int lane) {
+    const int n = T.n, m = T.m, mt = T.mt;
+    for (int i = lane; i < m; i += 32) row[i] = T.rsign[i] * S.v[i];
+    for (int j = lane; j < n; j += 32) row[m + j] = -col_dot(T.G, n, j, S.v, m);
+    for (int k = lane; k < T.kpre; k += 32) row[mt + k] = 0.0;
+}
+
 // ---- verification of the float32 "infeasible" verdicts -----------------------------------------------------------------------
 // The float32 ADMM certifies infeasibility with the dual INCREMENT of one iteration (qp_admm.cu) under a 1e-4 relative
 // margin.  Here the same increment is recomputed in float64 - one ADMM iteration from the sample's stored state - and
@@ -175,8 +184,11 @@ struct VerifyArgs {
     const double* Px; const double* Pc; const double* pre_lo; const double* pre_hi; int kpre;
     int* failed; int* n_failed;
     unsigned long long* row_proofs;     // nullable counter: verdicts proven by a single row
+    double* cert;                       // nullable [batch][mt + kpre]: the proof of every verified sample
 };
 
+// CERT: the certificate stores are a separate instantiation, so that a solve without certificates runs the same code as before
+template <bool CERT>
 __global__ void __launch_bounds__(kExactThreads) verify_kernel(const PolishTables T, const ExactTables E, const VerifyArgs A) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -197,10 +209,14 @@ __global__ void __launch_bounds__(kExactThreads) verify_kernel(const PolishTable
                              A.Pc[k] * cd;
             pre_ok = v <= A.pre_hi[k] && v >= A.pre_lo[k];
         }
-        if (!pre_ok) continue;                                         // infeasible whatever u is: nothing to verify
+        if (!pre_ok) {                                                 // infeasible whatever u is: nothing to verify
+            if (CERT) store_pre_certificate(A.cert + (size_t)sample * (mt + T.kpre), mt, T.kpre, A.Px, A.Pc, A.pre_lo, A.pre_hi, x0, cd, lane);
+            continue;
+        }
         __syncwarp();
         // single-row certificates: the bound of a row lies outside what G_i u can reach over the input box
         bool row_proof = false;
+        int proof_row = -1;                                            // the first such row of this lane, +-(i + 1)
         for (int i = lane; i < m; i += 32) {
             const double* gx = T.Gx + (size_t)i * 4;
             const double t0 = gx[0] * x0[0], t1 = gx[1] * x0[1], t2 = gx[2] * x0[2], t3 = gx[3] * x0[3], t4 = T.Gc[i] * cd;
@@ -209,8 +225,23 @@ __global__ void __launch_bounds__(kExactThreads) verify_kernel(const PolishTable
             const double slop = 1e-12 * (fabs(t0) + fabs(t1) + fabs(t2) + fabs(t3) + fabs(t4) + E.rowabs[i] + (isinf(hi) ? 0.0 : fabs(hi)) +
                                          (isinf(lo) ? 0.0 : fabs(lo)));
             row_proof = row_proof || (hi - shift < E.rowmin[i] - slop) || (lo - shift > E.rowmax[i] + slop);
+            if (CERT && row_proof && proof_row == -1) proof_row = hi - shift < E.rowmin[i] - slop ? i + 1 : -(i + 1);
         }
-        if (__any_sync(0xffffffffu, row_proof)) { if (lane == 0 && A.row_proofs) atomicAdd(A.row_proofs, 1ull); continue; }
+        if (__any_sync(0xffffffffu, row_proof)) {
+            if (lane == 0 && A.row_proofs) atomicAdd(A.row_proofs, 1ull);
+            if (CERT) {
+                // y = +-1 on that row, box part -G_i' y: the support value is (hi - shift) - rowmin (or rowmax - (lo - shift))
+                const unsigned proof_lanes = __ballot_sync(0xffffffffu, row_proof);
+                const int pr = __shfl_sync(0xffffffffu, proof_row, __ffs(proof_lanes) - 1);
+                const int i = abs(pr) - 1;
+                const double yi = pr > 0 ? 1.0 : -1.0;
+                double* row = A.cert + (size_t)sample * (mt + T.kpre);
+                for (int e = lane; e < m; e += 32) row[e] = e == i ? T.rsign[i] * yi : 0.0;
+                for (int j = lane; j < n; j += 32) row[m + j] = -T.G[(size_t)i * n + j] * yi;
+                for (int k = lane; k < T.kpre; k += 32) row[mt + k] = 0.0;
+            }
+            continue;
+        }
         exact_setup(T, E, S, x0, dx, cd, A.warm + (size_t)sample * mt, lane);
         bool proven = false;
         for (int round = 0; round < 3 && !proven; ++round) {           // the increment of the 1st, 2nd, 4th iteration from the state
@@ -220,6 +251,11 @@ __global__ void __launch_bounds__(kExactThreads) verify_kernel(const PolishTable
             for (int i = lane; i < m; i += 32) { const double wi = S.w[i]; S.v[i] = (wi - clampd(wi, S.l[i], S.h[i])) - S.yp[i]; }
             __syncwarp();
             proven = exact_farkas(T, S, lane);
+        }
+        if (CERT) {
+            double* row = A.cert + (size_t)sample * (mt + T.kpre);
+            if (proven) store_ray(T, S, row, lane);
+            else for (int e = lane; e < mt + T.kpre; e += 32) row[e] = 0.0;      // a proof stored earlier did not hold up
         }
         if (!proven && lane == 0) {
             A.status[sample] = kStatusNeedsMoreAdmm;
@@ -241,8 +277,10 @@ struct ExactArgs {
     double* u0; double* objective; double* u_full; int8_t* polished;
     unsigned long long* stats;
     unsigned long long* total_iters;
+    double* cert;                 // nullable [batch][mt + kpre]: the ray of every sample proven infeasible here
 };
 
+template <bool CERT>
 __global__ void __launch_bounds__(kExactThreads) exact_kernel(const PolishTables T, const ExactTables E, const ExactArgs A) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -292,6 +330,7 @@ __global__ void __launch_bounds__(kExactThreads) exact_kernel(const PolishTables
                 A.sign[(size_t)sample * mt + i] = (int8_t)((wi > S.h[i]) - (wi < S.l[i]));
             }
         }
+        if (CERT && verdict == CARMPC_QP_INFEASIBLE) store_ray(T, S, A.cert + (size_t)sample * (mt + T.kpre), lane);
         if (verdict != CARMPC_QP_SOLVED && A.u_full) for (int j = lane; j < n; j += 32) A.u_full[(size_t)sample * n + j] = NaN;
         if (lane == 0) {
             A.status[sample] = verdict;
@@ -337,15 +376,16 @@ int exact_fallback(QPHandle* q, const PolishBatch& pb_final, const int* d_list, 
     for (int c = 0; c < 4; ++c) a.xref[c] = pb_final.xref[c];
     a.warm = d_warm; a.sign = q->ws_sign; a.status = pb_final.status; a.iters = d_iters;
     a.u0 = pb_final.u0; a.objective = pb_final.objective; a.u_full = pb_final.u_full; a.polished = q->ws_polished;
-    a.stats = q->ws_polish_stats; a.total_iters = q->ws_total_iters;
+    a.stats = q->ws_polish_stats; a.total_iters = q->ws_total_iters; a.cert = q->cert;
     const int mt = q->polish.mt, nn = q->polish.n;
     // iteration budget: ~4e8 multiply-adds per sample (5000 iterations at N = 20, ~2600 at N = 80)
     const double macs = 2.0 * q->polish.m * nn + (double)nn * nn;
     a.max_iter = (int)std::max(1000.0, std::min(5000.0, 4.0e8 / std::max(1.0, macs)));
     const size_t smem = exact_smem(nn, mt);
-    { const int rc = kernel_config(reinterpret_cast<const void*>(exact_kernel), kExactThreads, smem, nullptr); if (rc != CARMPC_OK) return rc; }
+    void (*kernel)(const PolishTables, const ExactTables, const ExactArgs) = a.cert ? exact_kernel<true> : exact_kernel<false>;
+    { const int rc = kernel_config(reinterpret_cast<const void*>(kernel), kExactThreads, smem, nullptr); if (rc != CARMPC_OK) return rc; }
     const int blocks = std::max(1, std::min((n + 3) / 4, q->sm * 2));
-    exact_kernel<<<blocks, kExactThreads, smem, st>>>(q->polish, q->exact, a);
+    kernel<<<blocks, kExactThreads, smem, st>>>(q->polish, q->exact, a);
     CARMPC_CUDA(cudaGetLastError());
     // one more float64 polish from the float64 active sets; strict: an uncertified sample becomes "undecided"
     PolishBatch pb = pb_final;
@@ -364,12 +404,13 @@ int farkas_verify_launch(QPHandle* q, const int* d_list, int count, int* d_statu
     for (int c = 0; c < 4; ++c) a.xref[c] = xref[c];
     a.warm = d_warm; a.status = d_status;
     a.Px = q->admm.Px; a.Pc = q->admm.Pc; a.pre_lo = q->admm.pre_lo; a.pre_hi = q->admm.pre_hi; a.kpre = q->admm.kpre;
-    a.failed = d_failed; a.n_failed = d_n_failed;
+    a.failed = d_failed; a.n_failed = d_n_failed; a.cert = q->cert;
     const size_t smem = exact_smem(q->polish.n, q->polish.mt);
     int per_sm = 0;
-    { const int rc = kernel_config(reinterpret_cast<const void*>(verify_kernel), kExactThreads, smem, &per_sm); if (rc != CARMPC_OK) return rc; }
+    void (*kernel)(const PolishTables, const ExactTables, const VerifyArgs) = a.cert ? verify_kernel<true> : verify_kernel<false>;
+    { const int rc = kernel_config(reinterpret_cast<const void*>(kernel), kExactThreads, smem, &per_sm); if (rc != CARMPC_OK) return rc; }
     const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>((count + 3) / 4, (int64_t)q->sm * std::max(per_sm, 1)));
-    verify_kernel<<<blocks, kExactThreads, smem, st>>>(q->polish, q->exact, a);
+    kernel<<<blocks, kExactThreads, smem, st>>>(q->polish, q->exact, a);
     CARMPC_CUDA(cudaGetLastError());
     return CARMPC_OK;
 }

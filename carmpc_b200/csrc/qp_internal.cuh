@@ -166,7 +166,9 @@ struct PolishTables {
     const double* lo;        // [mt]
     const double* G;         // [m][n]      general rows (rows bounded only from below negated, as hi / lo)
     const double* Eg;        // [m]         row scaling of the ADMM (its dual iterate is in scaled units)
+    const double* rsign;     // [m]         -1 for a row the setup negated (bounded only from below), else +1
     int n, m, mt;
+    int kpre;                // u-independent rows: a certificate row has mt + kpre entries
 };
 
 struct PolishBatch {
@@ -207,6 +209,7 @@ struct PolishBatch {
     double* rec_lam;         // [records][32][5]
     int* rec_act;            // [records][33]   na (-1: no map), then the active rows in the order of Lam's rows
     int rec_write, rec_read;
+    double* cert;            // nullable [batch][mt + kpre]: multipliers of certified samples (carmpc_qp_solve_certified)
     unsigned long long* stats;   // nullable [20]: [r] samples certified after r repair rounds (r = 0..9), [10] not certified,
                                  // [11] round 0 taken from a multiplier map, [12] certified by a multiplier map alone,
                                  // [13] proven infeasible by the anchor's Farkas certificate (or the u-independent rows),
@@ -246,6 +249,7 @@ struct QPHost {
     std::vector<int2> segB;
     // polish (logical order, unscaled)
     std::vector<double> H, Hinv, F, G, Uu, AUu, AH, AHA, Gx, Gc, hi, lo;
+    std::vector<double> rsign;       // [m] -1 where a row bounded only from below was negated
     // tensor-core form: one part for the whole problem, or one per independent chain (sizes in t; pointers filled by the handle)
     TcTables tc;                     // = tc_parts[0].t
     std::vector<TcPart> tc_parts;
@@ -295,6 +299,24 @@ int exact_fallback(QPHandle* q, const PolishBatch& pb_final, const int* d_list, 
                    cudaStream_t st, int* h_handled, const int* d_count = nullptr);
 size_t admm_smem_bytes(const QPHost& h, int samples_per_lane, bool mats_in_smem);
 
+// Certificate rows (carmpc_qp_solve_certified) are in the caller's orientation: entry i of a general row the setup negated
+// changes sign, so that positive always means "against the upper bound" of the row as passed to carmpc_qp_create.
+// A violated u-independent row is an infeasibility proof by itself: y = +1 (above pre_hi) or -1 (below pre_lo) on the
+// first such row, zeros elsewhere (its G part is zero).  A non-finite state has no certificate: the row stays zero.
+// The whole warp writes the row.
+__device__ __forceinline__ void store_pre_certificate(double* row, int mt, int kpre, const double* Px, const double* Pc,
+                                                      const double* pre_lo, const double* pre_hi, const double (&x0)[4],
+                                                      double cd, int lane) {
+    for (int e = lane; e < mt + kpre; e += 32) row[e] = 0.0;
+    __syncwarp();
+    if (lane != 0) return;
+    for (int k = 0; k < kpre; ++k) {
+        const double v = Px[k * 4 + 0] * x0[0] + Px[k * 4 + 1] * x0[1] + Px[k * 4 + 2] * x0[2] + Px[k * 4 + 3] * x0[3] + Pc[k] * cd;
+        if (v > pre_hi[k]) { row[mt + k] = 1.0; return; }
+        if (v < pre_lo[k]) { row[mt + k] = -1.0; return; }
+    }
+}
+
 struct QPHandle : HandleBase {
     QPHost host;
     AdmmTables admm;
@@ -325,6 +347,8 @@ struct QPHandle : HandleBase {
     unsigned long long* ws_polish_stats = nullptr;   // [kPolishStats] histogram of the polish launches of the last solve
     int stats_hold = 0;
     int defer_total = 0;                         // closed loop: ws_total_iters accumulates over the steps, read once at the end
+    double* cert = nullptr;                      // carmpc_qp_solve_certified: [batch][mt + kpre] certificate rows, zeroed
+                                                 // by the entry point; every proof site below stores what it proved
     int certify_with_c = 0;                      // closed loop with a disturbance estimate: solve() also runs the filter /
                                                  // decide certificates on the disturbance-shifted bounds (the public
                                                  // entry points keep max_iter there)

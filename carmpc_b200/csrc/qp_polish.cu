@@ -170,6 +170,12 @@ __global__ void __launch_bounds__(kPolishThreads, 7) polish_kernel(const PolishT
                 }
             }
             if (proven_infeasible) {
+                if (B.cert) {
+                    // the anchor's exported row is the certificate its record holds (farkas_kernel mode 0 wrote it)
+                    double* row = B.cert + (size_t)sample * (mt + T.kpre);
+                    if (!pre_ok) store_pre_certificate(row, mt, T.kpre, B.Px, B.Pc, B.pre_lo, B.pre_hi, x0, cd, lane);
+                    else for (int e = lane; e < mt + T.kpre; e += 32) row[e] = B.cert[(size_t)sign_src * (mt + T.kpre) + e];
+                }
                 if (lane == 0) {
                     B.status[sample] = CARMPC_QP_INFEASIBLE;
                     if (B.iters_out) B.iters_out[sample] = 0;
@@ -486,6 +492,11 @@ __global__ void __launch_bounds__(kPolishThreads, 7) polish_kernel(const PolishT
         }
         if (certified && B.sign_out) for (int i = lane; i < mt; i += 32) B.sign_out[(size_t)sample * mt + i] = sgn[i];
         if (B.u_full) for (int j = lane; j < n; j += 32) B.u_full[(size_t)sample * n + j] = u[j];
+        // the multipliers this certificate checked (the row was zeroed by the entry point: only active rows are written)
+        if (certified && B.cert) {
+            double* row = B.cert + (size_t)sample * (mt + T.kpre);
+            for (int a = lane; a < na; a += 32) { const int i = act[a]; row[i] = i < m ? T.rsign[i] * rhs[a] : rhs[a]; }
+        }
         // Anchor of a seeded map: export the active rows and the affine multiplier map lambda(x0) = Lam [x0; 1] of this
         // critical region (five more right-hand sides through the factor already in shared memory).
         if (certified && b_rec_write && B.cdist == nullptr) {
@@ -527,11 +538,14 @@ struct FarkasArgs {
     int* status; const float* warm; const double* x0; int64_t stride;
     const double* cdist;                                               // nullable per-sample disturbance
     const int* rec_of; double* rec_lam; int* rec_act;                  // mode 0
+    double* cert;                                                      // nullable: rows of proven samples (mode 0: anchors)
     double* u0; double* objective; double* u_full; int8_t* polished;   // mode 1, 2 (nullable)
     int* survivors; int* n_survivors;                                  // mode 2
     unsigned long long* stats;
 };
 
+// CERT: the certificate store is a separate instantiation, so that a solve without certificates runs the same code as before
+template <bool CERT>
 __global__ void __launch_bounds__(128) farkas_kernel(const PolishTables T, const FarkasArgs F) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -588,6 +602,18 @@ __global__ void __launch_bounds__(128) farkas_kernel(const PolishTables T, const
             if (F.mode == 2 && lane == 0) F.survivors[atomicAdd(F.n_survivors, 1)] = sample;
             continue;
         }
+        if (CERT) {
+            // y as tested above, box part recomputed by the same expression (a mode-0 row replaces the anchor's own proof:
+            // it is the certificate its followers' support values S(x0) use)
+            double* row = F.cert + (size_t)sample * (mt + T.kpre);
+            for (int i = lane; i < m; i += 32) row[i] = T.rsign[i] * y[i];
+            for (int j = lane; j < n; j += 32) {
+                double s = 0.0;
+                for (int i = 0; i < m; ++i) s += T.G[(size_t)i * n + j] * y[i];
+                row[m + j] = -s;
+            }
+            for (int k = lane; k < T.kpre; k += 32) row[mt + k] = 0.0;
+        }
         if (F.mode == 0) {
             if (lane == 0) {
                 double* r = F.rec_lam + (size_t)rec * kPolishSmallActive * 5;
@@ -615,7 +641,8 @@ static int farkas_launch(QPHandle* qh, const FarkasArgs& f, cudaStream_t st) {
     if (f.count <= 0) return CARMPC_OK;
     const size_t smem = sizeof(double) * 4 * (size_t)qh->polish.m;
     const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>((f.count + 3) / 4, (int64_t)qh->sm * 8));
-    farkas_kernel<<<blocks, 128, smem, st>>>(qh->polish, f);
+    if (f.cert) farkas_kernel<true><<<blocks, 128, smem, st>>>(qh->polish, f);
+    else farkas_kernel<false><<<blocks, 128, smem, st>>>(qh->polish, f);
     CARMPC_CUDA(cudaGetLastError());
     return CARMPC_OK;
 }
@@ -624,7 +651,7 @@ int farkas_export_launch(QPHandle* qh, const int* d_anchors, int count, const in
                          const double* d_x0, int64_t stride, cudaStream_t st) {
     FarkasArgs f = {};
     f.list = d_anchors; f.count = count; f.mode = 0; f.status = const_cast<int*>(d_status); f.warm = d_warm; f.x0 = d_x0;
-    f.stride = stride; f.rec_of = qh->ws_rec_of; f.rec_lam = qh->ws_rec_lam; f.rec_act = qh->ws_rec_act;
+    f.stride = stride; f.rec_of = qh->ws_rec_of; f.rec_lam = qh->ws_rec_lam; f.rec_act = qh->ws_rec_act; f.cert = qh->cert;
     return farkas_launch(qh, f, st);
 }
 
@@ -635,6 +662,7 @@ int farkas_decide_launch(QPHandle* qh, const int* d_list, int count, int* d_stat
     f.list = d_list; f.count = count; f.count_dev = d_count; f.mode = 1; f.status = d_status; f.warm = d_warm; f.x0 = d_x0; f.stride = stride;
     f.cdist = d_c;
     f.u0 = d_u0; f.objective = d_objective; f.u_full = d_u_full; f.polished = d_polished; f.stats = qh->ws_polish_stats;
+    f.cert = qh->cert;
     return farkas_launch(qh, f, st);
 }
 
@@ -645,7 +673,7 @@ int farkas_filter_launch(QPHandle* qh, const int* d_list, int count, int* d_stat
     f.list = d_list; f.count = count; f.mode = 2; f.status = d_status; f.warm = d_warm; f.x0 = d_x0; f.stride = stride;
     f.cdist = d_c;
     f.u0 = d_u0; f.objective = d_objective; f.u_full = d_u_full; f.polished = d_polished; f.stats = qh->ws_polish_stats;
-    f.survivors = d_survivors; f.n_survivors = d_n_survivors;
+    f.survivors = d_survivors; f.n_survivors = d_n_survivors; f.cert = qh->cert;
     return farkas_launch(qh, f, st);
 }
 

@@ -149,6 +149,7 @@ int qp_host_setup(int n, int m_in, int kpre, const double* H_in, const double* F
     if (Gc_in) q.Gc.assign(Gc_in, Gc_in + m);
     q.hi.assign(mt, 0.0);
     q.lo.assign(mt, 0.0);
+    q.rsign.assign((size_t)m, 1.0);
     std::vector<char> live(m, 1);
     for (int i = 0; i < m; ++i) {
         double lo = lo_in[i], hi = hi_in[i];
@@ -158,6 +159,7 @@ int qp_host_setup(int n, int m_in, int kpre, const double* H_in, const double* F
             for (int j = 0; j < n; ++j) q.G[(size_t)i * n + j] = -q.G[(size_t)i * n + j];
             for (int c = 0; c < 4; ++c) q.Gx[(size_t)i * 4 + c] = -q.Gx[(size_t)i * 4 + c];
             q.Gc[i] = -q.Gc[i];
+            q.rsign[i] = -1.0;
             const double t = hi; hi = -lo; lo = -t;
         }
         q.hi[i] = hi;

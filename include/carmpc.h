@@ -258,6 +258,40 @@ int carmpc_qp_map_host(void* qp, const double* h_axes, const int32_t dims[4], co
                        const int32_t block[4], const double* h_xref, double* h_u0, double* h_objective,
                        int32_t* h_status, int32_t* h_iters, int64_t* h_seeded);
 
+/* carmpc_qp_solve_batch (d_seed == NULL: cold, no warm state) or carmpc_qp_solve_seeded (d_seed != NULL), with the same
+ * results, that also exports the certificate behind every verdict.  d_cert: batch x (m + n + k) float64, row-major per
+ * sample, in the row space of the handle: the m general rows, the n box rows and the k u-independent rows exactly as
+ * passed to carmpc_qp_create.  Positive means "against the upper bound", negative "against the lower bound".
+ *   CARMPC_QP_SOLVED      the multipliers of the float64 KKT certificate: H u + F (x0 - xref) + G' lam_g + lam_b = 0,
+ *                         non-zero only on rows the polish certified as active; zero on the k rows.
+ *   CARMPC_QP_INFEASIBLE  the Farkas ray y the library checked: G' y_g + y_b = 0 and the support value
+ *                         sum_i (y_i+ hi_i(x0, c) - y_i- lo_i(x0, c)) over all m + n + k rows is negative.  A violated
+ *                         u-independent row is y = +-1 on that row.  A non-finite state has no certificate (zero row).
+ *   CARMPC_QP_MAX_ITER    zeros.
+ * Returns CARMPC_ERR_INVALID when the handle has opts.polish == 0 (no certificate without the polish). */
+int carmpc_qp_solve_certified(void* qp, const double* d_x0, const double* h_xref, const double* d_c,
+                              const int32_t* d_seed, int64_t batch, double* d_u0, double* d_objective,
+                              int32_t* d_status, int32_t* d_iters, double* d_u_full, double* d_cert,
+                              int64_t* h_seeded, void* stream);
+
+/* Independent float64 checker of certificates for a QP in the general two-sided form
+ *     min 1/2 u'Hu + (F (x0 - xref))'u    lo - Gx x0 - Gc c <= G u <= hi - Gx x0 - Gc c ,   lb <= u <= ub
+ * with R general rows (a one-sided stack is lo = -inf), stated by the caller: it shares nothing with a QP handle.
+ * n <= 160, R <= 16000; Gc may be NULL.  H (n x n), F (n x 4), G (R x n), Gx (R x 4) row-major. */
+int carmpc_qp_checker_create(int n, int R, const double* h_H, const double* h_F, const double* h_G,
+                             const double* h_Gx, const double* h_Gc, const double* h_lo, const double* h_hi,
+                             const double* h_lb, const double* h_ub, void** handle);
+
+/* Checks one certificate row per sample (d_cert: batch x (R + n), general rows then box, sign convention of
+ * carmpc_qp_solve_certified) against d_status / d_u_full (batch x n).  d_x0: SoA 4 x batch; d_c nullable.
+ * d_resid: batch x 4 float64.  Status 0: [primal violation, stationarity, multiplier against an infinite bound,
+ * complementarity], all relative (qp_check.cu states the scales).  Status 1: [support value of the ray with its box part
+ * completed as -G'y_g, its rounding scale, |G'y_g + y_b|_inf of the given box part relative to max_j sum_i |G_ij y_i|,
+ * mass against infinite bounds]; the ray is a proof iff the last is 0 and support < -4e-12 scale.  Status 2: NaN. */
+int carmpc_qp_check(void* checker, const double* d_x0, const double* h_xref, const double* d_c, int64_t batch,
+                    const int32_t* d_status, const double* d_u_full, const double* d_cert, double* d_resid,
+                    void* stream);
+
 /* Host-buffer convenience: h_x0 is batch x 4 row-major (AoS, as the reference passes states). */
 int carmpc_qp_solve_host(void* qp, const double* h_x0, const double* h_xref, const double* h_c, int64_t batch,
                          double* h_u0 /* batch x 2 */, double* h_objective, int32_t* h_status,

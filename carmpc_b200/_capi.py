@@ -65,6 +65,7 @@ SIGNATURES = {
     "carmpc_qp_solve_seeded": (_i32, [_vp, _dp, _dp, _dp, _vp, _i64, _dp, _dp, _vp, _vp, _dp, ctypes.POINTER(_i64), _vp]),
     "carmpc_qp_solve_certified": (_i32, [_vp, _dp, _dp, _dp, _vp, _i64, _dp, _dp, _vp, _vp, _dp, _dp, ctypes.POINTER(_i64),
                                          _vp]),
+    "carmpc_qp_sensitivity": (_i32, [_vp, _dp, _dp, _i64, _vp, _dp, _dp, _i32, _dp, _dp, _vp, _vp]),
     "carmpc_qp_checker_create": (_i32, [_i32, _i32] + [_dp] * 9 + [ctypes.POINTER(_vp)]),
     "carmpc_qp_check": (_i32, [_vp, _dp, _dp, _dp, _i64, _vp, _dp, _dp, _dp, _vp]),
     "carmpc_qp_map_host": (_i32, [_vp, _dp, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32),

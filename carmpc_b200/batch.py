@@ -412,6 +412,38 @@ class BatchQP(_Handle):
             int(warm_in), int(warm_out), _stream_ptr(stream)))
         return out
 
+    def sensitivity(self, x0, out, c=None, rows: Optional[int] = None, stream=None) -> dict:
+        """Derivatives of a certified solve with respect to ``(x, y, psi, v, c)`` (``carmpc_qp_sensitivity``).
+
+        ``out``: the dict of ``solve(x0, c=c, want_u_full=True, want_certificate=True)`` (cold or seeded) for the same
+        ``x0`` and ``c``.  Returns CUDA tensors ``jac`` (B, rows, 5) = du/dp of the leading ``rows`` variables (default n;
+        2 gives the local gain du0/dp), ``grad_objective`` (B, 5) = dV/dp and ``flags`` (B,) int32 (the bits of
+        ``carmpc_b200.sensitivity``).  Samples with status != 0 get NaN and flags 0.  Nothing is synchronised."""
+        torch = _torch()
+        if not (x0.is_cuda and x0.dtype == torch.float64 and x0.dim() == 2 and x0.shape[0] == 4 and x0.is_contiguous()):
+            raise ValueError("x0 must be a contiguous (4, B) float64 CUDA tensor")
+        B = x0.shape[1]
+        if "u_full" not in out or "certificate" not in out:
+            raise ValueError("out must come from solve(..., want_u_full=True, want_certificate=True)")
+        width = self.m + self.n + len(self.pq.pre_hi)
+        for name, t, shape, dt in (("status", out["status"], (B,), torch.int32),
+                                   ("u_full", out["u_full"], (B, self.n), torch.float64),
+                                   ("certificate", out["certificate"], (B, width), torch.float64)):
+            if not (t.is_cuda and t.dtype == dt and tuple(t.shape) == shape and t.is_contiguous()):
+                raise ValueError(f"out[{name!r}] must be a contiguous {dt} CUDA tensor of shape {shape}")
+        if c is not None and not (c.is_cuda and c.dtype == torch.float64 and c.numel() == B and c.is_contiguous()):
+            raise ValueError("c must be a contiguous float64 CUDA tensor of B entries")
+        rows = self.n if rows is None else int(rows)
+        dev = x0.device
+        res = {"jac": torch.empty((B, rows, 5), dtype=torch.float64, device=dev),
+               "grad_objective": torch.empty((B, 5), dtype=torch.float64, device=dev),
+               "flags": torch.empty(B, dtype=torch.int32, device=dev)}
+        check(self._lib.carmpc_qp_sensitivity(
+            self._h, x0.data_ptr(), c.data_ptr() if c is not None else None, B, out["status"].data_ptr(),
+            out["u_full"].data_ptr(), out["certificate"].data_ptr(), rows, res["jac"].data_ptr(),
+            res["grad_objective"].data_ptr(), res["flags"].data_ptr(), _stream_ptr(stream)))
+        return res
+
     # ---- host arrays ---------------------------------------------------------------------------------
     def _host_result(self, B: int, want_u0=True, want_objective=True, want_u_full=False, pinned=False) -> QPResult:
         """Host result arrays; ``pinned``: page-locked buffers owned by this object and reused by the next call of the same

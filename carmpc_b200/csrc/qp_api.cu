@@ -709,6 +709,22 @@ int carmpc_qp_solve_certified(void* qp, const double* d_x0, const double* h_xref
     return rc;
 }
 
+int carmpc_qp_sensitivity(void* qp, const double* d_x0, const double* d_c, int64_t batch, const int32_t* d_status,
+                          const double* d_u_full, const double* d_cert, int rows, double* d_jac, double* d_grad_obj,
+                          int32_t* d_flags, void* stream) {
+    QPHandle* q = check_handle<QPHandle>(qp, kQP);
+    CARMPC_REQUIRE(q != nullptr, "not a QP handle");
+    CARMPC_REQUIRE(batch >= 0 && batch < (int64_t)1 << 31, "batch");
+    CARMPC_REQUIRE(rows >= 1 && rows <= q->host.n, "1 <= rows <= n");
+    CARMPC_REQUIRE(q->host.opts.polish != 0, "sensitivities need the certificates of the float64 polish (opts.polish = 1)");
+    if (batch == 0) return CARMPC_OK;
+    CARMPC_REQUIRE(d_x0 && d_status && d_u_full && d_cert && d_flags, "d_x0, d_status, d_u_full, d_cert and d_flags are required");
+    if (q->host_only) { set_error("carmpc_qp: this handle was created without a CUDA device; there is no CPU solver"); return CARMPC_ERR_CUDA; }
+    // reads only the handle's constant tables: no workspace, so no busy guard is needed
+    return sensitivity_launch(q, d_x0, d_c, batch, d_status, d_u_full, d_cert, rows, d_jac, d_grad_obj, d_flags,
+                              (cudaStream_t)stream);
+}
+
 int carmpc_qp_solve_host(void* qp, const double* h_x0, const double* h_xref, const double* h_c, int64_t batch,
                          double* h_u0, double* h_objective, int32_t* h_status, int32_t* h_iters, double* h_u_full) {
     QPHandle* q = check_handle<QPHandle>(qp, kQP);

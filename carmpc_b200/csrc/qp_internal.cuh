@@ -30,6 +30,10 @@ constexpr int kAdmmThreads = kAdmmWarps * 32;
 constexpr int kMaxN = 160;        // variables (2 x horizon 80)
 constexpr int kMaxM = 392;        // general rows (8 warps x 7 groups x 7 rows)
 constexpr int kPolishMaxActive = 64;
+// KKT tolerances of the polish's certificate (qp_polish.cu), shared with the sensitivity pass (qp_sensitivity.cu) so that
+// "a row at its bound" and "a multiplier of the right sign" mean what the certificate can distinguish:
+constexpr double kFeasTol = 1e-8;     // a row is satisfied when it exceeds its bound by at most this (absolute)
+constexpr double kSignTol = 1e-9;     // a multiplier is wrong-signed below -kSignTol (1 + max |lambda|)
 constexpr int kPolishStats = 20;       // counters of carmpc_qp_polish_stats
 constexpr int kFirstPassIters = 100;  // iteration cap of the first ADMM pass (stragglers continue in the second pass)
 
@@ -298,6 +302,10 @@ int farkas_verify_launch(QPHandle* q, const int* d_list, int count, int* d_statu
 int exact_fallback(QPHandle* q, const PolishBatch& pb_final, const int* d_list, int count, float* d_warm, int* d_iters,
                    cudaStream_t st, int* h_handled, const int* d_count = nullptr);
 size_t admm_smem_bytes(const QPHost& h, int samples_per_lane, bool mats_in_smem);
+// derivatives of certified solutions (qp_sensitivity.cu); d_x0 SoA with stride = batch, d_jac / d_grad nullable
+int sensitivity_launch(QPHandle* q, const double* d_x0, const double* d_c, int64_t batch, const int32_t* d_status,
+                       const double* d_u_full, const double* d_cert, int rows, double* d_jac, double* d_grad,
+                       int32_t* d_flags, cudaStream_t st);
 
 // Certificate rows (carmpc_qp_solve_certified) are in the caller's orientation: entry i of a general row the setup negated
 // changes sign, so that positive always means "against the upper bound" of the row as passed to carmpc_qp_create.

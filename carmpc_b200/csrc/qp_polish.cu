@@ -20,8 +20,6 @@ constexpr int kPolishRounds = 10;
 constexpr int kPolishSmallActive = 32;
 constexpr int kAddPerRound = 3;      // violated rows added to the active set per repair round
 constexpr int kPolishThreads = 128;
-constexpr double kFeasTol = 1e-8;
-constexpr double kSignTol = 1e-9;
 
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll

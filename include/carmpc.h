@@ -274,6 +274,25 @@ int carmpc_qp_solve_certified(void* qp, const double* d_x0, const double* h_xref
                               int32_t* d_status, int32_t* d_iters, double* d_u_full, double* d_cert,
                               int64_t* h_seeded, void* stream);
 
+/* Derivatives of certified solutions (carmpc_qp_solve_certified outputs) w.r.t. p = (x, y, psi, v, c): the state and
+ * the per-sample disturbance (its column is zero for a handle without Gc).  A solved sample's certificate row names its
+ * active rows S; on the critical region of S the optimal u is affine in p (explicit MPC), and
+ *   d_jac       batch x rows x 5 float64 (nullable): du_r/dp_k for the leading `rows` variables (1 <= rows <= n; rows = 2
+ *               is du0/dp, the local gain of the MPC law)
+ *   d_grad_obj  batch x 5 float64 (nullable): dV/dp of the returned objective V
+ *   d_flags     batch int32: bit 0 DERIVATIVE  u* is differentiable at p and d_jac is its derivative;
+ *               bit 1 WEAK  a row outside S is at a bound (within 1e-8) or a multiplier on S is within the sign tolerance
+ *                     (1e-9 (1 + max |lambda|)) of 0: d_jac is the derivative of the affine piece of S, a one-sided
+ *                     derivative for perturbations that keep those rows inactive;
+ *               bit 2 DEPENDENT  S is linearly dependent: d_jac comes from the independent subset (rows in index order);
+ *               bit 3 TOO_MANY_ROWS  more than 64 rows in S (no solver certificate has that many): d_jac is NaN.
+ * d_x0: SoA 4 x batch; d_c nullable (the disturbance of the solve); d_status, d_u_full (batch x n) and d_cert
+ * (batch x (m + n + k)) as the certified solve returned them.  Samples with status != 0: NaN in d_jac and d_grad_obj,
+ * flags 0.  Only enqueues work on `stream`.  CARMPC_ERR_INVALID for a handle with opts.polish == 0. */
+int carmpc_qp_sensitivity(void* qp, const double* d_x0, const double* d_c, int64_t batch, const int32_t* d_status,
+                          const double* d_u_full, const double* d_cert, int rows, double* d_jac,
+                          double* d_grad_obj, int32_t* d_flags, void* stream);
+
 /* Independent float64 checker of certificates for a QP in the general two-sided form
  *     min 1/2 u'Hu + (F (x0 - xref))'u    lo - Gx x0 - Gc c <= G u <= hi - Gx x0 - Gc c ,   lb <= u <= ub
  * with R general rows (a one-sided stack is lo = -inf), stated by the caller: it shares nothing with a QP handle.

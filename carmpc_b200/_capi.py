@@ -30,6 +30,12 @@ class DisturbanceModel(ctypes.Structure):
                 ("L2", ctypes.c_double * 3), ("Bd_plant", ctypes.c_double * 4), ("Cd_plant", ctypes.c_double * 3)]
 
 
+class LoopNoiseParams(ctypes.Structure):
+    """``carmpc_loop_noise`` (include/carmpc.h)."""
+    _fields_ = [("seed", ctypes.c_uint64), ("first_run", ctypes.c_int64), ("Lw", ctypes.c_double * 16),
+                ("Lv", ctypes.c_double * 16)]
+
+
 _vp, _dp, _i64, _i32 = ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int
 
 #: name -> (restype, argtypes); every function include/carmpc.h declares
@@ -79,6 +85,10 @@ SIGNATURES = {
     "carmpc_closed_loop_disturbance": (_i32, [_vp, _dp, _dp, _dp, ctypes.POINTER(DisturbanceModel), _dp, ctypes.c_double,
                                               ctypes.c_double, _i32, _i32, _dp, _dp, _dp, _dp, _i64, _dp, _dp, _vp, _dp,
                                               _dp, _dp, ctypes.POINTER(_i64), _vp]),
+    "carmpc_closed_loop_stochastic": (_i32, [_vp, _i32, _dp, _dp, _dp, _dp, ctypes.POINTER(DisturbanceModel), _dp,
+                                             ctypes.c_double, ctypes.c_double, _i32, _i32, _dp, _dp, _dp, _dp, _i64, _dp,
+                                             _dp, _vp, _dp, _dp, _dp, ctypes.POINTER(LoopNoiseParams), _dp, _i32, _vp, _vp,
+                                             _vp, ctypes.POINTER(_i64), _vp]),
     "carmpc_measure_peak": (_i32, [_i32, ctypes.POINTER(ctypes.c_double)]),
 }
 

@@ -506,13 +506,60 @@ class BatchQP(_Handle):
         return res
 
     # ---- Monte-Carlo closed loop ------------------------------------------------------------------------
+    @staticmethod
+    def _monitor_rows(monitor) -> np.ndarray:
+        """(rows, 5) [A | b] or (A, b) -> contiguous float64 (rows, 5)."""
+        if isinstance(monitor, (tuple, list)) and len(monitor) == 2:
+            A_, b_ = np.asarray(monitor[0], dtype=np.float64), np.asarray(monitor[1], dtype=np.float64).ravel()
+            if A_.ndim != 2 or A_.shape[1] != 4 or len(b_) != len(A_):
+                raise ValueError("monitor (A, b) must be (rows, 4) and (rows,)")
+            rows = np.hstack((A_, b_[:, None]))
+        else:
+            rows = np.asarray(monitor, dtype=np.float64)
+            if rows.ndim != 2 or rows.shape[1] != 5:
+                raise ValueError("monitor must be (rows, 5) [A | b] or (A, b)")
+        if not 1 <= len(rows) <= 512 or not np.isfinite(rows).all():
+            raise ValueError("monitor must have 1 to 512 finite rows")
+        return np.ascontiguousarray(rows)
+
+    def _closed_loop_stochastic(self, mode, x_init, steps, A_, B_, C_, L_, dm, xref, dt, l1, warm_start, xhat_init,
+                                dhat_init, d_plant, out, noise, monitor, stream) -> None:
+        """``carmpc_closed_loop_stochastic`` into ``out`` (adds the monitor's outputs when ``monitor`` is given)."""
+        torch = _torch()
+        R, dev = x_init.shape[1], x_init.device
+        params = noise.params() if noise is not None else None
+        rows = self._monitor_rows(monitor) if monitor is not None else None
+        if rows is not None:
+            out["violation_step"] = torch.empty(R, dtype=torch.int32, device=dev)
+            out["violation_row"] = torch.empty(R, dtype=torch.int32, device=dev)
+            out["violations_per_step"] = torch.empty(steps, dtype=torch.int32, device=dev)
+
+        def p(key):
+            return out[key].data_ptr() if key in out else None
+
+        total = ctypes.c_int64(0)
+        check(self._lib.carmpc_closed_loop_stochastic(
+            self._h, mode, _capi.ptr(A_), _capi.ptr(B_), _capi.ptr(C_), _capi.ptr(L_),
+            ctypes.byref(dm) if dm is not None else None, _capi.ptr(xref), float(dt), float(l1), int(steps),
+            int(warm_start), x_init.data_ptr(), xhat_init.data_ptr() if xhat_init is not None else None,
+            dhat_init.data_ptr() if dhat_init is not None else None, d_plant.data_ptr() if d_plant is not None else None,
+            R, p("final"), p("dhat"), p("fail_step"), p("traj"), p("inputs"), p("dhat_traj"),
+            ctypes.byref(params) if params is not None else None, _capi.ptr(rows), len(rows) if rows is not None else 0,
+            p("violation_step"), p("violation_row"), p("violations_per_step"), ctypes.byref(total), _stream_ptr(stream)))
+        out["total_iters"] = int(total.value)
+
     def closed_loop(self, x_init, steps: int, A, B, x_ref=None, C=None, L=None, xhat_init=None, dt: float = 0.2,
                     l1: float = 3.5, warm_start: bool = True, want_traj: bool = False, want_inputs: bool = False,
-                    stream=None) -> dict:
+                    noise=None, monitor=None, stream=None) -> dict:
         """Runs ``steps`` closed-loop steps for every column of ``x_init`` ((4, R) float64 CUDA tensor) against the
         nonlinear bicycle.  Output feedback when ``C`` and ``L`` are given (observer started at ``xhat_init`` or the
         true state), state feedback otherwise.  Returns ``final`` (4, R), ``fail_step`` (R,) int32 (-1: never
-        infeasible), optionally ``traj`` (steps, 4, R) and ``inputs`` (steps, 2, R), and ``total_iters``."""
+        infeasible), optionally ``traj`` (steps, 4, R) and ``inputs`` (steps, 2, R), and ``total_iters``.
+
+        ``noise``: a ``carmpc_b200.montecarlo.LoopNoise`` (process and measurement noise drawn on the device).
+        ``monitor``: (rows, 5) ``[A | b]`` or ``(A, b)``, e.g. ``montecarlo.plant_rows(controller)``; the true state is
+        checked against it after every plant step and ``violation_step`` (R,), ``violation_row`` (R,) (-1: none) and
+        ``violations_per_step`` (steps,) int32 are added to the result.  A violation does not stop a run."""
         torch = _torch()
         if not (x_init.is_cuda and x_init.dtype == torch.float64 and x_init.dim() == 2 and x_init.shape[0] == 4
                 and x_init.is_contiguous()):
@@ -530,6 +577,10 @@ class BatchQP(_Handle):
             out["traj"] = torch.empty((steps, 4, R), dtype=torch.float64, device=dev)
         if want_inputs:
             out["inputs"] = torch.empty((steps, 2, R), dtype=torch.float64, device=dev)
+        if noise is not None or monitor is not None:
+            self._closed_loop_stochastic(mode, x_init, steps, A_, B_, C_, L_, None, xref, dt, l1, warm_start, xhat_init,
+                                         None, None, out, noise, monitor, stream)
+            return out
         total = ctypes.c_int64(0)
         check(self._lib.carmpc_closed_loop(
             self._h, mode, _capi.ptr(A_), _capi.ptr(B_), _capi.ptr(C_), _capi.ptr(L_), _capi.ptr(xref), float(dt),
@@ -543,7 +594,7 @@ class BatchQP(_Handle):
     def closed_loop_disturbance(self, x_init, steps: int, A, B, C, Bd, Cd, L1, L2, x_ref=None, Bd_plant=None,
                                 Cd_plant=None, d_plant=None, xhat_init=None, dhat_init=None, dt: float = 0.2,
                                 l1: float = 3.5, warm_start=True, want_traj: bool = False, want_inputs: bool = False,
-                                want_dhat: bool = False, stream=None) -> dict:
+                                want_dhat: bool = False, noise=None, monitor=None, stream=None) -> dict:
         """Closed loops of the disturbance-estimating output-feedback controller (``MPCOutputFBWithDisturbance``,
         ``carmpc_closed_loop_disturbance``): the loop of ``closed_loop`` with a scalar disturbance estimate ``d^`` kept
         beside ``x^`` by the augmented observer (``Bd`` (4,), ``Cd`` (3,), gains ``L1`` (4, 3), ``L2`` (3,); no defaults,
@@ -552,7 +603,8 @@ class BatchQP(_Handle):
         run ((R,) float64 CUDA tensor, None: 0) through ``Bd_plant`` (4,) after its Euler step and ``Cd_plant`` (3,) in its
         output (None: zeros).  ``dhat_init``: (R,) CUDA tensor (None: 0).  ``warm_start``: 0 / 1 (True) / 2 as in
         ``closed_loop``.  Returns ``final`` (4, R), ``dhat`` (R,), ``fail_step`` (R,) int32, ``total_iters`` and
-        optionally ``traj`` (steps, 4, R), ``inputs`` (steps, 2, R), ``dhat_traj`` (steps, R)."""
+        optionally ``traj`` (steps, 4, R), ``inputs`` (steps, 2, R), ``dhat_traj`` (steps, R).  ``noise`` and ``monitor``
+        as in ``closed_loop`` (the measurement noise adds to ``C s + Cd_plant d_r``)."""
         torch = _torch()
         if not (x_init.is_cuda and x_init.dtype == torch.float64 and x_init.dim() == 2 and x_init.shape[0] == 4
                 and x_init.is_contiguous()):
@@ -590,6 +642,10 @@ class BatchQP(_Handle):
             out["inputs"] = torch.empty((steps, 2, R), dtype=torch.float64, device=dev)
         if want_dhat:
             out["dhat_traj"] = torch.empty((steps, R), dtype=torch.float64, device=dev)
+        if noise is not None or monitor is not None:
+            self._closed_loop_stochastic(2, x_init, steps, A_, B_, C_, None, dm, xref, dt, l1, warm_start, xhat_init,
+                                         dhat_init, d_plant, out, noise, monitor, stream)
+            return out
         total = ctypes.c_int64(0)
         check(self._lib.carmpc_closed_loop_disturbance(
             self._h, _capi.ptr(A_), _capi.ptr(B_), _capi.ptr(C_), ctypes.byref(dm), _capi.ptr(xref), float(dt),

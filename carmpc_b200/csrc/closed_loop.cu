@@ -15,11 +15,20 @@
 //
 // One thread per run for plant + observer (4 state and 2 input registers); the QPs of all live runs go through the
 // batched solver with the previous step's ADMM state as warm start.
+//
+// Noise and monitor (carmpc_closed_loop_stochastic, any mode): process noise Lw z_w is added to the plant state after
+// the Euler step (and after Bd_p d_r), the state is then checked against the caller's rows [a | b] with the membership
+// chain of K1 (a violation never stops a run), and measurement noise Lv z_v enters what the controller sees.  z_w, z_v
+// are four standard normals each from Philox4x64-10 (philox.cuh) at counter (first_run + run, step, 0 / 1, 0), key
+// (seed, 0): they depend on nothing but the global run id and the step, so warm-start mode, graph replay and batch
+// composition draw the same noise.  Both are compile-time switches of loop_advance_kernel: with both off it is the
+// code the two deterministic entry points always ran.
 #include <math.h>
 #include <string.h>
 
 #include <stdlib.h>
 
+#include "philox.cuh"
 #include "qp_internal.cuh"
 
 namespace carmpc {
@@ -33,17 +42,38 @@ struct LoopConst {
     int mode;            // 0 state feedback, 1 output feedback, 2 output feedback with a disturbance estimate
 };
 
-// plant step with the previous input, observer update, estimate -> QP input; builds the list of live runs
+// Noise factors of a call (carmpc_loop_noise): v = Lv z, w = Lw z, row-major 4 x 4.
+struct LoopNoise {
+    uint64_t seed;
+    int64_t first_run;
+    double Lw[16], Lv[16];
+};
+
+// Monitor rows (a loop-owned device copy, rows x 5) and its outputs (each nullable).
+struct LoopMonitor {
+    const double* Ab;
+    int rows;
+    int32_t* violation_step;        // runs: first step whose state violates a row, -1 none
+    int32_t* violation_row;         // runs: lowest violated row at that step, -1 none
+    int32_t* per_step;              // steps: runs violating at the step
+};
+
+// plant step with the previous input, observer update, estimate -> QP input; builds the list of live runs.
+// kNoise / kMonitor: process and measurement noise, monitor rows; step is the step number of host-driven steps.
+template <bool kNoise, bool kMonitor>
 __global__ void __launch_bounds__(256)
 loop_advance_kernel(const LoopConst K, int64_t runs, double* __restrict__ x, double* __restrict__ xhat,
                     const double* __restrict__ u_prev, const int32_t* __restrict__ fail_step,
                     double* __restrict__ est, int* __restrict__ live_list, int* __restrict__ live_count,
                     double* __restrict__ traj_step, const int* __restrict__ step_dev,
-                    double* __restrict__ dhat, const double* __restrict__ d_plant) {
+                    double* __restrict__ dhat, const double* __restrict__ d_plant, const LoopNoise N,
+                    const LoopMonitor M, int step) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= runs) return;
     // replayed steps (CUDA graph) read the step number on the device: traj_step is then the base of the trajectory
     if (traj_step != nullptr && step_dev != nullptr) traj_step += (size_t)*step_dev * 4 * runs;
+    if ((kNoise || kMonitor) && step_dev != nullptr) step = *step_dev;
+    bool viol = false;
     double s[4], u[2];
 #pragma unroll
     for (int c = 0; c < 4; ++c) s[c] = x[c * runs + i];
@@ -65,8 +95,41 @@ loop_advance_kernel(const LoopConst K, int64_t runs, double* __restrict__ x, dou
 #pragma unroll
             for (int c = 0; c < 4; ++c) s[c] = s[c] + K.Bdp[c] * dr;
         }
+        double vm[4] = {0.0, 0.0, 0.0, 0.0};      // measurement noise
+        if (kNoise) {
+            const uint64_t run = (uint64_t)(N.first_run + i);
+            double z[4];
+            normal4(N.seed, run, (uint64_t)step, 0, z);
+#pragma unroll
+            for (int c = 0; c < 4; ++c) {
+                double w = 0.0;
+#pragma unroll
+                for (int j = 0; j < 4; ++j) w += N.Lw[c * 4 + j] * z[j];
+                s[c] = s[c] + w;
+            }
+            normal4(N.seed, run, (uint64_t)step, 1, z);
+#pragma unroll
+            for (int c = 0; c < 4; ++c) {
+#pragma unroll
+                for (int j = 0; j < 4; ++j) vm[c] += N.Lv[c * 4 + j] * z[j];
+            }
+        }
 #pragma unroll
         for (int c = 0; c < 4; ++c) x[c * runs + i] = s[c];
+        if (kMonitor) {
+            // K1's mode-0 chain; a NaN never satisfies <=, so a non-finite state violates the first row
+            int bad = -1;
+            for (int r = 0; r < M.rows; ++r) {
+                const double* a = M.Ab + 5 * r;
+                const double lhs = fma(__ldg(a + 3), s[3], fma(__ldg(a + 2), s[2], fma(__ldg(a + 1), s[1], __ldg(a) * s[0])));
+                if (!(lhs <= __ldg(a + 4))) { bad = r; break; }
+            }
+            viol = bad >= 0;
+            if (viol) {
+                if (M.violation_step != nullptr && M.violation_step[i] < 0) M.violation_step[i] = step;
+                if (M.violation_row != nullptr && M.violation_row[i] < 0) M.violation_row[i] = bad;
+            }
+        }
         double e[4];
         if (K.mode == 2) {
             // augmented observer: y = C s + Cd_p d_r measured, innovation against C x^ + Cd d^
@@ -79,6 +142,7 @@ loop_advance_kernel(const LoopConst K, int64_t runs, double* __restrict__ x, dou
                 double y = K.Cdp[r] * dr, yh = K.Cd[r] * dh;
 #pragma unroll
                 for (int c = 0; c < 4; ++c) { y += K.C[r * 4 + c] * s[c]; yh += K.C[r * 4 + c] * xh[c]; }
+                if (kNoise) y += vm[r];
                 innov[r] = y - yh;
             }
             double dn = dh;
@@ -106,6 +170,7 @@ loop_advance_kernel(const LoopConst K, int64_t runs, double* __restrict__ x, dou
                 double y = 0, yh = 0;
 #pragma unroll
                 for (int c = 0; c < 4; ++c) { y += K.C[r * 4 + c] * s[c]; yh += K.C[r * 4 + c] * xh[c]; }
+                if (kNoise) y += vm[r];
                 innov[r] = y - yh;
             }
 #pragma unroll
@@ -122,11 +187,17 @@ loop_advance_kernel(const LoopConst K, int64_t runs, double* __restrict__ x, dou
             for (int c = 0; c < 4; ++c) xhat[c * runs + i] = e[c];
         } else {
 #pragma unroll
-            for (int c = 0; c < 4; ++c) e[c] = s[c];
+            for (int c = 0; c < 4; ++c) e[c] = kNoise ? s[c] + vm[c] : s[c];
         }
 #pragma unroll
         for (int c = 0; c < 4; ++c) est[c * runs + i] = e[c];
         live_list[atomicAdd(live_count, 1)] = (int)i;
+    }
+    if (kMonitor && M.per_step != nullptr) {
+        // one atomic per warp (and per group of threads that arrive together)
+        const unsigned act = __activemask();
+        const unsigned hit = __ballot_sync(act, viol);
+        if (hit != 0 && (int)(threadIdx.x & 31) == __ffs(act) - 1) atomicAdd(M.per_step + step, __popc(hit));
     }
     if (traj_step != nullptr) {
 #pragma unroll
@@ -178,10 +249,21 @@ struct LoopDisturbance {
     double* dhat_log;
 };
 
+// Noise and monitor of a run set: noise == nullptr draws none; monitor_rows == 0 checks none (outputs then null).
+struct LoopStochastic {
+    const LoopNoise* noise;
+    const double* h_monitor_Ab;
+    int monitor_rows;
+    int32_t* violation_step;
+    int32_t* violation_row;
+    int32_t* violations_per_step;
+};
+
 // The loop shared by every mode: host-driven first steps, then one captured CUDA graph with the step number on the device.
 int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int steps, int warm_start, const double* d_x_init,
                     const double* d_xhat_init, int64_t runs, double* d_final, int32_t* d_fail_step, double* d_traj,
-                    double* d_u_log, const LoopDisturbance& D, int64_t* h_total_iters, void* stream) {
+                    double* d_u_log, const LoopDisturbance& D, const LoopStochastic& Z, int64_t* h_total_iters,
+                    void* stream) {
     if (q->host_only) { set_error("carmpc_closed_loop: this QP handle was created without a CUDA device"); return CARMPC_ERR_CUDA; }
     QPBusyGuard guard(q->busy);
     CARMPC_REQUIRE(guard.acquired, "this QP handle is in use by another call (one call per handle at a time)");
@@ -200,11 +282,12 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
     int32_t* status = nullptr;
     int *live_list = nullptr, *live_count = nullptr;
     float* warm = nullptr;
+    double* monitor_Ab = nullptr;
     int rc = CARMPC_OK;
     auto cleanup = [&]() { if (st != user_st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); } if (ev) cudaEventDestroy(ev);
                            q->defer_total = 0; q->certify_with_c = 0;
                            cudaFree(xhat); cudaFree(est); cudaFree(u_prev); cudaFree(u0); cudaFree(status); cudaFree(live_list);
-                           cudaFree(live_count); cudaFree(warm); cudaFree(dhat_own); };
+                           cudaFree(live_count); cudaFree(warm); cudaFree(dhat_own); cudaFree(monitor_Ab); };
 #define TRY(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) { set_error("%s: %s", #call, cudaGetErrorString(e__)); cleanup(); return CARMPC_ERR_CUDA; } } while (0)
     TRY(cudaMalloc(&xhat, sizeof(double) * 4 * runs));
     TRY(cudaMalloc(&est, sizeof(double) * 4 * runs));
@@ -231,6 +314,27 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
     TRY(cudaMemsetAsync(u_prev, 0, sizeof(double) * 2 * runs, st));
     const int blocks = (int)((runs + 255) / 256);
     fill_i32<<<blocks, 256, 0, st>>>(d_fail_step, runs, -1);
+    // noise and monitor: kernel arguments by value (a captured graph keeps them), the rows in a buffer the loop owns
+    LoopNoise noise;
+    memset(&noise, 0, sizeof(noise));
+    if (Z.noise != nullptr) noise = *Z.noise;
+    LoopMonitor mon = {nullptr, 0, Z.violation_step, Z.violation_row, Z.violations_per_step};
+    if (Z.monitor_rows > 0) {
+        TRY(cudaMalloc(&monitor_Ab, sizeof(double) * 5 * Z.monitor_rows));
+        TRY(cudaMemcpyAsync(monitor_Ab, Z.h_monitor_Ab, sizeof(double) * 5 * Z.monitor_rows, cudaMemcpyHostToDevice, st));
+        mon.Ab = monitor_Ab;
+        mon.rows = Z.monitor_rows;
+        if (mon.violation_step) fill_i32<<<blocks, 256, 0, st>>>(mon.violation_step, runs, -1);
+        if (mon.violation_row) fill_i32<<<blocks, 256, 0, st>>>(mon.violation_row, runs, -1);
+        if (mon.per_step && steps > 0) TRY(cudaMemsetAsync(mon.per_step, 0, sizeof(int32_t) * steps, st));
+    }
+    const bool with_noise = Z.noise != nullptr, with_monitor = Z.monitor_rows > 0;
+    auto advance = [&](int k, double* traj_step, const int* step_dev) {
+        auto kern = with_noise ? (with_monitor ? loop_advance_kernel<true, true> : loop_advance_kernel<true, false>)
+                               : (with_monitor ? loop_advance_kernel<false, true> : loop_advance_kernel<false, false>);
+        kern<<<blocks, 256, 0, st>>>(K, runs, x, xhat, u_prev, d_fail_step, est, live_list, live_count, traj_step, step_dev,
+                                     dhat, D.d_plant, noise, mon, k);
+    };
     int64_t total_iters = 0;
     bool warm_valid = false;
     // the iteration total accumulates on the device over the steps (one read at the end instead of one per step)
@@ -244,9 +348,7 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
     auto enqueue_step = [&](int k, const int* step_dev) -> int {
         cudaError_t e = cudaMemsetAsync(live_count, 0, sizeof(int), st);
         if (e != cudaSuccess) { set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return CARMPC_ERR_CUDA; }
-        loop_advance_kernel<<<blocks, 256, 0, st>>>(K, runs, x, xhat, u_prev, d_fail_step, est, live_list, live_count,
-                                                    d_traj ? (step_dev ? d_traj : d_traj + (size_t)k * 4 * runs) : nullptr, step_dev,
-                                                    dhat, D.d_plant);
+        advance(k, d_traj ? (step_dev ? d_traj : d_traj + (size_t)k * 4 * runs) : nullptr, step_dev);
         const int rc2 = q->solve_enqueue(est, runs, h_xref, c_qp, live_list, live_count, runs, u0, status, warm, st);
         if (rc2 != CARMPC_OK) return rc2;
         loop_apply_kernel<<<blocks, 256, 0, st>>>(runs, k, live_list, (int)runs, live_count, u0, status, u_prev, d_fail_step, step_dev);
@@ -298,8 +400,7 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
             break;
         }
         TRY(cudaMemsetAsync(live_count, 0, sizeof(int), st));
-        loop_advance_kernel<<<blocks, 256, 0, st>>>(K, runs, x, xhat, u_prev, d_fail_step, est, live_list, live_count,
-                                                    d_traj ? d_traj + (size_t)k * 4 * runs : nullptr, nullptr, dhat, D.d_plant);
+        advance(k, d_traj ? d_traj + (size_t)k * 4 * runs : nullptr, nullptr);
         int live = 0;
         TRY(cudaMemcpyAsync(&live, live_count, sizeof(int), cudaMemcpyDeviceToHost, st));
         TRY(cudaStreamSynchronize(st));
@@ -357,8 +458,9 @@ extern "C" int carmpc_closed_loop(void* qp, int mode, const double* h_A, const d
     if (h_L) memcpy(K.L, h_L, sizeof(K.L));
     K.dt = dt; K.l1 = l1; K.mode = mode;
     const LoopDisturbance none = {nullptr, nullptr, nullptr, nullptr};
+    const LoopStochastic off = {nullptr, nullptr, 0, nullptr, nullptr, nullptr};
     return closed_loop_run(q, K, h_xref, steps, warm_start, d_x_init, d_xhat_init, runs, d_final, d_fail_step, d_traj, d_u_log,
-                           none, h_total_iters, stream);
+                           none, off, h_total_iters, stream);
 }
 
 extern "C" int carmpc_closed_loop_disturbance(void* qp, const double* h_A, const double* h_B, const double* h_C,
@@ -396,6 +498,81 @@ extern "C" int carmpc_closed_loop_disturbance(void* qp, const double* h_A, const
     memcpy(K.Cdp, dm->Cd_plant, sizeof(K.Cdp));
     K.dt = dt; K.l1 = l1; K.mode = 2;
     const LoopDisturbance D = {d_dhat_init, d_d_plant, d_dhat_final, d_dhat_log};
+    const LoopStochastic off = {nullptr, nullptr, 0, nullptr, nullptr, nullptr};
     return closed_loop_run(q, K, h_xref, steps, warm_start, d_x_init, d_xhat_init, runs, d_final, d_fail_step, d_traj, d_u_log,
-                           D, h_total_iters, stream);
+                           D, off, h_total_iters, stream);
+}
+
+extern "C" int carmpc_closed_loop_stochastic(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C,
+                                             const double* h_L, const carmpc_disturbance_model* dm, const double* h_xref,
+                                             double dt, double l1, int steps, int warm_start, const double* d_x_init,
+                                             const double* d_xhat_init, const double* d_dhat_init, const double* d_d_plant,
+                                             int64_t runs, double* d_final, double* d_dhat_final, int32_t* d_fail_step,
+                                             double* d_traj, double* d_u_log, double* d_dhat_log,
+                                             const carmpc_loop_noise* noise, const double* h_monitor_Ab, int monitor_rows,
+                                             int32_t* d_violation_step, int32_t* d_violation_row,
+                                             int32_t* d_violations_per_step, int64_t* h_total_iters, void* stream) {
+    QPHandle* q = check_handle<QPHandle>(qp, kQP);
+    CARMPC_REQUIRE(q != nullptr, "not a QP handle");
+    CARMPC_REQUIRE(mode >= 0 && mode <= 2, "mode must be 0 (state feedback), 1 (output feedback) or 2 (with a disturbance estimate)");
+    CARMPC_REQUIRE(h_A && h_B && h_xref, "null model pointer");
+    CARMPC_REQUIRE(mode != 1 || (h_C && h_L), "output feedback needs C and L");
+    CARMPC_REQUIRE(mode != 2 || (h_C && dm), "mode 2 needs C and a disturbance model");
+    CARMPC_REQUIRE(steps >= 0 && runs >= 0 && runs < (int64_t)1 << 31, "steps / runs");
+    CARMPC_REQUIRE(warm_start >= 0 && warm_start <= 2, "warm_start must be 0, 1 or 2");
+    CARMPC_REQUIRE(dt > 0 && l1 > 0, "dt, l1");
+    bool finite = true;
+    if (mode == 1)
+        for (int j = 0; j < 12; ++j) finite = finite && isfinite(h_L[j]);
+    if (mode == 2) {
+        const double* gains[] = {dm->Bd, dm->Cd, dm->L1, dm->L2, dm->Bd_plant, dm->Cd_plant};
+        const int counts[] = {4, 3, 12, 3, 4, 3};
+        for (int g = 0; g < 6; ++g)
+            for (int j = 0; j < counts[g]; ++j) finite = finite && isfinite(gains[g][j]);
+    }
+    CARMPC_REQUIRE(finite, "observer gains and the disturbance model must be finite");
+    if (noise != nullptr) {
+        for (int j = 0; j < 16; ++j) finite = finite && isfinite(noise->Lw[j]) && isfinite(noise->Lv[j]);
+        CARMPC_REQUIRE(finite, "noise factors Lw, Lv must be finite");
+        CARMPC_REQUIRE(noise->first_run >= 0 && noise->first_run <= INT64_MAX - runs, "first_run must be >= 0");
+    }
+    if (h_monitor_Ab != nullptr) {
+        CARMPC_REQUIRE(monitor_rows >= 1 && monitor_rows <= 512, "monitor_rows must be in [1, 512]");
+        for (int j = 0; j < 5 * monitor_rows; ++j) finite = finite && isfinite(h_monitor_Ab[j]);
+        CARMPC_REQUIRE(finite, "monitor rows must be finite");
+    } else {
+        CARMPC_REQUIRE(monitor_rows == 0, "monitor_rows without monitor rows");
+        CARMPC_REQUIRE(!d_violation_step && !d_violation_row && !d_violations_per_step, "monitor outputs without monitor rows");
+    }
+    if (h_total_iters) *h_total_iters = 0;
+    if (runs == 0) return CARMPC_OK;
+    CARMPC_REQUIRE(d_x_init && d_final && d_fail_step, "null device pointer");
+    LoopConst K;
+    memset(&K, 0, sizeof(K));
+    memcpy(K.A, h_A, sizeof(K.A));
+    memcpy(K.B, h_B, sizeof(K.B));
+    if (mode != 0) memcpy(K.C, h_C, sizeof(K.C));
+    if (mode == 1) memcpy(K.L, h_L, sizeof(K.L));
+    LoopDisturbance D = {nullptr, nullptr, nullptr, nullptr};
+    if (mode == 2) {
+        memcpy(K.L, dm->L1, sizeof(K.L));
+        memcpy(K.Bd, dm->Bd, sizeof(K.Bd));
+        memcpy(K.Cd, dm->Cd, sizeof(K.Cd));
+        memcpy(K.L2, dm->L2, sizeof(K.L2));
+        memcpy(K.Bdp, dm->Bd_plant, sizeof(K.Bdp));
+        memcpy(K.Cdp, dm->Cd_plant, sizeof(K.Cdp));
+        D = {d_dhat_init, d_d_plant, d_dhat_final, d_dhat_log};
+    }
+    K.dt = dt; K.l1 = l1; K.mode = mode;
+    LoopNoise nz;
+    if (noise != nullptr) {
+        nz.seed = noise->seed;
+        nz.first_run = noise->first_run;
+        memcpy(nz.Lw, noise->Lw, sizeof(nz.Lw));
+        memcpy(nz.Lv, noise->Lv, sizeof(nz.Lv));
+    }
+    const LoopStochastic Z = {noise ? &nz : nullptr, h_monitor_Ab, h_monitor_Ab ? monitor_rows : 0, d_violation_step,
+                              d_violation_row, d_violations_per_step};
+    return closed_loop_run(q, K, h_xref, steps, warm_start, d_x_init, d_xhat_init, runs, d_final, d_fail_step, d_traj, d_u_log,
+                           D, Z, h_total_iters, stream);
 }

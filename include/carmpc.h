@@ -390,6 +390,45 @@ int carmpc_closed_loop_disturbance(void* qp, const double* h_A, const double* h_
                                    double* d_dhat_final, int32_t* d_fail_step, double* d_traj, double* d_u_log,
                                    double* d_dhat_log, int64_t* h_total_iters, void* stream);
 
+/* Closed loops with random process and measurement noise, and a monitor of the true plant state (modes 0, 1, 2 of the two
+ * functions above).  Step k of a run still running at the start of step k:
+ *   s = s + dt * f(s, u_prev);   mode 2: s = s + Bd_plant * d_r;   s = s + Lw z_w      (process noise)
+ *   s is stored to d_final / d_traj, then checked against the monitor rows [a | b]: fma(a3, v, fma(a2, psi, fma(a1, y,
+ *   a0 * x))) <= b for every row (the chain of carmpc_membership_bitset mode 0; a non-finite state violates)
+ *   v = Lv z_v;   mode 0: the QP sees s + v[0..3];  mode 1: y = C s + v[0..2];  mode 2: y = C s + Cd_plant d_r + v[0..2]
+ *   observer and QP as in carmpc_closed_loop / carmpc_closed_loop_disturbance.
+ * z_w, z_v: four standard normals each.  Philox4x64-10 with key (seed, 0) at counter (first_run + run, k, j, 0), j = 0
+ * for z_w and 1 for z_v, gives words x0..x3; (x0, x1) and (x2, x3) each give two normals by Box-Muller:
+ *   ua = ((x0 >> 11) + 1) 2^-53,  ub = (x1 >> 11) 2^-53,  z0 = sqrt(-2 ln ua) cos(2 pi ub),  z1 = ... sin(2 pi ub).
+ * The draws depend only on (seed, first_run + run, k, j): not on the batch, warm_start or which runs still run, so a run
+ * set split over calls (first_run = the offset of each part) draws what one call would.
+ * A violation never stops a run.  d_violation_step / d_violation_row (runs int32, -1 none): the first step with a
+ * violation and the lowest violated row (caller's order) at that step.  d_violations_per_step (steps int32): runs
+ * violating at step k.  Stopped runs are neither moved nor counted; a run whose QP fails at step k was moved and checked
+ * at step k.
+ *   mode 0: h_C, h_L ignored;  mode 1: h_C, h_L (as carmpc_closed_loop);  mode 2: h_C and dm (h_L ignored).
+ *   d_dhat_init, d_d_plant, d_dhat_final, d_dhat_log: mode 2 only (as carmpc_closed_loop_disturbance).
+ *   noise (nullable: no noise).  h_monitor_Ab (nullable: no monitor): host rows x 5, 1 <= monitor_rows <= 512, finite;
+ *   the monitor outputs are nullable and need rows.
+ * With noise = NULL and no monitor the results are those of carmpc_closed_loop / carmpc_closed_loop_disturbance.
+ * CARMPC_ERR_INVALID for non-finite factors or gains, first_run < 0, bad monitor rows, monitor outputs without rows, mode
+ * 2 without dm; CARMPC_ERR_CUDA on a handle created without a device. */
+typedef struct carmpc_loop_noise {
+    uint64_t seed;
+    int64_t first_run;      /* global id of run 0 of this call */
+    double Lw[16];          /* process-noise factor, 4 x 4 row-major: w = Lw z_w   */
+    double Lv[16];          /* measurement-noise factor, 4 x 4 row-major: v = Lv z_v */
+} carmpc_loop_noise;
+
+int carmpc_closed_loop_stochastic(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C,
+                                  const double* h_L, const carmpc_disturbance_model* dm, const double* h_xref, double dt,
+                                  double l1, int steps, int warm_start, const double* d_x_init, const double* d_xhat_init,
+                                  const double* d_dhat_init, const double* d_d_plant, int64_t runs, double* d_final,
+                                  double* d_dhat_final, int32_t* d_fail_step, double* d_traj, double* d_u_log,
+                                  double* d_dhat_log, const carmpc_loop_noise* noise, const double* h_monitor_Ab,
+                                  int monitor_rows, int32_t* d_violation_step, int32_t* d_violation_row,
+                                  int32_t* d_violations_per_step, int64_t* h_total_iters, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Device micro-benchmarks used as roofline denominators that MEASURED_PEAKS.json does not carry.
  * which: 0 = FP32 FFMA TFLOP/s (uniform multiplier), 1 = FP64 DFMA TFLOP/s, 2 = HBM copy GB/s (read+write),

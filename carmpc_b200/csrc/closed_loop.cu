@@ -285,7 +285,6 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
     double* monitor_Ab = nullptr;
     int rc = CARMPC_OK;
     auto cleanup = [&]() { if (st != user_st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); } if (ev) cudaEventDestroy(ev);
-                           q->defer_total = 0; q->certify_with_c = 0;
                            cudaFree(xhat); cudaFree(est); cudaFree(u_prev); cudaFree(u0); cudaFree(status); cudaFree(live_list);
                            cudaFree(live_count); cudaFree(warm); cudaFree(dhat_own); cudaFree(monitor_Ab); };
 #define TRY(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) { set_error("%s: %s", #call, cudaGetErrorString(e__)); cleanup(); return CARMPC_ERR_CUDA; } } while (0)
@@ -341,15 +340,19 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
     rc = q->ensure_workspace(runs);
     if (rc != CARMPC_OK) { cleanup(); return rc; }
     TRY(cudaMemsetAsync(q->ws_total_iters, 0, sizeof(unsigned long long), st));
-    q->defer_total = 1;
-    // host-driven steps run the filter / decide certificates on the disturbance-shifted bounds too
-    q->certify_with_c = dist ? 1 : 0;
+    // the QP of every step: the live runs (est, indexed like the runs), warm-started once a step has run
+    SolveRequest req;
+    req.x0 = est; req.stride = runs; req.xref = h_xref; req.c = c_qp; req.idx = live_list;
+    req.u0 = u0; req.status = status; req.warm = warm; req.warm_out = warm ? 1 : 0; req.keep_total = 1;
+    req.certify_shifted = dist ? 1 : 0;       // host-driven steps certify on the disturbance-shifted bounds too
     // One enqueue-only step (every count stays on the device).  step_dev == nullptr: the step number k comes from the host.
     auto enqueue_step = [&](int k, const int* step_dev) -> int {
         cudaError_t e = cudaMemsetAsync(live_count, 0, sizeof(int), st);
         if (e != cudaSuccess) { set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return CARMPC_ERR_CUDA; }
         advance(k, d_traj ? (step_dev ? d_traj : d_traj + (size_t)k * 4 * runs) : nullptr, step_dev);
-        const int rc2 = q->solve_enqueue(est, runs, h_xref, c_qp, live_list, live_count, runs, u0, status, warm, st);
+        SolveRequest r = req;
+        r.count = runs; r.count_dev = live_count; r.warm_in = 1;
+        const int rc2 = q->solve_enqueue(r, st);
         if (rc2 != CARMPC_OK) return rc2;
         loop_apply_kernel<<<blocks, 256, 0, st>>>(runs, k, live_list, (int)runs, live_count, u0, status, u_prev, d_fail_step, step_dev);
         if (step_dev) {
@@ -406,8 +409,8 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
         TRY(cudaStreamSynchronize(st));
         if (live > 0) {
             // from the second step on, the active set certified at the previous step is tried first
-            rc = q->solve(est, runs, h_xref, c_qp, live_list, live, u0, nullptr, status, nullptr, nullptr, warm,
-                          warm_valid ? 1 : 0, warm ? 1 : 0, st, warm_valid ? 1 : 0);
+            req.count = live; req.warm_in = req.reuse = warm_valid ? 1 : 0;
+            rc = q->solve(req, st);
             if (rc != CARMPC_OK) { cleanup(); return rc; }
             warm_valid = warm != nullptr;
             loop_apply_kernel<<<(live + 255) / 256, 256, 0, st>>>(runs, k, live_list, live, nullptr, u0, status, u_prev, d_fail_step, nullptr);
@@ -417,7 +420,6 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
         if (D.dhat_log)   // the estimate the QP of this step used (unchanged for stopped runs)
             TRY(cudaMemcpyAsync(D.dhat_log + (size_t)k * runs, dhat, sizeof(double) * runs, cudaMemcpyDeviceToDevice, st));
     }
-    q->defer_total = 0;
     unsigned long long total_dev = 0;
     TRY(cudaMemcpyAsync(&total_dev, q->ws_total_iters, sizeof(total_dev), cudaMemcpyDeviceToHost, st));
     TRY(cudaStreamSynchronize(st));

@@ -86,6 +86,57 @@ __global__ void map_expand_kernel(const double* __restrict__ axes, MapGrid g, in
     seed[i] = (int)anchor;
 }
 
+// The base values of a request's polish and ADMM launches (both pipelines): every stage then sets its own list, counters and
+// pass-specific fields on a copy.
+PolishBatch polish_batch(QPHandle& q, const SolveRequest& r) {
+    PolishBatch pb;
+    memset(&pb, 0, sizeof(pb));
+    pb.x0 = r.x0; pb.stride = r.stride; pb.cdist = r.c;
+    for (int c = 0; c < 4; ++c) pb.xref[c] = r.xref[c];
+    pb.idx_list = r.idx; pb.count = (int)r.count; pb.count_dev = r.count_dev;
+    pb.sign = q.ws_sign; pb.u_admm = q.ws_u; pb.status = r.status ? r.status : q.ws_status;
+    pb.u0 = r.u0; pb.objective = r.objective; pb.u_full = r.u_full; pb.polished = q.ws_polished;
+    pb.n_failed = q.ws_counters + kCntFailed; pb.failed_list = q.ws_failed;
+    pb.rounds = q.host.opts.polish ? -1 : 0; pb.final_pass = q.host.opts.polish ? 0 : 1;
+    pb.stats = q.ws_polish_stats; pb.cert = r.cert;
+    // warm-started sequences and seeded maps keep the certified (repaired) active set
+    if ((r.warm && r.warm_out) || r.keep_sign) pb.sign_out = q.ws_sign;
+    if (r.records) {
+        pb.rec_of = q.ws_rec_of; pb.rec_lam = q.ws_rec_lam; pb.rec_act = q.ws_rec_act;
+        pb.rec_write = r.seed == nullptr;                 // anchors export, followers read (p0 in solve)
+    }
+    return pb;
+}
+
+AdmmBatch admm_batch(QPHandle& q, const SolveRequest& r) {
+    AdmmBatch ab;
+    memset(&ab, 0, sizeof(ab));
+    ab.x0 = r.x0; ab.stride = r.stride; ab.cdist = r.c;
+    for (int c = 0; c < 4; ++c) ab.xref[c] = r.xref[c];
+    ab.idx_list = r.idx; ab.count = (int)r.count; ab.count_dev = r.count_dev; ab.next = q.ws_counters + kCntNext;
+    ab.sign = q.ws_sign; ab.u_admm = q.ws_u; ab.status = r.status ? r.status : q.ws_status; ab.iters = r.iters ? r.iters : q.ws_iters;
+    // the ADMM state of every sample is kept (caller's buffer or the workspace): the second pass resumes from it
+    ab.warm = r.warm ? r.warm : q.ws_warm; ab.warm_in = r.warm ? r.warm_in : 0; ab.warm_out = 1;
+    ab.total_iters = q.ws_total_iters; ab.eps_scale = 1.f; ab.max_iter = q.host.opts.max_iter;
+    return ab;
+}
+
+// Results of the host-buffer entry points: u0 back to the caller's (batch x 2) layout, the rest as it is; synchronises.
+int download(QPHandle* q, int64_t batch, double* h_u0, double* h_objective, int32_t* h_status, int32_t* h_iters,
+             double* h_u_full, cudaStream_t st) {
+    if (h_u0) {
+        soa_to_aos_kernel<<<(int)((batch + 255) / 256), 256, 0, st>>>(q->io_u0, q->io_u0_aos, batch, 2);
+        CARMPC_CUDA(cudaMemcpyAsync(h_u0, q->io_u0_aos, sizeof(double) * 2 * batch, cudaMemcpyDeviceToHost, st));
+    }
+    if (h_objective) CARMPC_CUDA(cudaMemcpyAsync(h_objective, q->io_obj, sizeof(double) * batch, cudaMemcpyDeviceToHost, st));
+    CARMPC_CUDA(cudaMemcpyAsync(h_status, q->io_status, sizeof(int32_t) * batch, cudaMemcpyDeviceToHost, st));
+    if (h_iters) CARMPC_CUDA(cudaMemcpyAsync(h_iters, q->io_iters, sizeof(int32_t) * batch, cudaMemcpyDeviceToHost, st));
+    if (h_u_full) CARMPC_CUDA(cudaMemcpyAsync(h_u_full, q->io_full, sizeof(double) * (size_t)q->host.n * batch, cudaMemcpyDeviceToHost, st));
+    CARMPC_CUDA(cudaStreamSynchronize(st));
+    CARMPC_CUDA(cudaGetLastError());
+    return CARMPC_OK;
+}
+
 }  // namespace
 
 int QPHandle::ensure_io(int64_t batch, bool want_full) {
@@ -125,7 +176,7 @@ QPHandle::~QPHandle() {
 
 int QPHandle::ensure_workspace(int64_t batch) {
     if (ws_counters == nullptr) {
-        CARMPC_CUDA(cudaMalloc(&ws_counters, sizeof(int) * 16));
+        CARMPC_CUDA(cudaMalloc(&ws_counters, sizeof(int) * kCounters));
         CARMPC_CUDA(cudaMalloc(&ws_total_iters, sizeof(unsigned long long)));
         CARMPC_CUDA(cudaMalloc(&ws_polish_stats, sizeof(unsigned long long) * kPolishStats));
         CARMPC_CUDA(cudaMemset(ws_polish_stats, 0, sizeof(unsigned long long) * kPolishStats));
@@ -160,43 +211,18 @@ int QPHandle::ensure_workspace(int64_t batch) {
     return CARMPC_OK;
 }
 
-int QPHandle::solve(const double* d_x0, int64_t stride, const double* xref, const double* d_c, const int* d_idx,
-                    int64_t count, double* d_u0, double* d_objective, int32_t* d_status, int32_t* d_iters,
-                    double* d_u_full, float* d_warm, int warm_in, int warm_out, cudaStream_t st, int reuse_active_set,
-                    const int* d_seed, int keep_sign) {
-    // `stride` is the number of samples the per-sample arrays are sized for; `count` the number solved now
-    // (all of them, or those listed in d_idx).
+int QPHandle::solve(const SolveRequest& r, cudaStream_t st, SolveCounts* counts) {
     if (host_only) { set_error("carmpc_qp: this handle was created without a CUDA device; there is no CPU solver"); return CARMPC_ERR_CUDA; }
-    int rc = ensure_workspace(stride);
+    int rc = ensure_workspace(r.stride);
     if (rc != CARMPC_OK) return rc;
-    last_launches = 0;
+    SolveCounts own, &k = counts ? *counts : own;
+    k = SolveCounts();
     last_tc_samples = 0;
-    last_second_pass = 0;
-    last_reused = 0;
-    last_fallback = 0;
     CARMPC_CUDA(cudaMemsetAsync(ws_counters, 0, sizeof(int) * 8, st));
-    if (!defer_total) CARMPC_CUDA(cudaMemsetAsync(ws_total_iters, 0, sizeof(unsigned long long), st));
-    int* status = d_status ? d_status : ws_status;
-    int* iters = d_iters ? d_iters : ws_iters;
-
-    PolishBatch pb;
-    memset(&pb, 0, sizeof(pb));
-    pb.x0 = d_x0; pb.stride = stride; pb.cdist = d_c;
-    for (int c = 0; c < 4; ++c) pb.xref[c] = xref[c];
-    pb.idx_list = d_idx; pb.count = (int)count; pb.sign = ws_sign; pb.u_admm = ws_u; pb.status = status;
-    pb.u0 = d_u0; pb.objective = d_objective; pb.u_full = d_u_full; pb.polished = ws_polished;
-    pb.n_failed = ws_counters + 1; pb.failed_list = ws_failed;
-    pb.rounds = host.opts.polish ? -1 : 0;
-    pb.final_pass = host.opts.polish ? 0 : 1;
-    pb.stats = ws_polish_stats;
-    pb.cert = cert;
-    if (!stats_hold) CARMPC_CUDA(cudaMemsetAsync(ws_polish_stats, 0, sizeof(unsigned long long) * kPolishStats, st));
-    // warm-started sequences and seeded maps keep the certified (repaired) active set
-    if ((d_warm && warm_out) || keep_sign) pb.sign_out = ws_sign;
-    if (use_records) {
-        pb.rec_of = ws_rec_of; pb.rec_lam = ws_rec_lam; pb.rec_act = ws_rec_act;
-        pb.rec_write = d_seed == nullptr;                 // anchors export, followers read (p0 below)
-    }
+    if (!r.keep_total) CARMPC_CUDA(cudaMemsetAsync(ws_total_iters, 0, sizeof(unsigned long long), st));
+    PolishBatch pb = polish_batch(*this, r);
+    AdmmBatch ab = admm_batch(*this, r);
+    if (!r.hold_stats) CARMPC_CUDA(cudaMemsetAsync(ws_polish_stats, 0, sizeof(unsigned long long) * kPolishStats, st));
 
     // Active-set reuse (closed loop): consecutive QPs of a run mostly share their active set, so the set certified at
     // the previous step (kept in the workspace, same sample indexing) goes through the float64 polish first; only the
@@ -204,224 +230,186 @@ int QPHandle::solve(const double* d_x0, int64_t stride, const double* xref, cons
     // The empty active set first (polish_unconstrained_kernel): where the unconstrained minimiser satisfies every row it is
     // the optimum - certified in float64 by one thread, no iteration, no factorisation.  Closed-loop runs near their goal
     // live there; on the config-3 grid it settles 8.6 % of the states.  The rest (listed on the device) goes on.
-    const int* d_count = nullptr;                        // device-side count of the list the pipeline below works on
     if (host.opts.polish) {
         PolishBatch pu = pb;
-        pu.sign_out = ws_sign; pu.iters_out = iters;
-        rc = polish_unconstrained_launch(this, pu, ws_rest, ws_counters + 6, st);
+        pu.sign_out = ws_sign; pu.iters_out = ab.iters;
+        rc = polish_unconstrained_launch(this, pu, ws_rest, ws_counters + kCntRest, st);
         if (rc != CARMPC_OK) return rc;
-        ++last_launches;
-        d_idx = ws_rest;
-        d_count = ws_counters + 6;
-        pb.idx_list = d_idx; pb.count_dev = d_count;
+        ++k.launches;
+        pb.idx_list = ws_rest; pb.count_dev = ws_counters + kCntRest;
     }
-    if (reuse_active_set && host.opts.polish) {
+    if (r.reuse && host.opts.polish) {
         PolishBatch p0 = pb;
-        p0.rounds = 4; p0.final_pass = 0; p0.n_failed = ws_counters + 5; p0.failed_list = ws_failed0;
+        p0.rounds = 4; p0.final_pass = 0; p0.n_failed = ws_counters + kCntReuseFailed; p0.failed_list = ws_failed0;
         p0.precheck = 1; p0.Px = admm.Px; p0.Pc = admm.Pc; p0.pre_lo = admm.pre_lo; p0.pre_hi = admm.pre_hi; p0.kpre = admm.kpre;
-        p0.sign_out = ws_sign; p0.iters_out = iters; p0.seed = d_seed;
-        p0.rec_write = 0; p0.rec_read = use_records && d_seed != nullptr;
+        p0.sign_out = ws_sign; p0.iters_out = ab.iters; p0.seed = r.seed;
+        p0.rec_write = 0; p0.rec_read = r.records && r.seed != nullptr;
         rc = polish_launch(this, p0, st);
         if (rc != CARMPC_OK) return rc;
-        ++last_launches;
-        int n_failed0 = 0, n_rest = 0;
-        CARMPC_CUDA(cudaMemcpyAsync(&n_failed0, ws_counters + 5, sizeof(int), cudaMemcpyDeviceToHost, st));
-        CARMPC_CUDA(cudaMemcpyAsync(&n_rest, ws_counters + 6, sizeof(int), cudaMemcpyDeviceToHost, st));
+        ++k.launches;
+        int n_failed0 = 0;
+        CARMPC_CUDA(cudaMemcpyAsync(&n_failed0, ws_counters + kCntReuseFailed, sizeof(int), cudaMemcpyDeviceToHost, st));
         CARMPC_CUDA(cudaStreamSynchronize(st));
-        last_reused = count - n_failed0;
-        (void)n_rest;
-        if (n_failed0 == 0) { last_total_iters = 0; return CARMPC_OK; }        // (deferred totals: nothing was added)
-        d_idx = ws_failed0;
-        count = n_failed0;
-        d_count = nullptr;
-        pb.idx_list = d_idx; pb.count = (int)count; pb.count_dev = nullptr;
+        k.reused = r.count - n_failed0;
+        if (n_failed0 == 0) { last_total_iters = 0; last_launches = k.launches; return CARMPC_OK; }   // no iteration
+        pb.idx_list = ws_failed0; pb.count = n_failed0; pb.count_dev = nullptr;
     }
 
-    AdmmBatch ab;
-    memset(&ab, 0, sizeof(ab));
-    ab.x0 = d_x0; ab.stride = stride; ab.cdist = d_c;
-    for (int c = 0; c < 4; ++c) ab.xref[c] = xref[c];
-    ab.idx_list = d_idx; ab.count = (int)count; ab.count_dev = d_count; ab.next = ws_counters + 0;
-    ab.sign = ws_sign; ab.u_admm = ws_u; ab.status = status; ab.iters = iters;
-    // the ADMM state of every sample is kept (caller's buffer or the workspace): the second pass resumes from it
-    ab.warm = d_warm ? d_warm : ws_warm; ab.warm_in = d_warm ? warm_in : 0; ab.warm_out = 1;
-    ab.total_iters = ws_total_iters; ab.eps_scale = 1.f; ab.max_iter = host.opts.max_iter; ab.iters_accumulate = 0;
+    ab.idx_list = pb.idx_list; ab.count = pb.count; ab.count_dev = pb.count_dev;
     // First pass capped at kFirstPassIters: on the region-of-attraction grid every solvable state converges within 90
     // iterations and only barely infeasible states run longer (up to ~400).  On 128-sample tiles such stragglers hold a
     // whole tile at ~10 us per iteration; handed to the second pass they continue on narrow tiles (~3 us per iteration).
     // The cap does not depend on the batch, so a state sees the same iteration schedule however it is batched (cold grid,
     // seeded map, alone): the statuses of cold solves are path-independent.  Warm-started solves (closed-loop steps: small
     // batches on narrow tiles, where a second pass only adds launches) keep the full budget.
-    if (host.opts.polish && !(d_warm && warm_in))
+    if (host.opts.polish && !(r.warm && r.warm_in))
         ab.max_iter = std::min(ab.max_iter, std::max(kFirstPassIters, admm.check_every));
     ab.write_u = host.opts.polish ? 0 : 1;        // with the polish on, only the final pass may fall back to the iterate
     rc = admm_launch(this, ab, st);
     if (rc != CARMPC_OK) return rc;
-    ++last_launches;
+    ++k.launches;
 
     rc = polish_launch(this, pb, st);
     if (rc != CARMPC_OK) return rc;
-    ++last_launches;
+    ++k.launches;
 
     int n_failed = 0;
     if (host.opts.polish) {
         // "infeasible" verdicts of the float32 ADMM are accepted only with a float64 Farkas certificate of their final
         // dual iterate (or a violated u-independent row); the others join the list of the second pass
-        rc = farkas_verify_launch(this, d_idx, (int)count, status, ab.warm, d_x0, stride, d_c, xref, ws_failed, ws_counters + 1, st, d_count);
+        rc = farkas_verify_launch(this, pb, pb.idx_list, pb.count, pb.count_dev, ab.warm, ws_failed, ws_counters + kCntFailed, st);
         if (rc != CARMPC_OK) return rc;
-        ++last_launches;
-        CARMPC_CUDA(cudaMemcpyAsync(&n_failed, ws_counters + 1, sizeof(int), cudaMemcpyDeviceToHost, st));
+        ++k.launches;
+        CARMPC_CUDA(cudaMemcpyAsync(&n_failed, ws_counters + kCntFailed, sizeof(int), cudaMemcpyDeviceToHost, st));
         CARMPC_CUDA(cudaStreamSynchronize(st));
     }
     const int* second_list = ws_failed;
     // The certificate kernels take the disturbance shift as well; the public entry points keep their results with a
-    // disturbance (max_iter instead of a certified "infeasible"), only the closed loop turns them on (certify_with_c).
-    const bool certify = d_c == nullptr || certify_with_c;
+    // disturbance (max_iter instead of a certified "infeasible"), only the closed loop turns them on (certify_shifted).
+    const bool certify = r.c == nullptr || r.certify_shifted;
     if (n_failed > 0 && certify) {
         // most of what the first pass could not settle is barely infeasible: the exact certificate test on the first-pass
         // state removes those before the (long) tighter pass
-        CARMPC_CUDA(cudaMemsetAsync(ws_counters + 7, 0, sizeof(int), st));
-        rc = farkas_filter_launch(this, ws_failed, n_failed, status, ab.warm, d_x0, stride, d_c, d_u0, d_objective, d_u_full,
-                                  ws_polished, ws_overflow, ws_counters + 7, st);
+        CARMPC_CUDA(cudaMemsetAsync(ws_counters + kCntSurvivors, 0, sizeof(int), st));
+        rc = farkas_filter_launch(this, pb, ws_failed, n_failed, ab.warm, ws_overflow, ws_counters + kCntSurvivors, st);
         if (rc != CARMPC_OK) return rc;
-        ++last_launches;
-        CARMPC_CUDA(cudaMemcpyAsync(&n_failed, ws_counters + 7, sizeof(int), cudaMemcpyDeviceToHost, st));
+        ++k.launches;
+        CARMPC_CUDA(cudaMemcpyAsync(&n_failed, ws_counters + kCntSurvivors, sizeof(int), cudaMemcpyDeviceToHost, st));
         CARMPC_CUDA(cudaStreamSynchronize(st));
         // the survivors move to ws_failed (the polish launches below reuse ws_overflow)
         if (n_failed > 0) CARMPC_CUDA(cudaMemcpyAsync(ws_failed, ws_overflow, sizeof(int) * n_failed, cudaMemcpyDeviceToDevice, st));
     }
     if (n_failed > 0) {
         // second pass on the samples whose active set the polish could not certify: tighter ADMM, then accept
-        last_second_pass = n_failed;
-        ab.idx_list = second_list; ab.count = n_failed; ab.count_dev = nullptr; ab.next = ws_counters + 2; ab.eps_scale = 0.01f;
+        ab.idx_list = second_list; ab.count = n_failed; ab.count_dev = nullptr; ab.next = ws_counters + kCntNext2; ab.eps_scale = 0.01f;
         ab.max_iter = host.opts.max_iter;
         ab.warm_in = 1; ab.iters_accumulate = 1; ab.write_u = 1;
         rc = admm_launch(this, ab, st);
         if (rc != CARMPC_OK) return rc;
-        pb.idx_list = second_list; pb.count = n_failed; pb.count_dev = nullptr; pb.n_failed = ws_counters + 3; pb.final_pass = 1;
+        pb.idx_list = second_list; pb.count = n_failed; pb.count_dev = nullptr; pb.n_failed = ws_counters + kCntFinal; pb.final_pass = 1;
         rc = polish_launch(this, pb, st);
         if (rc != CARMPC_OK) return rc;
         // whoever is still at "max_iter" is almost always barely infeasible: the dual iterate of its final ADMM state,
         // evaluated exactly, settles it
         if (certify) {
-            rc = farkas_decide_launch(this, second_list, n_failed, status, ab.warm, d_x0, stride, d_c, d_u0, d_objective,
-                                      d_u_full, ws_polished, st);
+            rc = farkas_decide_launch(this, pb, second_list, n_failed, nullptr, ab.warm, st);
             if (rc != CARMPC_OK) return rc;
-            ++last_launches;
+            ++k.launches;
         }
-        last_launches += 2;
+        k.launches += 2;
         if (host.opts.polish) {
             // second-pass "infeasible" verdicts need their float64 certificate as well (unverified ones join the fallback)
-            CARMPC_CUDA(cudaMemsetAsync(ws_counters + 13, 0, sizeof(int), st));
-            rc = farkas_verify_launch(this, second_list, n_failed, status, ab.warm, d_x0, stride, d_c, xref, ws_overflow, ws_counters + 13, st);
+            CARMPC_CUDA(cudaMemsetAsync(ws_counters + kCntVerify2, 0, sizeof(int), st));
+            rc = farkas_verify_launch(this, pb, second_list, n_failed, nullptr, ab.warm, ws_overflow, ws_counters + kCntVerify2, st);
             if (rc != CARMPC_OK) return rc;
             // whatever is still without a proof (no KKT certificate, or out of iterations): float64 fallback
             int handled = 0;
-            rc = exact_fallback(this, pb, second_list, n_failed, ab.warm, iters, st, &handled);
+            rc = exact_fallback(this, pb, second_list, n_failed, nullptr, ab.warm, ab.iters, st, &handled);
             if (rc != CARMPC_OK) return rc;
-            last_launches += handled > 0 ? 4 : 1;
-            last_fallback = handled;
+            k.launches += handled > 0 ? 4 : 1;
         }
     }
-    if (defer_total) { last_total_iters = 0; return CARMPC_OK; }
-    unsigned long long total = 0;
-    CARMPC_CUDA(cudaMemcpyAsync(&total, ws_total_iters, sizeof(total), cudaMemcpyDeviceToHost, st));
-    CARMPC_CUDA(cudaStreamSynchronize(st));
-    last_total_iters = (int64_t)total;
+    if (!r.keep_total) {
+        unsigned long long total = 0;
+        CARMPC_CUDA(cudaMemcpyAsync(&total, ws_total_iters, sizeof(total), cudaMemcpyDeviceToHost, st));
+        CARMPC_CUDA(cudaStreamSynchronize(st));
+        k.iters = (int64_t)total;
+    }
+    last_total_iters = k.iters; last_launches = k.launches;
     return CARMPC_OK;
 }
 
-int QPHandle::solve_enqueue(const double* d_x0, int64_t stride, const double* xref, const double* d_c, const int* d_idx,
-                            const int* d_count, int64_t max_count, double* d_u0, int32_t* d_status, float* d_warm,
-                            cudaStream_t st) {
+int QPHandle::solve_enqueue(const SolveRequest& r, cudaStream_t st) {
     if (host_only) { set_error("carmpc_qp: this handle was created without a CUDA device; there is no CPU solver"); return CARMPC_ERR_CUDA; }
     if (!host.opts.polish) { set_error("solve_enqueue needs the float64 polish (opts.polish = 1)"); return CARMPC_ERR_INVALID; }
-    int rc = ensure_workspace(stride);
+    int rc = ensure_workspace(r.stride);
     if (rc != CARMPC_OK) return rc;
-    CARMPC_CUDA(cudaMemsetAsync(ws_counters, 0, sizeof(int) * 16, st));
-    const int cap = (int)max_count;
-    int* status = d_status;
+    CARMPC_CUDA(cudaMemsetAsync(ws_counters, 0, sizeof(int) * kCounters, st));
+    const int cap = (int)r.count;
 
-    // every stage below (pu, p0, the polish passes, ab, the certificates, the fallback) sees the same disturbance d_c
-    PolishBatch pb;
-    memset(&pb, 0, sizeof(pb));
-    pb.x0 = d_x0; pb.stride = stride; pb.cdist = d_c;
-    for (int c = 0; c < 4; ++c) pb.xref[c] = xref[c];
-    pb.sign = ws_sign; pb.u_admm = ws_u; pb.status = status; pb.u0 = d_u0; pb.polished = ws_polished;
-    pb.rounds = -1; pb.stats = ws_polish_stats; pb.sign_out = ws_sign;
+    // every stage below (pu, p0, the polish passes, ab, the certificates, the fallback) sees the same disturbance r.c
+    PolishBatch pb = polish_batch(*this, r);
+    AdmmBatch ab = admm_batch(*this, r);
 
     // 0. the empty active set (runs near their goal: the unconstrained minimiser is feasible), one thread per run
     PolishBatch pu = pb;
-    pu.idx_list = d_idx; pu.count = cap; pu.count_dev = d_count; pu.iters_out = ws_iters;
-    rc = polish_unconstrained_launch(this, pu, ws_rest, ws_counters + 6, st);
+    pu.iters_out = ab.iters;
+    rc = polish_unconstrained_launch(this, pu, ws_rest, ws_counters + kCntRest, st);
     if (rc != CARMPC_OK) return rc;
     // 1. the active set certified at the previous step, straight into the float64 polish
     PolishBatch p0 = pb;
-    p0.idx_list = ws_rest; p0.count = cap; p0.count_dev = ws_counters + 6;
-    p0.rounds = 4; p0.final_pass = 0; p0.n_failed = ws_counters + 5; p0.failed_list = ws_failed0;
+    p0.idx_list = ws_rest; p0.count = cap; p0.count_dev = ws_counters + kCntRest;
+    p0.rounds = 4; p0.final_pass = 0; p0.n_failed = ws_counters + kCntReuseFailed; p0.failed_list = ws_failed0;
     p0.precheck = 1; p0.Px = admm.Px; p0.Pc = admm.Pc; p0.pre_lo = admm.pre_lo; p0.pre_hi = admm.pre_hi; p0.kpre = admm.kpre;
-    p0.iters_out = ws_iters;
+    p0.iters_out = ab.iters;
     rc = polish_launch(this, p0, st);
     if (rc != CARMPC_OK) return rc;
 
     // 2. ADMM (warm-started from the previous step's state) for the runs whose set changed, then the polish
-    AdmmBatch ab;
-    memset(&ab, 0, sizeof(ab));
-    ab.x0 = d_x0; ab.stride = stride; ab.cdist = d_c;
-    for (int c = 0; c < 4; ++c) ab.xref[c] = xref[c];
-    ab.idx_list = ws_failed0; ab.count = cap; ab.count_dev = ws_counters + 5; ab.narrow = 1; ab.next = ws_counters + 0;
-    ab.sign = ws_sign; ab.u_admm = ws_u; ab.status = status; ab.iters = ws_iters;
-    ab.warm = d_warm; ab.warm_in = 1; ab.warm_out = 1;
-    ab.total_iters = ws_total_iters; ab.eps_scale = 1.f; ab.max_iter = host.opts.max_iter;
+    ab.idx_list = ws_failed0; ab.count = cap; ab.count_dev = ws_counters + kCntReuseFailed; ab.narrow = 1;
     rc = admm_launch(this, ab, st);
     if (rc != CARMPC_OK) return rc;
-    pb.idx_list = ws_failed0; pb.count = cap; pb.count_dev = ws_counters + 5;
-    pb.n_failed = ws_counters + 1; pb.failed_list = ws_failed; pb.final_pass = 0;
+    pb.idx_list = ws_failed0; pb.count = cap; pb.count_dev = ws_counters + kCntReuseFailed;
     rc = polish_launch(this, pb, st);
     if (rc != CARMPC_OK) return rc;
-    rc = farkas_verify_launch(this, ws_failed0, cap, status, d_warm, d_x0, stride, d_c, xref, ws_failed, ws_counters + 1, st,
-                              ws_counters + 5);
+    rc = farkas_verify_launch(this, pb, ws_failed0, cap, ws_counters + kCntReuseFailed, r.warm, ws_failed, ws_counters + kCntFailed, st);
     if (rc != CARMPC_OK) return rc;
 
     // 3. second pass (tighter) for what is still open, then the float64 fallback: all sized on the device, almost always empty
-    ab.idx_list = ws_failed; ab.count_dev = ws_counters + 1; ab.next = ws_counters + 2; ab.eps_scale = 0.01f;
+    ab.idx_list = ws_failed; ab.count_dev = ws_counters + kCntFailed; ab.next = ws_counters + kCntNext2; ab.eps_scale = 0.01f;
     ab.iters_accumulate = 1; ab.write_u = 1;
     rc = admm_launch(this, ab, st);
     if (rc != CARMPC_OK) return rc;
-    pb.idx_list = ws_failed; pb.count_dev = ws_counters + 1; pb.n_failed = ws_counters + 3; pb.final_pass = 1;
+    pb.idx_list = ws_failed; pb.count_dev = ws_counters + kCntFailed; pb.n_failed = ws_counters + kCntFinal; pb.final_pass = 1;
     rc = polish_launch(this, pb, st);
     if (rc != CARMPC_OK) return rc;
-    rc = farkas_decide_launch(this, ws_failed, cap, status, d_warm, d_x0, stride, d_c, d_u0, nullptr, nullptr, ws_polished, st,
-                              ws_counters + 1);
+    rc = farkas_decide_launch(this, pb, ws_failed, cap, ws_counters + kCntFailed, r.warm, st);
     if (rc != CARMPC_OK) return rc;
-    rc = farkas_verify_launch(this, ws_failed, cap, status, d_warm, d_x0, stride, d_c, xref, ws_overflow, ws_counters + 13, st,
-                              ws_counters + 1);
+    rc = farkas_verify_launch(this, pb, ws_failed, cap, ws_counters + kCntFailed, r.warm, ws_overflow, ws_counters + kCntVerify2, st);
     if (rc != CARMPC_OK) return rc;
     int handled = 0;
-    return exact_fallback(this, pb, ws_failed, cap, d_warm, ws_iters, st, &handled, ws_counters + 1);
+    return exact_fallback(this, pb, ws_failed, cap, ws_counters + kCntFailed, r.warm, ab.iters, st, &handled);
 }
 
-int QPHandle::solve_seeded(const double* d_x0, int64_t batch, const double* xref, const double* d_c, const int* d_seed,
-                           double* d_u0, double* d_objective, int32_t* d_status, int32_t* d_iters, double* d_u_full,
-                           cudaStream_t st) {
+int QPHandle::solve_seeded(const SolveRequest& r, cudaStream_t st, SolveCounts* counts) {
     if (host_only) { set_error("carmpc_qp: this handle was created without a CUDA device; there is no CPU solver"); return CARMPC_ERR_CUDA; }
     if (!host.opts.polish) { set_error("carmpc_qp_solve_seeded needs the float64 polish (opts.polish = 1)"); return CARMPC_ERR_INVALID; }
+    const int64_t batch = r.stride;
     int rc = ensure_workspace(batch);
     if (rc != CARMPC_OK) return rc;
-    struct ResetOnExit { int& flag; ~ResetOnExit() { flag = 0; } } reset_records{use_records}, reset_hold{stats_hold};   // also on error returns
     CARMPC_CUDA(cudaMemsetAsync(ws_polish_stats, 0, sizeof(unsigned long long) * kPolishStats, st));
-    stats_hold = 1;                                       // the histogram covers anchors and followers
-    CARMPC_CUDA(cudaMemsetAsync(ws_counters + 8, 0, sizeof(int) * 2, st));
-    CARMPC_CUDA(cudaMemsetAsync(d_status, 0, sizeof(int32_t) * batch, st));     // followers enter the polish as "not infeasible"
-    split_seeds_kernel<<<(int)((batch + 255) / 256), 256, 0, st>>>(d_seed, (int)batch, ws_anchor, ws_follow, ws_counters + 8,
-                                                                   ws_rec_of);
+    CARMPC_CUDA(cudaMemsetAsync(ws_counters + kCntAnchors, 0, sizeof(int) * 2, st));
+    CARMPC_CUDA(cudaMemsetAsync(r.status, 0, sizeof(int32_t) * batch, st));     // followers enter the polish as "not infeasible"
+    split_seeds_kernel<<<(int)((batch + 255) / 256), 256, 0, st>>>(r.seed, (int)batch, ws_anchor, ws_follow,
+                                                                   ws_counters + kCntAnchors, ws_rec_of);
     int n_split[2] = {0, 0};
-    CARMPC_CUDA(cudaMemcpyAsync(n_split, ws_counters + 8, sizeof(int) * 2, cudaMemcpyDeviceToHost, st));
+    CARMPC_CUDA(cudaMemcpyAsync(n_split, ws_counters + kCntAnchors, sizeof(int) * 2, cudaMemcpyDeviceToHost, st));
     CARMPC_CUDA(cudaStreamSynchronize(st));
+    SolveRequest part = r;
+    part.hold_stats = 1; part.keep_sign = 1;              // the histogram covers anchors and followers
     // multiplier maps of the anchors (1.4 KB each); skipped when there is a per-sample disturbance or too many anchors
     constexpr size_t kRecLam = sizeof(double) * 32 * 5, kRecAct = sizeof(int) * 33;
-    use_records = 0;
-    if (d_c == nullptr && n_split[0] > 0 && n_split[1] > 0 && (size_t)n_split[0] * (kRecLam + kRecAct) <= ((size_t)1 << 30)) {
+    if (r.c == nullptr && n_split[0] > 0 && n_split[1] > 0 && (size_t)n_split[0] * (kRecLam + kRecAct) <= ((size_t)1 << 30)) {
         if (n_split[0] > rec_cap) {
             cudaFree(ws_rec_lam); cudaFree(ws_rec_act); ws_rec_lam = nullptr; ws_rec_act = nullptr; rec_cap = 0;
             CARMPC_CUDA(cudaMalloc(&ws_rec_lam, kRecLam * n_split[0]));
@@ -429,30 +417,29 @@ int QPHandle::solve_seeded(const double* d_x0, int64_t batch, const double* xref
             rec_cap = n_split[0];
         }
         CARMPC_CUDA(cudaMemsetAsync(ws_rec_act, 0xFF, kRecAct * n_split[0], st));      // na = -1: no map yet
-        use_records = 1;
+        part.records = 1;
     }
-    int64_t iters_sum = 0, launches = 1, second = 0;
+    SolveCounts sum, k;
+    sum.launches = 1;
     if (n_split[0] > 0) {
-        rc = solve(d_x0, batch, xref, d_c, ws_anchor, n_split[0], d_u0, d_objective, d_status, d_iters, d_u_full, nullptr, 0, 0, st,
-                   0, nullptr, 1);
+        part.idx = ws_anchor; part.count = n_split[0]; part.reuse = 0; part.seed = nullptr;
+        rc = solve(part, st, &k);
         if (rc != CARMPC_OK) return rc;
-        iters_sum += last_total_iters; launches += last_launches; second += last_second_pass;
-        if (use_records && n_split[1] > 0) {
-            rc = farkas_export_launch(this, ws_anchor, n_split[0], d_status, ws_warm, d_x0, batch, st);
+        sum.iters += k.iters; sum.launches += k.launches;
+        if (part.records && n_split[1] > 0) {
+            rc = farkas_export_launch(this, polish_batch(*this, part), ws_anchor, n_split[0], ws_warm, st);
             if (rc != CARMPC_OK) return rc;
-            ++launches;
+            ++sum.launches;
         }
     }
-    int64_t reused = 0;
     if (n_split[1] > 0) {
-        rc = solve(d_x0, batch, xref, d_c, ws_follow, n_split[1], d_u0, d_objective, d_status, d_iters, d_u_full, nullptr, 0, 0, st,
-                   1, d_seed, 1);
+        part.idx = ws_follow; part.count = n_split[1]; part.reuse = 1; part.seed = r.seed;
+        rc = solve(part, st, &k);
         if (rc != CARMPC_OK) return rc;
-        iters_sum += last_total_iters; launches += last_launches; second += last_second_pass; reused = last_reused;
+        sum.iters += k.iters; sum.launches += k.launches; sum.reused = k.reused;
     }
-    use_records = 0;
-    last_total_iters = iters_sum; last_launches = launches; last_second_pass = second; last_reused = reused;
-    last_anchors = n_split[0];
+    last_total_iters = sum.iters; last_launches = sum.launches;
+    if (counts) *counts = sum;
     return CARMPC_OK;
 }
 
@@ -656,9 +643,11 @@ int carmpc_qp_solve_batch(void* qp, const double* d_x0, const double* h_xref, co
     CARMPC_REQUIRE(d_x0 && d_status, "d_x0 and d_status are required");
     QPBusyGuard guard(q->busy);
     CARMPC_REQUIRE(guard.acquired, "this QP handle is in use by another call (one call per handle at a time)");
-    q->use_records = 0;
-    return q->solve(d_x0, batch, h_xref, d_c, nullptr, batch, d_u0, d_objective, d_status, d_iters, d_u_full, d_warm,
-                    warm_in, warm_out, (cudaStream_t)stream);
+    SolveRequest r;
+    r.x0 = d_x0; r.stride = r.count = batch; r.xref = h_xref; r.c = d_c;
+    r.u0 = d_u0; r.objective = d_objective; r.status = d_status; r.iters = d_iters; r.u_full = d_u_full;
+    r.warm = d_warm; r.warm_in = warm_in; r.warm_out = warm_out;
+    return q->solve(r, (cudaStream_t)stream);
 }
 
 int carmpc_qp_solve_seeded(void* qp, const double* d_x0, const double* h_xref, const double* d_c, const int32_t* d_seed,
@@ -673,9 +662,12 @@ int carmpc_qp_solve_seeded(void* qp, const double* d_x0, const double* h_xref, c
     CARMPC_REQUIRE(d_x0 && d_status && d_seed, "d_x0, d_status and d_seed are required");
     QPBusyGuard guard(q->busy);
     CARMPC_REQUIRE(guard.acquired, "this QP handle is in use by another call (one call per handle at a time)");
-    const int rc = q->solve_seeded(d_x0, batch, h_xref, d_c, d_seed, d_u0, d_objective, d_status, d_iters, d_u_full,
-                                   (cudaStream_t)stream);
-    if (rc == CARMPC_OK && h_seeded) *h_seeded = q->last_reused;
+    SolveRequest r;
+    r.x0 = d_x0; r.stride = r.count = batch; r.xref = h_xref; r.c = d_c; r.seed = d_seed;
+    r.u0 = d_u0; r.objective = d_objective; r.status = d_status; r.iters = d_iters; r.u_full = d_u_full;
+    SolveCounts k;
+    const int rc = q->solve_seeded(r, (cudaStream_t)stream, &k);
+    if (rc == CARMPC_OK && h_seeded) *h_seeded = k.reused;
     return rc;
 }
 
@@ -696,16 +688,13 @@ int carmpc_qp_solve_certified(void* qp, const double* d_x0, const double* h_xref
     cudaStream_t st = (cudaStream_t)stream;
     const size_t width = (size_t)q->host.m + q->host.n + q->host.kpre;
     CARMPC_CUDA(cudaMemsetAsync(d_cert, 0, sizeof(double) * width * batch, st));
-    struct ResetOnExit { double*& p; ~ResetOnExit() { p = nullptr; } } reset_cert{q->cert};     // also on error returns
-    q->cert = d_cert;
-    int rc;
-    if (d_seed != nullptr) {
-        rc = q->solve_seeded(d_x0, batch, h_xref, d_c, d_seed, d_u0, d_objective, d_status, d_iters, d_u_full, st);
-        if (rc == CARMPC_OK && h_seeded) *h_seeded = q->last_reused;
-    } else {
-        q->use_records = 0;
-        rc = q->solve(d_x0, batch, h_xref, d_c, nullptr, batch, d_u0, d_objective, d_status, d_iters, d_u_full, nullptr, 0, 0, st);
-    }
+    SolveRequest r;
+    r.x0 = d_x0; r.stride = r.count = batch; r.xref = h_xref; r.c = d_c; r.seed = d_seed;
+    r.u0 = d_u0; r.objective = d_objective; r.status = d_status; r.iters = d_iters; r.u_full = d_u_full; r.cert = d_cert;
+    if (d_seed == nullptr) return q->solve(r, st);
+    SolveCounts k;
+    const int rc = q->solve_seeded(r, st, &k);
+    if (rc == CARMPC_OK && h_seeded) *h_seeded = k.reused;
     return rc;
 }
 
@@ -735,29 +724,20 @@ int carmpc_qp_solve_host(void* qp, const double* h_x0, const double* h_xref, con
     if (q->host_only) { set_error("carmpc_qp: this handle was created without a CUDA device; there is no CPU solver"); return CARMPC_ERR_CUDA; }
     QPBusyGuard guard(q->busy);
     CARMPC_REQUIRE(guard.acquired, "this QP handle is in use by another call (one call per handle at a time)");
-    const int n = q->host.n;
     int rc = q->ensure_io(batch, h_u_full != nullptr);
     if (rc != CARMPC_OK) return rc;
     cudaStream_t st = nullptr;
-    const int blocks = (int)((batch + 255) / 256);
     // states arrive as the reference passes them (batch x 4, row-major): one copy, re-laid out to SoA on the device
     CARMPC_CUDA(cudaMemcpyAsync(q->io_x0_aos, h_x0, sizeof(double) * 4 * batch, cudaMemcpyHostToDevice, st));
-    aos_to_soa_kernel<<<blocks, 256, 0, st>>>(q->io_x0_aos, q->io_x0, batch, 4);
+    aos_to_soa_kernel<<<(int)((batch + 255) / 256), 256, 0, st>>>(q->io_x0_aos, q->io_x0, batch, 4);
     if (h_c) CARMPC_CUDA(cudaMemcpyAsync(q->io_c, h_c, sizeof(double) * batch, cudaMemcpyHostToDevice, st));
-    rc = q->solve(q->io_x0, batch, h_xref, h_c ? q->io_c : nullptr, nullptr, batch, q->io_u0, q->io_obj, q->io_status,
-                  q->io_iters, h_u_full ? q->io_full : nullptr, nullptr, 0, 0, st);
+    SolveRequest r;
+    r.x0 = q->io_x0; r.stride = r.count = batch; r.xref = h_xref; r.c = h_c ? q->io_c : nullptr;
+    r.u0 = q->io_u0; r.objective = q->io_obj; r.status = q->io_status; r.iters = q->io_iters;
+    r.u_full = h_u_full ? q->io_full : nullptr;
+    rc = q->solve(r, st);
     if (rc != CARMPC_OK) return rc;
-    if (h_u0) {
-        soa_to_aos_kernel<<<blocks, 256, 0, st>>>(q->io_u0, q->io_u0_aos, batch, 2);
-        CARMPC_CUDA(cudaMemcpyAsync(h_u0, q->io_u0_aos, sizeof(double) * 2 * batch, cudaMemcpyDeviceToHost, st));
-    }
-    if (h_objective) CARMPC_CUDA(cudaMemcpyAsync(h_objective, q->io_obj, sizeof(double) * batch, cudaMemcpyDeviceToHost, st));
-    CARMPC_CUDA(cudaMemcpyAsync(h_status, q->io_status, sizeof(int32_t) * batch, cudaMemcpyDeviceToHost, st));
-    if (h_iters) CARMPC_CUDA(cudaMemcpyAsync(h_iters, q->io_iters, sizeof(int32_t) * batch, cudaMemcpyDeviceToHost, st));
-    if (h_u_full) CARMPC_CUDA(cudaMemcpyAsync(h_u_full, q->io_full, sizeof(double) * (size_t)n * batch, cudaMemcpyDeviceToHost, st));
-    CARMPC_CUDA(cudaStreamSynchronize(st));
-    CARMPC_CUDA(cudaGetLastError());
-    return CARMPC_OK;
+    return download(q, batch, h_u0, h_objective, h_status, h_iters, h_u_full, st);
 }
 
 int carmpc_qp_map_host(void* qp, const double* h_axes, const int32_t dims[4], const int32_t axis_to_state[4],
@@ -794,26 +774,19 @@ int carmpc_qp_map_host(void* qp, const double* h_axes, const int32_t dims[4], co
     CARMPC_CUDA(cudaMemcpyAsync(q->io_axes, h_axes, sizeof(double) * off, cudaMemcpyHostToDevice, st));
     map_expand_kernel<<<(int)((n + 255) / 256), 256, 0, st>>>(q->io_axes, g, n, q->io_x0, q->io_seed);
     CARMPC_CUDA(cudaGetLastError());
-    q->use_records = 0;
+    SolveRequest r;
+    r.x0 = q->io_x0; r.stride = r.count = n; r.xref = h_xref;
+    r.u0 = h_u0 ? q->io_u0 : nullptr; r.objective = h_objective ? q->io_obj : nullptr; r.status = q->io_status; r.iters = q->io_iters;
     if (blocked && q->host.opts.polish) {
-        rc = q->solve_seeded(q->io_x0, n, h_xref, nullptr, q->io_seed, h_u0 ? q->io_u0 : nullptr, h_objective ? q->io_obj : nullptr,
-                             q->io_status, q->io_iters, nullptr, st);
-        if (rc == CARMPC_OK && h_seeded) *h_seeded = q->last_reused;
+        r.seed = q->io_seed;
+        SolveCounts k;
+        rc = q->solve_seeded(r, st, &k);
+        if (rc == CARMPC_OK && h_seeded) *h_seeded = k.reused;
     } else {
-        rc = q->solve(q->io_x0, n, h_xref, nullptr, nullptr, n, h_u0 ? q->io_u0 : nullptr, h_objective ? q->io_obj : nullptr,
-                      q->io_status, q->io_iters, nullptr, nullptr, 0, 0, st);
+        rc = q->solve(r, st);
     }
     if (rc != CARMPC_OK) return rc;
-    if (h_u0) {
-        soa_to_aos_kernel<<<(int)((n + 255) / 256), 256, 0, st>>>(q->io_u0, q->io_u0_aos, n, 2);
-        CARMPC_CUDA(cudaMemcpyAsync(h_u0, q->io_u0_aos, sizeof(double) * 2 * n, cudaMemcpyDeviceToHost, st));
-    }
-    if (h_objective) CARMPC_CUDA(cudaMemcpyAsync(h_objective, q->io_obj, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
-    CARMPC_CUDA(cudaMemcpyAsync(h_status, q->io_status, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, st));
-    if (h_iters) CARMPC_CUDA(cudaMemcpyAsync(h_iters, q->io_iters, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, st));
-    CARMPC_CUDA(cudaStreamSynchronize(st));
-    CARMPC_CUDA(cudaGetLastError());
-    return CARMPC_OK;
+    return download(q, n, h_u0, h_objective, h_status, h_iters, nullptr, st);
 }
 
 int carmpc_qp_polish_stats(void* qp, int64_t* h_hist20) {

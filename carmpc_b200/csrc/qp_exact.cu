@@ -352,13 +352,13 @@ static size_t exact_smem(int n, int mt) { return sizeof(double) * (kExactThreads
 
 // After the second pass: everything in `d_list` that is still unproven goes through the float64 ADMM; converged samples
 // get one more polish (strict: no certificate -> CARMPC_QP_MAX_ITER).  Returns the number of samples handled.
-int exact_fallback(QPHandle* q, const PolishBatch& pb_final, const int* d_list, int count, float* d_warm, int* d_iters,
-                   cudaStream_t st, int* h_handled, const int* d_count) {
+int exact_fallback(QPHandle* q, const PolishBatch& b, const int* d_list, int count, const int* d_count, float* d_warm,
+                   int* d_iters, cudaStream_t st, int* h_handled) {
     *h_handled = 0;
     if (count <= 0) return CARMPC_OK;
-    int* n_unproven = q->ws_counters + 11;
+    int* n_unproven = q->ws_counters + kCntUnproven;
     CARMPC_CUDA(cudaMemsetAsync(n_unproven, 0, sizeof(int), st));
-    collect_unproven_kernel<<<std::min((count + 255) / 256, 64), 256, 0, st>>>(d_list, count, d_count, pb_final.status, q->ws_polished,
+    collect_unproven_kernel<<<std::min((count + 255) / 256, 64), 256, 0, st>>>(d_list, count, d_count, b.status, b.polished,
                                                                           q->ws_unproven, n_unproven);
     int n = 0;
     if (d_count == nullptr) {
@@ -372,11 +372,11 @@ int exact_fallback(QPHandle* q, const PolishBatch& pb_final, const int* d_list, 
     ExactArgs a;
     memset(&a, 0, sizeof(a));
     a.list = q->ws_unproven; a.count_dev = n_unproven; a.count_max = d_count == nullptr ? n : count;
-    a.x0 = pb_final.x0; a.stride = pb_final.stride; a.cdist = pb_final.cdist;
-    for (int c = 0; c < 4; ++c) a.xref[c] = pb_final.xref[c];
-    a.warm = d_warm; a.sign = q->ws_sign; a.status = pb_final.status; a.iters = d_iters;
-    a.u0 = pb_final.u0; a.objective = pb_final.objective; a.u_full = pb_final.u_full; a.polished = q->ws_polished;
-    a.stats = q->ws_polish_stats; a.total_iters = q->ws_total_iters; a.cert = q->cert;
+    a.x0 = b.x0; a.stride = b.stride; a.cdist = b.cdist;
+    for (int c = 0; c < 4; ++c) a.xref[c] = b.xref[c];
+    a.warm = d_warm; a.sign = q->ws_sign; a.status = b.status; a.iters = d_iters;
+    a.u0 = b.u0; a.objective = b.objective; a.u_full = b.u_full; a.polished = b.polished;
+    a.stats = b.stats; a.total_iters = q->ws_total_iters; a.cert = b.cert;
     const int mt = q->polish.mt, nn = q->polish.n;
     // iteration budget: ~4e8 multiply-adds per sample (5000 iterations at N = 20, ~2600 at N = 80)
     const double macs = 2.0 * q->polish.m * nn + (double)nn * nn;
@@ -388,23 +388,22 @@ int exact_fallback(QPHandle* q, const PolishBatch& pb_final, const int* d_list, 
     kernel<<<blocks, kExactThreads, smem, st>>>(q->polish, q->exact, a);
     CARMPC_CUDA(cudaGetLastError());
     // one more float64 polish from the float64 active sets; strict: an uncertified sample becomes "undecided"
-    PolishBatch pb = pb_final;
+    PolishBatch pb = b;
     pb.idx_list = q->ws_unproven; pb.count = d_count == nullptr ? n : count; pb.count_dev = d_count == nullptr ? nullptr : n_unproven;
-    pb.n_failed = q->ws_counters + 12; pb.final_pass = 2; pb.rounds = 40;
+    pb.n_failed = q->ws_counters + kCntExactFinal; pb.final_pass = 2; pb.rounds = 40;
     return polish_launch(q, pb, st);
 }
 
-int farkas_verify_launch(QPHandle* q, const int* d_list, int count, int* d_status, const float* d_warm, const double* d_x0,
-                         int64_t stride, const double* d_c, const double* xref, int* d_failed, int* d_n_failed, cudaStream_t st,
-                         const int* d_count) {
+int farkas_verify_launch(QPHandle* q, const PolishBatch& b, const int* d_list, int count, const int* d_count,
+                         const float* d_warm, int* d_failed, int* d_n_failed, cudaStream_t st) {
     if (count <= 0) return CARMPC_OK;
     VerifyArgs a;
     memset(&a, 0, sizeof(a));
-    a.list = d_list; a.count = count; a.count_dev = d_count; a.x0 = d_x0; a.stride = stride; a.cdist = d_c;
-    for (int c = 0; c < 4; ++c) a.xref[c] = xref[c];
-    a.warm = d_warm; a.status = d_status;
+    a.list = d_list; a.count = count; a.count_dev = d_count; a.x0 = b.x0; a.stride = b.stride; a.cdist = b.cdist;
+    for (int c = 0; c < 4; ++c) a.xref[c] = b.xref[c];
+    a.warm = d_warm; a.status = b.status;
     a.Px = q->admm.Px; a.Pc = q->admm.Pc; a.pre_lo = q->admm.pre_lo; a.pre_hi = q->admm.pre_hi; a.kpre = q->admm.kpre;
-    a.failed = d_failed; a.n_failed = d_n_failed; a.cert = q->cert;
+    a.failed = d_failed; a.n_failed = d_n_failed; a.cert = b.cert;
     const size_t smem = exact_smem(q->polish.n, q->polish.mt);
     int per_sm = 0;
     void (*kernel)(const PolishTables, const ExactTables, const VerifyArgs) = a.cert ? verify_kernel<true> : verify_kernel<false>;

@@ -269,6 +269,52 @@ int qp_host_setup(int n, int m, int k, const double* H, const double* F, const d
                   const double* Px, const double* Pc, const double* pre_lo, const double* pre_hi,
                   const carmpc_qp_opts& opts, QPHost* out);
 
+// What one solve is asked to do (host only).  QPHandle::solve / solve_enqueue / solve_seeded take it whole, so that no
+// option of a call is left on the handle for the next one.  Device pointers; outputs are nullable except status.
+struct SolveRequest {
+    const double* x0 = nullptr; int64_t stride = 0;   // SoA x0[c * stride + sample]; every per-sample array has stride
+    const double* xref = nullptr;    // host, 4 values
+    const double* c = nullptr;       // nullable per-sample disturbance: every stage shifts its bounds by Gc c
+    const int* idx = nullptr; int64_t count = 0;       // the samples solved now: idx[0 .. count) (null idx: 0 .. count)
+    const int* count_dev = nullptr;  // solve_enqueue: the number of listed samples lives here (count is an upper bound)
+    double *u0 = nullptr, *objective = nullptr, *u_full = nullptr;
+    int32_t *status = nullptr, *iters = nullptr;
+    double* cert = nullptr;          // [stride][mt + kpre] certificate rows, zeroed by the caller
+    float* warm = nullptr;           // ADMM state [stride][mt] (null: the workspace's)
+    int warm_in = 0, warm_out = 0;
+    int reuse = 0;                   // try the certified active set kept in the workspace first
+    const int* seed = nullptr;       // with reuse: sample i starts from the certified set of sample seed[i]
+    int keep_sign = 0;               // write certified active sets back to the workspace
+    int records = 0;                 // seeded solve: anchors export multiplier maps, followers read them
+    int hold_stats = 0;              // keep counting into the polish histogram instead of zeroing it
+    int keep_total = 0;              // closed loop: the iteration total accumulates on the device, read once at the end
+    int certify_shifted = 0;         // run the filter / decide certificates with a disturbance too (the public entry
+                                     // points keep max_iter there)
+};
+
+// What a solve did (also published as last_total_iters / last_launches for carmpc_qp_last_stats): ADMM iterations (0
+// with keep_total), kernel launches, samples certified from the reused active set
+struct SolveCounts { int64_t iters = 0, launches = 0, reused = 0; };
+
+// Counters of the solve pipeline (QPHandle::ws_counters, 16 ints).  The indices are fixed: solve() zeroes [0, 8) per call,
+// solve_enqueue() [0, 16), solve_seeded() the split pair [8, 10).
+constexpr int kCntNext = 0;          // ADMM work counter, first pass
+constexpr int kCntFailed = 1;        // first-pass samples the polish could not certify (list ws_failed)
+constexpr int kCntNext2 = 2;         // ADMM work counter, second pass
+constexpr int kCntFinal = 3;         // n_failed of the final polish (a final pass lists nothing)
+constexpr int kCntOverflow = 4;      // polish samples over the small active-set budget (list ws_overflow)
+constexpr int kCntReuseFailed = 5;   // samples the reused active set did not certify (list ws_failed0)
+constexpr int kCntRest = 6;          // samples the empty active set did not settle (list ws_rest)
+constexpr int kCntSurvivors = 7;     // samples the Farkas filter did not prove infeasible (list ws_overflow)
+constexpr int kCntAnchors = 8;       // seeded split: anchors (list ws_anchor), then followers (list ws_follow) at 9
+constexpr int kCntUnproven = 11;     // samples the second pass left without a proof (list ws_unproven)
+constexpr int kCntExactFinal = 12;   // n_failed of the fallback's polish (a final pass lists nothing)
+constexpr int kCntVerify2 = 13;      // second-pass "infeasible" verdicts without a certificate (list ws_overflow)
+constexpr int kCounters = 16;
+// ws_overflow holds three lists in turn: the polish's overflow (kCntOverflow, refilled by every polish launch), the Farkas
+// filter's survivors (kCntSurvivors, copied to ws_failed at once) and the second verify's failures (kCntVerify2, never
+// read back: the exact fallback finds them by their status).
+
 struct QPHandle;
 struct QPBusyGuard {
     std::atomic<bool>* flag;
@@ -283,24 +329,22 @@ bool admm_tc_usable(const QPHandle* q, const AdmmBatch& b);
 int polish_launch(QPHandle* q, const PolishBatch& b, cudaStream_t st);
 // the empty active set tried first (one thread per sample); samples it does not settle are appended to d_rest
 int polish_unconstrained_launch(QPHandle* q, const PolishBatch& b, int* d_rest, int* d_n_rest, cudaStream_t st);
+// The certificate launches take the per-sample arrays (x0, c, status, outputs), the histogram and the certificate rows
+// from the call's polish batch `b`, and work on the samples d_list[0 .. count) (d_count: the count lives on the device).
 // infeasible anchors of a seeded map: turn the ADMM dual iterate into an exact Farkas certificate, affine in x0
-int farkas_export_launch(QPHandle* q, const int* d_anchors, int count, const int* d_status, const float* d_warm,
-                         const double* d_x0, int64_t stride, cudaStream_t st);
+int farkas_export_launch(QPHandle* q, const PolishBatch& b, const int* d_list, int count, const float* d_warm, cudaStream_t st);
 // before the second pass: samples the certificate of their first-pass state proves infeasible are done, the rest is listed
-int farkas_filter_launch(QPHandle* q, const int* d_list, int count, int* d_status, const float* d_warm, const double* d_x0,
-                         int64_t stride, const double* d_c, double* d_u0, double* d_objective, double* d_u_full,
-                         int8_t* d_polished, int* d_survivors, int* d_n_survivors, cudaStream_t st);
+int farkas_filter_launch(QPHandle* q, const PolishBatch& b, const int* d_list, int count, const float* d_warm,
+                         int* d_survivors, int* d_n_survivors, cudaStream_t st);
 // samples that ran out of ADMM iterations: a valid certificate from their final ADMM state makes them proven infeasible
-int farkas_decide_launch(QPHandle* q, const int* d_list, int count, int* d_status, const float* d_warm, const double* d_x0,
-                         int64_t stride, const double* d_c, double* d_u0, double* d_objective, double* d_u_full,
-                         int8_t* d_polished, cudaStream_t st, const int* d_count = nullptr);
+int farkas_decide_launch(QPHandle* q, const PolishBatch& b, const int* d_list, int count, const int* d_count,
+                         const float* d_warm, cudaStream_t st);
 // ADMM verdicts "infeasible" are only accepted with a float64 certificate: the others re-enter the second pass
-int farkas_verify_launch(QPHandle* q, const int* d_list, int count, int* d_status, const float* d_warm, const double* d_x0,
-                         int64_t stride, const double* d_c, const double* xref, int* d_failed, int* d_n_failed, cudaStream_t st,
-                         const int* d_count = nullptr);
-// float64 fallback for what the second pass could not prove (qp_exact.cu)
-int exact_fallback(QPHandle* q, const PolishBatch& pb_final, const int* d_list, int count, float* d_warm, int* d_iters,
-                   cudaStream_t st, int* h_handled, const int* d_count = nullptr);
+int farkas_verify_launch(QPHandle* q, const PolishBatch& b, const int* d_list, int count, const int* d_count,
+                         const float* d_warm, int* d_failed, int* d_n_failed, cudaStream_t st);
+// float64 fallback for what the second pass could not prove (qp_exact.cu); *h_handled: the number of samples it took
+int exact_fallback(QPHandle* q, const PolishBatch& b, const int* d_list, int count, const int* d_count, float* d_warm,
+                   int* d_iters, cudaStream_t st, int* h_handled);
 size_t admm_smem_bytes(const QPHost& h, int samples_per_lane, bool mats_in_smem);
 // derivatives of certified solutions (qp_sensitivity.cu); d_x0 SoA with stride = batch, d_jac / d_grad nullable
 int sensitivity_launch(QPHandle* q, const double* d_x0, const double* d_c, int64_t batch, const int32_t* d_status,
@@ -351,18 +395,10 @@ struct QPHandle : HandleBase {
     double* ws_rec_lam = nullptr;                // multiplier maps of the anchors (grown on demand, capped)
     int* ws_rec_act = nullptr;
     int64_t rec_cap = 0;
-    int use_records = 0;                         // set by solve_seeded for the two solve() calls it makes
     unsigned long long* ws_polish_stats = nullptr;   // [kPolishStats] histogram of the polish launches of the last solve
-    int stats_hold = 0;
-    int defer_total = 0;                         // closed loop: ws_total_iters accumulates over the steps, read once at the end
-    double* cert = nullptr;                      // carmpc_qp_solve_certified: [batch][mt + kpre] certificate rows, zeroed
-                                                 // by the entry point; every proof site below stores what it proved
-    int certify_with_c = 0;                      // closed loop with a disturbance estimate: solve() also runs the filter /
-                                                 // decide certificates on the disturbance-shifted bounds (the public
-                                                 // entry points keep max_iter there)
     int* ws_overflow = nullptr;
     int* ws_unproven = nullptr;                  // samples the second pass left without a proof (float64 fallback)
-    int* ws_counters = nullptr;                  // [0] work counter, [1] n_failed
+    int* ws_counters = nullptr;                  // [kCounters], indices kCnt*
     unsigned long long* ws_total_iters = nullptr;
     int8_t* ws_polished = nullptr;
     float* ws_warm = nullptr;                    // ADMM state of every sample (warm start of the second pass)
@@ -373,7 +409,7 @@ struct QPHandle : HandleBase {
     int32_t *io_status = nullptr, *io_iters = nullptr, *io_seed = nullptr;
     double* io_axes = nullptr;                   // grid axes of carmpc_qp_map_host
     int ensure_io(int64_t batch, bool want_full);
-    int64_t last_total_iters = 0, last_launches = 0, last_second_pass = 0, last_fallback = 0;
+    int64_t last_total_iters = 0, last_launches = 0;   // carmpc_qp_last_stats: the counts of the last (seeded) solve
     int sm = 148;
     bool host_only = false;
     // per-call state lives in the handle (workspace, counters): one call at a time.  A second call entering while one is
@@ -381,23 +417,14 @@ struct QPHandle : HandleBase {
     std::atomic<bool> busy{false};
     ~QPHandle() override;
     int ensure_workspace(int64_t batch);
-    // full solve on device buffers (all pointers device; any output may be null except status)
-    int solve(const double* d_x0, int64_t stride, const double* xref, const double* d_c, const int* d_idx, int64_t count,
-              double* d_u0, double* d_objective, int32_t* d_status, int32_t* d_iters, double* d_u_full, float* d_warm,
-              int warm_in, int warm_out, cudaStream_t st, int reuse_active_set = 0, const int* d_seed = nullptr,
-              int keep_sign = 0);
+    // full solve on device buffers; counts (nullable) receives what the call did
+    int solve(const SolveRequest& r, cudaStream_t st, SolveCounts* counts = nullptr);
     // The same pipeline for a warm-started sequence (closed loop), with every sample count left on the device: the list
-    // d_idx holds *d_count <= max_count entries, the previous step's certified active sets are tried first, and nothing
+    // r.idx holds *r.count_dev <= r.count entries, the previous step's certified active sets are tried first, and nothing
     // is read back - the call only enqueues (no host synchronisation), so consecutive steps run back to back on the GPU.
-    // d_c (nullable): per-sample disturbance estimate, indexed like d_x0; every stage shifts its bounds by Gc c.
-    int solve_enqueue(const double* d_x0, int64_t stride, const double* xref, const double* d_c, const int* d_idx,
-                      const int* d_count, int64_t max_count, double* d_u0, int32_t* d_status, float* d_warm, cudaStream_t st);
+    int solve_enqueue(const SolveRequest& r, cudaStream_t st);
     // anchors (seed[i] == i or out of range) cold, then every other sample from its anchor's certified active set
-    int solve_seeded(const double* d_x0, int64_t batch, const double* xref, const double* d_c, const int* d_seed,
-                     double* d_u0, double* d_objective, int32_t* d_status, int32_t* d_iters, double* d_u_full,
-                     cudaStream_t st);
-    int64_t last_reused = 0;                     // samples certified from the reused active set in the last solve
-    int64_t last_anchors = 0;                    // seeded solve: samples solved cold
+    int solve_seeded(const SolveRequest& r, cudaStream_t st, SolveCounts* counts = nullptr);
 };
 
 }  // namespace carmpc

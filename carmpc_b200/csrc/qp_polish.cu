@@ -645,33 +645,31 @@ static int farkas_launch(QPHandle* qh, const FarkasArgs& f, cudaStream_t st) {
     return CARMPC_OK;
 }
 
-int farkas_export_launch(QPHandle* qh, const int* d_anchors, int count, const int* d_status, const float* d_warm,
-                         const double* d_x0, int64_t stride, cudaStream_t st) {
+// the per-sample arrays, the histogram and the certificate rows of the call
+static FarkasArgs farkas_args(const PolishBatch& b, const int* d_list, int count, const int* d_count, int mode,
+                              const float* d_warm) {
     FarkasArgs f = {};
-    f.list = d_anchors; f.count = count; f.mode = 0; f.status = const_cast<int*>(d_status); f.warm = d_warm; f.x0 = d_x0;
-    f.stride = stride; f.rec_of = qh->ws_rec_of; f.rec_lam = qh->ws_rec_lam; f.rec_act = qh->ws_rec_act; f.cert = qh->cert;
+    f.list = d_list; f.count = count; f.count_dev = d_count; f.mode = mode; f.status = b.status; f.warm = d_warm;
+    f.x0 = b.x0; f.stride = b.stride; f.cdist = b.cdist;
+    f.u0 = b.u0; f.objective = b.objective; f.u_full = b.u_full; f.polished = b.polished; f.stats = b.stats; f.cert = b.cert;
+    return f;
+}
+
+int farkas_export_launch(QPHandle* qh, const PolishBatch& b, const int* d_list, int count, const float* d_warm, cudaStream_t st) {
+    FarkasArgs f = farkas_args(b, d_list, count, nullptr, 0, d_warm);
+    f.rec_of = b.rec_of; f.rec_lam = b.rec_lam; f.rec_act = b.rec_act;
     return farkas_launch(qh, f, st);
 }
 
-int farkas_decide_launch(QPHandle* qh, const int* d_list, int count, int* d_status, const float* d_warm, const double* d_x0,
-                         int64_t stride, const double* d_c, double* d_u0, double* d_objective, double* d_u_full,
-                         int8_t* d_polished, cudaStream_t st, const int* d_count) {
-    FarkasArgs f = {};
-    f.list = d_list; f.count = count; f.count_dev = d_count; f.mode = 1; f.status = d_status; f.warm = d_warm; f.x0 = d_x0; f.stride = stride;
-    f.cdist = d_c;
-    f.u0 = d_u0; f.objective = d_objective; f.u_full = d_u_full; f.polished = d_polished; f.stats = qh->ws_polish_stats;
-    f.cert = qh->cert;
-    return farkas_launch(qh, f, st);
+int farkas_decide_launch(QPHandle* qh, const PolishBatch& b, const int* d_list, int count, const int* d_count,
+                         const float* d_warm, cudaStream_t st) {
+    return farkas_launch(qh, farkas_args(b, d_list, count, d_count, 1, d_warm), st);
 }
 
-int farkas_filter_launch(QPHandle* qh, const int* d_list, int count, int* d_status, const float* d_warm, const double* d_x0,
-                         int64_t stride, const double* d_c, double* d_u0, double* d_objective, double* d_u_full,
-                         int8_t* d_polished, int* d_survivors, int* d_n_survivors, cudaStream_t st) {
-    FarkasArgs f = {};
-    f.list = d_list; f.count = count; f.mode = 2; f.status = d_status; f.warm = d_warm; f.x0 = d_x0; f.stride = stride;
-    f.cdist = d_c;
-    f.u0 = d_u0; f.objective = d_objective; f.u_full = d_u_full; f.polished = d_polished; f.stats = qh->ws_polish_stats;
-    f.survivors = d_survivors; f.n_survivors = d_n_survivors; f.cert = qh->cert;
+int farkas_filter_launch(QPHandle* qh, const PolishBatch& b, const int* d_list, int count, const float* d_warm,
+                         int* d_survivors, int* d_n_survivors, cudaStream_t st) {
+    FarkasArgs f = farkas_args(b, d_list, count, nullptr, 2, d_warm);
+    f.survivors = d_survivors; f.n_survivors = d_n_survivors;
     return farkas_launch(qh, f, st);
 }
 
@@ -829,12 +827,12 @@ int polish_launch(QPHandle* qh, const PolishBatch& b_in, cudaStream_t st) {
         b.na_cap = full; b.overflow_list = nullptr; b.n_overflow = nullptr;
         return polish_launch_cap(qh, b, st);
     }
-    CARMPC_CUDA(cudaMemsetAsync(qh->ws_counters + 4, 0, sizeof(int), st));
-    b.na_cap = kPolishSmallActive; b.overflow_list = qh->ws_overflow; b.n_overflow = qh->ws_counters + 4;
+    CARMPC_CUDA(cudaMemsetAsync(qh->ws_counters + kCntOverflow, 0, sizeof(int), st));
+    b.na_cap = kPolishSmallActive; b.overflow_list = qh->ws_overflow; b.n_overflow = qh->ws_counters + kCntOverflow;
     int rc = polish_launch_cap(qh, b, st);
     if (rc != CARMPC_OK) return rc;
     // the overflow launch reads its sample count on the device (no host round trip; with nothing listed its CTAs exit at once)
-    b.na_cap = full; b.idx_list = qh->ws_overflow; b.count_dev = qh->ws_counters + 4; b.overflow_list = nullptr; b.n_overflow = nullptr;
+    b.na_cap = full; b.idx_list = qh->ws_overflow; b.count_dev = qh->ws_counters + kCntOverflow; b.overflow_list = nullptr; b.n_overflow = nullptr;
     return polish_launch_cap(qh, b, st);
 }
 

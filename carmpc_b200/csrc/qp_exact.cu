@@ -12,7 +12,8 @@
 // from the sample's float32 ADMM state; at every check the dual iterate y = E (w - clip(w)), completed with box
 // multipliers y_b = -G'y so that A'y = 0 holds exactly, is evaluated as a Farkas certificate (the test of
 // farkas_kernel, qp_polish.cu).  A converged sample hands its active set (the signs of w against its bounds) to one
-// more float64 polish, which certifies it or leaves it undecided.
+// more float64 polish, which certifies it or leaves it undecided; a sample still out of iterations goes to the same polish
+// with the active set its float32 passes left.
 #include <math.h>
 #include <string.h>
 
@@ -340,7 +341,9 @@ __global__ void __launch_bounds__(kExactThreads) exact_kernel(const PolishTables
                 if (A.u0) { A.u0[sample] = NaN; A.u0[A.stride + sample] = NaN; }
                 if (A.objective) A.objective[sample] = verdict == CARMPC_QP_INFEASIBLE ? INFINITY : NaN;
                 if (A.polished) A.polished[sample] = 0;
-                if (A.stats) atomicAdd(A.stats + (verdict == CARMPC_QP_INFEASIBLE ? 18 : 19), 1ull);
+                // a max_iter sample still goes through the strict polish below (from the active set its ADMM passes left),
+                // which counts it once, as solved (17) or undecided (19)
+                if (A.stats && verdict == CARMPC_QP_INFEASIBLE) atomicAdd(A.stats + 18, 1ull);
             }
         }
     }
@@ -350,8 +353,9 @@ static size_t exact_smem(int n, int mt) { return sizeof(double) * (kExactThreads
 
 }  // namespace
 
-// After the second pass: everything in `d_list` that is still unproven goes through the float64 ADMM; converged samples
-// get one more polish (strict: no certificate -> CARMPC_QP_MAX_ITER).  Returns the number of samples handled.
+// After the second pass: everything in `d_list` that is still unproven goes through the float64 ADMM; the samples it does
+// not prove infeasible get one more polish (strict: no certificate -> CARMPC_QP_MAX_ITER).  Returns the number of samples
+// handled.
 int exact_fallback(QPHandle* q, const PolishBatch& b, const int* d_list, int count, const int* d_count, float* d_warm,
                    int* d_iters, cudaStream_t st, int* h_handled) {
     *h_handled = 0;

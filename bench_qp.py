@@ -169,7 +169,7 @@ def run_qp_bench(args, rank, world, dev, barrier):
         res["cpu_baseline"] = cpu_qp_rate()
 
     # ---- config 3 as a region-of-attraction MAP: anchors of a sub-lattice solved cold, every other grid point first tries its
-    # anchor's certified active set in the float64 polish (carmpc_qp_solve_seeded); identical results, fewer ADMM iterations
+    # anchor's certified active set in the float64 polish (carmpc_qp_solve with d_seed); identical results, fewer ADMM iterations
     if not args.skip_seeded and full_grid:
         from carmpc_b200.grids import lattice_seeds
         dims = [len(a) for a in axes]
@@ -207,7 +207,7 @@ def run_qp_bench(args, rank, world, dev, barrier):
         res["seeded_map"] = {"metric": "horizon-20 QPs/s (region-of-attraction map, active sets seeded from lattice anchors)",
                              "value": seeded[best]["qps"], "unit": "QPs/s", "ms_per_step": seeded[best]["ms"],
                              "block": best, "by_block": seeded,
-                             "call": "carmpc_qp_solve_seeded (same certified optima and flags as the cold solve)"}
+                             "call": "carmpc_qp_solve with d_seed (same certified optima and flags as the cold solve)"}
     if not args.skip_seeded and full_grid and world == 1:
         # end to end for the map: grid axes on the host in, status / u0 / objective on the host out
         blk0 = blocks[0]

@@ -67,10 +67,8 @@ SIGNATURES = {
     "carmpc_qp_default_opts": (None, [ctypes.POINTER(QPOpts)]),
     "carmpc_qp_create": (_i32, [_i32, _i32, _i32] + [_dp] * 13 + [ctypes.POINTER(QPOpts), ctypes.POINTER(_vp)]),
     "carmpc_qp_get_setup": (_i32, [_vp, _i32, _dp, _i32]),
-    "carmpc_qp_solve_batch": (_i32, [_vp, _dp, _dp, _dp, _i64, _dp, _dp, _vp, _vp, _dp, _vp, _i32, _i32, _vp]),
-    "carmpc_qp_solve_seeded": (_i32, [_vp, _dp, _dp, _dp, _vp, _i64, _dp, _dp, _vp, _vp, _dp, ctypes.POINTER(_i64), _vp]),
-    "carmpc_qp_solve_certified": (_i32, [_vp, _dp, _dp, _dp, _vp, _i64, _dp, _dp, _vp, _vp, _dp, _dp, ctypes.POINTER(_i64),
-                                         _vp]),
+    "carmpc_qp_solve": (_i32, [_vp, _dp, _dp, _dp, _vp, _i64, _dp, _dp, _vp, _vp, _dp, _vp, _i32, _i32, _dp,
+                               ctypes.POINTER(_i64), _vp]),
     "carmpc_qp_sensitivity": (_i32, [_vp, _dp, _dp, _i64, _vp, _dp, _dp, _i32, _dp, _dp, _vp, _vp]),
     "carmpc_qp_checker_create": (_i32, [_i32, _i32] + [_dp] * 9 + [ctypes.POINTER(_vp)]),
     "carmpc_qp_check": (_i32, [_vp, _dp, _dp, _dp, _i64, _vp, _dp, _dp, _dp, _vp]),
@@ -80,15 +78,9 @@ SIGNATURES = {
     "carmpc_qp_polish_stats": (_i32, [_vp, ctypes.POINTER(_i64)]),
     "carmpc_qp_last_stats": (_i32, [_vp, ctypes.POINTER(_i64), ctypes.POINTER(_i64)]),
     "carmpc_qp_tensor_mode": (_i32, [_vp, _i32, ctypes.POINTER(_i64)]),
-    "carmpc_closed_loop": (_i32, [_vp, _i32, _dp, _dp, _dp, _dp, _dp, ctypes.c_double, ctypes.c_double, _i32,
-                                  _i32, _dp, _dp, _i64, _dp, _vp, _dp, _dp, ctypes.POINTER(_i64), _vp]),
-    "carmpc_closed_loop_disturbance": (_i32, [_vp, _dp, _dp, _dp, ctypes.POINTER(DisturbanceModel), _dp, ctypes.c_double,
-                                              ctypes.c_double, _i32, _i32, _dp, _dp, _dp, _dp, _i64, _dp, _dp, _vp, _dp,
-                                              _dp, _dp, ctypes.POINTER(_i64), _vp]),
-    "carmpc_closed_loop_stochastic": (_i32, [_vp, _i32, _dp, _dp, _dp, _dp, ctypes.POINTER(DisturbanceModel), _dp,
-                                             ctypes.c_double, ctypes.c_double, _i32, _i32, _dp, _dp, _dp, _dp, _i64, _dp,
-                                             _dp, _vp, _dp, _dp, _dp, ctypes.POINTER(LoopNoiseParams), _dp, _i32, _vp, _vp,
-                                             _vp, ctypes.POINTER(_i64), _vp]),
+    "carmpc_closed_loop": (_i32, [_vp, _i32, _dp, _dp, _dp, _dp, ctypes.POINTER(DisturbanceModel), _dp, ctypes.c_double,
+                                  ctypes.c_double, _i32, _i32, _dp, _dp, _dp, _dp, _i64, _dp, _dp, _vp, _dp, _dp, _dp,
+                                  ctypes.POINTER(LoopNoiseParams), _dp, _i32, _vp, _vp, _vp, ctypes.POINTER(_i64), _vp]),
     "carmpc_measure_peak": (_i32, [_i32, ctypes.POINTER(ctypes.c_double)]),
 }
 

@@ -363,7 +363,7 @@ class BatchQP(_Handle):
         ``out["seeded"]`` counts the samples that needed no ADMM iteration.  Same results as the cold solve.
 
         ``want_certificate``: also ``out["certificate"]``, a (B, m + n + k) float64 CUDA tensor in the row space of the
-        handle (``carmpc_qp_solve_certified``): the KKT multipliers of solved samples, the Farkas ray of infeasible ones,
+        handle (``d_cert`` of ``carmpc_qp_solve``): the KKT multipliers of solved samples, the Farkas ray of infeasible ones,
         zeros for undecided ones.  The other outputs are bit-identical to a solve without it (not with ``warm``)."""
         torch = _torch()
         if not (x0.is_cuda and x0.dtype == torch.float64 and x0.dim() == 2 and x0.shape[0] == 4 and x0.is_contiguous()):
@@ -388,28 +388,17 @@ class BatchQP(_Handle):
             if warm is not None:
                 raise ValueError("certificates are exported by cold and seeded solves, not warm-started ones")
             out["certificate"] = torch.empty((B, self.m + self.n + len(self.pq.pre_hi)), dtype=torch.float64, device=dev)
-            seeded = ctypes.c_int64(0)
-            check(self._lib.carmpc_qp_solve_certified(
-                self._h, x0.data_ptr(), _capi.ptr(xref), c.data_ptr() if c is not None else None,
-                seed.data_ptr() if seed is not None else None, B, out["u0"].data_ptr(), out["objective"].data_ptr(),
-                out["status"].data_ptr(), out["iters"].data_ptr(), out["u_full"].data_ptr() if want_u_full else None,
-                out["certificate"].data_ptr(), ctypes.byref(seeded), _stream_ptr(stream)))
-            if seed is not None:
-                out["seeded"] = int(seeded.value)
-            return out
+
+        def p(t):
+            return t.data_ptr() if t is not None else None
+
+        seeded = ctypes.c_int64(0)
+        check(self._lib.carmpc_qp_solve(
+            self._h, x0.data_ptr(), _capi.ptr(xref), p(c), p(seed), B, out["u0"].data_ptr(), out["objective"].data_ptr(),
+            out["status"].data_ptr(), out["iters"].data_ptr(), p(out.get("u_full")), p(warm), int(warm_in), int(warm_out),
+            p(out.get("certificate")), ctypes.byref(seeded), _stream_ptr(stream)))
         if seed is not None:
-            seeded = ctypes.c_int64(0)
-            check(self._lib.carmpc_qp_solve_seeded(
-                self._h, x0.data_ptr(), _capi.ptr(xref), c.data_ptr() if c is not None else None, seed.data_ptr(), B,
-                out["u0"].data_ptr(), out["objective"].data_ptr(), out["status"].data_ptr(), out["iters"].data_ptr(),
-                out["u_full"].data_ptr() if want_u_full else None, ctypes.byref(seeded), _stream_ptr(stream)))
             out["seeded"] = int(seeded.value)
-            return out
-        check(self._lib.carmpc_qp_solve_batch(
-            self._h, x0.data_ptr(), _capi.ptr(xref), c.data_ptr() if c is not None else None, B,
-            out["u0"].data_ptr(), out["objective"].data_ptr(), out["status"].data_ptr(), out["iters"].data_ptr(),
-            out["u_full"].data_ptr() if want_u_full else None, warm.data_ptr() if warm is not None else None,
-            int(warm_in), int(warm_out), _stream_ptr(stream)))
         return out
 
     def sensitivity(self, x0, out, c=None, rows: Optional[int] = None, stream=None) -> dict:
@@ -522,13 +511,37 @@ class BatchQP(_Handle):
             raise ValueError("monitor must have 1 to 512 finite rows")
         return np.ascontiguousarray(rows)
 
-    def _closed_loop_stochastic(self, mode, x_init, steps, A_, B_, C_, L_, dm, xref, dt, l1, warm_start, xhat_init,
-                                dhat_init, d_plant, out, noise, monitor, stream) -> None:
-        """``carmpc_closed_loop_stochastic`` into ``out`` (adds the monitor's outputs when ``monitor`` is given)."""
+    def _closed_loop(self, mode, x_init, steps, A, B, C, L, dm, x_ref, dt, l1, warm_start, xhat_init, dhat_init, d_plant,
+                     want_traj, want_inputs, want_dhat, noise, monitor, stream) -> dict:
+        """``carmpc_closed_loop`` in ``mode`` 0, 1 or 2 (``dm``: a ``DisturbanceModel``): checks the device inputs, then
+        returns the outputs the ``want_*`` flags, the mode and the monitor ask for, and ``total_iters``."""
         torch = _torch()
+        if not (x_init.is_cuda and x_init.dtype == torch.float64 and x_init.dim() == 2 and x_init.shape[0] == 4
+                and x_init.is_contiguous()):
+            raise ValueError("x_init must be a contiguous (4, R) float64 CUDA tensor")
         R, dev = x_init.shape[1], x_init.device
+        for name, t in (("d_plant", d_plant), ("dhat_init", dhat_init)):
+            if t is not None and not (t.is_cuda and t.dtype == torch.float64 and t.numel() == R and t.is_contiguous()):
+                raise ValueError(f"{name} must be a contiguous float64 CUDA tensor of R elements")
+        if xhat_init is not None and not (xhat_init.is_cuda and xhat_init.dtype == torch.float64
+                                          and tuple(xhat_init.shape) == (4, R) and xhat_init.is_contiguous()):
+            raise ValueError("xhat_init must be a contiguous (4, R) float64 CUDA tensor")
+        xref = _f64(self.pq.goal if x_ref is None else x_ref)
+        A_, B_ = _f64(A), _f64(B)
+        C_ = _f64(C) if C is not None else None
+        L_ = _f64(L) if L is not None else None
         params = noise.params() if noise is not None else None
         rows = self._monitor_rows(monitor) if monitor is not None else None
+        out = {"final": torch.empty((4, R), dtype=torch.float64, device=dev)}
+        if mode == 2:
+            out["dhat"] = torch.empty(R, dtype=torch.float64, device=dev)
+        out["fail_step"] = torch.empty(R, dtype=torch.int32, device=dev)
+        if want_traj:
+            out["traj"] = torch.empty((steps, 4, R), dtype=torch.float64, device=dev)
+        if want_inputs:
+            out["inputs"] = torch.empty((steps, 2, R), dtype=torch.float64, device=dev)
+        if want_dhat:
+            out["dhat_traj"] = torch.empty((steps, R), dtype=torch.float64, device=dev)
         if rows is not None:
             out["violation_step"] = torch.empty(R, dtype=torch.int32, device=dev)
             out["violation_row"] = torch.empty(R, dtype=torch.int32, device=dev)
@@ -538,7 +551,7 @@ class BatchQP(_Handle):
             return out[key].data_ptr() if key in out else None
 
         total = ctypes.c_int64(0)
-        check(self._lib.carmpc_closed_loop_stochastic(
+        check(self._lib.carmpc_closed_loop(
             self._h, mode, _capi.ptr(A_), _capi.ptr(B_), _capi.ptr(C_), _capi.ptr(L_),
             ctypes.byref(dm) if dm is not None else None, _capi.ptr(xref), float(dt), float(l1), int(steps),
             int(warm_start), x_init.data_ptr(), xhat_init.data_ptr() if xhat_init is not None else None,
@@ -547,6 +560,7 @@ class BatchQP(_Handle):
             ctypes.byref(params) if params is not None else None, _capi.ptr(rows), len(rows) if rows is not None else 0,
             p("violation_step"), p("violation_row"), p("violations_per_step"), ctypes.byref(total), _stream_ptr(stream)))
         out["total_iters"] = int(total.value)
+        return out
 
     def closed_loop(self, x_init, steps: int, A, B, x_ref=None, C=None, L=None, xhat_init=None, dt: float = 0.2,
                     l1: float = 3.5, warm_start: bool = True, want_traj: bool = False, want_inputs: bool = False,
@@ -560,43 +574,15 @@ class BatchQP(_Handle):
         ``monitor``: (rows, 5) ``[A | b]`` or ``(A, b)``, e.g. ``montecarlo.plant_rows(controller)``; the true state is
         checked against it after every plant step and ``violation_step`` (R,), ``violation_row`` (R,) (-1: none) and
         ``violations_per_step`` (steps,) int32 are added to the result.  A violation does not stop a run."""
-        torch = _torch()
-        if not (x_init.is_cuda and x_init.dtype == torch.float64 and x_init.dim() == 2 and x_init.shape[0] == 4
-                and x_init.is_contiguous()):
-            raise ValueError("x_init must be a contiguous (4, R) float64 CUDA tensor")
-        R = x_init.shape[1]
-        dev = x_init.device
-        mode = 1 if C is not None else 0
-        xref = _f64(self.pq.goal if x_ref is None else x_ref)
-        A_, B_ = _f64(A), _f64(B)
-        C_ = _f64(C) if C is not None else None
-        L_ = _f64(L) if L is not None else None
-        out = {"final": torch.empty((4, R), dtype=torch.float64, device=dev),
-               "fail_step": torch.empty(R, dtype=torch.int32, device=dev)}
-        if want_traj:
-            out["traj"] = torch.empty((steps, 4, R), dtype=torch.float64, device=dev)
-        if want_inputs:
-            out["inputs"] = torch.empty((steps, 2, R), dtype=torch.float64, device=dev)
-        if noise is not None or monitor is not None:
-            self._closed_loop_stochastic(mode, x_init, steps, A_, B_, C_, L_, None, xref, dt, l1, warm_start, xhat_init,
-                                         None, None, out, noise, monitor, stream)
-            return out
-        total = ctypes.c_int64(0)
-        check(self._lib.carmpc_closed_loop(
-            self._h, mode, _capi.ptr(A_), _capi.ptr(B_), _capi.ptr(C_), _capi.ptr(L_), _capi.ptr(xref), float(dt),
-            float(l1), int(steps), int(warm_start), x_init.data_ptr(),
-            xhat_init.data_ptr() if xhat_init is not None else None, R, out["final"].data_ptr(),
-            out["fail_step"].data_ptr(), out["traj"].data_ptr() if want_traj else None,
-            out["inputs"].data_ptr() if want_inputs else None, ctypes.byref(total), _stream_ptr(stream)))
-        out["total_iters"] = int(total.value)
-        return out
+        return self._closed_loop(1 if C is not None else 0, x_init, steps, A, B, C, L, None, x_ref, dt, l1, warm_start,
+                                 xhat_init, None, None, want_traj, want_inputs, False, noise, monitor, stream)
 
     def closed_loop_disturbance(self, x_init, steps: int, A, B, C, Bd, Cd, L1, L2, x_ref=None, Bd_plant=None,
                                 Cd_plant=None, d_plant=None, xhat_init=None, dhat_init=None, dt: float = 0.2,
                                 l1: float = 3.5, warm_start=True, want_traj: bool = False, want_inputs: bool = False,
                                 want_dhat: bool = False, noise=None, monitor=None, stream=None) -> dict:
         """Closed loops of the disturbance-estimating output-feedback controller (``MPCOutputFBWithDisturbance``,
-        ``carmpc_closed_loop_disturbance``): the loop of ``closed_loop`` with a scalar disturbance estimate ``d^`` kept
+        ``carmpc_closed_loop`` mode 2): the loop of ``closed_loop`` with a scalar disturbance estimate ``d^`` kept
         beside ``x^`` by the augmented observer (``Bd`` (4,), ``Cd`` (3,), gains ``L1`` (4, 3), ``L2`` (3,); no defaults,
         see ``carmpc_b200.observer``), and the QP of each run taking ``d^`` as its disturbance.  This handle's ``Gc`` must
         come from a controller with the same ``Bd`` (or be zero).  The plant gets a constant disturbance ``d_plant`` per
@@ -605,18 +591,6 @@ class BatchQP(_Handle):
         ``closed_loop``.  Returns ``final`` (4, R), ``dhat`` (R,), ``fail_step`` (R,) int32, ``total_iters`` and
         optionally ``traj`` (steps, 4, R), ``inputs`` (steps, 2, R), ``dhat_traj`` (steps, R).  ``noise`` and ``monitor``
         as in ``closed_loop`` (the measurement noise adds to ``C s + Cd_plant d_r``)."""
-        torch = _torch()
-        if not (x_init.is_cuda and x_init.dtype == torch.float64 and x_init.dim() == 2 and x_init.shape[0] == 4
-                and x_init.is_contiguous()):
-            raise ValueError("x_init must be a contiguous (4, R) float64 CUDA tensor")
-        R = x_init.shape[1]
-        dev = x_init.device
-        for name, t in (("d_plant", d_plant), ("dhat_init", dhat_init)):
-            if t is not None and not (t.is_cuda and t.dtype == torch.float64 and t.numel() == R and t.is_contiguous()):
-                raise ValueError(f"{name} must be a contiguous float64 CUDA tensor of R elements")
-        if xhat_init is not None and not (xhat_init.is_cuda and xhat_init.dtype == torch.float64
-                                          and tuple(xhat_init.shape) == (4, R) and xhat_init.is_contiguous()):
-            raise ValueError("xhat_init must be a contiguous (4, R) float64 CUDA tensor")
 
         def vec(a, n, name):
             v = _f64(a).ravel()
@@ -631,30 +605,5 @@ class BatchQP(_Handle):
         dm.L2[:] = vec(L2, 3, "L2").tolist()
         dm.Bd_plant[:] = vec(np.zeros(4) if Bd_plant is None else Bd_plant, 4, "Bd_plant").tolist()
         dm.Cd_plant[:] = vec(np.zeros(3) if Cd_plant is None else Cd_plant, 3, "Cd_plant").tolist()
-        xref = _f64(self.pq.goal if x_ref is None else x_ref)
-        A_, B_, C_ = _f64(A), _f64(B), _f64(C)
-        out = {"final": torch.empty((4, R), dtype=torch.float64, device=dev),
-               "dhat": torch.empty(R, dtype=torch.float64, device=dev),
-               "fail_step": torch.empty(R, dtype=torch.int32, device=dev)}
-        if want_traj:
-            out["traj"] = torch.empty((steps, 4, R), dtype=torch.float64, device=dev)
-        if want_inputs:
-            out["inputs"] = torch.empty((steps, 2, R), dtype=torch.float64, device=dev)
-        if want_dhat:
-            out["dhat_traj"] = torch.empty((steps, R), dtype=torch.float64, device=dev)
-        if noise is not None or monitor is not None:
-            self._closed_loop_stochastic(2, x_init, steps, A_, B_, C_, None, dm, xref, dt, l1, warm_start, xhat_init,
-                                         dhat_init, d_plant, out, noise, monitor, stream)
-            return out
-        total = ctypes.c_int64(0)
-        check(self._lib.carmpc_closed_loop_disturbance(
-            self._h, _capi.ptr(A_), _capi.ptr(B_), _capi.ptr(C_), ctypes.byref(dm), _capi.ptr(xref), float(dt),
-            float(l1), int(steps), int(warm_start), x_init.data_ptr(),
-            xhat_init.data_ptr() if xhat_init is not None else None,
-            dhat_init.data_ptr() if dhat_init is not None else None,
-            d_plant.data_ptr() if d_plant is not None else None, R, out["final"].data_ptr(), out["dhat"].data_ptr(),
-            out["fail_step"].data_ptr(), out["traj"].data_ptr() if want_traj else None,
-            out["inputs"].data_ptr() if want_inputs else None, out["dhat_traj"].data_ptr() if want_dhat else None,
-            ctypes.byref(total), _stream_ptr(stream)))
-        out["total_iters"] = int(total.value)
-        return out
+        return self._closed_loop(2, x_init, steps, A, B, C, None, dm, x_ref, dt, l1, warm_start, xhat_init, dhat_init,
+                                 d_plant, want_traj, want_inputs, want_dhat, noise, monitor, stream)

@@ -6,7 +6,7 @@
 // the state itself for state feedback, then one condensed QP per run (lib/mpc.py:461-478 / :318-335).  A run whose QP is
 // infeasible stops there, as the reference raises OutsideTheRegionOfAttractionError.
 //
-// The disturbance mode (carmpc_closed_loop_disturbance) is the controller for constant disturbances
+// The disturbance mode (mode 2) is the controller for constant disturbances
 // (MPCOutputFBWithDisturbance): the plant gets a constant per-run disturbance d_r after its Euler step (Bd_p d_r) and in
 // its output (Cd_p d_r); the augmented observer keeps a scalar estimate d^ beside x^,
 //     i = y - C x^ - Cd d^ ,   x^' = A x^ + Bd d^ + B u_prev + L1 i ,   d^' = d^ + L2 . i ,
@@ -16,13 +16,13 @@
 // One thread per run for plant + observer (4 state and 2 input registers); the QPs of all live runs go through the
 // batched solver with the previous step's ADMM state as warm start.
 //
-// Noise and monitor (carmpc_closed_loop_stochastic, any mode): process noise Lw z_w is added to the plant state after
+// Noise and monitor (any mode): process noise Lw z_w is added to the plant state after
 // the Euler step (and after Bd_p d_r), the state is then checked against the caller's rows [a | b] with the membership
 // chain of K1 (a violation never stops a run), and measurement noise Lv z_v enters what the controller sees.  z_w, z_v
 // are four standard normals each from Philox4x64-10 (philox.cuh) at counter (first_run + run, step, 0 / 1, 0), key
 // (seed, 0): they depend on nothing but the global run id and the step, so warm-start mode, graph replay and batch
-// composition draw the same noise.  Both are compile-time switches of loop_advance_kernel: with both off it is the
-// code the two deterministic entry points always ran.
+// composition draw the same noise.  Both are compile-time switches of loop_advance_kernel: with both off it has none of
+// their code.
 #include <math.h>
 #include <string.h>
 
@@ -437,83 +437,13 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
 using namespace carmpc;
 
 extern "C" int carmpc_closed_loop(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C,
-                                  const double* h_L, const double* h_xref, double dt, double l1, int steps,
-                                  int warm_start, const double* d_x_init, const double* d_xhat_init, int64_t runs,
-                                  double* d_final, int32_t* d_fail_step, double* d_traj, double* d_u_log,
-                                  int64_t* h_total_iters, void* stream) {
-    QPHandle* q = check_handle<QPHandle>(qp, kQP);
-    CARMPC_REQUIRE(q != nullptr, "not a QP handle");
-    CARMPC_REQUIRE(mode == 0 || mode == 1, "mode must be 0 (state feedback) or 1 (output feedback)");
-    CARMPC_REQUIRE(h_A && h_B && h_xref, "null model pointer");
-    CARMPC_REQUIRE(mode == 0 || (h_C && h_L), "output feedback needs C and L");
-    CARMPC_REQUIRE(steps >= 0 && runs >= 0 && runs < (int64_t)1 << 31, "steps / runs");
-    CARMPC_REQUIRE(warm_start >= 0 && warm_start <= 2, "warm_start must be 0, 1 or 2");
-    CARMPC_REQUIRE(dt > 0 && l1 > 0, "dt, l1");
-    if (h_total_iters) *h_total_iters = 0;
-    if (runs == 0) return CARMPC_OK;
-    CARMPC_REQUIRE(d_x_init && d_final && d_fail_step, "null device pointer");
-    LoopConst K;
-    memset(&K, 0, sizeof(K));
-    memcpy(K.A, h_A, sizeof(K.A));
-    memcpy(K.B, h_B, sizeof(K.B));
-    if (h_C) memcpy(K.C, h_C, sizeof(K.C));
-    if (h_L) memcpy(K.L, h_L, sizeof(K.L));
-    K.dt = dt; K.l1 = l1; K.mode = mode;
-    const LoopDisturbance none = {nullptr, nullptr, nullptr, nullptr};
-    const LoopStochastic off = {nullptr, nullptr, 0, nullptr, nullptr, nullptr};
-    return closed_loop_run(q, K, h_xref, steps, warm_start, d_x_init, d_xhat_init, runs, d_final, d_fail_step, d_traj, d_u_log,
-                           none, off, h_total_iters, stream);
-}
-
-extern "C" int carmpc_closed_loop_disturbance(void* qp, const double* h_A, const double* h_B, const double* h_C,
-                                              const carmpc_disturbance_model* dm, const double* h_xref, double dt, double l1,
-                                              int steps, int warm_start, const double* d_x_init, const double* d_xhat_init,
-                                              const double* d_dhat_init, const double* d_d_plant, int64_t runs,
-                                              double* d_final, double* d_dhat_final, int32_t* d_fail_step, double* d_traj,
-                                              double* d_u_log, double* d_dhat_log, int64_t* h_total_iters, void* stream) {
-    QPHandle* q = check_handle<QPHandle>(qp, kQP);
-    CARMPC_REQUIRE(q != nullptr, "not a QP handle");
-    CARMPC_REQUIRE(h_A && h_B && h_C && h_xref, "null model pointer");
-    CARMPC_REQUIRE(dm != nullptr, "null disturbance model");
-    CARMPC_REQUIRE(steps >= 0 && runs >= 0 && runs < (int64_t)1 << 31, "steps / runs");
-    CARMPC_REQUIRE(warm_start >= 0 && warm_start <= 2, "warm_start must be 0, 1 or 2");
-    CARMPC_REQUIRE(dt > 0 && l1 > 0, "dt, l1");
-    bool finite = true;
-    const double* gains[] = {dm->Bd, dm->Cd, dm->L1, dm->L2, dm->Bd_plant, dm->Cd_plant};
-    const int counts[] = {4, 3, 12, 3, 4, 3};
-    for (int g = 0; g < 6; ++g)
-        for (int j = 0; j < counts[g]; ++j) finite = finite && isfinite(gains[g][j]);
-    CARMPC_REQUIRE(finite, "disturbance model and observer gains must be finite");
-    if (h_total_iters) *h_total_iters = 0;
-    if (runs == 0) return CARMPC_OK;
-    CARMPC_REQUIRE(d_x_init && d_final && d_fail_step, "null device pointer");
-    LoopConst K;
-    memset(&K, 0, sizeof(K));
-    memcpy(K.A, h_A, sizeof(K.A));
-    memcpy(K.B, h_B, sizeof(K.B));
-    memcpy(K.C, h_C, sizeof(K.C));
-    memcpy(K.L, dm->L1, sizeof(K.L));
-    memcpy(K.Bd, dm->Bd, sizeof(K.Bd));
-    memcpy(K.Cd, dm->Cd, sizeof(K.Cd));
-    memcpy(K.L2, dm->L2, sizeof(K.L2));
-    memcpy(K.Bdp, dm->Bd_plant, sizeof(K.Bdp));
-    memcpy(K.Cdp, dm->Cd_plant, sizeof(K.Cdp));
-    K.dt = dt; K.l1 = l1; K.mode = 2;
-    const LoopDisturbance D = {d_dhat_init, d_d_plant, d_dhat_final, d_dhat_log};
-    const LoopStochastic off = {nullptr, nullptr, 0, nullptr, nullptr, nullptr};
-    return closed_loop_run(q, K, h_xref, steps, warm_start, d_x_init, d_xhat_init, runs, d_final, d_fail_step, d_traj, d_u_log,
-                           D, off, h_total_iters, stream);
-}
-
-extern "C" int carmpc_closed_loop_stochastic(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C,
-                                             const double* h_L, const carmpc_disturbance_model* dm, const double* h_xref,
-                                             double dt, double l1, int steps, int warm_start, const double* d_x_init,
-                                             const double* d_xhat_init, const double* d_dhat_init, const double* d_d_plant,
-                                             int64_t runs, double* d_final, double* d_dhat_final, int32_t* d_fail_step,
-                                             double* d_traj, double* d_u_log, double* d_dhat_log,
-                                             const carmpc_loop_noise* noise, const double* h_monitor_Ab, int monitor_rows,
-                                             int32_t* d_violation_step, int32_t* d_violation_row,
-                                             int32_t* d_violations_per_step, int64_t* h_total_iters, void* stream) {
+                                  const double* h_L, const carmpc_disturbance_model* dm, const double* h_xref, double dt,
+                                  double l1, int steps, int warm_start, const double* d_x_init, const double* d_xhat_init,
+                                  const double* d_dhat_init, const double* d_d_plant, int64_t runs, double* d_final,
+                                  double* d_dhat_final, int32_t* d_fail_step, double* d_traj, double* d_u_log,
+                                  double* d_dhat_log, const carmpc_loop_noise* noise, const double* h_monitor_Ab,
+                                  int monitor_rows, int32_t* d_violation_step, int32_t* d_violation_row,
+                                  int32_t* d_violations_per_step, int64_t* h_total_iters, void* stream) {
     QPHandle* q = check_handle<QPHandle>(qp, kQP);
     CARMPC_REQUIRE(q != nullptr, "not a QP handle");
     CARMPC_REQUIRE(mode >= 0 && mode <= 2, "mode must be 0 (state feedback), 1 (output feedback) or 2 (with a disturbance estimate)");

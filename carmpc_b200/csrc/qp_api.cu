@@ -393,7 +393,7 @@ int QPHandle::solve_enqueue(const SolveRequest& r, cudaStream_t st) {
 
 int QPHandle::solve_seeded(const SolveRequest& r, cudaStream_t st, SolveCounts* counts) {
     if (host_only) { set_error("carmpc_qp: this handle was created without a CUDA device; there is no CPU solver"); return CARMPC_ERR_CUDA; }
-    if (!host.opts.polish) { set_error("carmpc_qp_solve_seeded needs the float64 polish (opts.polish = 1)"); return CARMPC_ERR_INVALID; }
+    if (!host.opts.polish) { set_error("carmpc_qp_solve with seeds needs the float64 polish (opts.polish = 1)"); return CARMPC_ERR_INVALID; }
     const int64_t batch = r.stride;
     int rc = ensure_workspace(batch);
     if (rc != CARMPC_OK) return rc;
@@ -632,65 +632,30 @@ int carmpc_qp_get_setup(void* qp, int which, double* h_out, int capacity) {
     return cnt;
 }
 
-int carmpc_qp_solve_batch(void* qp, const double* d_x0, const double* h_xref, const double* d_c, int64_t batch,
-                          double* d_u0, double* d_objective, int32_t* d_status, int32_t* d_iters, double* d_u_full,
-                          float* d_warm, int warm_in, int warm_out, void* stream) {
+int carmpc_qp_solve(void* qp, const double* d_x0, const double* h_xref, const double* d_c, const int32_t* d_seed,
+                    int64_t batch, double* d_u0, double* d_objective, int32_t* d_status, int32_t* d_iters, double* d_u_full,
+                    float* d_warm, int warm_in, int warm_out, double* d_cert, int64_t* h_seeded, void* stream) {
     QPHandle* q = check_handle<QPHandle>(qp, kQP);
     CARMPC_REQUIRE(q != nullptr, "not a QP handle");
     CARMPC_REQUIRE(batch >= 0 && batch < (int64_t)1 << 31, "batch");
     CARMPC_REQUIRE(h_xref != nullptr, "h_xref");
+    CARMPC_REQUIRE(d_warm == nullptr || (d_seed == nullptr && d_cert == nullptr),
+                   "d_warm is a starting point of its own: it cannot be combined with d_seed or d_cert");
+    CARMPC_REQUIRE(q->host.opts.polish != 0 || (d_seed == nullptr && d_cert == nullptr),
+                   "seeds and certificates need the float64 polish (opts.polish = 1)");
+    if (h_seeded) *h_seeded = 0;
     if (batch == 0) { q->last_total_iters = 0; q->last_launches = 0; return CARMPC_OK; }
     CARMPC_REQUIRE(d_x0 && d_status, "d_x0 and d_status are required");
-    QPBusyGuard guard(q->busy);
-    CARMPC_REQUIRE(guard.acquired, "this QP handle is in use by another call (one call per handle at a time)");
-    SolveRequest r;
-    r.x0 = d_x0; r.stride = r.count = batch; r.xref = h_xref; r.c = d_c;
-    r.u0 = d_u0; r.objective = d_objective; r.status = d_status; r.iters = d_iters; r.u_full = d_u_full;
-    r.warm = d_warm; r.warm_in = warm_in; r.warm_out = warm_out;
-    return q->solve(r, (cudaStream_t)stream);
-}
-
-int carmpc_qp_solve_seeded(void* qp, const double* d_x0, const double* h_xref, const double* d_c, const int32_t* d_seed,
-                           int64_t batch, double* d_u0, double* d_objective, int32_t* d_status, int32_t* d_iters,
-                           double* d_u_full, int64_t* h_seeded, void* stream) {
-    QPHandle* q = check_handle<QPHandle>(qp, kQP);
-    CARMPC_REQUIRE(q != nullptr, "not a QP handle");
-    CARMPC_REQUIRE(batch >= 0 && batch < (int64_t)1 << 31, "batch");
-    CARMPC_REQUIRE(h_xref != nullptr, "h_xref");
-    if (h_seeded) *h_seeded = 0;
-    if (batch == 0) { q->last_total_iters = 0; q->last_launches = 0; return CARMPC_OK; }
-    CARMPC_REQUIRE(d_x0 && d_status && d_seed, "d_x0, d_status and d_seed are required");
-    QPBusyGuard guard(q->busy);
-    CARMPC_REQUIRE(guard.acquired, "this QP handle is in use by another call (one call per handle at a time)");
-    SolveRequest r;
-    r.x0 = d_x0; r.stride = r.count = batch; r.xref = h_xref; r.c = d_c; r.seed = d_seed;
-    r.u0 = d_u0; r.objective = d_objective; r.status = d_status; r.iters = d_iters; r.u_full = d_u_full;
-    SolveCounts k;
-    const int rc = q->solve_seeded(r, (cudaStream_t)stream, &k);
-    if (rc == CARMPC_OK && h_seeded) *h_seeded = k.reused;
-    return rc;
-}
-
-int carmpc_qp_solve_certified(void* qp, const double* d_x0, const double* h_xref, const double* d_c, const int32_t* d_seed,
-                              int64_t batch, double* d_u0, double* d_objective, int32_t* d_status, int32_t* d_iters,
-                              double* d_u_full, double* d_cert, int64_t* h_seeded, void* stream) {
-    QPHandle* q = check_handle<QPHandle>(qp, kQP);
-    CARMPC_REQUIRE(q != nullptr, "not a QP handle");
-    CARMPC_REQUIRE(batch >= 0 && batch < (int64_t)1 << 31, "batch");
-    CARMPC_REQUIRE(h_xref != nullptr, "h_xref");
-    CARMPC_REQUIRE(q->host.opts.polish != 0, "certificates come from the float64 polish (opts.polish = 1)");
-    if (h_seeded) *h_seeded = 0;
-    if (batch == 0) { q->last_total_iters = 0; q->last_launches = 0; return CARMPC_OK; }
-    CARMPC_REQUIRE(d_x0 && d_status && d_cert, "d_x0, d_status and d_cert are required");
     QPBusyGuard guard(q->busy);
     CARMPC_REQUIRE(guard.acquired, "this QP handle is in use by another call (one call per handle at a time)");
     if (q->host_only) { set_error("carmpc_qp: this handle was created without a CUDA device; there is no CPU solver"); return CARMPC_ERR_CUDA; }
     cudaStream_t st = (cudaStream_t)stream;
     const size_t width = (size_t)q->host.m + q->host.n + q->host.kpre;
-    CARMPC_CUDA(cudaMemsetAsync(d_cert, 0, sizeof(double) * width * batch, st));
+    if (d_cert) CARMPC_CUDA(cudaMemsetAsync(d_cert, 0, sizeof(double) * width * batch, st));
     SolveRequest r;
     r.x0 = d_x0; r.stride = r.count = batch; r.xref = h_xref; r.c = d_c; r.seed = d_seed;
     r.u0 = d_u0; r.objective = d_objective; r.status = d_status; r.iters = d_iters; r.u_full = d_u_full; r.cert = d_cert;
+    r.warm = d_warm; r.warm_in = warm_in; r.warm_out = warm_out;
     if (d_seed == nullptr) return q->solve(r, st);
     SolveCounts k;
     const int rc = q->solve_seeded(r, st, &k);

@@ -213,7 +213,7 @@ struct PolishBatch {
     double* rec_lam;         // [records][32][5]
     int* rec_act;            // [records][33]   na (-1: no map), then the active rows in the order of Lam's rows
     int rec_write, rec_read;
-    double* cert;            // nullable [batch][mt + kpre]: multipliers of certified samples (carmpc_qp_solve_certified)
+    double* cert;            // nullable [batch][mt + kpre]: multipliers of certified samples (carmpc_qp_solve d_cert)
     unsigned long long* stats;   // nullable [20]: [r] samples certified after r repair rounds (r = 0..9), [10] not certified,
                                  // [11] round 0 taken from a multiplier map, [12] certified by a multiplier map alone,
                                  // [13] proven infeasible by the anchor's Farkas certificate (or the u-independent rows),
@@ -351,7 +351,7 @@ int sensitivity_launch(QPHandle* q, const double* d_x0, const double* d_c, int64
                        const double* d_u_full, const double* d_cert, int rows, double* d_jac, double* d_grad,
                        int32_t* d_flags, cudaStream_t st);
 
-// Certificate rows (carmpc_qp_solve_certified) are in the caller's orientation: entry i of a general row the setup negated
+// Certificate rows (carmpc_qp_solve d_cert) are in the caller's orientation: entry i of a general row the setup negated
 // changes sign, so that positive always means "against the upper bound" of the row as passed to carmpc_qp_create.
 // A violated u-independent row is an infeasibility proof by itself: y = +1 (above pre_hi) or -1 (below pre_lo) on the
 // first such row, zeros elsewhere (its G part is zero).  A non-finite state has no certificate: the row stays zero.

@@ -1,6 +1,6 @@
 // Derivatives of certified QP solutions with respect to the initial state and the disturbance (carmpc_qp_sensitivity).
 //
-// A solved sample's certificate row y (carmpc_qp_solve_certified) names its active rows S = {i : y_i != 0} among the m
+// A solved sample's certificate row y (carmpc_qp_solve d_cert) names its active rows S = {i : y_i != 0} among the m
 // general and n box rows, A = [G; I].  On the critical region of S the solution is affine in p = (x0, c):
 //       M lambda = AUu_S (x0 - xref) + Gx_S x0 + Gc_S c - b_S ,   u = Uu (x0 - xref) - AH_S' lambda ,   M = A_S H^-1 A_S'
 // hence (box rows: Gx = Gc = 0)

@@ -2,7 +2,7 @@
 
 ``LoopNoise`` describes the process and measurement noise of ``BatchQP.closed_loop(..., noise=...)`` and
 ``BatchQP.closed_loop_disturbance(..., noise=...)``; ``plant_rows`` gives a controller's own state rows as a monitor for
-the ``monitor=`` argument of the same calls.  The noise is drawn on the device (``carmpc_closed_loop_stochastic``,
+the ``monitor=`` argument of the same calls.  The noise is drawn on the device (``carmpc_closed_loop``,
 Philox4x64-10 at counter (first_run + run, step, 0 / 1, 0), key (seed, 0)), so it depends only on the seed, the global run
 id and the step: a run set split over calls or GPUs with ``first_run`` offsets draws what one call would.
 """

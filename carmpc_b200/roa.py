@@ -46,7 +46,7 @@ def feasibility_map(controller, axes: Sequence[np.ndarray], x_ref=None, batch_so
     """Feasibility flag of every point of the tensor grid ``axes`` (C order, x slowest ... v fastest): True where the
     controller's QP is feasible.  Solved on the GPU (no CPU fallback).  ``seeded`` (default) solves only a sub-lattice
     of anchors cold and certifies every other point from its anchor's active set / Farkas certificate
-    (``carmpc_qp_solve_seeded``: same flags, 1.7 - 4.6 x faster on 10^6-point maps).
+    (``carmpc_qp_solve`` with seeds: same flags, 1.7 - 4.6 x faster on 10^6-point maps).
 
     Every True is backed by a float64 KKT certificate and every False by a float64 Farkas certificate.  A point the
     solver could prove neither way (status 2: degenerate states within ~1e-7 of the boundary of the region) is not

@@ -228,53 +228,46 @@ int carmpc_qp_get_setup(void* qp, int which, double* h_out, int capacity);
  *   d_status    batch int32 (CARMPC_QP_*)
  *   d_iters     batch int32
  *   d_u_full    batch x n float64, row-major per sample (u_horizon of the reference)
- * d_warm (nullable): batch x (m + n) float32 solver state, read if warm_in != 0, written if warm_out != 0.
+ * Three optional uses, each selected by its pointer (all NULL: every sample cold):
+ *   d_warm   batch x (m + n) float32 solver state, read if warm_in != 0, written if warm_out != 0.
+ *   d_seed   region-of-attraction maps (the grid search of the reference's paper section III-E: lib/mpc.py:318-338
+ *            evaluated on a grid of initial states): neighbouring states mostly share their active set, so only a
+ *            sub-lattice of "anchor" samples is solved cold (ADMM + polish); every other sample i first tries the
+ *            certified active set of its anchor d_seed[i] in the float64 polish (one Schur-complement solve + KKT
+ *            certificate, repaired a few rounds) and runs ADMM iterations only if that does not certify (set too
+ *            different, or outside the region of attraction).  batch int32; d_seed[i] == i (or out of range) marks an
+ *            anchor; a follower's seed must be an anchor.  Results are the same certified optima / infeasibility flags
+ *            as the cold solve, whatever the seeds are.
+ *   d_cert   the certificate behind every verdict, with the same other results as the solve without it (cold or
+ *            seeded).  batch x (m + n + k) float64, row-major per sample, in the row space of the handle: the m general
+ *            rows, the n box rows and the k u-independent rows exactly as passed to carmpc_qp_create.  Positive means
+ *            "against the upper bound", negative "against the lower bound".
+ *     CARMPC_QP_SOLVED      the multipliers of the float64 KKT certificate: H u + F (x0 - xref) + G' lam_g + lam_b = 0,
+ *                           non-zero only on rows the polish certified as active; zero on the k rows.
+ *     CARMPC_QP_INFEASIBLE  the Farkas ray y the library checked: G' y_g + y_b = 0 and the support value
+ *                           sum_i (y_i+ hi_i(x0, c) - y_i- lo_i(x0, c)) over all m + n + k rows is negative.  A violated
+ *                           u-independent row is y = +-1 on that row.  A non-finite state has no certificate (zero row).
+ *     CARMPC_QP_MAX_ITER    zeros.
+ * h_seeded (nullable): number of samples certified from their seed without any ADMM iteration (0 without d_seed).
+ * CARMPC_ERR_INVALID for d_warm together with d_seed or d_cert, and for d_seed or d_cert on a handle with
+ * opts.polish == 0 (seeds and certificates come from the polish); CARMPC_ERR_CUDA on a handle created without a device.
  * The call synchronises `stream` (it reads back how many samples need the second, tighter pass). */
-int carmpc_qp_solve_batch(void* qp, const double* d_x0, const double* h_xref, const double* d_c,
-                          int64_t batch, double* d_u0, double* d_objective, int32_t* d_status,
-                          int32_t* d_iters, double* d_u_full, float* d_warm, int warm_in, int warm_out,
-                          void* stream);
-
-/* Region-of-attraction maps (the grid search of the reference's paper section III-E: lib/mpc.py:318-338 evaluated
- * on a grid of initial states): neighbouring states mostly share their active set, so only a sub-lattice of
- * "anchor" samples is solved cold (ADMM + polish); every other sample i first tries the certified active set of its
- * anchor d_seed[i] in the float64 polish (one Schur-complement solve + KKT certificate, repaired a few rounds) and
- * runs ADMM iterations only if that does not certify (set too different, or outside the region of attraction).
- * d_seed: batch int32; d_seed[i] == i (or out of range) marks an anchor; a follower's seed must be an anchor.
- * Results are the same certified optima / infeasibility flags as carmpc_qp_solve_batch, whatever the seeds are.
- * h_seeded (nullable): number of samples certified from their seed without any ADMM iteration. */
-int carmpc_qp_solve_seeded(void* qp, const double* d_x0, const double* h_xref, const double* d_c,
-                           const int32_t* d_seed, int64_t batch, double* d_u0, double* d_objective,
-                           int32_t* d_status, int32_t* d_iters, double* d_u_full, int64_t* h_seeded,
-                           void* stream);
+int carmpc_qp_solve(void* qp, const double* d_x0, const double* h_xref, const double* d_c, const int32_t* d_seed,
+                    int64_t batch, double* d_u0, double* d_objective, int32_t* d_status, int32_t* d_iters,
+                    double* d_u_full, float* d_warm, int warm_in, int warm_out, double* d_cert, int64_t* h_seeded,
+                    void* stream);
 
 /* Region-of-attraction map from the host: the states are the C-order tensor grid of four axes (h_axes: the axes
  * concatenated, dims[k] points each, 1..4096; axis k is state component axis_to_state[k]), expanded on the device.
  * block (nullable = every point cold): points per axis of the lattice blocks whose centre points are the anchors
- * of carmpc_qp_solve_seeded.  Outputs as carmpc_qp_solve_host (h_u0 batch x 2 row-major, any may be NULL except
+ * of the seeded carmpc_qp_solve.  Outputs as carmpc_qp_solve_host (h_u0 batch x 2 row-major, any may be NULL except
  * h_status); batch = dims[0] dims[1] dims[2] dims[3].  This is the sampled counterpart of the reference's exact
  * but impractical projection lib/in_adm_set.py:4-77 ("grid search" of the paper, section III-E). */
 int carmpc_qp_map_host(void* qp, const double* h_axes, const int32_t dims[4], const int32_t axis_to_state[4],
                        const int32_t block[4], const double* h_xref, double* h_u0, double* h_objective,
                        int32_t* h_status, int32_t* h_iters, int64_t* h_seeded);
 
-/* carmpc_qp_solve_batch (d_seed == NULL: cold, no warm state) or carmpc_qp_solve_seeded (d_seed != NULL), with the same
- * results, that also exports the certificate behind every verdict.  d_cert: batch x (m + n + k) float64, row-major per
- * sample, in the row space of the handle: the m general rows, the n box rows and the k u-independent rows exactly as
- * passed to carmpc_qp_create.  Positive means "against the upper bound", negative "against the lower bound".
- *   CARMPC_QP_SOLVED      the multipliers of the float64 KKT certificate: H u + F (x0 - xref) + G' lam_g + lam_b = 0,
- *                         non-zero only on rows the polish certified as active; zero on the k rows.
- *   CARMPC_QP_INFEASIBLE  the Farkas ray y the library checked: G' y_g + y_b = 0 and the support value
- *                         sum_i (y_i+ hi_i(x0, c) - y_i- lo_i(x0, c)) over all m + n + k rows is negative.  A violated
- *                         u-independent row is y = +-1 on that row.  A non-finite state has no certificate (zero row).
- *   CARMPC_QP_MAX_ITER    zeros.
- * Returns CARMPC_ERR_INVALID when the handle has opts.polish == 0 (no certificate without the polish). */
-int carmpc_qp_solve_certified(void* qp, const double* d_x0, const double* h_xref, const double* d_c,
-                              const int32_t* d_seed, int64_t batch, double* d_u0, double* d_objective,
-                              int32_t* d_status, int32_t* d_iters, double* d_u_full, double* d_cert,
-                              int64_t* h_seeded, void* stream);
-
-/* Derivatives of certified solutions (carmpc_qp_solve_certified outputs) w.r.t. p = (x, y, psi, v, c): the state and
+/* Derivatives of certified solutions (carmpc_qp_solve outputs with d_cert) w.r.t. p = (x, y, psi, v, c): the state and
  * the per-sample disturbance (its column is zero for a handle without Gc).  A solved sample's certificate row names its
  * active rows S; on the critical region of S the optimal u is affine in p (explicit MPC), and
  *   d_jac       batch x rows x 5 float64 (nullable): du_r/dp_k for the leading `rows` variables (1 <= rows <= n; rows = 2
@@ -302,7 +295,7 @@ int carmpc_qp_checker_create(int n, int R, const double* h_H, const double* h_F,
                              const double* h_lb, const double* h_ub, void** handle);
 
 /* Checks one certificate row per sample (d_cert: batch x (R + n), general rows then box, sign convention of
- * carmpc_qp_solve_certified) against d_status / d_u_full (batch x n).  d_x0: SoA 4 x batch; d_c nullable.
+ * carmpc_qp_solve's d_cert) against d_status / d_u_full (batch x n).  d_x0: SoA 4 x batch; d_c nullable.
  * d_resid: batch x 4 float64.  Status 0: [primal violation, stationarity, multiplier against an infinite bound,
  * complementarity], all relative (qp_check.cu states the scales).  Status 1: [support value of the ray with its box part
  * completed as -G'y_g, its rounding scale, |G'y_g + y_b|_inf of the given box part relative to max_j sum_i |G_ij y_i|,
@@ -349,70 +342,50 @@ int carmpc_qp_tensor_mode(void* qp, int mode, int64_t* h_info);
 
 /* ------------------------------------------------------------------------------------------------
  * Monte-Carlo closed loop against the nonlinear bicycle (lib/simulator.py:51-69), in the order of
- * examples/run_MPCOutputFB.py:29-41: plant step with the previous input (first [0,0]), observer
- * update (mode 1, lib/mpc.py:448) or direct state (mode 0), QP, repeat.
+ * examples/run_MPCOutputFB.py:29-41.  Step k of a run still running at the start of step k:
+ *   s = s + dt * f(s, u_prev)  (u_prev = [0, 0] at the first step);   mode 2: s = s + Bd_plant * d_r;
+ *   s = s + Lw z_w  (process noise)
+ *   s is stored to d_final / d_traj, then checked against the monitor rows [a | b]: fma(a3, v, fma(a2, psi, fma(a1, y,
+ *   a0 * x))) <= b for every row (the chain of carmpc_membership_bitset mode 0; a non-finite state violates)
+ *   v = Lv z_v  (measurement noise), then the controller:
+ *   mode 0  state feedback: the QP at x0 = s + v[0..3];
+ *   mode 1  output feedback (lib/mpc.py:448): y = C s + v[0..2],  x^' = A x^ + B u_prev + L (y - C x^),  QP at x0 = x^';
+ *   mode 2  the disturbance-estimating controller (MPCOutputFBWithDisturbance, lib/mpc.py:329-396), with a constant
+ *           scalar disturbance d_r per run and an augmented observer:  y = C s + Cd_plant d_r + v[0..2],
+ *           i = y - C x^ - Cd d^,  x^' = A x^ + Bd d^ + B u_prev + L1 i,  d^' = d^ + L2 . i;
+ *           QP at x0 = x^', c = d^' (bounds shifted by Gc c).  The QP handle's Gc must describe the same Bd
+ *           (BatchQP.from_controller of a controller with that Bd); a handle whose Gc is zero is allowed (c then has no
+ *           effect).  "Infeasible" verdicts carry a float64 certificate of the disturbance-shifted problem; a non-finite
+ *           d^ or state of one run makes that run's QP infeasible.
+ * A run whose QP is infeasible or undecided at step k stops there (the reference raises) and keeps its state.
  *   h_A (4x4), h_B (4x2), h_C (3x4), h_L (4x3) row-major; dt, l1 as in the reference (0.2, 3.5).
- *   d_x_init, d_xhat_init: SoA 4 x runs.  d_final: SoA 4 x runs.  d_fail_step: int32, -1 = none.
+ *   mode 0: h_C, h_L ignored;  mode 1: h_C, h_L;  mode 2: h_C and dm (h_L ignored).
+ *   d_x_init, d_xhat_init (nullable: x_init): SoA 4 x runs.  d_final: SoA 4 x runs.  d_fail_step: int32, -1 = none.
  *   d_traj (nullable): steps x 4 x runs float64.  d_u_log (nullable): steps x 2 x runs.
- * A run whose QP is infeasible at step t stops there (the reference raises) and keeps its state.
+ *   mode 2 only: dm: model and gains (L1 4x3 row-major).  d_dhat_init (nullable: 0), d_d_plant (nullable: 0, the
+ *   per-run d_r), d_dhat_final (nullable): runs float64.  d_dhat_log (nullable): steps x runs, d^ the QP of each step used.
  * warm_start: 0 = every QP cold; 1 = the previous step's certified active set / ADMM state is reused and the steps are
  * only enqueued (every sample count stays on the device, no host synchronisation inside the loop); 2 = the same reuse
- * with host-sized launches (three count read-backs per step: the round-1 form, kept to time one against the other). */
-int carmpc_closed_loop(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C,
-                       const double* h_L, const double* h_xref, double dt, double l1, int steps, int warm_start,
-                       const double* d_x_init, const double* d_xhat_init, int64_t runs, double* d_final,
-                       int32_t* d_fail_step, double* d_traj, double* d_u_log, int64_t* h_total_iters,
-                       void* stream);
-
-/* Closed loops of the disturbance-estimating output-feedback controller (MPCOutputFBWithDisturbance, lib/mpc.py:329-396):
- * the same loop, with a constant scalar disturbance per run and an augmented observer.  Step k of a run:
- *   s  = s + dt * f(s, u_prev);   s = s + Bd_plant * d_r          (plant: Euler step, then the true disturbance)
- *   y  = C s + Cd_plant * d_r
- *   i  = y - C x^ - Cd d^;   x^' = A x^ + Bd d^ + B u_prev + L1 i;   d^' = d^ + L2 . i
- *   QP at x0 = x^', c = d^' (bounds shifted by Gc c), x_ref = h_xref
- * The QP handle's Gc must describe the same Bd (BatchQP.from_controller of a controller with that Bd); a handle whose Gc
- * is zero is allowed (c then has no effect).  Infeasible or undecided QPs stop the run (d_fail_step), as in
- * carmpc_closed_loop; "infeasible" verdicts carry a float64 certificate of the disturbance-shifted problem.
- * Non-finite gains are rejected; a non-finite d^ or state of one run makes that run's QP infeasible.
- *   dm: model and gains (L1 4x3 row-major).  d_x_init, d_xhat_init (nullable: x_init): SoA 4 x runs.
- *   d_dhat_init (nullable: 0), d_d_plant (nullable: 0, the per-run d_r), d_dhat_final (nullable): runs float64.
- *   d_traj, d_u_log as in carmpc_closed_loop; d_dhat_log (nullable): steps x runs, d^ the QP of each step used.
- * warm_start 0 / 1 / 2 as in carmpc_closed_loop. */
+ * with host-sized launches (three count read-backs per step: the round-1 form, kept to time one against the other).
+ * noise (nullable: no noise).  z_w, z_v: four standard normals each.  Philox4x64-10 with key (seed, 0) at counter
+ * (first_run + run, k, j, 0), j = 0 for z_w and 1 for z_v, gives words x0..x3; (x0, x1) and (x2, x3) each give two
+ * normals by Box-Muller:
+ *   ua = ((x0 >> 11) + 1) 2^-53,  ub = (x1 >> 11) 2^-53,  z0 = sqrt(-2 ln ua) cos(2 pi ub),  z1 = ... sin(2 pi ub).
+ * The draws depend only on (seed, first_run + run, k, j): not on the batch, warm_start or which runs still run, so a run
+ * set split over calls (first_run = the offset of each part) draws what one call would.
+ * h_monitor_Ab (nullable: no monitor): host rows x 5, 1 <= monitor_rows <= 512, finite.  A violation never stops a run.
+ * The monitor outputs are nullable and need rows: d_violation_step / d_violation_row (runs int32, -1 none): the first
+ * step with a violation and the lowest violated row (caller's order) at that step.  d_violations_per_step (steps
+ * int32): runs violating at step k.  Stopped runs are neither moved nor counted; a run whose QP fails at step k was
+ * moved and checked at step k.
+ * Noise and monitor are compile-time switches of the step kernel: a loop without them pays nothing for them.
+ * CARMPC_ERR_INVALID for non-finite factors or gains, first_run < 0, bad monitor rows, monitor outputs without rows, mode
+ * 2 without dm; CARMPC_ERR_CUDA on a handle created without a device. */
 typedef struct carmpc_disturbance_model {
     double Bd[4], Cd[3], L1[12], L2[3];   /* controller: disturbance model and observer gains (L1 4x3 row-major) */
     double Bd_plant[4], Cd_plant[3];      /* how the true per-run disturbance enters the plant state / output    */
 } carmpc_disturbance_model;
 
-int carmpc_closed_loop_disturbance(void* qp, const double* h_A, const double* h_B, const double* h_C,
-                                   const carmpc_disturbance_model* dm, const double* h_xref, double dt, double l1,
-                                   int steps, int warm_start, const double* d_x_init, const double* d_xhat_init,
-                                   const double* d_dhat_init, const double* d_d_plant, int64_t runs, double* d_final,
-                                   double* d_dhat_final, int32_t* d_fail_step, double* d_traj, double* d_u_log,
-                                   double* d_dhat_log, int64_t* h_total_iters, void* stream);
-
-/* Closed loops with random process and measurement noise, and a monitor of the true plant state (modes 0, 1, 2 of the two
- * functions above).  Step k of a run still running at the start of step k:
- *   s = s + dt * f(s, u_prev);   mode 2: s = s + Bd_plant * d_r;   s = s + Lw z_w      (process noise)
- *   s is stored to d_final / d_traj, then checked against the monitor rows [a | b]: fma(a3, v, fma(a2, psi, fma(a1, y,
- *   a0 * x))) <= b for every row (the chain of carmpc_membership_bitset mode 0; a non-finite state violates)
- *   v = Lv z_v;   mode 0: the QP sees s + v[0..3];  mode 1: y = C s + v[0..2];  mode 2: y = C s + Cd_plant d_r + v[0..2]
- *   observer and QP as in carmpc_closed_loop / carmpc_closed_loop_disturbance.
- * z_w, z_v: four standard normals each.  Philox4x64-10 with key (seed, 0) at counter (first_run + run, k, j, 0), j = 0
- * for z_w and 1 for z_v, gives words x0..x3; (x0, x1) and (x2, x3) each give two normals by Box-Muller:
- *   ua = ((x0 >> 11) + 1) 2^-53,  ub = (x1 >> 11) 2^-53,  z0 = sqrt(-2 ln ua) cos(2 pi ub),  z1 = ... sin(2 pi ub).
- * The draws depend only on (seed, first_run + run, k, j): not on the batch, warm_start or which runs still run, so a run
- * set split over calls (first_run = the offset of each part) draws what one call would.
- * A violation never stops a run.  d_violation_step / d_violation_row (runs int32, -1 none): the first step with a
- * violation and the lowest violated row (caller's order) at that step.  d_violations_per_step (steps int32): runs
- * violating at step k.  Stopped runs are neither moved nor counted; a run whose QP fails at step k was moved and checked
- * at step k.
- *   mode 0: h_C, h_L ignored;  mode 1: h_C, h_L (as carmpc_closed_loop);  mode 2: h_C and dm (h_L ignored).
- *   d_dhat_init, d_d_plant, d_dhat_final, d_dhat_log: mode 2 only (as carmpc_closed_loop_disturbance).
- *   noise (nullable: no noise).  h_monitor_Ab (nullable: no monitor): host rows x 5, 1 <= monitor_rows <= 512, finite;
- *   the monitor outputs are nullable and need rows.
- * With noise = NULL and no monitor the results are those of carmpc_closed_loop / carmpc_closed_loop_disturbance.
- * CARMPC_ERR_INVALID for non-finite factors or gains, first_run < 0, bad monitor rows, monitor outputs without rows, mode
- * 2 without dm; CARMPC_ERR_CUDA on a handle created without a device. */
 typedef struct carmpc_loop_noise {
     uint64_t seed;
     int64_t first_run;      /* global id of run 0 of this call */
@@ -420,14 +393,14 @@ typedef struct carmpc_loop_noise {
     double Lv[16];          /* measurement-noise factor, 4 x 4 row-major: v = Lv z_v */
 } carmpc_loop_noise;
 
-int carmpc_closed_loop_stochastic(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C,
-                                  const double* h_L, const carmpc_disturbance_model* dm, const double* h_xref, double dt,
-                                  double l1, int steps, int warm_start, const double* d_x_init, const double* d_xhat_init,
-                                  const double* d_dhat_init, const double* d_d_plant, int64_t runs, double* d_final,
-                                  double* d_dhat_final, int32_t* d_fail_step, double* d_traj, double* d_u_log,
-                                  double* d_dhat_log, const carmpc_loop_noise* noise, const double* h_monitor_Ab,
-                                  int monitor_rows, int32_t* d_violation_step, int32_t* d_violation_row,
-                                  int32_t* d_violations_per_step, int64_t* h_total_iters, void* stream);
+int carmpc_closed_loop(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C, const double* h_L,
+                       const carmpc_disturbance_model* dm, const double* h_xref, double dt, double l1, int steps,
+                       int warm_start, const double* d_x_init, const double* d_xhat_init, const double* d_dhat_init,
+                       const double* d_d_plant, int64_t runs, double* d_final, double* d_dhat_final,
+                       int32_t* d_fail_step, double* d_traj, double* d_u_log, double* d_dhat_log,
+                       const carmpc_loop_noise* noise, const double* h_monitor_Ab, int monitor_rows,
+                       int32_t* d_violation_step, int32_t* d_violation_row, int32_t* d_violations_per_step,
+                       int64_t* h_total_iters, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Device micro-benchmarks used as roofline denominators that MEASURED_PEAKS.json does not carry.

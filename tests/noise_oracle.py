@@ -1,4 +1,4 @@
-"""CPU restatement of the closed loops' noise (carmpc_closed_loop_stochastic): Philox4x64-10 and the Box-Muller step in
+"""CPU restatement of the closed loops' noise (carmpc_closed_loop): Philox4x64-10 and the Box-Muller step in
 numpy, and the noisy loop of the three modes with exact QPs, built on ``oracle/carmpc_oracle.py`` and
 ``tests/disturbance_oracle.py`` (both used unchanged).
 
@@ -70,7 +70,7 @@ def numpy_philox_block(counter, key):
 
 
 def noisy_closed_loop(mode, A, B, C, L, x_init, steps, solve, Lw, Lv, seed, first_run=0, dist=None, monitor=None):
-    """The loop of carmpc_closed_loop_stochastic for mode 0 (state feedback), 1 (output feedback, gain L) or 2
+    """The loop of carmpc_closed_loop for mode 0 (state feedback), 1 (output feedback, gain L) or 2
     (``dist`` = (Bd, Cd, L1, L2, Bd_plant, Cd_plant, d_plant)).  ``solve(x (B, 4), d (B,)) -> (u0 (B, 2), status)``.
     ``monitor``: (rows, 5) [A | b] checked with numpy's A @ s <= b.  Returns a dict of final, fail_step, traj (steps, R,
     4), inputs (steps, R, 2), dhat, dhat_traj and, with a monitor, violation_step, violation_row, violations_per_step."""

@@ -12,11 +12,11 @@ def _declared_functions():
     return sorted(set(re.findall(r"\b(carmpc_[a-z0-9_]+)\s*\(", src)))
 
 
-def test_header_declares_the_documented_surface():
+def test_header_declares_the_public_entry_points():
     names = _declared_functions()
     for must in ("carmpc_polytope_create", "carmpc_membership_bitset", "carmpc_membership_grid",
                  "carmpc_membership_bitset_host", "carmpc_rollout_create", "carmpc_rollout_bitset",
-                 "carmpc_qp_create", "carmpc_qp_solve_batch", "carmpc_qp_solve_host", "carmpc_closed_loop",
+                 "carmpc_qp_create", "carmpc_qp_solve", "carmpc_qp_solve_host", "carmpc_closed_loop",
                  "carmpc_destroy", "carmpc_last_error"):
         assert must in names
 

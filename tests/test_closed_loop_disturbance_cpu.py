@@ -1,6 +1,6 @@
 """Disturbance-estimating output feedback without a GPU: the oracle's augmented observer against the controller's own,
-the observer-gain helper (and the instability of the reference's gains), argument checks of
-carmpc_closed_loop_disturbance."""
+the observer-gain helper (and the instability of the reference's gains), argument checks of carmpc_closed_loop in
+mode 2."""
 import ctypes
 import math
 
@@ -78,10 +78,10 @@ def test_helper_gain_is_stable_and_the_reference_gain_is_not(ctl):
 def _call(lib, qp, dm, runs=4, steps=3, warm_start=1, dt=0.2, l1=3.5, A=True, ptr=16):
     mat = np.zeros(16)
     p = ctypes.c_void_p(ptr)
-    return lib.carmpc_closed_loop_disturbance(qp, mat.ctypes.data if A else None, mat.ctypes.data, mat.ctypes.data,
-                                              ctypes.byref(dm) if dm is not None else None, mat.ctypes.data, dt, l1,
-                                              steps, warm_start, p, None, None, None, runs, p, None, p, None, None, None,
-                                              None, None)
+    return lib.carmpc_closed_loop(qp, 2, mat.ctypes.data if A else None, mat.ctypes.data, mat.ctypes.data, None,
+                                  ctypes.byref(dm) if dm is not None else None, mat.ctypes.data, dt, l1, steps, warm_start,
+                                  p, None, None, None, runs, p, None, p, None, None, None, None, None, 0, None, None, None,
+                                  None, None)
 
 
 def _model():
@@ -93,7 +93,7 @@ def _model():
     return dm
 
 
-def test_entry_point_argument_errors(ctl):
+def test_closed_loop_mode_2_argument_errors(ctl):
     from carmpc_b200 import _capi
     from carmpc_b200.batch import BatchQP
     lib = _capi.load()
@@ -116,13 +116,13 @@ def test_entry_point_argument_errors(ctl):
     # no runs: nothing to do, whatever the pointers
     total = ctypes.c_int64(7)
     mat = np.zeros(16)
-    assert lib.carmpc_closed_loop_disturbance(bq._h, mat.ctypes.data, mat.ctypes.data, mat.ctypes.data, ctypes.byref(dm),
-                                              mat.ctypes.data, 0.2, 3.5, 5, 1, None, None, None, None, 0, None, None,
-                                              None, None, None, None, ctypes.byref(total), None) == 0
+    assert lib.carmpc_closed_loop(bq._h, 2, mat.ctypes.data, mat.ctypes.data, mat.ctypes.data, None, ctypes.byref(dm),
+                                  mat.ctypes.data, 0.2, 3.5, 5, 1, None, None, None, None, 0, None, None, None, None, None,
+                                  None, None, None, 0, None, None, None, ctypes.byref(total), None) == 0
     assert total.value == 0
 
 
-def test_host_only_handle_is_a_cuda_error(ctl):
+def test_closed_loop_mode_2_on_a_host_only_handle_is_a_cuda_error(ctl):
     """A handle created without a CUDA device keeps its host setup; the loop fails loudly instead of computing."""
     try:
         import torch

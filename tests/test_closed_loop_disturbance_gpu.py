@@ -1,4 +1,4 @@
-"""Closed loops of the disturbance-estimating output-feedback controller (carmpc_closed_loop_disturbance) on RoadEnv,
+"""Closed loops of the disturbance-estimating output-feedback controller (carmpc_closed_loop mode 2) on RoadEnv,
 horizon 20: parity with the oracle's loop (exact QPs on the disturbance-shifted bounds), the reference's unstable gains,
 reduction to the plain output-feedback loop, config-4 size, and the offset-free property the controller is for."""
 import os

@@ -1,6 +1,6 @@
 """Noisy closed loops without a GPU: the Philox4x64-10 / Box-Muller restatement against numpy.random.Philox and the
 normal distribution, the noise factors of montecarlo.LoopNoise, montecarlo.plant_rows against MPC.state_constraint, and
-the argument checks of carmpc_closed_loop_stochastic."""
+the argument checks of carmpc_closed_loop."""
 import ctypes
 import math
 
@@ -121,7 +121,7 @@ def test_monitor_argument_forms():
             BatchQP._monitor_rows(bad)
 
 
-# ---- carmpc_closed_loop_stochastic argument checks ----------------------------------------------------------------
+# ---- carmpc_closed_loop argument checks ---------------------------------------------------------------------------
 @pytest.fixture(scope="module")
 def handle():
     from carmpc_b200.batch import BatchQP
@@ -163,14 +163,14 @@ def _call(lib, qp, mode=1, dm="model", noise="noise", rows=_ROWS, monitor_rows=N
         monitor_rows = len(rows) if rows is not None else 0
     rows_ptr = np.ascontiguousarray(rows).ctypes.data if rows is not None else None
     vs, vr, vp = (ctypes.c_void_p(64) if o else None for o in outs)
-    return lib.carmpc_closed_loop_stochastic(
+    return lib.carmpc_closed_loop(
         qp, mode, mat.ctypes.data, mat.ctypes.data, mat.ctypes.data if C else None, mat.ctypes.data if L else None,
         ctypes.byref(dm) if dm is not None else None, mat.ctypes.data, dt, l1, steps, warm_start, p, None, None, None, runs,
         p, None, p, None, None, None, ctypes.byref(noise) if noise is not None else None, rows_ptr, monitor_rows, vs, vr,
         vp, None, None)
 
 
-def test_entry_point_argument_errors(handle):
+def test_closed_loop_argument_errors(handle):
     from carmpc_b200 import _capi
     lib = _capi.load()
     h = handle._h
@@ -215,13 +215,13 @@ def test_entry_point_argument_errors(handle):
     # no runs: nothing to do once the arguments are valid
     total = ctypes.c_int64(7)
     mat = np.zeros(16)
-    assert lib.carmpc_closed_loop_stochastic(h, 0, mat.ctypes.data, mat.ctypes.data, None, None, None, mat.ctypes.data,
-                                             0.2, 3.5, 5, 1, None, None, None, None, 0, None, None, None, None, None,
-                                             None, None, None, 0, None, None, None, ctypes.byref(total), None) == 0
+    assert lib.carmpc_closed_loop(h, 0, mat.ctypes.data, mat.ctypes.data, None, None, None, mat.ctypes.data, 0.2, 3.5, 5,
+                                  1, None, None, None, None, 0, None, None, None, None, None, None, None, None, 0, None,
+                                  None, None, ctypes.byref(total), None) == 0
     assert total.value == 0
 
 
-def test_host_only_handle_is_a_cuda_error(handle):
+def test_closed_loop_on_a_host_only_handle_is_a_cuda_error(handle):
     """Valid arguments on a handle created without a CUDA device: the loop fails loudly instead of computing."""
     try:
         import torch
@@ -235,3 +235,37 @@ def test_host_only_handle_is_a_cuda_error(handle):
         assert _call(lib, handle._h, mode=mode) == -2
         assert b"without a CUDA device" in lib.carmpc_last_error()
     assert _call(lib, handle._h, noise=None, rows=None, outs=(False, False, False)) == -2
+
+
+def _flagged_empty(torch, shape):
+    """An empty float64 host tensor that reports is_cuda: it reaches BatchQP's own checks without a GPU.  With no runs
+    the library checks every argument and returns without touching a pointer."""
+    class Flagged(torch.Tensor):
+        @property
+        def is_cuda(self):
+            return True
+
+    return torch.empty(shape, dtype=torch.float64).as_subclass(Flagged)
+
+
+def test_loops_refuse_a_non_finite_gain_and_a_misshaped_xhat_init(handle):
+    """closed_loop with output feedback refuses a non-finite observer gain L, and both loops refuse an xhat_init that is
+    not (4, R), before any device work."""
+    import torch
+    from types import SimpleNamespace
+    from carmpc_b200._capi import CarmpcError
+    x0 = _flagged_empty(torch, (4, 0))
+    A, B, C, L = np.eye(4), np.zeros((4, 2)), np.zeros((3, 4)), np.zeros((4, 3))
+    kw = dict(C=C, stream=SimpleNamespace(cuda_stream=None))          # the legacy default stream; nothing is enqueued
+    assert handle.closed_loop(x0, 3, A, B, L=L, **kw)["total_iters"] == 0
+    for bad in (math.nan, math.inf):
+        L_bad = L.copy()
+        L_bad[2, 1] = bad
+        with pytest.raises(CarmpcError, match="finite"):
+            handle.closed_loop(x0, 3, A, B, L=L_bad, **kw)
+    xhat = _flagged_empty(torch, (4, 2))
+    with pytest.raises(ValueError, match="xhat_init"):
+        handle.closed_loop(x0, 3, A, B, L=L, xhat_init=xhat, **kw)
+    with pytest.raises(ValueError, match="xhat_init"):
+        handle.closed_loop_disturbance(x0, 3, A, B, C, np.ones(4), np.ones(3), L, np.zeros(3), xhat_init=xhat,
+                                       stream=kw["stream"])

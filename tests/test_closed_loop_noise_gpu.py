@@ -1,5 +1,5 @@
-"""Closed loops with random process and measurement noise and a monitor of the true plant (carmpc_closed_loop_stochastic)
-on RoadEnv, horizon 20: without noise and monitor it is the deterministic loop bit for bit; the device draws are the
+"""Closed loops with random process and measurement noise and a monitor of the true plant (carmpc_closed_loop) on RoadEnv,
+horizon 20: zero noise factors and a monitor leave the loop bit for bit as it is without them; the device draws are the
 restated Philox4x64-10 normals; parity with the restated noisy loop (exact QPs) in the three modes; the monitor's outputs
 equal the C membership oracle's on the stored trajectories; reproducibility across calls and run-set splits; config-4
 size."""
@@ -101,10 +101,9 @@ def _assert_draws(out, x_init, Lw, seed, first_run=0):
 
 # ---- 1. off is off ----------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("warm_start", [0, 1, 2])
-def test_off_is_the_deterministic_loop(torch_cuda, plain, dist, warm_start):
-    """noise = NULL and no monitor through the new entry point: torch.equal to carmpc_closed_loop (modes 0, 1) and to
-    carmpc_closed_loop_disturbance, 2000 runs x 60 steps (graph-replayed steps with warm_start 1).  Zero factors and a
-    monitor change nothing either."""
+def test_zero_noise_and_monitor_change_nothing(torch_cuda, plain, dist, warm_start):
+    """Zero noise factors, a monitor, or both change nothing: torch.equal to the plain loop in modes 0, 1 and 2, 2000
+    runs x 60 steps (graph-replayed steps with warm_start 1)."""
     torch = torch_cuda
     from carmpc_b200.lib.mpc import _C_XYV, _L_OBSERVER
     from carmpc_b200.montecarlo import LoopNoise, plant_rows
@@ -117,29 +116,10 @@ def test_off_is_the_deterministic_loop(torch_cuda, plain, dist, warm_start):
     rows = plant_rows(ctl)
     keys = ("final", "fail_step", "traj", "inputs")
 
-    def direct(handle, mode, **kw):
-        """the new entry point with noise = NULL and no monitor"""
-        out = {"final": torch.empty((4, R), dtype=torch.float64, device="cuda"),
-               "fail_step": torch.empty(R, dtype=torch.int32, device="cuda"),
-               "traj": torch.empty((T, 4, R), dtype=torch.float64, device="cuda"),
-               "inputs": torch.empty((T, 2, R), dtype=torch.float64, device="cuda")}
-        if mode == 2:
-            out["dhat"] = torch.empty(R, dtype=torch.float64, device="cuda")
-            out["dhat_traj"] = torch.empty((T, R), dtype=torch.float64, device="cuda")
-        handle._closed_loop_stochastic(mode, x0, T, kw["A"], kw["B"], kw.get("C"), kw.get("L"), kw.get("dm"), X_REF, 0.2,
-                                       3.5, warm_start, None, None, kw.get("d_plant"), out, None, None, None)
-        return out
-
     for mode in (0, 1):
         C, L = (_C_XYV, _L_OBSERVER) if mode else (None, None)
         ref = bq.closed_loop(x0, T, ctl.A, ctl.B, x_ref=X_REF, C=C, L=L, warm_start=warm_start, want_traj=True,
                              want_inputs=True)
-        new = direct(bq, mode, A=np.ascontiguousarray(ctl.A, dtype=float), B=np.ascontiguousarray(ctl.B, dtype=float),
-                     C=None if C is None else np.ascontiguousarray(C, dtype=float),
-                     L=None if L is None else np.ascontiguousarray(L, dtype=float))
-        for k in keys:
-            assert torch.equal(new[k], ref[k]), (mode, k)
-        assert new["total_iters"] == ref["total_iters"]
         ok = (ref["fail_step"] < 0).float().mean().item()
         assert 0.05 < ok < 0.95
         for noise, monitor in ((zero, None), (None, rows), (zero, rows)):
@@ -148,19 +128,10 @@ def test_off_is_the_deterministic_loop(torch_cuda, plain, dist, warm_start):
             for k in keys:
                 assert torch.equal(o[k], ref[k]), (mode, k, noise is None)
 
-    from carmpc_b200 import _capi
     Bd, Cd, L1, L2 = gains
     dkw = dict(x_ref=X_REF, Bd_plant=np.ones(4), d_plant=d_r, warm_start=warm_start, want_traj=True, want_inputs=True,
                want_dhat=True)
     ref = dbq.closed_loop_disturbance(x0, T, dctl.A, dctl.B, dctl.C, Bd, Cd, L1, L2, **dkw)
-    dm = _capi.DisturbanceModel()
-    dm.Bd[:], dm.Cd[:], dm.L1[:], dm.L2[:] = Bd.tolist(), Cd.tolist(), np.ravel(L1).tolist(), np.ravel(L2).tolist()
-    dm.Bd_plant[:], dm.Cd_plant[:] = [1.0] * 4, [0.0] * 3
-    new = direct(dbq, 2, A=np.ascontiguousarray(dctl.A, dtype=float), B=np.ascontiguousarray(dctl.B, dtype=float),
-                 C=np.ascontiguousarray(dctl.C, dtype=float), dm=dm, d_plant=d_r)
-    for k in keys + ("dhat", "dhat_traj"):
-        assert torch.equal(new[k], ref[k]), k
-    assert new["total_iters"] == ref["total_iters"]
     o = dbq.closed_loop_disturbance(x0, T, dctl.A, dctl.B, dctl.C, Bd, Cd, L1, L2, noise=zero, monitor=rows, **dkw)
     for k in keys + ("dhat", "dhat_traj"):
         assert torch.equal(o[k], ref[k]), k

@@ -154,7 +154,7 @@ def test_to_one_sided_rejects_a_wrong_width():
         to_one_sided(pq, torch.zeros((2, pq.m + pq.n)))
 
 
-def test_checker_and_certified_solve_reject_bad_arguments_without_a_gpu():
+def test_checker_and_solve_reject_bad_arguments_without_a_gpu():
     from carmpc_b200 import _capi
     from carmpc_b200.certificate import QPChecker
     lib = _capi.load()
@@ -170,14 +170,26 @@ def test_checker_and_certified_solve_reject_bad_arguments_without_a_gpu():
     assert lib.carmpc_qp_checker_create(2, 0, p(bad), p(F2), None, None, None, None, None, p(z), p(z), ctypes.byref(h)) == -1
     xref = np.zeros(4)
     assert lib.carmpc_qp_check(None, None, p(xref), None, 1, None, None, None, None, None) == -1
-    assert lib.carmpc_qp_solve_certified(None, None, p(xref), None, None, 1, None, None, None, None, None, None, None, None) == -1
+    fake = ctypes.c_void_p(64)            # never dereferenced: every call below is refused before any device work
+
+    def solve(qp, seed=None, warm=None, cert=None, batch=1):
+        return lib.carmpc_qp_solve(qp, None, p(xref), None, seed, batch, None, None, None, None, None, warm, 0, 0, cert, None,
+                                   None)
+
+    assert solve(None, cert=fake) == -1
     # a well-formed checker can be created without a device (its check calls then fail)
     chk = QPChecker(I2, F2, np.ones((1, 2)), np.zeros((1, 4)), [-np.inf], [1.0], -np.ones(2), np.ones(2))
     assert chk.R == 1 and chk._h
-    # the polish is what produces certificates: a handle without it is refused before any device work
+    # the polish is what produces certificates and reuses seeds: a handle without it is refused
     from carmpc_b200.batch import BatchQP
     pq = _parametric("RoadEnv", "RoadEnv", None, 3)
     bq = BatchQP(pq, polish=0)
-    assert lib.carmpc_qp_solve_certified(bq._h, None, p(xref), None, None, 1, None, None, None, None, None, None, None,
-                                         None) == -1
-    assert b"polish" in lib.carmpc_last_error()
+    for kw in (dict(cert=fake), dict(seed=fake), dict(cert=fake, batch=0), dict(seed=fake, batch=0)):
+        assert solve(bq._h, **kw) == -1, kw
+        assert b"polish" in lib.carmpc_last_error()
+    # a warm state is a starting point of its own: not with seeds or certificates, on any handle
+    for handle in (bq, BatchQP(pq)):
+        for kw in (dict(seed=fake), dict(cert=fake), dict(seed=fake, cert=fake)):
+            for batch in (1, 0):
+                assert solve(handle._h, warm=fake, batch=batch, **kw) == -1, (kw, batch)
+                assert b"d_warm" in lib.carmpc_last_error()

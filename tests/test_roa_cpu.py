@@ -83,7 +83,7 @@ def test_exact_projection_matches_lp_feasibility():
 
 
 def test_lattice_seeds_form_a_single_level_forest():
-    """Seed maps of carmpc_qp_solve_seeded: anchors name themselves, every follower names an anchor of its own block, and
+    """Seed maps of the seeded carmpc_qp_solve: anchors name themselves, every follower names an anchor of its own block, and
     shard-local maps never point outside the shard (SURVEY 8e: contiguous index ranges per rank)."""
     from carmpc_b200.grids import lattice_seeds, shard_range
     dims = (12, 10, 3, 4)

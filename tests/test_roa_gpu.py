@@ -56,7 +56,7 @@ def test_feasibility_map_matches_exact_projection_at_tiny_horizon():
 
 
 def test_seeded_and_cold_feasibility_maps_are_identical():
-    """The default map goes through carmpc_qp_solve_seeded (lattice anchors + active-set / Farkas reuse); its flags must
+    """The default map goes through the seeded carmpc_qp_solve (lattice anchors + active-set / Farkas reuse); its flags must
     equal the cold solve's point for point, for the default block and for odd ones."""
     c = make_controller(make_env("RoadOneCarEnv", [29.9, 1.5, 0, 0]), 20)
     axes = _grid(40, 48, 4, 5)

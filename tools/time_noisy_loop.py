@@ -1,8 +1,8 @@
 """Times config 4 (RoadEnv, N = 20, output feedback, 10^5 runs x 200 steps against the nonlinear bicycle) with noise and
-monitor (``carmpc_closed_loop_stochastic``).  Four arms, alternating, in one process: the existing ``closed_loop``; the new
-entry point with everything off; the monitor alone (the controller's plant rows); noise and monitor.  Prints one JSON
-object: ms per loop (every repetition, min and median), ADMM iterations per solved QP, failed runs, runs with a
-violation, with the GPU name and power limit read in the same run.
+monitor (``carmpc_closed_loop``).  Three arms, alternating, in one process: ``closed_loop`` without noise and monitor; the
+monitor alone (the controller's plant rows); noise and monitor.  Prints one JSON object: ms per loop (every repetition,
+min and median), ADMM iterations per solved QP, failed runs, runs with a violation, with the GPU name and power limit
+read in the same run.
 
     python tools/time_noisy_loop.py [--runs 100000] [--steps 200] [--reps 5] [--out result.json]
 """
@@ -63,16 +63,8 @@ def main():
     rows = plant_rows(ctl)
     noise = LoopNoise(PROCESS_STD, MEASUREMENT_STD, seed=0)
 
-    def everything_off(steps):
-        out = {"final": torch.empty((4, R), dtype=torch.float64, device="cuda"),
-               "fail_step": torch.empty(R, dtype=torch.int32, device="cuda")}
-        bq._closed_loop_stochastic(1, x_init, steps, A, B, C, L, None, x_ref, 0.2, 3.5, 1, None, None, None, out, None,
-                                   None, None)
-        return out
-
     arms = {
         "closed_loop": lambda steps: bq.closed_loop(x_init, steps, A, B, x_ref=x_ref, C=C, L=L),
-        "stochastic_off": everything_off,
         "monitor_only": lambda steps: bq.closed_loop(x_init, steps, A, B, x_ref=x_ref, C=C, L=L, monitor=rows),
         "noise_and_monitor": lambda steps: bq.closed_loop(x_init, steps, A, B, x_ref=x_ref, C=C, L=L, monitor=rows,
                                                           noise=noise),

@@ -108,6 +108,7 @@ struct Polytope : HandleBase {
     HostStage stage;
     std::vector<double> h_rows;      // rows x 5 in device order (host copy, for re-ordering)
     bool tuned = false;              // row order already adapted to a sample set
+    bool interleave = false;         // groups of the scan in interleaved order (set by the pilot, see ticket_group)
     Staging staging;                 // geometry of the bulk-async scan (carmpc_scan_staging)
     unsigned long long* d_work = nullptr;   // [2] work counters of the scan kernel (self-resetting)
     double* d_axes = nullptr;        // grid axes of carmpc_membership_grid (4 x 4096 doubles at most)
@@ -131,6 +132,7 @@ struct Rollout : HandleBase {
     std::vector<double> h_rows64;    // every expanded row as built: [rows][5] = g (4), b' (absolute coordinates)
     std::vector<RowF32> h_rows32;    // host copy (re-ordered by the pilot)
     bool tuned = false;
+    bool interleave = false;
     Staging staging;
     unsigned long long* d_work = nullptr;
     HostStage stage;
@@ -154,6 +156,7 @@ struct ScreenConst {         // float32 error-bound constants of the polytope
 
 constexpr int kExit64 = 4;       // rows between "whole warp already outside" votes, float64 path
 constexpr int kRowBlock = 8;     // ... float32 screen (the float32 row image is padded to a multiple of it)
+constexpr int kFirstRows = 2;    // ... except the first vote of the float32 screen, which comes after two rows (screen32)
 
 // Largest bound beta(p) = beta0 + beta1 |p|_1 for which the screen may decide.  Every intermediate of a row's float32 chain
 // is at most (|b_r| + sum |a_rk| |p_k|) (1 + 2^-21) <= (bmax + l1max |p|_1) (1 + 2^-21), and the constants are built with
@@ -240,6 +243,28 @@ __device__ __forceinline__ void decide_exact(const double* __restrict__ s_rows, 
     else rollout64(s_rows, es, x, y, p, v, in);
 }
 
+// ROWS consecutive float32 rows on the thread's samples, in pairs: the four fmas of a row run as FFMA2 (same IEEE result
+// per sample as fmaf, half the issue slots)
+template <int ROWS>
+__device__ __forceinline__ void screen_rows(const RowF32* __restrict__ rows, const f32x2 (&x2)[kNS / 2],
+                                            const f32x2 (&y2)[kNS / 2], const f32x2 (&p2)[kNS / 2],
+                                            const f32x2 (&v2)[kNS / 2], float (&mmin)[kNS]) {
+#pragma unroll
+    for (int r = 0; r < ROWS; ++r) {
+        const RowF32 q = rows[r];
+        const f32x2 a0 = pack2(q.na0, q.na0), a1 = pack2(q.na1, q.na1), a2 = pack2(q.na2, q.na2), a3 = pack2(q.na3, q.na3);
+        const f32x2 b = pack2(q.b, q.b);
+#pragma unroll
+        for (int k = 0; k < kNS / 2; ++k) {
+            const f32x2 m2 = ffma2(a3, v2[k], ffma2(a2, p2[k], ffma2(a1, y2[k], ffma2(a0, x2[k], b))));
+            float m_lo, m_hi;
+            unpack2(m2, m_lo, m_hi);
+            mmin[2 * k] = fminf(mmin[2 * k], m_lo);       // a NaN margin is ignored here; NaN inputs are caught by the bound
+            mmin[2 * k + 1] = fminf(mmin[2 * k + 1], m_hi);
+        }
+    }
+}
+
 // float32 screen: in[k] becomes "surely inside"; returns through amb[k] the samples only the float64 chain can decide
 __device__ __forceinline__ void screen32(const RowF32* __restrict__ s_rows32, int rows_padded, const ScreenConst sc,
                                          const float (&xf)[kNS], const float (&yf)[kNS], const float (&pf)[kNS],
@@ -253,32 +278,27 @@ __device__ __forceinline__ void screen32(const RowF32* __restrict__ s_rows32, in
         ibeta[k] = fmaf(sc.in1, psum, sc.in0);
         mmin[k] = in[k] ? kScreenMaxBound : -INFINITY;       // padding lanes count as "already outside"; for the cap see below
     }
-    // samples in pairs: the four fmas of a row run as FFMA2 (same IEEE result per sample as fmaf, half the issue slots)
     f32x2 x2[kNS / 2], y2[kNS / 2], p2[kNS / 2], v2[kNS / 2];
 #pragma unroll
     for (int k = 0; k < kNS / 2; ++k) {
         x2[k] = pack2(xf[2 * k], xf[2 * k + 1]); y2[k] = pack2(yf[2 * k], yf[2 * k + 1]);
         p2[k] = pack2(pf[2 * k], pf[2 * k + 1]); v2[k] = pack2(vf[2 * k], vf[2 * k + 1]);
     }
-    for (int r0 = 0; r0 < rows_padded; r0 += kRowBlock) {
+    auto warp_out = [&]() {                                  // every sample of the warp already surely outside
         bool all_out = true;
 #pragma unroll
         for (int k = 0; k < kNS; ++k) all_out &= mmin[k] < nbeta[k];
-        if (__all_sync(0xffffffffu, all_out)) break;          // every sample of the warp already surely outside
-#pragma unroll
-        for (int r = 0; r < kRowBlock; ++r) {
-            const RowF32 q = s_rows32[r0 + r];
-            const f32x2 a0 = pack2(q.na0, q.na0), a1 = pack2(q.na1, q.na1), a2 = pack2(q.na2, q.na2), a3 = pack2(q.na3, q.na3);
-            const f32x2 b = pack2(q.b, q.b);
-#pragma unroll
-            for (int k = 0; k < kNS / 2; ++k) {
-                const f32x2 m2 = ffma2(a3, v2[k], ffma2(a2, p2[k], ffma2(a1, y2[k], ffma2(a0, x2[k], b))));
-                float m_lo, m_hi;
-                unpack2(m2, m_lo, m_hi);
-                mmin[2 * k] = fminf(mmin[2 * k], m_lo);       // a NaN margin is ignored here; NaN inputs are caught by the bound
-                mmin[2 * k + 1] = fminf(mmin[2 * k + 1], m_hi);
-            }
-        }
+        return __all_sync(0xffffffffu, all_out);
+    };
+    // Rows in blocks of kRowBlock with a vote before each, except that the first block is cut after kFirstRows rows for
+    // one more vote: the row order puts the axis-aligned bounds first, and on a grid most warp tiles that lie beyond one
+    // of them are rejected whole by the first two rows (config 2: 7.4 instead of 12.1 rows per 128-sample tile,
+    // tools/scan_row_model.py).  The row order and padding are unchanged; only a warp that is done stops sooner.
+    for (int r0 = 0; r0 < rows_padded; r0 += kRowBlock) {
+        screen_rows<kFirstRows>(s_rows32 + r0, x2, y2, p2, v2, mmin);
+        if (r0 == 0 && warp_out()) break;
+        screen_rows<kRowBlock - kFirstRows>(s_rows32 + r0 + kFirstRows, x2, y2, p2, v2, mmin);
+        if (r0 + kRowBlock < rows_padded && warp_out()) break;
     }
 #pragma unroll
     for (int k = 0; k < kNS; ++k) {
@@ -463,12 +483,37 @@ membership_kernel(const double* __restrict__ g_rows, const RowF32* __restrict__ 
 // __syncwarp()s, and lane 0 immediately refills the stage.  Warps never wait for each other (the early exits make
 // their tiles very unequal), and the bytes in flight do not depend on register allocation.
 //
-// Work unit of a warp: a GROUP of 8 consecutive tiles = 1024 samples = 32 bitset words, handed out round-robin over
-// all warps of the grid.  The 32 words of a group are collected one per lane and leave as ONE 128-byte store per
+// Work unit of a warp: a GROUP of 8 consecutive tiles = 1024 samples = 32 bitset words, handed out dynamically in the
+// interleaved order of ticket_group.  The 32 words of a group are collected one per lane and leave as ONE 128-byte store per
 // destination (the local bitset and, for a sharded scan, every peer's copy over NVLink).
 constexpr int kTile = 32 * kNS;                 // samples per warp tile
 constexpr int kGroupTiles = 8;                  // tiles per group
 constexpr int kGroup = kTile * kGroupTiles;     // samples per group (1024)
+
+// Order in which the groups are handed out.  The warps in flight at any moment cover only a few per cent of the groups,
+// so in index order the whole GPU works on one region of the sample set at a time, and where the cost per sample depends
+// on the region (config 2: the x < 30 half of the grid is issue-bound, the other half is bound by HBM) the kernel takes
+// the issue-bound phase PLUS the memory-bound phase.  Instead the groups are cut into kStripes contiguous stripes and
+// consecutive tickets of the work counter go to different stripes, so that both kinds of work are in flight together.
+// Each group stays 1024 contiguous samples.  Measured on config 2 (B200, 1000 W, tools/scan_halves.py): 8, 16, 32, 64 and
+// 256 stripes scan the grid in 0.479 - 0.482 ms against 0.493 ms for 4, 0.498 ms for 2 and 0.500 ms for one (index
+// order); 16 is also the fastest for the rollout-form screen (0.487 ms against 0.493 - 0.504 ms for 8 - 256).
+// On samples whose cost does NOT depend on the index the interleaved order measured 3 - 7 % slower (10^8 uniform random
+// samples: 1.16 against 1.09 ms, cause not established), so it is only used where the row-order pilot saw the cost vary
+// along the index (cost_varies_along_index); everywhere else the groups go out in index order.
+constexpr uint64_t kStripes = 16;
+
+// group of ticket t: stripe s holds q + (s < r) groups (q = n_groups / kStripes, r = n_groups % kStripes) and starts at
+// s q + min(s, r); ticket t < kStripes q is group t / kStripes of stripe t % kStripes, the last r tickets are the last
+// groups of the first r stripes.  A bijection of [0, n_groups); tickets >= n_groups stay past the end.  Without
+// `interleave` the ticket is the group (index order).
+__device__ __forceinline__ int64_t ticket_group(unsigned long long t, int64_t n_groups, bool interleave) {
+    const uint64_t n = (uint64_t)n_groups, q = n / kStripes, r = n % kStripes;
+    if (!interleave || t >= n) return (int64_t)t;
+    const uint64_t s = t < kStripes * q ? t % kStripes : t - kStripes * q;
+    const uint64_t k = t < kStripes * q ? t / kStripes : q;
+    return (int64_t)(s * q + min(s, r) + k);
+}
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -497,7 +542,7 @@ template <int MODE, int KIND, int THREADS, int STAGES, int TPS>
 __global__ void __launch_bounds__(THREADS)
 membership_tma_kernel(const double* __restrict__ g_rows, const RowF32* __restrict__ g_rows32, const ExactSpec es, int rows_padded,
                       const ScreenConst sc, const double* __restrict__ gx, const double* __restrict__ gy,
-                      const double* __restrict__ gp, const double* __restrict__ gv, int64_t n_groups,
+                      const double* __restrict__ gp, const double* __restrict__ gv, int64_t n_groups, bool interleave,
                       const BitSink sink, unsigned long long* __restrict__ count, unsigned long long* __restrict__ work) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr int kWarps = THREADS / 32;
@@ -523,7 +568,7 @@ membership_tma_kernel(const double* __restrict__ g_rows, const RowF32* __restric
 
     // Groups are handed out dynamically (one atomic per 1024 samples): their cost varies a lot (a warp leaves a tile as soon
     // as every sample is rejected) and, on tensor grids, periodically in the sample index, so a static round-robin leaves
-    // some warps with systematically more work and the kernel with a long tail.
+    // some warps with systematically more work and the kernel with a long tail.  Tickets become groups through ticket_group.
     // Producer (lane 0): group pg, next slot ps of it, running slot count pj; it is never more than one group ahead of
     // the consumer (STAGES <= slots per group), so the consumer's next group is always the producer's current one.
     static_assert(STAGES <= kSlotsPerGroup, "the producer may be at most one group ahead");
@@ -538,9 +583,9 @@ membership_tma_kernel(const double* __restrict__ g_rows, const RowF32* __restric
         for (int a = 0; a < 4; ++a)
             bulk_load(w_stage + ((size_t)stage * 4 + a) * kSlot, src[a] + sample, kArrayBytes, w_bar + stage);
         ++pj;
-        if (++ps == kSlotsPerGroup) { ps = 0; pg = (int64_t)atomicAdd(work, 1ull); }
+        if (++ps == kSlotsPerGroup) { ps = 0; pg = ticket_group(atomicAdd(work, 1ull), n_groups, interleave); }
     };
-    if (lane == 0) pg = (int64_t)atomicAdd(work, 1ull);
+    if (lane == 0) pg = ticket_group(atomicAdd(work, 1ull), n_groups, interleave);
     int64_t group = __shfl_sync(0xffffffffu, pg, 0);
     if (lane == 0)
         for (int s = 0; s < STAGES; ++s) advance();
@@ -842,7 +887,7 @@ static bool staging_supported(const Staging& g) {
 
 template <int KIND, int THREADS, int STAGES, int TPS>
 static int launch_tma(const double* d_exact, const RowF32* d_rows32, const ExactSpec& es, int rows_padded, const ScreenConst& sc,
-                      const double* x, const double* y, const double* p, const double* v, int64_t n_groups,
+                      const double* x, const double* y, const double* p, const double* v, int64_t n_groups, bool interleave,
                       const BitSink& sink, unsigned long long* count, unsigned long long* work, size_t smem, cudaStream_t st) {
     auto kernel = membership_tma_kernel<1, KIND, THREADS, STAGES, TPS>;
     // the function attribute is per device and the occupancy depends on smem only through the row count, which rarely
@@ -861,7 +906,7 @@ static int launch_tma(const double* d_exact, const RowF32* d_rows32, const Exact
     }
     const int64_t n_units = (n_groups + THREADS / 32 - 1) / (THREADS / 32);
     kernel<<<grid_blocks(n_units, per_sm_cached[dev]), THREADS, smem, st>>>(d_exact, d_rows32, es, rows_padded, sc, x, y, p, v,
-                                                                      n_groups, sink, count, work);
+                                                                      n_groups, interleave, sink, count, work);
     CARMPC_CUDA(cudaGetLastError());
     return CARMPC_OK;
 }
@@ -871,7 +916,7 @@ template <int KIND>
 static int launch_scan(const double* d_exact, const RowF32* d_rows32, const ExactSpec es, int rows_padded,
                        const ScreenConst sc, const double* x, const double* y, const double* p, const double* v,
                        int64_t n, BitSink sink, unsigned long long* count, unsigned long long* work, int mode, const Staging& geo,
-                       cudaStream_t st) {
+                       bool interleave, cudaStream_t st) {
     if (n == 0) return CARMPC_OK;
     const bool vec = ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y) |
                        reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(v)) & 15) == 0;
@@ -884,7 +929,8 @@ static int launch_scan(const double* d_exact, const RowF32* d_rows32, const Exac
         int rc = CARMPC_ERR_UNSUPPORTED;
 #define TMA_CASE(T, S, P)                                                                                              \
         if (geo.threads == T && geo.stages == S && geo.tps == P)                                                           \
-            rc = launch_tma<KIND, T, S, P>(d_exact, d_rows32, es, rows_padded, sc, x, y, p, v, n_groups, sink, count, work, smem, st)
+            rc = launch_tma<KIND, T, S, P>(d_exact, d_rows32, es, rows_padded, sc, x, y, p, v, n_groups, interleave, sink, count, \
+                                           work, smem, st)
         TMA_CASE(256, 3, 1); TMA_CASE(128, 3, 1); TMA_CASE(128, 4, 1); TMA_CASE(128, 2, 2);
         TMA_CASE(128, 3, 2); TMA_CASE(256, 2, 1); TMA_CASE(128, 2, 1); TMA_CASE(256, 2, 2);
 #undef TMA_CASE
@@ -923,7 +969,7 @@ static int launch_membership(Polytope* P, const double* x, const double* y, cons
     es.len = P->rows * 5;
     es.rows = P->rows;
     return launch_scan<0>(P->d_rows, P->d_rows32, es, pad_rows(P->rows), screen_const(P), x, y, p, v, n, sink, count, work, mode,
-                          P->staging, st);
+                          P->staging, P->interleave, st);
 }
 
 static int launch_rollout(Rollout* R, const double* x, const double* y, const double* p, const double* v, int64_t n,
@@ -936,7 +982,8 @@ static int launch_rollout(Rollout* R, const double* x, const double* y, const do
         es.s = R->s; es.rin = R->rin; es.k_steps = R->k_steps; es.input_mode = R->input_mode;
         ScreenConst sc;
         sc.beta0 = R->beta0; sc.beta1 = R->beta1; sc.in0 = R->in0; sc.in1 = R->in1;
-        return launch_scan<1>(R->d_data, R->d_rows32, es, R->rows_padded, sc, x, y, p, v, n, sink, count, work, 1, R->staging, st);
+        return launch_scan<1>(R->d_data, R->d_rows32, es, R->rows_padded, sc, x, y, p, v, n, sink, count, work, 1, R->staging, R->interleave,
+                              st);
     }
     const size_t smem = sizeof(double) * (20 + 5 * R->s + 5 * R->rin);
     const int64_t n_chunks = (n + kThreads - 1) / kThreads;
@@ -1005,6 +1052,23 @@ pilot_kernel(const double* __restrict__ g_rows, int rows, const double* __restri
     masks[k] = m;
 }
 
+// Whether the cost of a sample changes along the sample index enough for the interleaved group order to pay
+// (ticket_group).  cost[k]: rows the screen runs on pilot sample k (taken at index k * stride, so in index order) until
+// one rejects it, in the new row order, or all of them.  The mean cost of the costliest of kStripes index ranges is
+// compared with the cheapest: 7.6x on config 2's grid, 1.15 - 1.19x on uniform random samples (65,536 pilot samples).
+static bool cost_varies_along_index(const std::vector<int>& cost) {
+    const size_t per = cost.size() / kStripes;
+    if (per == 0) return false;
+    double lo = INFINITY, hi = 0.0;
+    for (size_t s = 0; s < kStripes; ++s) {
+        double sum = 0.0;
+        for (size_t k = s * per; k < (s + 1) * per; ++k) sum += cost[k];
+        lo = std::min(lo, sum);
+        hi = std::max(hi, sum);
+    }
+    return hi > 2.0 * lo;
+}
+
 static int upload_rows(Polytope* P, cudaStream_t st) {
     const int rows = P->rows;
     std::vector<RowF32> r32(pad_rows(rows) > 0 ? pad_rows(rows) : 8);
@@ -1027,6 +1091,7 @@ static int tune_row_order(Polytope* P, const double* x, const double* y, const d
                           cudaStream_t st) {
     const int rows = P->rows;
     P->tuned = true;
+    P->interleave = false;
     if (rows < 2 || rows > 64 || n < 1024) return CARMPC_OK;
     const int n_sub = (int)std::min<int64_t>(1 << 16, n);
     const int64_t stride = n / n_sub;
@@ -1058,6 +1123,14 @@ static int tune_row_order(Polytope* P, const double* x, const double* y, const d
         alive.resize(w);
     }
     for (int r = 0; r < rows; ++r) if (!used[r]) order.push_back(r);       // the rest keeps its relative order
+    std::vector<int> rank(rows), cost(n_sub);
+    for (int i = 0; i < rows; ++i) rank[order[i]] = i;
+    for (int k = 0; k < n_sub; ++k) {
+        int c = rows;
+        for (unsigned long long t = masks[k]; t; t &= t - 1) c = std::min(c, rank[__builtin_ctzll(t)] + 1);
+        cost[k] = c;
+    }
+    P->interleave = cost_varies_along_index(cost);
     std::vector<double> sorted(5 * rows);
     for (int i = 0; i < rows; ++i)
         for (int k = 0; k < 5; ++k) sorted[5 * i + k] = P->h_rows[5 * order[i] + k];
@@ -1088,6 +1161,7 @@ pilot32_kernel(const RowF32* __restrict__ g_rows32, int rows, int words, const d
 static int tune_rollout_order(Rollout* R, const double* x, const double* y, const double* p, const double* v, int64_t n,
                               cudaStream_t st) {
     R->tuned = true;
+    R->interleave = false;
     const int rows = R->rows32;
     if (rows < 2 || n < 1024 || R->d_rows32 == nullptr) return CARMPC_OK;
     const int words = (rows + 63) / 64;
@@ -1127,6 +1201,15 @@ static int tune_rollout_order(Rollout* R, const double* x, const double* y, cons
         alive.resize(w);
     }
     for (int r = 0; r < rows; ++r) if (!used[r]) order.push_back(r);       // the rest keeps its relative order
+    std::vector<int> rank(rows), cost(n_sub);
+    for (int i = 0; i < rows; ++i) rank[order[i]] = i;
+    for (int k = 0; k < n_sub; ++k) {
+        int c = rows;
+        for (int w = 0; w < words; ++w)
+            for (unsigned long long t = masks[(size_t)k * words + w]; t; t &= t - 1) c = std::min(c, rank[64 * w + __builtin_ctzll(t)] + 1);
+        cost[k] = c;
+    }
+    R->interleave = cost_varies_along_index(cost);
     std::vector<RowF32> sorted(R->h_rows32);
     for (int i = 0; i < rows; ++i) sorted[i] = R->h_rows32[order[i]];
     R->h_rows32.swap(sorted);

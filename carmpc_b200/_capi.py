@@ -36,6 +36,12 @@ class LoopNoiseParams(ctypes.Structure):
                 ("Lv", ctypes.c_double * 16)]
 
 
+class LoopGoal(ctypes.Structure):
+    """``carmpc_loop_goal`` (include/carmpc.h)."""
+    _fields_ = [("h_Ab", ctypes.c_void_p), ("rows", ctypes.c_int32), ("d_arrival_step", ctypes.c_void_p),
+                ("d_arrivals_per_step", ctypes.c_void_p)]
+
+
 _vp, _dp, _i64, _i32 = ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int
 
 #: name -> (restype, argtypes); every function include/carmpc.h declares
@@ -81,6 +87,10 @@ SIGNATURES = {
     "carmpc_closed_loop": (_i32, [_vp, _i32, _dp, _dp, _dp, _dp, ctypes.POINTER(DisturbanceModel), _dp, ctypes.c_double,
                                   ctypes.c_double, _i32, _i32, _dp, _dp, _dp, _dp, _i64, _dp, _dp, _vp, _dp, _dp, _dp,
                                   ctypes.POINTER(LoopNoiseParams), _dp, _i32, _vp, _vp, _vp, ctypes.POINTER(_i64), _vp]),
+    "carmpc_closed_loop_goal": (_i32, [_vp, _i32, _dp, _dp, _dp, _dp, ctypes.POINTER(DisturbanceModel), _dp,
+                                       ctypes.c_double, ctypes.c_double, _i32, _i32, _dp, _dp, _dp, _dp, _i64, _dp, _dp,
+                                       _vp, _dp, _dp, _dp, ctypes.POINTER(LoopNoiseParams), _dp, _i32, _vp, _vp, _vp,
+                                       ctypes.POINTER(LoopGoal), ctypes.POINTER(_i64), _vp]),
     "carmpc_measure_peak": (_i32, [_i32, ctypes.POINTER(ctypes.c_double)]),
 }
 

@@ -512,9 +512,9 @@ class BatchQP(_Handle):
         return np.ascontiguousarray(rows)
 
     def _closed_loop(self, mode, x_init, steps, A, B, C, L, dm, x_ref, dt, l1, warm_start, xhat_init, dhat_init, d_plant,
-                     want_traj, want_inputs, want_dhat, noise, monitor, stream) -> dict:
-        """``carmpc_closed_loop`` in ``mode`` 0, 1 or 2 (``dm``: a ``DisturbanceModel``): checks the device inputs, then
-        returns the outputs the ``want_*`` flags, the mode and the monitor ask for, and ``total_iters``."""
+                     want_traj, want_inputs, want_dhat, noise, monitor, goal, stream) -> dict:
+        """``carmpc_closed_loop_goal`` in ``mode`` 0, 1 or 2 (``dm``: a ``DisturbanceModel``): checks the device inputs,
+        then returns the outputs the ``want_*`` flags, the mode, the monitor and the goal ask for, and ``total_iters``."""
         torch = _torch()
         if not (x_init.is_cuda and x_init.dtype == torch.float64 and x_init.dim() == 2 and x_init.shape[0] == 4
                 and x_init.is_contiguous()):
@@ -532,6 +532,7 @@ class BatchQP(_Handle):
         L_ = _f64(L) if L is not None else None
         params = noise.params() if noise is not None else None
         rows = self._monitor_rows(monitor) if monitor is not None else None
+        goal_rows = self._monitor_rows(goal) if goal is not None else None
         out = {"final": torch.empty((4, R), dtype=torch.float64, device=dev)}
         if mode == 2:
             out["dhat"] = torch.empty(R, dtype=torch.float64, device=dev)
@@ -546,25 +547,32 @@ class BatchQP(_Handle):
             out["violation_step"] = torch.empty(R, dtype=torch.int32, device=dev)
             out["violation_row"] = torch.empty(R, dtype=torch.int32, device=dev)
             out["violations_per_step"] = torch.empty(steps, dtype=torch.int32, device=dev)
+        if goal_rows is not None:
+            out["arrival_step"] = torch.empty(R, dtype=torch.int32, device=dev)
+            out["arrivals_per_step"] = torch.empty(steps, dtype=torch.int32, device=dev)
 
         def p(key):
             return out[key].data_ptr() if key in out else None
 
+        g = None
+        if goal_rows is not None:
+            g = _capi.LoopGoal(goal_rows.ctypes.data, len(goal_rows), p("arrival_step"), p("arrivals_per_step"))
         total = ctypes.c_int64(0)
-        check(self._lib.carmpc_closed_loop(
+        check(self._lib.carmpc_closed_loop_goal(
             self._h, mode, _capi.ptr(A_), _capi.ptr(B_), _capi.ptr(C_), _capi.ptr(L_),
             ctypes.byref(dm) if dm is not None else None, _capi.ptr(xref), float(dt), float(l1), int(steps),
             int(warm_start), x_init.data_ptr(), xhat_init.data_ptr() if xhat_init is not None else None,
             dhat_init.data_ptr() if dhat_init is not None else None, d_plant.data_ptr() if d_plant is not None else None,
             R, p("final"), p("dhat"), p("fail_step"), p("traj"), p("inputs"), p("dhat_traj"),
             ctypes.byref(params) if params is not None else None, _capi.ptr(rows), len(rows) if rows is not None else 0,
-            p("violation_step"), p("violation_row"), p("violations_per_step"), ctypes.byref(total), _stream_ptr(stream)))
+            p("violation_step"), p("violation_row"), p("violations_per_step"), ctypes.byref(g) if g is not None else None,
+            ctypes.byref(total), _stream_ptr(stream)))
         out["total_iters"] = int(total.value)
         return out
 
     def closed_loop(self, x_init, steps: int, A, B, x_ref=None, C=None, L=None, xhat_init=None, dt: float = 0.2,
                     l1: float = 3.5, warm_start: bool = True, want_traj: bool = False, want_inputs: bool = False,
-                    noise=None, monitor=None, stream=None) -> dict:
+                    noise=None, monitor=None, goal=None, stream=None) -> dict:
         """Runs ``steps`` closed-loop steps for every column of ``x_init`` ((4, R) float64 CUDA tensor) against the
         nonlinear bicycle.  Output feedback when ``C`` and ``L`` are given (observer started at ``xhat_init`` or the
         true state), state feedback otherwise.  Returns ``final`` (4, R), ``fail_step`` (R,) int32 (-1: never
@@ -573,14 +581,20 @@ class BatchQP(_Handle):
         ``noise``: a ``carmpc_b200.montecarlo.LoopNoise`` (process and measurement noise drawn on the device).
         ``monitor``: (rows, 5) ``[A | b]`` or ``(A, b)``, e.g. ``montecarlo.plant_rows(controller)``; the true state is
         checked against it after every plant step and ``violation_step`` (R,), ``violation_row`` (R,) (-1: none) and
-        ``violations_per_step`` (steps,) int32 are added to the result.  A violation does not stop a run."""
+        ``violations_per_step`` (steps,) int32 are added to the result.  A violation does not stop a run.
+
+        ``goal``: (rows, 5) ``[A | b]`` or ``(A, b)``, e.g. ``montecarlo.goal_box(controller.goal)``; a run whose true
+        state satisfies every row after a plant step, and whose QP of that step is solved, stops there (the reference's
+        loops break at the goal): its ``final`` state is that state and the step's input is not applied.  A QP that is not
+        solved at the same step is a failure, as in the reference.  ``arrival_step`` (R,) (-1: none) and
+        ``arrivals_per_step`` (steps,) int32 are added to the result."""
         return self._closed_loop(1 if C is not None else 0, x_init, steps, A, B, C, L, None, x_ref, dt, l1, warm_start,
-                                 xhat_init, None, None, want_traj, want_inputs, False, noise, monitor, stream)
+                                 xhat_init, None, None, want_traj, want_inputs, False, noise, monitor, goal, stream)
 
     def closed_loop_disturbance(self, x_init, steps: int, A, B, C, Bd, Cd, L1, L2, x_ref=None, Bd_plant=None,
                                 Cd_plant=None, d_plant=None, xhat_init=None, dhat_init=None, dt: float = 0.2,
                                 l1: float = 3.5, warm_start=True, want_traj: bool = False, want_inputs: bool = False,
-                                want_dhat: bool = False, noise=None, monitor=None, stream=None) -> dict:
+                                want_dhat: bool = False, noise=None, monitor=None, goal=None, stream=None) -> dict:
         """Closed loops of the disturbance-estimating output-feedback controller (``MPCOutputFBWithDisturbance``,
         ``carmpc_closed_loop`` mode 2): the loop of ``closed_loop`` with a scalar disturbance estimate ``d^`` kept
         beside ``x^`` by the augmented observer (``Bd`` (4,), ``Cd`` (3,), gains ``L1`` (4, 3), ``L2`` (3,); no defaults,
@@ -589,8 +603,8 @@ class BatchQP(_Handle):
         run ((R,) float64 CUDA tensor, None: 0) through ``Bd_plant`` (4,) after its Euler step and ``Cd_plant`` (3,) in its
         output (None: zeros).  ``dhat_init``: (R,) CUDA tensor (None: 0).  ``warm_start``: 0 / 1 (True) / 2 as in
         ``closed_loop``.  Returns ``final`` (4, R), ``dhat`` (R,), ``fail_step`` (R,) int32, ``total_iters`` and
-        optionally ``traj`` (steps, 4, R), ``inputs`` (steps, 2, R), ``dhat_traj`` (steps, R).  ``noise`` and ``monitor``
-        as in ``closed_loop`` (the measurement noise adds to ``C s + Cd_plant d_r``)."""
+        optionally ``traj`` (steps, 4, R), ``inputs`` (steps, 2, R), ``dhat_traj`` (steps, R).  ``noise``, ``monitor`` and
+        ``goal`` as in ``closed_loop`` (the measurement noise adds to ``C s + Cd_plant d_r``)."""
 
         def vec(a, n, name):
             v = _f64(a).ravel()
@@ -606,4 +620,4 @@ class BatchQP(_Handle):
         dm.Bd_plant[:] = vec(np.zeros(4) if Bd_plant is None else Bd_plant, 4, "Bd_plant").tolist()
         dm.Cd_plant[:] = vec(np.zeros(3) if Cd_plant is None else Cd_plant, 3, "Cd_plant").tolist()
         return self._closed_loop(2, x_init, steps, A, B, C, None, dm, x_ref, dt, l1, warm_start, xhat_init, dhat_init,
-                                 d_plant, want_traj, want_inputs, want_dhat, noise, monitor, stream)
+                                 d_plant, want_traj, want_inputs, want_dhat, noise, monitor, goal, stream)

@@ -23,6 +23,13 @@
 // (seed, 0): they depend on nothing but the global run id and the step, so warm-start mode, graph replay and batch
 // composition draw the same noise.  Both are compile-time switches of loop_advance_kernel: with both off it has none of
 // their code.
+//
+// Goal (any mode): the caller's goal rows [a | b] are checked on the same true plant state as the monitor, with the same
+// chain.  The run still solves its QP at that step, so a QP that is not solved stops the run as a failure first (the
+// reference raises before it tests the goal); a solved QP with the state inside stops the run as arrived: its input is
+// not applied and it is never moved, solved or counted again.  The verdict of the rows waits for the QP's in a loop-owned
+// byte per run.  A third compile-time switch of loop_advance_kernel and loop_apply_kernel: with it off both are the
+// kernels without a goal.
 #include <math.h>
 #include <string.h>
 
@@ -58,16 +65,26 @@ struct LoopMonitor {
     int32_t* per_step;              // steps: runs violating at the step
 };
 
+// Goal rows (a loop-owned device copy, rows x 5), the pending verdict of the rows (loop-owned) and the outputs.
+struct LoopGoal {
+    const double* Ab;
+    int rows;
+    uint8_t* inside;                // runs: the state of this step satisfied every row (read once its QP is known)
+    int32_t* arrival_step;          // runs: step of arrival, -1 none
+    int32_t* per_step;              // steps (nullable): runs arriving at the step
+};
+
 // plant step with the previous input, observer update, estimate -> QP input; builds the list of live runs.
-// kNoise / kMonitor: process and measurement noise, monitor rows; step is the step number of host-driven steps.
-template <bool kNoise, bool kMonitor>
+// kNoise / kMonitor / kGoal: process and measurement noise, monitor rows, goal rows; step is the step number of
+// host-driven steps.
+template <bool kNoise, bool kMonitor, bool kGoal>
 __global__ void __launch_bounds__(256)
 loop_advance_kernel(const LoopConst K, int64_t runs, double* __restrict__ x, double* __restrict__ xhat,
                     const double* __restrict__ u_prev, const int32_t* __restrict__ fail_step,
                     double* __restrict__ est, int* __restrict__ live_list, int* __restrict__ live_count,
                     double* __restrict__ traj_step, const int* __restrict__ step_dev,
                     double* __restrict__ dhat, const double* __restrict__ d_plant, const LoopNoise N,
-                    const LoopMonitor M, int step) {
+                    const LoopMonitor M, int step, const LoopGoal G) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= runs) return;
     // replayed steps (CUDA graph) read the step number on the device: traj_step is then the base of the trajectory
@@ -77,7 +94,7 @@ loop_advance_kernel(const LoopConst K, int64_t runs, double* __restrict__ x, dou
     double s[4], u[2];
 #pragma unroll
     for (int c = 0; c < 4; ++c) s[c] = x[c * runs + i];
-    const bool alive = fail_step[i] < 0;
+    const bool alive = fail_step[i] < 0 && (!kGoal || G.arrival_step[i] < 0);
     if (alive) {
         u[0] = u_prev[i];
         u[1] = u_prev[runs + i];
@@ -129,6 +146,16 @@ loop_advance_kernel(const LoopConst K, int64_t runs, double* __restrict__ x, dou
                 if (M.violation_step != nullptr && M.violation_step[i] < 0) M.violation_step[i] = step;
                 if (M.violation_row != nullptr && M.violation_row[i] < 0) M.violation_row[i] = bad;
             }
+        }
+        if (kGoal) {
+            // the monitor's chain; a non-finite state is never inside (an infinite coordinate may satisfy a row)
+            bool in = isfinite(s[0]) && isfinite(s[1]) && isfinite(s[2]) && isfinite(s[3]);
+            for (int r = 0; in && r < G.rows; ++r) {
+                const double* a = G.Ab + 5 * r;
+                const double lhs = fma(__ldg(a + 3), s[3], fma(__ldg(a + 2), s[2], fma(__ldg(a + 1), s[1], __ldg(a) * s[0])));
+                in = lhs <= __ldg(a + 4);
+            }
+            G.inside[i] = in ? 1 : 0;
         }
         double e[4];
         if (K.mode == 2) {
@@ -205,21 +232,35 @@ loop_advance_kernel(const LoopConst K, int64_t runs, double* __restrict__ x, dou
     }
 }
 
-// take the QP results of the live runs: new input, or mark the run as failed at this step
+// take the QP results of the live runs: new input, or mark the run as failed at this step; kGoal: a solved run whose state
+// was inside the goal arrives instead of taking its input
+template <bool kGoal>
 __global__ void __launch_bounds__(256)
 loop_apply_kernel(int64_t runs, int step, const int* __restrict__ live_list, int live, const int* __restrict__ live_dev,
                   const double* __restrict__ u0, const int32_t* __restrict__ status, double* __restrict__ u_prev,
-                  int32_t* __restrict__ fail_step, const int* __restrict__ step_dev) {
+                  int32_t* __restrict__ fail_step, const int* __restrict__ step_dev, const LoopGoal G) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (live_dev != nullptr) live = min(live, *live_dev);
     if (step_dev != nullptr) step = *step_dev;
     if (q >= live) return;
     const int i = live_list[q];
+    bool arrived = false;
     if (status[i] == CARMPC_QP_SOLVED) {
-        u_prev[i] = u0[i];
-        u_prev[runs + i] = u0[runs + i];
+        if (kGoal && G.inside[i]) {
+            G.arrival_step[i] = step;
+            arrived = true;
+        } else {
+            u_prev[i] = u0[i];
+            u_prev[runs + i] = u0[runs + i];
+        }
     } else {
         fail_step[i] = step;
+    }
+    if (kGoal && G.per_step != nullptr) {
+        // one atomic per warp, as the monitor's count
+        const unsigned act = __activemask();
+        const unsigned hit = __ballot_sync(act, arrived);
+        if (hit != 0 && (int)(threadIdx.x & 31) == __ffs(act) - 1) atomicAdd(G.per_step + step, __popc(hit));
     }
 }
 
@@ -239,6 +280,11 @@ __global__ void loop_set_kernel(int* step_dev, int v) { *step_dev = v; }
 __global__ void fill_i32(int32_t* p, int64_t n, int32_t v) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) p[i] = v;
+}
+
+template <bool kNoise, bool kMonitor>
+auto advance_variant(bool goal) {
+    return goal ? loop_advance_kernel<kNoise, kMonitor, true> : loop_advance_kernel<kNoise, kMonitor, false>;
 }
 
 // Mode-2 state and logs of a run set (all nullable: d^ starts at 0, d_r is 0, d^ is kept in a buffer of the driver).
@@ -262,8 +308,8 @@ struct LoopStochastic {
 // The loop shared by every mode: host-driven first steps, then one captured CUDA graph with the step number on the device.
 int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int steps, int warm_start, const double* d_x_init,
                     const double* d_xhat_init, int64_t runs, double* d_final, int32_t* d_fail_step, double* d_traj,
-                    double* d_u_log, const LoopDisturbance& D, const LoopStochastic& Z, int64_t* h_total_iters,
-                    void* stream) {
+                    double* d_u_log, const LoopDisturbance& D, const LoopStochastic& Z, const carmpc_loop_goal* goal,
+                    int64_t* h_total_iters, void* stream) {
     if (q->host_only) { set_error("carmpc_closed_loop: this QP handle was created without a CUDA device"); return CARMPC_ERR_CUDA; }
     QPBusyGuard guard(q->busy);
     CARMPC_REQUIRE(guard.acquired, "this QP handle is in use by another call (one call per handle at a time)");
@@ -282,11 +328,13 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
     int32_t* status = nullptr;
     int *live_list = nullptr, *live_count = nullptr;
     float* warm = nullptr;
-    double* monitor_Ab = nullptr;
+    double *monitor_Ab = nullptr, *goal_Ab = nullptr;
+    uint8_t* inside = nullptr;
     int rc = CARMPC_OK;
     auto cleanup = [&]() { if (st != user_st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); } if (ev) cudaEventDestroy(ev);
                            cudaFree(xhat); cudaFree(est); cudaFree(u_prev); cudaFree(u0); cudaFree(status); cudaFree(live_list);
-                           cudaFree(live_count); cudaFree(warm); cudaFree(dhat_own); cudaFree(monitor_Ab); };
+                           cudaFree(live_count); cudaFree(warm); cudaFree(dhat_own); cudaFree(monitor_Ab);
+                           cudaFree(goal_Ab); cudaFree(inside); };
 #define TRY(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) { set_error("%s: %s", #call, cudaGetErrorString(e__)); cleanup(); return CARMPC_ERR_CUDA; } } while (0)
     TRY(cudaMalloc(&xhat, sizeof(double) * 4 * runs));
     TRY(cudaMalloc(&est, sizeof(double) * 4 * runs));
@@ -327,13 +375,25 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
         if (mon.violation_row) fill_i32<<<blocks, 256, 0, st>>>(mon.violation_row, runs, -1);
         if (mon.per_step && steps > 0) TRY(cudaMemsetAsync(mon.per_step, 0, sizeof(int32_t) * steps, st));
     }
-    const bool with_noise = Z.noise != nullptr, with_monitor = Z.monitor_rows > 0;
+    // goal: rows and the pending verdict in buffers the loop owns, fixed addresses like every other buffer of the step
+    LoopGoal gl = {nullptr, 0, nullptr, nullptr, nullptr};
+    if (goal != nullptr) {
+        TRY(cudaMalloc(&goal_Ab, sizeof(double) * 5 * goal->rows));
+        TRY(cudaMalloc(&inside, runs));
+        TRY(cudaMemcpyAsync(goal_Ab, goal->h_Ab, sizeof(double) * 5 * goal->rows, cudaMemcpyHostToDevice, st));
+        TRY(cudaMemsetAsync(inside, 0, runs, st));
+        gl = {goal_Ab, goal->rows, inside, goal->d_arrival_step, goal->d_arrivals_per_step};
+        fill_i32<<<blocks, 256, 0, st>>>(gl.arrival_step, runs, -1);
+        if (gl.per_step && steps > 0) TRY(cudaMemsetAsync(gl.per_step, 0, sizeof(int32_t) * steps, st));
+    }
+    const bool with_noise = Z.noise != nullptr, with_monitor = Z.monitor_rows > 0, with_goal = goal != nullptr;
     auto advance = [&](int k, double* traj_step, const int* step_dev) {
-        auto kern = with_noise ? (with_monitor ? loop_advance_kernel<true, true> : loop_advance_kernel<true, false>)
-                               : (with_monitor ? loop_advance_kernel<false, true> : loop_advance_kernel<false, false>);
+        auto kern = with_noise ? (with_monitor ? advance_variant<true, true>(with_goal) : advance_variant<true, false>(with_goal))
+                               : (with_monitor ? advance_variant<false, true>(with_goal) : advance_variant<false, false>(with_goal));
         kern<<<blocks, 256, 0, st>>>(K, runs, x, xhat, u_prev, d_fail_step, est, live_list, live_count, traj_step, step_dev,
-                                     dhat, D.d_plant, noise, mon, k);
+                                     dhat, D.d_plant, noise, mon, k, gl);
     };
+    auto apply = with_goal ? loop_apply_kernel<true> : loop_apply_kernel<false>;
     int64_t total_iters = 0;
     bool warm_valid = false;
     // the iteration total accumulates on the device over the steps (one read at the end instead of one per step)
@@ -354,7 +414,7 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
         r.count = runs; r.count_dev = live_count; r.warm_in = 1;
         const int rc2 = q->solve_enqueue(r, st);
         if (rc2 != CARMPC_OK) return rc2;
-        loop_apply_kernel<<<blocks, 256, 0, st>>>(runs, k, live_list, (int)runs, live_count, u0, status, u_prev, d_fail_step, step_dev);
+        apply<<<blocks, 256, 0, st>>>(runs, k, live_list, (int)runs, live_count, u0, status, u_prev, d_fail_step, step_dev, gl);
         if (step_dev) {
             if (d_u_log || D.dhat_log)
                 loop_log_kernel<<<(int)((2 * runs + 255) / 256), 256, 0, st>>>(runs, u_prev, d_u_log, dhat, D.dhat_log, step_dev);
@@ -413,7 +473,7 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
             rc = q->solve(req, st);
             if (rc != CARMPC_OK) { cleanup(); return rc; }
             warm_valid = warm != nullptr;
-            loop_apply_kernel<<<(live + 255) / 256, 256, 0, st>>>(runs, k, live_list, live, nullptr, u0, status, u_prev, d_fail_step, nullptr);
+            apply<<<(live + 255) / 256, 256, 0, st>>>(runs, k, live_list, live, nullptr, u0, status, u_prev, d_fail_step, nullptr, gl);
         }
         if (d_u_log)      // the input each run will apply at the next plant step (unchanged for stopped runs)
             TRY(cudaMemcpyAsync(d_u_log + (size_t)k * 2 * runs, u_prev, sizeof(double) * 2 * runs, cudaMemcpyDeviceToDevice, st));
@@ -436,14 +496,15 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
 
 using namespace carmpc;
 
-extern "C" int carmpc_closed_loop(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C,
-                                  const double* h_L, const carmpc_disturbance_model* dm, const double* h_xref, double dt,
-                                  double l1, int steps, int warm_start, const double* d_x_init, const double* d_xhat_init,
-                                  const double* d_dhat_init, const double* d_d_plant, int64_t runs, double* d_final,
-                                  double* d_dhat_final, int32_t* d_fail_step, double* d_traj, double* d_u_log,
-                                  double* d_dhat_log, const carmpc_loop_noise* noise, const double* h_monitor_Ab,
-                                  int monitor_rows, int32_t* d_violation_step, int32_t* d_violation_row,
-                                  int32_t* d_violations_per_step, int64_t* h_total_iters, void* stream) {
+extern "C" int carmpc_closed_loop_goal(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C,
+                                       const double* h_L, const carmpc_disturbance_model* dm, const double* h_xref,
+                                       double dt, double l1, int steps, int warm_start, const double* d_x_init,
+                                       const double* d_xhat_init, const double* d_dhat_init, const double* d_d_plant,
+                                       int64_t runs, double* d_final, double* d_dhat_final, int32_t* d_fail_step,
+                                       double* d_traj, double* d_u_log, double* d_dhat_log, const carmpc_loop_noise* noise,
+                                       const double* h_monitor_Ab, int monitor_rows, int32_t* d_violation_step,
+                                       int32_t* d_violation_row, int32_t* d_violations_per_step,
+                                       const carmpc_loop_goal* goal, int64_t* h_total_iters, void* stream) {
     QPHandle* q = check_handle<QPHandle>(qp, kQP);
     CARMPC_REQUIRE(q != nullptr, "not a QP handle");
     CARMPC_REQUIRE(mode >= 0 && mode <= 2, "mode must be 0 (state feedback), 1 (output feedback) or 2 (with a disturbance estimate)");
@@ -476,6 +537,13 @@ extern "C" int carmpc_closed_loop(void* qp, int mode, const double* h_A, const d
         CARMPC_REQUIRE(monitor_rows == 0, "monitor_rows without monitor rows");
         CARMPC_REQUIRE(!d_violation_step && !d_violation_row && !d_violations_per_step, "monitor outputs without monitor rows");
     }
+    if (goal != nullptr) {
+        CARMPC_REQUIRE(goal->rows >= 1 && goal->rows <= 512, "goal rows must be in [1, 512]");
+        CARMPC_REQUIRE(goal->h_Ab != nullptr, "null goal rows");
+        for (int j = 0; j < 5 * goal->rows; ++j) finite = finite && isfinite(goal->h_Ab[j]);
+        CARMPC_REQUIRE(finite, "goal rows must be finite");
+        CARMPC_REQUIRE(goal->d_arrival_step != nullptr, "a goal needs d_arrival_step");
+    }
     if (h_total_iters) *h_total_iters = 0;
     if (runs == 0) return CARMPC_OK;
     CARMPC_REQUIRE(d_x_init && d_final && d_fail_step, "null device pointer");
@@ -506,5 +574,19 @@ extern "C" int carmpc_closed_loop(void* qp, int mode, const double* h_A, const d
     const LoopStochastic Z = {noise ? &nz : nullptr, h_monitor_Ab, h_monitor_Ab ? monitor_rows : 0, d_violation_step,
                               d_violation_row, d_violations_per_step};
     return closed_loop_run(q, K, h_xref, steps, warm_start, d_x_init, d_xhat_init, runs, d_final, d_fail_step, d_traj, d_u_log,
-                           D, Z, h_total_iters, stream);
+                           D, Z, goal, h_total_iters, stream);
+}
+
+extern "C" int carmpc_closed_loop(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C,
+                                  const double* h_L, const carmpc_disturbance_model* dm, const double* h_xref, double dt,
+                                  double l1, int steps, int warm_start, const double* d_x_init, const double* d_xhat_init,
+                                  const double* d_dhat_init, const double* d_d_plant, int64_t runs, double* d_final,
+                                  double* d_dhat_final, int32_t* d_fail_step, double* d_traj, double* d_u_log,
+                                  double* d_dhat_log, const carmpc_loop_noise* noise, const double* h_monitor_Ab,
+                                  int monitor_rows, int32_t* d_violation_step, int32_t* d_violation_row,
+                                  int32_t* d_violations_per_step, int64_t* h_total_iters, void* stream) {
+    return carmpc_closed_loop_goal(qp, mode, h_A, h_B, h_C, h_L, dm, h_xref, dt, l1, steps, warm_start, d_x_init,
+                                   d_xhat_init, d_dhat_init, d_d_plant, runs, d_final, d_dhat_final, d_fail_step, d_traj,
+                                   d_u_log, d_dhat_log, noise, h_monitor_Ab, monitor_rows, d_violation_step,
+                                   d_violation_row, d_violations_per_step, nullptr, h_total_iters, stream);
 }

@@ -1,8 +1,8 @@
-"""Monte-Carlo closed loops with random noise, and the rows that say whether the true plant stayed safe.
+"""Monte-Carlo closed loops with random noise, the rows that say whether the true plant stayed safe, and goal rows.
 
 ``LoopNoise`` describes the process and measurement noise of ``BatchQP.closed_loop(..., noise=...)`` and
 ``BatchQP.closed_loop_disturbance(..., noise=...)``; ``plant_rows`` gives a controller's own state rows as a monitor for
-the ``monitor=`` argument of the same calls.  The noise is drawn on the device (``carmpc_closed_loop``,
+the ``monitor=`` argument of the same calls; ``goal_box`` gives the reference's arrival test as rows for ``goal=``.  The noise is drawn on the device (``carmpc_closed_loop``,
 Philox4x64-10 at counter (first_run + run, step, 0 / 1, 0), key (seed, 0)), so it depends only on the seed, the global run
 id and the step: a run set split over calls or GPUs with ``first_run`` offsets draws what one call would.
 """
@@ -79,3 +79,17 @@ def plant_rows(controller, terminal_set: bool = False) -> np.ndarray:
         At, bt = controller.terminal_constraint()
         rows = np.vstack((rows, np.hstack((np.asarray(At, dtype=np.float64)[:, -4:], np.asarray(bt, dtype=np.float64)[:, None]))))
     return np.ascontiguousarray(rows)
+
+
+def goal_box(goal, tol: float = 0.1) -> np.ndarray:
+    """The reference's arrival test ``np.all(np.abs(state - goal) <= tol)`` (examples/run_MPCStateFB.py) as (8, 5) rows
+    ``[+-e_c | +-goal_c + tol]`` for the ``goal=`` argument of the closed loops.  The rows test ``s_c <= fl(g_c + tol)``
+    and ``-s_c <= fl(-g_c + tol)``; within an ulp of a face that can differ from ``fl(|s_c - g_c|) <= tol``."""
+    g = np.asarray(goal, dtype=np.float64).ravel()
+    if g.shape != (4,) or not np.isfinite(g).all() or not (np.isfinite(tol) and tol >= 0):
+        raise ValueError("goal must be 4 finite numbers and tol finite and >= 0")
+    rows = np.zeros((8, 5))
+    for c in range(4):
+        rows[2 * c, c], rows[2 * c, 4] = 1.0, g[c] + tol
+        rows[2 * c + 1, c], rows[2 * c + 1, 4] = -1.0, -g[c] + tol
+    return rows

@@ -13,10 +13,14 @@ conventions (absolute coordinates, unit-norm rows):
 * ``hull_polytope(points)``                   - convex hull -> merged, unit-normalised facets;
 * ``region_of_attraction(controller, axes)``  - the three above in sequence;
 * ``exact_feasible_set(G, Gx, w)``            - Fourier-Motzkin with LP redundancy removal after every elimination
-                                                (tiny horizons only; the cross-check of the tests).
+                                                (tiny horizons only; the cross-check of the tests);
+* ``closed_loop_map(controller, axes)``       - the region of attraction by closed-loop convergence (the paper's
+                                                criterion): the nonlinear bicycle under the MPC law from every grid point,
+                                                run on the GPU until it reaches the goal, its QP fails, or the steps end.
 
 The feasible set F = {x0 : exists u, G u <= w - Gx x0} is convex, so  hull(feasible samples) is an inner
-approximation of F and no infeasible sample may lie inside it - the property the tests check at every size.
+approximation of F and no infeasible sample may lie inside it - the property the tests check at every size.  The
+closed-loop map is not convex in general, so it is returned as flags only, never hulled.
 """
 from __future__ import annotations
 
@@ -160,3 +164,38 @@ def exact_feasible_set(G: np.ndarray, Gx: np.ndarray, w: np.ndarray) -> tuple[np
         P, phi = red.A, -red.b
         C, H = P[:, :C.shape[1]], P[:, C.shape[1]:]
     return C, -phi
+
+
+def closed_loop_map(controller, axes: Sequence[np.ndarray], steps: int = 200, goal=None, x_ref=None, batch_solver=None,
+                    noise=None) -> dict:
+    """Closed-loop convergence from every point of the tensor grid ``axes`` (C order, x slowest ... v fastest): the
+    nonlinear bicycle under ``controller``'s MPC law, in the order of the reference's loops (examples/run_MPCStateFB.py,
+    run_MPCOutputFB.py), one run per grid point on the GPU (``BatchQP.closed_loop`` with a goal).  ``MPCStateFB`` runs
+    state feedback; ``MPCOutputFB`` output feedback with its ``C`` and ``L``, the observer started at the true state.
+    ``goal``: rows as for ``closed_loop`` (default ``montecarlo.goal_box(controller.goal, 0.1)``, the reference's test).
+    ``noise``: an optional ``montecarlo.LoopNoise``.
+
+    Returns flat C-order numpy arrays: ``reached`` (bool), ``arrival_step`` and ``fail_step`` (int32, -1 none) and
+    ``outcome`` (int8): 0 reached the goal, 1 stopped by a QP that was not solved, 2 neither within ``steps``."""
+    import torch
+    from .batch import BatchQP
+    from .grids import materialise_grid
+    from .lib.mpc import MPCOutputFB, MPCStateFB
+    from .lib.simulator import CarTrailerDimension
+    from .montecarlo import goal_box
+    if isinstance(controller, MPCOutputFB):
+        C, L = controller.C, controller.L
+    elif isinstance(controller, MPCStateFB):
+        C = L = None
+    else:
+        raise TypeError("closed_loop_map needs an MPCStateFB or an MPCOutputFB controller")
+    bq = batch_solver if batch_solver is not None else BatchQP.from_controller(controller)
+    x0 = torch.stack(materialise_grid(axes, device="cuda")).contiguous()
+    out = bq.closed_loop(x0, steps, controller.A, controller.B, x_ref=x_ref, C=C, L=L, dt=controller.dt,
+                         l1=CarTrailerDimension.l1, noise=noise,
+                         goal=goal_box(controller.goal, 0.1) if goal is None else goal)
+    arrival = out["arrival_step"].cpu().numpy()
+    fail = out["fail_step"].cpu().numpy()
+    reached = arrival >= 0
+    outcome = np.where(reached, 0, np.where(fail >= 0, 1, 2)).astype(np.int8)
+    return {"reached": reached, "arrival_step": arrival, "fail_step": fail, "outcome": outcome}

@@ -379,8 +379,21 @@ int carmpc_qp_tensor_mode(void* qp, int mode, int64_t* h_info);
  * int32): runs violating at step k.  Stopped runs are neither moved nor counted; a run whose QP fails at step k was
  * moved and checked at step k.
  * Noise and monitor are compile-time switches of the step kernel: a loop without them pays nothing for them.
+ * goal (carmpc_closed_loop_goal only; nullable: runs never stop at a goal): runs that reach a goal stop there, as the
+ * reference's loops break on  all(|state - goal| <= 0.1).  h_Ab: host rows x 5 [a | b], 1 <= rows <= 512, finite (the
+ * loop copies them).  At step k the run is inside when s (the true state above, after the Euler step, Bd_plant d_r and
+ * the process noise) is finite and satisfies every row with the monitor's chain.  The initial state is not tested.  The
+ * run still solves its step-k QP, and then:
+ *   QP not solved               d_fail_step = k, d_arrival_step stays -1 (the reference raises before its goal test);
+ *   QP solved and s inside      d_arrival_step = k; the step-k input is not applied (d_u_log keeps the previous input,
+ *                               as for a failed run), d_final = s, and the run is never moved, observed, solved,
+ *                               monitored or counted again.
+ * A run is running while d_fail_step < 0 and d_arrival_step < 0.  d_arrival_step (runs int32, required): -1 or the
+ * step of arrival.  d_arrivals_per_step (steps int32, nullable): runs arriving at step k.  Replayed steps read k on the
+ * device; nothing of the goal is read back to the host.
  * CARMPC_ERR_INVALID for non-finite factors or gains, first_run < 0, bad monitor rows, monitor outputs without rows, mode
- * 2 without dm; CARMPC_ERR_CUDA on a handle created without a device. */
+ * 2 without dm, bad or null goal rows, a goal without d_arrival_step; CARMPC_ERR_CUDA on a handle created without a
+ * device.  carmpc_closed_loop is carmpc_closed_loop_goal with goal = NULL. */
 typedef struct carmpc_disturbance_model {
     double Bd[4], Cd[3], L1[12], L2[3];   /* controller: disturbance model and observer gains (L1 4x3 row-major) */
     double Bd_plant[4], Cd_plant[3];      /* how the true per-run disturbance enters the plant state / output    */
@@ -393,6 +406,13 @@ typedef struct carmpc_loop_noise {
     double Lv[16];          /* measurement-noise factor, 4 x 4 row-major: v = Lv z_v */
 } carmpc_loop_noise;
 
+typedef struct carmpc_loop_goal {
+    const double* h_Ab;              /* rows x 5 [a | b], host */
+    int32_t rows;                    /* 1..512 */
+    int32_t* d_arrival_step;         /* runs int32, required: step of arrival, -1 none */
+    int32_t* d_arrivals_per_step;    /* steps int32, nullable */
+} carmpc_loop_goal;
+
 int carmpc_closed_loop(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C, const double* h_L,
                        const carmpc_disturbance_model* dm, const double* h_xref, double dt, double l1, int steps,
                        int warm_start, const double* d_x_init, const double* d_xhat_init, const double* d_dhat_init,
@@ -401,6 +421,15 @@ int carmpc_closed_loop(void* qp, int mode, const double* h_A, const double* h_B,
                        const carmpc_loop_noise* noise, const double* h_monitor_Ab, int monitor_rows,
                        int32_t* d_violation_step, int32_t* d_violation_row, int32_t* d_violations_per_step,
                        int64_t* h_total_iters, void* stream);
+
+int carmpc_closed_loop_goal(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C, const double* h_L,
+                            const carmpc_disturbance_model* dm, const double* h_xref, double dt, double l1, int steps,
+                            int warm_start, const double* d_x_init, const double* d_xhat_init, const double* d_dhat_init,
+                            const double* d_d_plant, int64_t runs, double* d_final, double* d_dhat_final,
+                            int32_t* d_fail_step, double* d_traj, double* d_u_log, double* d_dhat_log,
+                            const carmpc_loop_noise* noise, const double* h_monitor_Ab, int monitor_rows,
+                            int32_t* d_violation_step, int32_t* d_violation_row, int32_t* d_violations_per_step,
+                            const carmpc_loop_goal* goal, int64_t* h_total_iters, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Device micro-benchmarks used as roofline denominators that MEASURED_PEAKS.json does not carry.

@@ -36,10 +36,10 @@ class LoopNoiseParams(ctypes.Structure):
                 ("Lv", ctypes.c_double * 16)]
 
 
-class LoopGoal(ctypes.Structure):
-    """``carmpc_loop_goal`` (include/carmpc.h)."""
-    _fields_ = [("h_Ab", ctypes.c_void_p), ("rows", ctypes.c_int32), ("d_arrival_step", ctypes.c_void_p),
-                ("d_arrivals_per_step", ctypes.c_void_p)]
+class LoopRows(ctypes.Structure):
+    """``carmpc_loop_rows`` (include/carmpc.h): the rows and outputs of a closed loop's monitor or goal."""
+    _fields_ = [("h_Ab", ctypes.c_void_p), ("rows", ctypes.c_int32), ("d_step", ctypes.c_void_p),
+                ("d_row", ctypes.c_void_p), ("d_per_step", ctypes.c_void_p)]
 
 
 _vp, _dp, _i64, _i32 = ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int
@@ -86,11 +86,8 @@ SIGNATURES = {
     "carmpc_qp_tensor_mode": (_i32, [_vp, _i32, ctypes.POINTER(_i64)]),
     "carmpc_closed_loop": (_i32, [_vp, _i32, _dp, _dp, _dp, _dp, ctypes.POINTER(DisturbanceModel), _dp, ctypes.c_double,
                                   ctypes.c_double, _i32, _i32, _dp, _dp, _dp, _dp, _i64, _dp, _dp, _vp, _dp, _dp, _dp,
-                                  ctypes.POINTER(LoopNoiseParams), _dp, _i32, _vp, _vp, _vp, ctypes.POINTER(_i64), _vp]),
-    "carmpc_closed_loop_goal": (_i32, [_vp, _i32, _dp, _dp, _dp, _dp, ctypes.POINTER(DisturbanceModel), _dp,
-                                       ctypes.c_double, ctypes.c_double, _i32, _i32, _dp, _dp, _dp, _dp, _i64, _dp, _dp,
-                                       _vp, _dp, _dp, _dp, ctypes.POINTER(LoopNoiseParams), _dp, _i32, _vp, _vp, _vp,
-                                       ctypes.POINTER(LoopGoal), ctypes.POINTER(_i64), _vp]),
+                                  ctypes.POINTER(LoopNoiseParams), ctypes.POINTER(LoopRows), ctypes.POINTER(LoopRows),
+                                  ctypes.POINTER(_i64), _vp]),
     "carmpc_measure_peak": (_i32, [_i32, ctypes.POINTER(ctypes.c_double)]),
 }
 

@@ -513,7 +513,7 @@ class BatchQP(_Handle):
 
     def _closed_loop(self, mode, x_init, steps, A, B, C, L, dm, x_ref, dt, l1, warm_start, xhat_init, dhat_init, d_plant,
                      want_traj, want_inputs, want_dhat, noise, monitor, goal, stream) -> dict:
-        """``carmpc_closed_loop_goal`` in ``mode`` 0, 1 or 2 (``dm``: a ``DisturbanceModel``): checks the device inputs,
+        """``carmpc_closed_loop`` in ``mode`` 0, 1 or 2 (``dm``: a ``DisturbanceModel``): checks the device inputs,
         then returns the outputs the ``want_*`` flags, the mode, the monitor and the goal ask for, and ``total_iters``."""
         torch = _torch()
         if not (x_init.is_cuda and x_init.dtype == torch.float64 and x_init.dim() == 2 and x_init.shape[0] == 4
@@ -554,19 +554,21 @@ class BatchQP(_Handle):
         def p(key):
             return out[key].data_ptr() if key in out else None
 
-        g = None
-        if goal_rows is not None:
-            g = _capi.LoopGoal(goal_rows.ctypes.data, len(goal_rows), p("arrival_step"), p("arrivals_per_step"))
+        def loop_rows(Ab, step, row, per_step):
+            if Ab is None:
+                return None
+            return ctypes.byref(_capi.LoopRows(Ab.ctypes.data, len(Ab), p(step), p(row), p(per_step)))
+
         total = ctypes.c_int64(0)
-        check(self._lib.carmpc_closed_loop_goal(
+        check(self._lib.carmpc_closed_loop(
             self._h, mode, _capi.ptr(A_), _capi.ptr(B_), _capi.ptr(C_), _capi.ptr(L_),
             ctypes.byref(dm) if dm is not None else None, _capi.ptr(xref), float(dt), float(l1), int(steps),
             int(warm_start), x_init.data_ptr(), xhat_init.data_ptr() if xhat_init is not None else None,
             dhat_init.data_ptr() if dhat_init is not None else None, d_plant.data_ptr() if d_plant is not None else None,
             R, p("final"), p("dhat"), p("fail_step"), p("traj"), p("inputs"), p("dhat_traj"),
-            ctypes.byref(params) if params is not None else None, _capi.ptr(rows), len(rows) if rows is not None else 0,
-            p("violation_step"), p("violation_row"), p("violations_per_step"), ctypes.byref(g) if g is not None else None,
-            ctypes.byref(total), _stream_ptr(stream)))
+            ctypes.byref(params) if params is not None else None,
+            loop_rows(rows, "violation_step", "violation_row", "violations_per_step"),
+            loop_rows(goal_rows, "arrival_step", None, "arrivals_per_step"), ctypes.byref(total), _stream_ptr(stream)))
         out["total_iters"] = int(total.value)
         return out
 

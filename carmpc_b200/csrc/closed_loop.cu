@@ -56,27 +56,37 @@ struct LoopNoise {
     double Lw[16], Lv[16];
 };
 
-// Monitor rows (a loop-owned device copy, rows x 5) and its outputs (each nullable).
-struct LoopMonitor {
+// A monitor's or a goal's row set on the device (carmpc_loop_rows): the rows in a loop-owned copy, rows x 5, and the
+// outputs.
+struct LoopRows {
     const double* Ab;
     int rows;
-    int32_t* violation_step;        // runs: first step whose state violates a row, -1 none
-    int32_t* violation_row;         // runs: lowest violated row at that step, -1 none
-    int32_t* per_step;              // steps: runs violating at the step
+    int32_t* step;                  // runs: monitor - first step whose state violates a row; goal - arrival step; -1 none
+    int32_t* row;                   // runs (monitor only, nullable): lowest violated row at that step, -1 none
+    int32_t* per_step;              // steps (nullable): runs violating / arriving at the step
 };
 
-// Goal rows (a loop-owned device copy, rows x 5), the pending verdict of the rows (loop-owned) and the outputs.
-struct LoopGoal {
-    const double* Ab;
-    int rows;
-    uint8_t* inside;                // runs: the state of this step satisfied every row (read once its QP is known)
-    int32_t* arrival_step;          // runs: step of arrival, -1 none
-    int32_t* per_step;              // steps (nullable): runs arriving at the step
-};
+// K1's mode-0 chain: the first row the state violates, -1 none.  A NaN never satisfies <=.
+__device__ __forceinline__ int first_violated(const LoopRows& R, const double s[4]) {
+    for (int r = 0; r < R.rows; ++r) {
+        const double* a = R.Ab + 5 * r;
+        const double lhs = fma(__ldg(a + 3), s[3], fma(__ldg(a + 2), s[2], fma(__ldg(a + 1), s[1], __ldg(a) * s[0])));
+        if (!(lhs <= __ldg(a + 4))) return r;
+    }
+    return -1;
+}
+
+// per_step[step] += the threads with hit, one atomic per warp (and per group of threads that arrive together)
+__device__ __forceinline__ void count_per_warp(int32_t* per_step, int step, bool hit) {
+    const unsigned act = __activemask();
+    const unsigned h = __ballot_sync(act, hit);
+    if (h != 0 && (int)(threadIdx.x & 31) == __ffs(act) - 1) atomicAdd(per_step + step, __popc(h));
+}
 
 // plant step with the previous input, observer update, estimate -> QP input; builds the list of live runs.
 // kNoise / kMonitor / kGoal: process and measurement noise, monitor rows, goal rows; step is the step number of
-// host-driven steps.
+// host-driven steps.  kGoal: inside (loop-owned, runs) keeps whether the state of this step is inside the goal until
+// loop_apply_kernel knows its QP.
 template <bool kNoise, bool kMonitor, bool kGoal>
 __global__ void __launch_bounds__(256)
 loop_advance_kernel(const LoopConst K, int64_t runs, double* __restrict__ x, double* __restrict__ xhat,
@@ -84,7 +94,7 @@ loop_advance_kernel(const LoopConst K, int64_t runs, double* __restrict__ x, dou
                     double* __restrict__ est, int* __restrict__ live_list, int* __restrict__ live_count,
                     double* __restrict__ traj_step, const int* __restrict__ step_dev,
                     double* __restrict__ dhat, const double* __restrict__ d_plant, const LoopNoise N,
-                    const LoopMonitor M, int step, const LoopGoal G) {
+                    const LoopRows M, int step, const LoopRows G, uint8_t* inside) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= runs) return;
     // replayed steps (CUDA graph) read the step number on the device: traj_step is then the base of the trajectory
@@ -94,7 +104,7 @@ loop_advance_kernel(const LoopConst K, int64_t runs, double* __restrict__ x, dou
     double s[4], u[2];
 #pragma unroll
     for (int c = 0; c < 4; ++c) s[c] = x[c * runs + i];
-    const bool alive = fail_step[i] < 0 && (!kGoal || G.arrival_step[i] < 0);
+    const bool alive = fail_step[i] < 0 && (!kGoal || G.step[i] < 0);
     if (alive) {
         u[0] = u_prev[i];
         u[1] = u_prev[runs + i];
@@ -134,29 +144,17 @@ loop_advance_kernel(const LoopConst K, int64_t runs, double* __restrict__ x, dou
 #pragma unroll
         for (int c = 0; c < 4; ++c) x[c * runs + i] = s[c];
         if (kMonitor) {
-            // K1's mode-0 chain; a NaN never satisfies <=, so a non-finite state violates the first row
-            int bad = -1;
-            for (int r = 0; r < M.rows; ++r) {
-                const double* a = M.Ab + 5 * r;
-                const double lhs = fma(__ldg(a + 3), s[3], fma(__ldg(a + 2), s[2], fma(__ldg(a + 1), s[1], __ldg(a) * s[0])));
-                if (!(lhs <= __ldg(a + 4))) { bad = r; break; }
-            }
+            // a non-finite state violates the first row
+            const int bad = first_violated(M, s);
             viol = bad >= 0;
             if (viol) {
-                if (M.violation_step != nullptr && M.violation_step[i] < 0) M.violation_step[i] = step;
-                if (M.violation_row != nullptr && M.violation_row[i] < 0) M.violation_row[i] = bad;
+                if (M.step != nullptr && M.step[i] < 0) M.step[i] = step;
+                if (M.row != nullptr && M.row[i] < 0) M.row[i] = bad;
             }
         }
-        if (kGoal) {
-            // the monitor's chain; a non-finite state is never inside (an infinite coordinate may satisfy a row)
-            bool in = isfinite(s[0]) && isfinite(s[1]) && isfinite(s[2]) && isfinite(s[3]);
-            for (int r = 0; in && r < G.rows; ++r) {
-                const double* a = G.Ab + 5 * r;
-                const double lhs = fma(__ldg(a + 3), s[3], fma(__ldg(a + 2), s[2], fma(__ldg(a + 1), s[1], __ldg(a) * s[0])));
-                in = lhs <= __ldg(a + 4);
-            }
-            G.inside[i] = in ? 1 : 0;
-        }
+        // a non-finite state is never inside (an infinite coordinate may satisfy a row)
+        if (kGoal)
+            inside[i] = isfinite(s[0]) && isfinite(s[1]) && isfinite(s[2]) && isfinite(s[3]) && first_violated(G, s) == -1;
         double e[4];
         if (K.mode == 2) {
             // augmented observer: y = C s + Cd_p d_r measured, innovation against C x^ + Cd d^
@@ -220,12 +218,7 @@ loop_advance_kernel(const LoopConst K, int64_t runs, double* __restrict__ x, dou
         for (int c = 0; c < 4; ++c) est[c * runs + i] = e[c];
         live_list[atomicAdd(live_count, 1)] = (int)i;
     }
-    if (kMonitor && M.per_step != nullptr) {
-        // one atomic per warp (and per group of threads that arrive together)
-        const unsigned act = __activemask();
-        const unsigned hit = __ballot_sync(act, viol);
-        if (hit != 0 && (int)(threadIdx.x & 31) == __ffs(act) - 1) atomicAdd(M.per_step + step, __popc(hit));
-    }
+    if (kMonitor && M.per_step != nullptr) count_per_warp(M.per_step, step, viol);
     if (traj_step != nullptr) {
 #pragma unroll
         for (int c = 0; c < 4; ++c) traj_step[c * runs + i] = s[c];
@@ -238,7 +231,8 @@ template <bool kGoal>
 __global__ void __launch_bounds__(256)
 loop_apply_kernel(int64_t runs, int step, const int* __restrict__ live_list, int live, const int* __restrict__ live_dev,
                   const double* __restrict__ u0, const int32_t* __restrict__ status, double* __restrict__ u_prev,
-                  int32_t* __restrict__ fail_step, const int* __restrict__ step_dev, const LoopGoal G) {
+                  int32_t* __restrict__ fail_step, const int* __restrict__ step_dev, const LoopRows G,
+                  const uint8_t* inside) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (live_dev != nullptr) live = min(live, *live_dev);
     if (step_dev != nullptr) step = *step_dev;
@@ -246,8 +240,8 @@ loop_apply_kernel(int64_t runs, int step, const int* __restrict__ live_list, int
     const int i = live_list[q];
     bool arrived = false;
     if (status[i] == CARMPC_QP_SOLVED) {
-        if (kGoal && G.inside[i]) {
-            G.arrival_step[i] = step;
+        if (kGoal && inside[i]) {
+            G.step[i] = step;
             arrived = true;
         } else {
             u_prev[i] = u0[i];
@@ -256,12 +250,7 @@ loop_apply_kernel(int64_t runs, int step, const int* __restrict__ live_list, int
     } else {
         fail_step[i] = step;
     }
-    if (kGoal && G.per_step != nullptr) {
-        // one atomic per warp, as the monitor's count
-        const unsigned act = __activemask();
-        const unsigned hit = __ballot_sync(act, arrived);
-        if (hit != 0 && (int)(threadIdx.x & 31) == __ffs(act) - 1) atomicAdd(G.per_step + step, __popc(hit));
-    }
+    if (kGoal && G.per_step != nullptr) count_per_warp(G.per_step, step, arrived);
 }
 
 // replayed steps: the input (and disturbance-estimate) logs of this step, then the step number moves on (one thread, after
@@ -295,21 +284,27 @@ struct LoopDisturbance {
     double* dhat_log;
 };
 
-// Noise and monitor of a run set: noise == nullptr draws none; monitor_rows == 0 checks none (outputs then null).
-struct LoopStochastic {
-    const LoopNoise* noise;
-    const double* h_monitor_Ab;
-    int monitor_rows;
-    int32_t* violation_step;
-    int32_t* violation_row;
-    int32_t* violations_per_step;
-};
+// The device side of a row set (h == nullptr: none, *d all null): the rows copied into the loop-owned buffer *Ab, the step
+// and row outputs set to -1, the per-step count to 0.
+cudaError_t rows_to_device(const carmpc_loop_rows* h, int64_t runs, int steps, cudaStream_t st, double** Ab, LoopRows* d) {
+    *d = {nullptr, 0, nullptr, nullptr, nullptr};
+    if (h == nullptr) return cudaSuccess;
+    cudaError_t e = cudaMalloc(Ab, sizeof(double) * 5 * h->rows);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(*Ab, h->h_Ab, sizeof(double) * 5 * h->rows, cudaMemcpyHostToDevice, st);
+    if (e != cudaSuccess) return e;
+    const int blocks = (int)((runs + 255) / 256);
+    if (h->d_step) fill_i32<<<blocks, 256, 0, st>>>(h->d_step, runs, -1);
+    if (h->d_row) fill_i32<<<blocks, 256, 0, st>>>(h->d_row, runs, -1);
+    if (h->d_per_step && steps > 0) e = cudaMemsetAsync(h->d_per_step, 0, sizeof(int32_t) * steps, st);
+    *d = {*Ab, h->rows, h->d_step, h->d_row, h->d_per_step};
+    return e;
+}
 
 // The loop shared by every mode: host-driven first steps, then one captured CUDA graph with the step number on the device.
 int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int steps, int warm_start, const double* d_x_init,
                     const double* d_xhat_init, int64_t runs, double* d_final, int32_t* d_fail_step, double* d_traj,
-                    double* d_u_log, const LoopDisturbance& D, const LoopStochastic& Z, const carmpc_loop_goal* goal,
-                    int64_t* h_total_iters, void* stream) {
+                    double* d_u_log, const LoopDisturbance& D, const carmpc_loop_noise* noise,
+                    const carmpc_loop_rows* monitor, const carmpc_loop_rows* goal, int64_t* h_total_iters, void* stream) {
     if (q->host_only) { set_error("carmpc_closed_loop: this QP handle was created without a CUDA device"); return CARMPC_ERR_CUDA; }
     QPBusyGuard guard(q->busy);
     CARMPC_REQUIRE(guard.acquired, "this QP handle is in use by another call (one call per handle at a time)");
@@ -361,37 +356,29 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
     TRY(cudaMemsetAsync(u_prev, 0, sizeof(double) * 2 * runs, st));
     const int blocks = (int)((runs + 255) / 256);
     fill_i32<<<blocks, 256, 0, st>>>(d_fail_step, runs, -1);
-    // noise and monitor: kernel arguments by value (a captured graph keeps them), the rows in a buffer the loop owns
-    LoopNoise noise;
-    memset(&noise, 0, sizeof(noise));
-    if (Z.noise != nullptr) noise = *Z.noise;
-    LoopMonitor mon = {nullptr, 0, Z.violation_step, Z.violation_row, Z.violations_per_step};
-    if (Z.monitor_rows > 0) {
-        TRY(cudaMalloc(&monitor_Ab, sizeof(double) * 5 * Z.monitor_rows));
-        TRY(cudaMemcpyAsync(monitor_Ab, Z.h_monitor_Ab, sizeof(double) * 5 * Z.monitor_rows, cudaMemcpyHostToDevice, st));
-        mon.Ab = monitor_Ab;
-        mon.rows = Z.monitor_rows;
-        if (mon.violation_step) fill_i32<<<blocks, 256, 0, st>>>(mon.violation_step, runs, -1);
-        if (mon.violation_row) fill_i32<<<blocks, 256, 0, st>>>(mon.violation_row, runs, -1);
-        if (mon.per_step && steps > 0) TRY(cudaMemsetAsync(mon.per_step, 0, sizeof(int32_t) * steps, st));
+    // noise, monitor and goal: kernel arguments by value (a captured graph keeps them); the rows and the goal's pending
+    // verdict in buffers the loop owns, fixed addresses like every other buffer of the step
+    LoopNoise nz;
+    memset(&nz, 0, sizeof(nz));
+    if (noise != nullptr) {
+        nz.seed = noise->seed;
+        nz.first_run = noise->first_run;
+        memcpy(nz.Lw, noise->Lw, sizeof(nz.Lw));
+        memcpy(nz.Lv, noise->Lv, sizeof(nz.Lv));
     }
-    // goal: rows and the pending verdict in buffers the loop owns, fixed addresses like every other buffer of the step
-    LoopGoal gl = {nullptr, 0, nullptr, nullptr, nullptr};
+    LoopRows mon, gl;
+    TRY(rows_to_device(monitor, runs, steps, st, &monitor_Ab, &mon));
+    TRY(rows_to_device(goal, runs, steps, st, &goal_Ab, &gl));
     if (goal != nullptr) {
-        TRY(cudaMalloc(&goal_Ab, sizeof(double) * 5 * goal->rows));
         TRY(cudaMalloc(&inside, runs));
-        TRY(cudaMemcpyAsync(goal_Ab, goal->h_Ab, sizeof(double) * 5 * goal->rows, cudaMemcpyHostToDevice, st));
         TRY(cudaMemsetAsync(inside, 0, runs, st));
-        gl = {goal_Ab, goal->rows, inside, goal->d_arrival_step, goal->d_arrivals_per_step};
-        fill_i32<<<blocks, 256, 0, st>>>(gl.arrival_step, runs, -1);
-        if (gl.per_step && steps > 0) TRY(cudaMemsetAsync(gl.per_step, 0, sizeof(int32_t) * steps, st));
     }
-    const bool with_noise = Z.noise != nullptr, with_monitor = Z.monitor_rows > 0, with_goal = goal != nullptr;
+    const bool with_noise = noise != nullptr, with_monitor = monitor != nullptr, with_goal = goal != nullptr;
     auto advance = [&](int k, double* traj_step, const int* step_dev) {
         auto kern = with_noise ? (with_monitor ? advance_variant<true, true>(with_goal) : advance_variant<true, false>(with_goal))
                                : (with_monitor ? advance_variant<false, true>(with_goal) : advance_variant<false, false>(with_goal));
         kern<<<blocks, 256, 0, st>>>(K, runs, x, xhat, u_prev, d_fail_step, est, live_list, live_count, traj_step, step_dev,
-                                     dhat, D.d_plant, noise, mon, k, gl);
+                                     dhat, D.d_plant, nz, mon, k, gl, inside);
     };
     auto apply = with_goal ? loop_apply_kernel<true> : loop_apply_kernel<false>;
     int64_t total_iters = 0;
@@ -414,7 +401,7 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
         r.count = runs; r.count_dev = live_count; r.warm_in = 1;
         const int rc2 = q->solve_enqueue(r, st);
         if (rc2 != CARMPC_OK) return rc2;
-        apply<<<blocks, 256, 0, st>>>(runs, k, live_list, (int)runs, live_count, u0, status, u_prev, d_fail_step, step_dev, gl);
+        apply<<<blocks, 256, 0, st>>>(runs, k, live_list, (int)runs, live_count, u0, status, u_prev, d_fail_step, step_dev, gl, inside);
         if (step_dev) {
             if (d_u_log || D.dhat_log)
                 loop_log_kernel<<<(int)((2 * runs + 255) / 256), 256, 0, st>>>(runs, u_prev, d_u_log, dhat, D.dhat_log, step_dev);
@@ -473,7 +460,7 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
             rc = q->solve(req, st);
             if (rc != CARMPC_OK) { cleanup(); return rc; }
             warm_valid = warm != nullptr;
-            apply<<<(live + 255) / 256, 256, 0, st>>>(runs, k, live_list, live, nullptr, u0, status, u_prev, d_fail_step, nullptr, gl);
+            apply<<<(live + 255) / 256, 256, 0, st>>>(runs, k, live_list, live, nullptr, u0, status, u_prev, d_fail_step, nullptr, gl, inside);
         }
         if (d_u_log)      // the input each run will apply at the next plant step (unchanged for stopped runs)
             TRY(cudaMemcpyAsync(d_u_log + (size_t)k * 2 * runs, u_prev, sizeof(double) * 2 * runs, cudaMemcpyDeviceToDevice, st));
@@ -491,20 +478,34 @@ int closed_loop_run(QPHandle* q, const LoopConst& K, const double* h_xref, int s
     return CARMPC_OK;
 }
 
+// The checks of a monitor's or a goal's row set (nullptr: none); a goal needs d_step and has no d_row.
+int check_rows(const carmpc_loop_rows* R, bool goal) {
+    if (R == nullptr) return CARMPC_OK;
+    const char* use = goal ? "goal" : "monitor";
+#define ROWS_REQUIRE(cond, fmt) do { if (!(cond)) { set_error("invalid argument: " fmt, use); return CARMPC_ERR_INVALID; } } while (0)
+    ROWS_REQUIRE(R->rows >= 1 && R->rows <= 512, "%s rows must be in [1, 512]");
+    ROWS_REQUIRE(R->h_Ab != nullptr, "null %s rows");
+    bool finite = true;
+    for (int j = 0; j < 5 * R->rows; ++j) finite = finite && isfinite(R->h_Ab[j]);
+    ROWS_REQUIRE(finite, "%s rows must be finite");
+    ROWS_REQUIRE(!goal || R->d_step != nullptr, "a %s needs d_step");
+    ROWS_REQUIRE(!goal || R->d_row == nullptr, "a %s has no d_row");
+#undef ROWS_REQUIRE
+    return CARMPC_OK;
+}
+
 }  // namespace
 }  // namespace carmpc
 
 using namespace carmpc;
 
-extern "C" int carmpc_closed_loop_goal(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C,
-                                       const double* h_L, const carmpc_disturbance_model* dm, const double* h_xref,
-                                       double dt, double l1, int steps, int warm_start, const double* d_x_init,
-                                       const double* d_xhat_init, const double* d_dhat_init, const double* d_d_plant,
-                                       int64_t runs, double* d_final, double* d_dhat_final, int32_t* d_fail_step,
-                                       double* d_traj, double* d_u_log, double* d_dhat_log, const carmpc_loop_noise* noise,
-                                       const double* h_monitor_Ab, int monitor_rows, int32_t* d_violation_step,
-                                       int32_t* d_violation_row, int32_t* d_violations_per_step,
-                                       const carmpc_loop_goal* goal, int64_t* h_total_iters, void* stream) {
+extern "C" int carmpc_closed_loop(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C,
+                                  const double* h_L, const carmpc_disturbance_model* dm, const double* h_xref, double dt,
+                                  double l1, int steps, int warm_start, const double* d_x_init, const double* d_xhat_init,
+                                  const double* d_dhat_init, const double* d_d_plant, int64_t runs, double* d_final,
+                                  double* d_dhat_final, int32_t* d_fail_step, double* d_traj, double* d_u_log,
+                                  double* d_dhat_log, const carmpc_loop_noise* noise, const carmpc_loop_rows* monitor,
+                                  const carmpc_loop_rows* goal, int64_t* h_total_iters, void* stream) {
     QPHandle* q = check_handle<QPHandle>(qp, kQP);
     CARMPC_REQUIRE(q != nullptr, "not a QP handle");
     CARMPC_REQUIRE(mode >= 0 && mode <= 2, "mode must be 0 (state feedback), 1 (output feedback) or 2 (with a disturbance estimate)");
@@ -529,21 +530,9 @@ extern "C" int carmpc_closed_loop_goal(void* qp, int mode, const double* h_A, co
         CARMPC_REQUIRE(finite, "noise factors Lw, Lv must be finite");
         CARMPC_REQUIRE(noise->first_run >= 0 && noise->first_run <= INT64_MAX - runs, "first_run must be >= 0");
     }
-    if (h_monitor_Ab != nullptr) {
-        CARMPC_REQUIRE(monitor_rows >= 1 && monitor_rows <= 512, "monitor_rows must be in [1, 512]");
-        for (int j = 0; j < 5 * monitor_rows; ++j) finite = finite && isfinite(h_monitor_Ab[j]);
-        CARMPC_REQUIRE(finite, "monitor rows must be finite");
-    } else {
-        CARMPC_REQUIRE(monitor_rows == 0, "monitor_rows without monitor rows");
-        CARMPC_REQUIRE(!d_violation_step && !d_violation_row && !d_violations_per_step, "monitor outputs without monitor rows");
-    }
-    if (goal != nullptr) {
-        CARMPC_REQUIRE(goal->rows >= 1 && goal->rows <= 512, "goal rows must be in [1, 512]");
-        CARMPC_REQUIRE(goal->h_Ab != nullptr, "null goal rows");
-        for (int j = 0; j < 5 * goal->rows; ++j) finite = finite && isfinite(goal->h_Ab[j]);
-        CARMPC_REQUIRE(finite, "goal rows must be finite");
-        CARMPC_REQUIRE(goal->d_arrival_step != nullptr, "a goal needs d_arrival_step");
-    }
+    int rc = check_rows(monitor, false);
+    if (rc == CARMPC_OK) rc = check_rows(goal, true);
+    if (rc != CARMPC_OK) return rc;
     if (h_total_iters) *h_total_iters = 0;
     if (runs == 0) return CARMPC_OK;
     CARMPC_REQUIRE(d_x_init && d_final && d_fail_step, "null device pointer");
@@ -564,29 +553,6 @@ extern "C" int carmpc_closed_loop_goal(void* qp, int mode, const double* h_A, co
         D = {d_dhat_init, d_d_plant, d_dhat_final, d_dhat_log};
     }
     K.dt = dt; K.l1 = l1; K.mode = mode;
-    LoopNoise nz;
-    if (noise != nullptr) {
-        nz.seed = noise->seed;
-        nz.first_run = noise->first_run;
-        memcpy(nz.Lw, noise->Lw, sizeof(nz.Lw));
-        memcpy(nz.Lv, noise->Lv, sizeof(nz.Lv));
-    }
-    const LoopStochastic Z = {noise ? &nz : nullptr, h_monitor_Ab, h_monitor_Ab ? monitor_rows : 0, d_violation_step,
-                              d_violation_row, d_violations_per_step};
     return closed_loop_run(q, K, h_xref, steps, warm_start, d_x_init, d_xhat_init, runs, d_final, d_fail_step, d_traj, d_u_log,
-                           D, Z, goal, h_total_iters, stream);
-}
-
-extern "C" int carmpc_closed_loop(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C,
-                                  const double* h_L, const carmpc_disturbance_model* dm, const double* h_xref, double dt,
-                                  double l1, int steps, int warm_start, const double* d_x_init, const double* d_xhat_init,
-                                  const double* d_dhat_init, const double* d_d_plant, int64_t runs, double* d_final,
-                                  double* d_dhat_final, int32_t* d_fail_step, double* d_traj, double* d_u_log,
-                                  double* d_dhat_log, const carmpc_loop_noise* noise, const double* h_monitor_Ab,
-                                  int monitor_rows, int32_t* d_violation_step, int32_t* d_violation_row,
-                                  int32_t* d_violations_per_step, int64_t* h_total_iters, void* stream) {
-    return carmpc_closed_loop_goal(qp, mode, h_A, h_B, h_C, h_L, dm, h_xref, dt, l1, steps, warm_start, d_x_init,
-                                   d_xhat_init, d_dhat_init, d_d_plant, runs, d_final, d_dhat_final, d_fail_step, d_traj,
-                                   d_u_log, d_dhat_log, noise, h_monitor_Ab, monitor_rows, d_violation_step,
-                                   d_violation_row, d_violations_per_step, nullptr, h_total_iters, stream);
+                           D, noise, monitor, goal, h_total_iters, stream);
 }

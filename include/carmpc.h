@@ -373,27 +373,25 @@ int carmpc_qp_tensor_mode(void* qp, int mode, int64_t* h_info);
  *   ua = ((x0 >> 11) + 1) 2^-53,  ub = (x1 >> 11) 2^-53,  z0 = sqrt(-2 ln ua) cos(2 pi ub),  z1 = ... sin(2 pi ub).
  * The draws depend only on (seed, first_run + run, k, j): not on the batch, warm_start or which runs still run, so a run
  * set split over calls (first_run = the offset of each part) draws what one call would.
- * h_monitor_Ab (nullable: no monitor): host rows x 5, 1 <= monitor_rows <= 512, finite.  A violation never stops a run.
- * The monitor outputs are nullable and need rows: d_violation_step / d_violation_row (runs int32, -1 none): the first
- * step with a violation and the lowest violated row (caller's order) at that step.  d_violations_per_step (steps
- * int32): runs violating at step k.  Stopped runs are neither moved nor counted; a run whose QP fails at step k was
- * moved and checked at step k.
- * Noise and monitor are compile-time switches of the step kernel: a loop without them pays nothing for them.
- * goal (carmpc_closed_loop_goal only; nullable: runs never stop at a goal): runs that reach a goal stop there, as the
- * reference's loops break on  all(|state - goal| <= 0.1).  h_Ab: host rows x 5 [a | b], 1 <= rows <= 512, finite (the
- * loop copies them).  At step k the run is inside when s (the true state above, after the Euler step, Bd_plant d_r and
- * the process noise) is finite and satisfies every row with the monitor's chain.  The initial state is not tested.  The
- * run still solves its step-k QP, and then:
- *   QP not solved               d_fail_step = k, d_arrival_step stays -1 (the reference raises before its goal test);
- *   QP solved and s inside      d_arrival_step = k; the step-k input is not applied (d_u_log keeps the previous input,
- *                               as for a failed run), d_final = s, and the run is never moved, observed, solved,
- *                               monitored or counted again.
- * A run is running while d_fail_step < 0 and d_arrival_step < 0.  d_arrival_step (runs int32, required): -1 or the
- * step of arrival.  d_arrivals_per_step (steps int32, nullable): runs arriving at step k.  Replayed steps read k on the
- * device; nothing of the goal is read back to the host.
- * CARMPC_ERR_INVALID for non-finite factors or gains, first_run < 0, bad monitor rows, monitor outputs without rows, mode
- * 2 without dm, bad or null goal rows, a goal without d_arrival_step; CARMPC_ERR_CUDA on a handle created without a
- * device.  carmpc_closed_loop is carmpc_closed_loop_goal with goal = NULL. */
+ * monitor and goal (each nullable: none) are row sets carmpc_loop_rows: h_Ab, host rows x 5 [a | b], 1 <= rows <= 512,
+ * finite (the loop copies them), tested on s with the chain above.  The loop sets d_step and d_row (runs int32) to -1
+ * and d_per_step (steps int32) to 0 before the first step.  Stopped runs are neither moved nor tested nor counted.
+ *   monitor: a violation (s fails a row) never stops a run.  d_step (nullable): the first step with a violation;
+ *     d_row (runs int32, nullable): the lowest violated row (caller's order) at that step, -1 none; d_per_step: runs
+ *     violating at step k.  A run whose QP fails at step k was moved and checked at step k.
+ *   goal: runs that reach it stop there, as the reference's loops break on  all(|state - goal| <= 0.1).  At step k the
+ *     run is inside when s is finite and satisfies every row.  The initial state is not tested.  The run still solves
+ *     its step-k QP, and then:
+ *       QP not solved               d_fail_step = k, d_step stays -1 (the reference raises before its goal test);
+ *       QP solved and s inside      d_step = k; the step-k input is not applied (d_u_log keeps the previous input, as
+ *                                   for a failed run), d_final = s, and the run is never moved, observed, solved,
+ *                                   monitored or counted again.
+ *     A run is running while d_fail_step < 0 and the goal's d_step < 0.  d_step is required and d_row must be NULL;
+ *     d_per_step: runs arriving at step k.  Replayed steps read k on the device; nothing of the goal is read back to
+ *     the host.
+ * Noise, monitor and goal are compile-time switches of the step kernels: a loop without them pays nothing for them.
+ * CARMPC_ERR_INVALID for non-finite factors or gains, first_run < 0, mode 2 without dm, bad or null rows of a monitor or
+ * a goal, a goal without d_step or with d_row; CARMPC_ERR_CUDA on a handle created without a device. */
 typedef struct carmpc_disturbance_model {
     double Bd[4], Cd[3], L1[12], L2[3];   /* controller: disturbance model and observer gains (L1 4x3 row-major) */
     double Bd_plant[4], Cd_plant[3];      /* how the true per-run disturbance enters the plant state / output    */
@@ -406,30 +404,21 @@ typedef struct carmpc_loop_noise {
     double Lv[16];          /* measurement-noise factor, 4 x 4 row-major: v = Lv z_v */
 } carmpc_loop_noise;
 
-typedef struct carmpc_loop_goal {
-    const double* h_Ab;              /* rows x 5 [a | b], host */
-    int32_t rows;                    /* 1..512 */
-    int32_t* d_arrival_step;         /* runs int32, required: step of arrival, -1 none */
-    int32_t* d_arrivals_per_step;    /* steps int32, nullable */
-} carmpc_loop_goal;
+typedef struct carmpc_loop_rows {
+    const double* h_Ab;     /* rows x 5 [a | b], host, copied by the loop */
+    int32_t rows;           /* 1..512 */
+    int32_t* d_step;        /* runs int32: monitor - first violating step; goal - arrival step; -1 none */
+    int32_t* d_row;         /* runs int32, monitor only (nullable): lowest violated row at that step */
+    int32_t* d_per_step;    /* steps int32 (nullable): runs violating / arriving at step k */
+} carmpc_loop_rows;
 
 int carmpc_closed_loop(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C, const double* h_L,
                        const carmpc_disturbance_model* dm, const double* h_xref, double dt, double l1, int steps,
                        int warm_start, const double* d_x_init, const double* d_xhat_init, const double* d_dhat_init,
                        const double* d_d_plant, int64_t runs, double* d_final, double* d_dhat_final,
                        int32_t* d_fail_step, double* d_traj, double* d_u_log, double* d_dhat_log,
-                       const carmpc_loop_noise* noise, const double* h_monitor_Ab, int monitor_rows,
-                       int32_t* d_violation_step, int32_t* d_violation_row, int32_t* d_violations_per_step,
+                       const carmpc_loop_noise* noise, const carmpc_loop_rows* monitor, const carmpc_loop_rows* goal,
                        int64_t* h_total_iters, void* stream);
-
-int carmpc_closed_loop_goal(void* qp, int mode, const double* h_A, const double* h_B, const double* h_C, const double* h_L,
-                            const carmpc_disturbance_model* dm, const double* h_xref, double dt, double l1, int steps,
-                            int warm_start, const double* d_x_init, const double* d_xhat_init, const double* d_dhat_init,
-                            const double* d_d_plant, int64_t runs, double* d_final, double* d_dhat_final,
-                            int32_t* d_fail_step, double* d_traj, double* d_u_log, double* d_dhat_log,
-                            const carmpc_loop_noise* noise, const double* h_monitor_Ab, int monitor_rows,
-                            int32_t* d_violation_step, int32_t* d_violation_row, int32_t* d_violations_per_step,
-                            const carmpc_loop_goal* goal, int64_t* h_total_iters, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Device micro-benchmarks used as roofline denominators that MEASURED_PEAKS.json does not carry.

@@ -1,4 +1,4 @@
-"""CPU restatement of closed loops that stop at a goal (carmpc_closed_loop_goal), built on
+"""CPU restatement of closed loops that stop at a goal (carmpc_closed_loop with a goal), built on
 ``oracle/carmpc_oracle.py`` (used unchanged).
 
 TEST INFRASTRUCTURE ONLY.  ``closed_loop`` is ``oracle.carmpc_oracle.closed_loop`` with the goal test of the reference's

@@ -80,8 +80,7 @@ def _call(lib, qp, dm, runs=4, steps=3, warm_start=1, dt=0.2, l1=3.5, A=True, pt
     p = ctypes.c_void_p(ptr)
     return lib.carmpc_closed_loop(qp, 2, mat.ctypes.data if A else None, mat.ctypes.data, mat.ctypes.data, None,
                                   ctypes.byref(dm) if dm is not None else None, mat.ctypes.data, dt, l1, steps, warm_start,
-                                  p, None, None, None, runs, p, None, p, None, None, None, None, None, 0, None, None, None,
-                                  None, None)
+                                  p, None, None, None, runs, p, None, p, None, None, None, None, None, None, None, None)
 
 
 def _model():
@@ -118,7 +117,7 @@ def test_closed_loop_mode_2_argument_errors(ctl):
     mat = np.zeros(16)
     assert lib.carmpc_closed_loop(bq._h, 2, mat.ctypes.data, mat.ctypes.data, mat.ctypes.data, None, ctypes.byref(dm),
                                   mat.ctypes.data, 0.2, 3.5, 5, 1, None, None, None, None, 0, None, None, None, None, None,
-                                  None, None, None, 0, None, None, None, ctypes.byref(total), None) == 0
+                                  None, None, None, None, ctypes.byref(total), None) == 0
     assert total.value == 0
 
 

@@ -1,4 +1,4 @@
-"""Closed loops that stop at a goal, without a GPU: the argument checks of carmpc_closed_loop_goal, montecarlo.goal_box
+"""Closed loops that stop at a goal, without a GPU: the argument checks of carmpc_closed_loop's goal, montecarlo.goal_box
 against the reference's arrival test, and the oracle's derivation of arrival and failure steps from a trajectory."""
 import ctypes
 import math
@@ -9,7 +9,7 @@ import pytest
 from conftest import make_env, make_controller
 
 
-# ---- carmpc_closed_loop_goal argument checks ----------------------------------------------------------------------
+# ---- carmpc_closed_loop argument checks of the goal ---------------------------------------------------------------
 @pytest.fixture(scope="module")
 def handle():
     from carmpc_b200.batch import BatchQP
@@ -19,20 +19,20 @@ def handle():
 _BOX = np.array([[1.0, 0.0, 0.0, 0.0, 30.1], [-1.0, 0.0, 0.0, 0.0, -29.9]])
 
 
-def _call(lib, qp, goal, runs=4, steps=3):
+def _call(lib, qp, goal, runs=4, steps=3, monitor=None):
     mat = np.zeros(16)
     p = ctypes.c_void_p(16)
-    return lib.carmpc_closed_loop_goal(
+    return lib.carmpc_closed_loop(
         qp, 0, mat.ctypes.data, mat.ctypes.data, None, None, None, mat.ctypes.data, 0.2, 3.5, steps, 1, p, None, None,
-        None, runs, p, None, p, None, None, None, None, None, 0, None, None, None,
+        None, runs, p, None, p, None, None, None, None, ctypes.byref(monitor) if monitor is not None else None,
         ctypes.byref(goal) if goal is not None else None, None, None)
 
 
-def _goal(rows=_BOX, n=None, arrival=True, per_step=False):
+def _goal(rows=_BOX, n=None, arrival=True, row=False, per_step=False):
     from carmpc_b200 import _capi
     rows = np.ascontiguousarray(rows, dtype=np.float64) if rows is not None else None
-    g = _capi.LoopGoal(rows.ctypes.data if rows is not None else None, len(rows) if n is None else n,
-                       64 if arrival else None, 128 if per_step else None)
+    g = _capi.LoopRows(rows.ctypes.data if rows is not None else None, len(rows) if n is None else n,
+                       64 if arrival else None, 96 if row else None, 128 if per_step else None)
     g._keep = rows                       # the rows must outlive the call
     return g
 
@@ -45,7 +45,8 @@ def test_goal_argument_errors(handle):
     for runs in (0, 4):                     # checked before the early return of an empty run set
         assert _call(lib, h, _goal(n=0), runs=runs) == -1 and b"goal rows" in err()
         assert _call(lib, h, _goal(np.tile(_BOX, (257, 1)), n=513), runs=runs) == -1 and b"goal rows" in err()
-        assert _call(lib, h, _goal(arrival=False), runs=runs) == -1 and b"d_arrival_step" in err()
+        assert _call(lib, h, _goal(arrival=False), runs=runs) == -1 and b"a goal needs d_step" in err()
+        assert _call(lib, h, _goal(row=True), runs=runs) == -1 and b"a goal has no d_row" in err()
         assert _call(lib, h, _goal(rows=None, n=2), runs=runs) == -1 and b"null goal rows" in err()
         for bad in (math.nan, math.inf, -math.inf):
             for r, c in ((0, 4), (1, 0), (1, 3)):
@@ -59,6 +60,17 @@ def test_goal_argument_errors(handle):
 
 def _valid_goals():
     return (_goal(), _goal(per_step=True), _goal(np.tile(_BOX, (256, 1)), n=512), None)
+
+
+def test_monitor_and_goal_together_pass_the_checks(handle):
+    """One row set as the monitor (every output set) and another as the goal: valid together, each checked as its use."""
+    from carmpc_b200 import _capi
+    lib = _capi.load()
+    rows = np.ascontiguousarray(np.tile(_BOX, (2, 1)))
+    monitor = _capi.LoopRows(rows.ctypes.data, len(rows), 256, 320, 384)
+    assert _call(lib, handle._h, _goal(per_step=True), runs=0, monitor=monitor) == 0
+    assert _call(lib, handle._h, _goal(arrival=False), runs=0, monitor=monitor) == -1
+    assert b"a goal needs d_step" in lib.carmpc_last_error()
 
 
 def test_goal_loop_on_a_host_only_handle_is_a_cuda_error(handle):

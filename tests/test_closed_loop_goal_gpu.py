@@ -1,7 +1,7 @@
-"""Closed loops that stop at a goal (carmpc_closed_loop_goal) on the GPU: a goal that is never met changes nothing, bit
-for bit, in every mode and warm-start form; parity with the restated loop (exact QPs) on RoadEnv; at size (10^4 runs x
-200 steps, graph-replayed steps) the arrival and failure steps are those of the loop without a goal; the map by
-closed-loop convergence against the reference's own loop; the example end to end."""
+"""Closed loops that stop at a goal (carmpc_closed_loop with a goal) on the GPU: a goal that is never met changes
+nothing, bit for bit, in every mode and warm-start form; parity with the restated loop (exact QPs) on RoadEnv; at size
+(10^4 runs x 200 steps, graph-replayed steps) the arrival and failure steps are those of the loop without a goal; the
+map by closed-loop convergence against the reference's own loop; the example end to end."""
 import importlib
 import os
 import sys

@@ -151,23 +151,29 @@ def _noise(**kw):
 _ROWS = np.array([[0.0, 1.0, 0.0, 0.0, 2.5], [0.0, -1.0, 0.0, 0.0, 2.5]])
 
 
-def _call(lib, qp, mode=1, dm="model", noise="noise", rows=_ROWS, monitor_rows=None, outs=(True, True, True), runs=4,
-          steps=3, warm_start=1, dt=0.2, l1=3.5, C=True, L=True, ptr=16):
+def _monitor(rows=_ROWS, n=None):
+    from carmpc_b200 import _capi
+    rows = np.ascontiguousarray(rows) if rows is not None else None
+    m = _capi.LoopRows(rows.ctypes.data if rows is not None else None, len(rows) if n is None else n, 64, 96, 128)
+    m._keep = rows                       # the rows must outlive the call
+    return m
+
+
+def _call(lib, qp, mode=1, dm="model", noise="noise", monitor="monitor", runs=4, steps=3, warm_start=1, dt=0.2, l1=3.5,
+          C=True, L=True, ptr=16):
     mat = np.zeros(16)
     p = ctypes.c_void_p(ptr)
     if isinstance(dm, str):
         dm = _model()
     if isinstance(noise, str):
         noise = _noise()
-    if monitor_rows is None:
-        monitor_rows = len(rows) if rows is not None else 0
-    rows_ptr = np.ascontiguousarray(rows).ctypes.data if rows is not None else None
-    vs, vr, vp = (ctypes.c_void_p(64) if o else None for o in outs)
+    if isinstance(monitor, str):
+        monitor = _monitor()
     return lib.carmpc_closed_loop(
         qp, mode, mat.ctypes.data, mat.ctypes.data, mat.ctypes.data if C else None, mat.ctypes.data if L else None,
         ctypes.byref(dm) if dm is not None else None, mat.ctypes.data, dt, l1, steps, warm_start, p, None, None, None, runs,
-        p, None, p, None, None, None, ctypes.byref(noise) if noise is not None else None, rows_ptr, monitor_rows, vs, vr,
-        vp, None, None)
+        p, None, p, None, None, None, ctypes.byref(noise) if noise is not None else None,
+        ctypes.byref(monitor) if monitor is not None else None, None, None, None)
 
 
 def test_closed_loop_argument_errors(handle):
@@ -200,24 +206,22 @@ def test_closed_loop_argument_errors(handle):
     assert _call(lib, h, noise=_noise(first_run=-1)) == -1 and b"first_run" in err()
     assert _call(lib, h, noise=_noise(first_run=2 ** 63 - 2)) == -1           # first_run + runs overflows
     # monitor rows
-    assert _call(lib, h, monitor_rows=0) == -1 and b"monitor_rows" in err()
-    assert _call(lib, h, rows=np.tile(_ROWS, (257, 1)), monitor_rows=513) == -1
+    assert _call(lib, h, monitor=_monitor(n=0)) == -1 and b"monitor rows" in err()
+    assert _call(lib, h, monitor=_monitor(np.tile(_ROWS, (257, 1)), n=513)) == -1
     for bad in (math.nan, math.inf):
         r = _ROWS.copy()
         r[1, 4] = bad
-        assert _call(lib, h, rows=r) == -1 and b"finite" in err()
+        assert _call(lib, h, monitor=_monitor(r)) == -1 and b"finite" in err()
         r = _ROWS.copy()
         r[0, 2] = bad
-        assert _call(lib, h, rows=r) == -1
-    for outs in ((True, False, False), (False, True, False), (False, False, True)):
-        assert _call(lib, h, rows=None, outs=outs) == -1 and b"without monitor rows" in err()
-    assert _call(lib, h, rows=None, monitor_rows=2, outs=(False, False, False)) == -1
+        assert _call(lib, h, monitor=_monitor(r)) == -1
+    assert _call(lib, h, monitor=_monitor(None, n=2)) == -1
     # no runs: nothing to do once the arguments are valid
     total = ctypes.c_int64(7)
     mat = np.zeros(16)
     assert lib.carmpc_closed_loop(h, 0, mat.ctypes.data, mat.ctypes.data, None, None, None, mat.ctypes.data, 0.2, 3.5, 5,
-                                  1, None, None, None, None, 0, None, None, None, None, None, None, None, None, 0, None,
-                                  None, None, ctypes.byref(total), None) == 0
+                                  1, None, None, None, None, 0, None, None, None, None, None, None, None, None, None,
+                                  ctypes.byref(total), None) == 0
     assert total.value == 0
 
 
@@ -234,7 +238,7 @@ def test_closed_loop_on_a_host_only_handle_is_a_cuda_error(handle):
     for mode in (0, 1, 2):
         assert _call(lib, handle._h, mode=mode) == -2
         assert b"without a CUDA device" in lib.carmpc_last_error()
-    assert _call(lib, handle._h, noise=None, rows=None, outs=(False, False, False)) == -2
+    assert _call(lib, handle._h, noise=None, monitor=None) == -2
 
 
 def _flagged_empty(torch, shape):

@@ -1,5 +1,5 @@
-"""Times closed loops that stop at a goal (``carmpc_closed_loop_goal``), in one process, with the GPU name and power
-limit read in the same run.  Prints one JSON object.
+"""Times closed loops that stop at a goal (``carmpc_closed_loop`` with a goal), in one process, with the GPU name and
+power limit read in the same run.  Prints one JSON object.
 
 1. Config 4 (RoadEnv, N = 20, output feedback, 10^5 runs x 200 steps against the nonlinear bicycle, the initial states of
    bench_qp.py's config 4) without a goal and with ``montecarlo.goal_box(goal, 0.1)``, alternating, ``--reps`` loops
